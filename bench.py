@@ -2,6 +2,7 @@
 """bench.py -- the PSULVSB hot path on B200 (BASELINE.json metric: registrations/s at N = 5000, 95 % outliers).
 
     python bench.py --gpus N --steps K --warmup W [--config cfgA|cfgB|cfgC|cfgD|bunny] [--impl reference]
+                    [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs; SURVEY.md section 8d).  One STEP = one pass of the hot path
 (RobustRegistrationSolver::solve, registration.cc:622-1535) over one batch of synthetic input, fixed seeds.
@@ -253,6 +254,33 @@ def compare_with_oracle(sols, refs, final_inlier_sets=None):
     if mism:
         out["first_mismatches"] = mism[:4]
     return out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def solution_arrays(sols):
+    """What a caller of the solve entry points receives, one row per registration, as float64 arrays."""
+    out = {"rotation": np.stack([s.R for s in sols]), "translation": np.stack([s.t for s in sols])}
+    for f in ("valid", "scale", "final_inlier_count", "host_rounds", "local_iters", "n_line_vectors", "n_reduced",
+              "final_C", "refined", "escalations", "borderline_pairs", "status"):
+        out[f] = np.array([getattr(s, f) for s in sols], dtype=np.float64)
+    return out
+
+
+def dump_outputs(directory: str, arrays: dict, rank: int):
+    """Writes arrays as DIR/<name>.npy (float64; DIR/<name>.rank<r>.npy for ranks > 0).  Should they exceed 64 MB in
+    all, a fixed, seeded sample of their rows is written instead, with the row indices as DIR/sampled_rows.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        n = max(a.shape[0] for a in arrays.values())
+        rows = np.sort(np.random.default_rng(0).choice(n, int(n * DUMP_LIMIT_BYTES / total), replace=False))
+        arrays = {k: (a[rows] if a.shape[0] == n else a) for k, a in arrays.items()}
+        arrays["sampled_rows"] = rows.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + (f".rank{rank}" if rank else "") + ".npy"), a)
 
 
 def cpu_cores() -> int:
@@ -609,6 +637,8 @@ def run_cfgA(args, c, strong_total: int = 0):
             sets = final_inlier_sets(c, params, probs, seeds, min(n_cpu, 8))
             line["parity"] = compare_with_oracle(sols[:n_cpu], refs, sets)
     barrier(c)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, solution_arrays(r["sols"]), rank)
     return line, params
 
 
@@ -672,7 +702,8 @@ def stage_k1(c, n=100_000, steps=3, warmup=2):
 
 
 def stage_k4(c, n=50_000, H=1 << 20, steps=5, warmup=3, with_e2e=False):
-    """cfg-D: hypotheses sharded over the ranks; psulvsb_score_batch_sharded ends with the 8-byte ncclAllReduce(max)."""
+    """cfg-D: hypotheses sharded over the ranks; psulvsb_score_batch_sharded ends with the 8-byte ncclAllReduce(max).
+    -> (summary, outputs of the last step: this rank's inlier counts and the global best)."""
     torch, capi = c.torch, c.capi
     from psulvsb_b200 import sharding, stages
 
@@ -744,6 +775,7 @@ def stage_k4(c, n=50_000, H=1 << 20, steps=5, warmup=3, with_e2e=False):
     units = H * n
     peak = c.world * c.sms * 128 * f * 1e6 / 1e9
     ach = units * 16 / (ms / 1e3) / 1e9
+    outputs = {"inlier_counts": counts.cpu().numpy(), "best_count": [cnt], "best_hypothesis": [hid]}
     return {"case": "hypothesis scoring sweep (cfg-D)", "n": n, "hypotheses": H, "n_gpus": c.world, "units": units,
             "ms": ms, "scores_per_s": units / (ms / 1e3),
             "best": {"count": cnt, "hypothesis": hid, "expected_hypothesis": H // 3},
@@ -753,15 +785,17 @@ def stage_k4(c, n=50_000, H=1 << 20, steps=5, warmup=3, with_e2e=False):
             "clocks": stage_clocks, "e2e": e2e,
             "hbm_hypothesis_stream_gbs": H * 96 / c.world / (ms / 1e3) / 1e9,
             "sharding": "hypotheses sliced across ranks; one 8-byte ncclAllReduce(max) of (count<<32 | ~id) on the same "
-                        "stream, inside psulvsb_score_batch_sharded"}
+                        "stream, inside psulvsb_score_batch_sharded"}, outputs
 
 
 def run_cfgD(args, c):
-    steps, W = max(args.steps, 3), max(args.warmup, 3)
+    steps, W = args.steps, max(args.warmup, 3)
     sampler = ClockSampler(c.local_rank)
     sampler.start()
-    s = stage_k4(c, steps=steps, warmup=W, with_e2e=True)
+    s, outputs = stage_k4(c, steps=steps, warmup=W, with_e2e=True)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs, c.rank)
     if c.rank != 0:
         return None
     return {"metric": "hypothesis-point scores/s", "value": s["scores_per_s"], "unit": "scores/s", "n_gpus": c.world,
@@ -781,7 +815,7 @@ def run_cfgB(args, c):
     pair = synth.make_pair(n, 0.99, 4242, side=30.0)
     prob = capi.HostProblem(pair["src"], pair["dst"])
     params = capi.default_params(seed=11, **PARAM_KW)
-    steps, W = max(1, min(args.steps, 5)), 2
+    steps, W = args.steps, 2
     solve = (lambda: c.h.solve_sharded(params, prob)) if c.world > 1 else (lambda: c.h.solve(params, prob)[0])
     sampler = ClockSampler(c.local_rank)
     sampler.start()
@@ -798,6 +832,8 @@ def run_cfgB(args, c):
     wall = (time.perf_counter() - t0) * 1e3
     clocks = sampler.stop()
     dev_max, wall_max, k1_max = max_over_ranks(c, dev, wall, k1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, solution_arrays([sol]), c.rank)
     if c.rank != 0:
         return None
     f_mhz = clocks["sm_mhz"] or 1965.0
@@ -847,7 +883,7 @@ def run_bunny(args, c):
                                          [p["dst"] for p in cases])
         return [capi.HostProblem(sr, tr, p["src"], p["dst"], keep, rmap) for (keep, sr, tr, rmap, _), p in zip(res, cases)]
 
-    steps, W = max(1, min(args.steps, 10)), 3
+    steps, W = args.steps, 3
     probs = prefilter_all()
     r = timed_resident(c, params, probs, seeds, steps, W)
     barrier(c)
@@ -867,6 +903,8 @@ def run_bunny(args, c):
         c.h.solve(params, prefilter(i))
         lat.append((time.perf_counter() - t0) * 1e3)
     dev_max, e2e_max = max_over_ranks(c, r["dev_ms"], e2e_ms)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, solution_arrays(r["sols"]), c.rank)
     if c.rank != 0:
         return None
     errs = [c.synth.rotation_error(s.R, p["R"]) for s, p in zip(sols, cases)]
@@ -929,7 +967,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="cfgA: skip stages / variants (kernel tuning runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy "
+                         "(float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
@@ -939,7 +984,7 @@ def main():
     if args.config in ("cfgA", "cfgC"):
         line, params = run_cfgA(args, c, CFGC_PAIRS if args.config == "cfgC" else 0)
         if args.config == "cfgA" and not args.no_extras:
-            stages = {"k1_100k": stage_k1(c), "k4_1Mx50k": stage_k4(c)}
+            stages = {"k1_100k": stage_k1(c), "k4_1Mx50k": stage_k4(c)[0]}
             n_check = 0 if args.no_cpu_baseline else 16
             variants = {
                 "mode2_prefilter_selfupdate": run_variant(

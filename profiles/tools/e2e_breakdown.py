@@ -1,5 +1,5 @@
 import sys, time, numpy as np
-sys.path.insert(0,'/root/repo')
+sys.path.insert(0, '.')
 import psulvsb_b200
 from psulvsb_b200 import capi, synth
 import bench

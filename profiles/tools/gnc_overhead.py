@@ -1,5 +1,5 @@
 import sys, numpy as np, torch
-sys.path.insert(0,'/root/repo')
+sys.path.insert(0, '.')
 import psulvsb_b200
 from psulvsb_b200 import capi, stages, synth
 pair = synth.make_pair(5000, 0.95, 3)

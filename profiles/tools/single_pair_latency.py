@@ -1,5 +1,5 @@
 import sys, json, numpy as np, time
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, '.')
 import psulvsb_b200
 from psulvsb_b200 import capi, synth
 kw = dict(noise_bound=0.05, cbar2=1.0, estimate_scaling=0, rotation_max_iterations=100, rotation_gnc_factor=1.4, rotation_cost_threshold=0.005, wallclock_cap_s=0.0)

@@ -1,7 +1,7 @@
 """Small end-to-end + stage run for compute-sanitizer (memcheck): every kernel family once."""
 import sys
 import numpy as np
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, '.')
 import psulvsb_b200
 from psulvsb_b200 import capi, stages, synth, io
 import torch
