@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpsulvsb_b200.so")
 
 OK, ERR_INVALID, ERR_CUDA, ERR_NO_DEVICE, ERR_CAPACITY, ERR_UNSUPPORTED, ERR_INTERNAL = range(7)
-DOMAIN_L_SAMPLED, DOMAIN_BASIC, DOMAIN_UNIFORM, DOMAIN_SCALE = 1, 2, 3, 4
+DOMAIN_L_SAMPLED, DOMAIN_BASIC, DOMAIN_UNIFORM, DOMAIN_SCALE, DOMAIN_TUPLE = 1, 2, 3, 4, 5
 
 # every symbol include/psulvsb.h declares (checked by tests/test_capi_symbols.py against the header)
 SYMBOLS = [
@@ -31,6 +31,7 @@ SYMBOLS = [
     "psulvsb_comm_unique_id", "psulvsb_comm_create", "psulvsb_comm_destroy", "psulvsb_comm_rank", "psulvsb_comm_world",
     "psulvsb_comm_allreduce_sum_u32", "psulvsb_comm_allreduce_max_u64", "psulvsb_score_batch_sharded",
     "psulvsb_solve_sharded", "psulvsb_shard_row_range",
+    "psulvsb_fpfh_workspace_bytes", "psulvsb_fpfh", "psulvsb_fpfh_host", "psulvsb_feature_nn", "psulvsb_match_host",
 ]
 UNIQUE_ID_BYTES = 128
 
@@ -230,6 +231,13 @@ def _declare(L: C.CDLL) -> None:
     L.psulvsb_solve_sharded.argtypes = [_vp, C.POINTER(Params), C.POINTER(Problem), C.POINTER(Solution), C.POINTER(Trace)]
     L.psulvsb_shard_row_range.argtypes = [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]
     L.psulvsb_score_one.argtypes = [_vp, _vp, _vp, C.c_int, C.c_double, _vp, _vp, C.c_double, _vp, _vp, _vp]
+    L.psulvsb_fpfh_workspace_bytes.argtypes = [C.c_int]
+    L.psulvsb_fpfh_workspace_bytes.restype = _ull
+    L.psulvsb_fpfh.argtypes = [_vp, _vp, C.c_int, C.c_double, C.c_double, C.POINTER(C.c_double), _vp, _vp, _vp]
+    L.psulvsb_fpfh_host.argtypes = [_vp, C.c_int, C.c_double, C.c_double, C.POINTER(C.c_double), _vp, _vp]
+    L.psulvsb_feature_nn.argtypes = [_vp, _vp, C.c_int, _vp, C.c_int, _vp, _vp]
+    L.psulvsb_match_host.argtypes = [_vp, C.c_int, _vp, C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_double, C.c_uint64,
+                                     _vp, C.c_longlong, C.POINTER(C.c_longlong)]
     for name in SYMBOLS:
         getattr(L, name)  # AttributeError here = the library does not export what the header declares
 

@@ -39,8 +39,6 @@ DebugKnobs& debug_knobs() {
   return k;
 }
 
-namespace {
-
 int need_device() {
   int n = 0;
   if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) {
@@ -49,6 +47,8 @@ int need_device() {
   }
   return PSULVSB_OK;
 }
+
+namespace {
 
 // single job descriptor -> device, freed in stream order after the kernels that read it
 template <typename T>

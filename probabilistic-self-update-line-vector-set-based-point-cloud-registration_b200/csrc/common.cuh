@@ -33,6 +33,9 @@ int fail(int code, const std::string& msg);
     }                                                                                               \
   } while (0)
 
+// PSULVSB_ERR_NO_DEVICE (with its message) when no CUDA device is visible, else PSULVSB_OK
+int need_device();
+
 // SMs of the current device (cudaDevAttrMultiProcessorCount, cached per device): every grid is sized from it
 int sm_count();
 

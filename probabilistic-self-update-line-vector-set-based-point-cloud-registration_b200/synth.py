@@ -81,3 +81,11 @@ def prefilter(pair: dict, seed: int, *, keep_inlier: float = 0.6, keep_outlier: 
 def rotation_error(Ra: np.ndarray, Rb: np.ndarray) -> float:
     c = (np.trace(Ra.T @ Rb) - 1.0) / 2.0
     return float(abs(np.arccos(np.clip(c, -1.0, 1.0))))
+
+
+def make_surface(n: int, seed: int) -> np.ndarray:
+    """n points (3xn) on the seeded smooth surface z = 0.3 sin(2x) cos(3y) + 0.1 x y over [0, 2]^2: the synthetic
+    cloud of the FPFH tests and benchmark (about 20 neighbours within r = 0.08 at n = 5 000)."""
+    rng = np.random.default_rng(seed)
+    x, y = rng.uniform(0.0, 2.0, n), rng.uniform(0.0, 2.0, n)
+    return np.stack([x, y, 0.3 * np.sin(2 * x) * np.cos(3 * y) + 0.1 * x * y])
