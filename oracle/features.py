@@ -5,22 +5,25 @@ TEST INFRASTRUCTURE ONLY.  It follows the section's definitions, not the kernels
 (then the same FP32 distance test), sums in numpy's order.  Where a result can legitimately differ from the device
 because of summation order or a last-bit difference of acos / atan2, the item is flagged *fragile*:
   - a pair whose bin argument lies within 1e-5 of an integer, or whose |a1| and |a2| differ, by at most 1e-6
-    relative + 1e-7 (the swap test);
-  - a neighbour with |d^2 - r^2| <= 1e-6 r^2;
+    relative + 1e-7 (the swap test); such a pair moves one count of each histogram at most, so a descriptor is
+    fragile only when its fragile pairs could move it by more than SOFT_L1 (L1) in all;
+  - a neighbour with |d^2 - r^2| <= 1e-6 r^2 (every descriptor it reaches is fragile);
   - a normal whose two smallest eigenvalues are within 1e-6 relative, or that lies within 1e-7 of perpendicular to
     the viewpoint direction;
-  - a descriptor nearest neighbour whose best and second-best distances differ by less than 1e-6 relative;
-  - a tuple trial within 1e-6 relative of a ratio bound.
+  - a descriptor nearest neighbour whose best and second-best distances differ, by less than 1e-6 relative;
+  - a tuple trial with an edge within 1e-6 relative of a ratio bound while its other edges pass or are as near.
 """
 import math
 
 import numpy as np
+from scipy import sparse
 from scipy.spatial import cKDTree
 
 BINS = 11
 DIM = 33
 DOMAIN_TUPLE = 5
 MAX_TUPLES = 1000
+SOFT_L1 = 5e-4   # how far fragile pairs may move a descriptor (L1) before the descriptor counts as fragile
 
 
 def _f32(points):
@@ -132,8 +135,10 @@ def bin_args(f1, f2, f3):
                      11.0 * (f2.astype(np.float64) + 1.0) / 2.0, 11.0 * (f3.astype(np.float64) + 1.0) / 2.0], axis=1)
 
 
-def fpfh(points, normal_radius, feature_radius, viewpoint=(0.0, 0.0, 0.0), normals=None):
-    """(features n x 33 float32, normals 3xn, fragile [n]) following DESIGN.md section 10."""
+def fpfh(points, normal_radius, feature_radius, viewpoint=(0.0, 0.0, 0.0), normals=None, bounds=False):
+    """(features n x 33 float32, normals 3xn, fragile [n]) following DESIGN.md section 10.  With bounds, also
+    (hard [n], soft_l1 [n]): hard = a fragile neighbour set reaches the descriptor; otherwise the device's
+    descriptor lies within soft_l1 (L1, plus rounding) of this one."""
     P = np.asarray(points, dtype=np.float64)
     n = P.shape[1]
     nfrag = np.zeros(n, dtype=bool)
@@ -148,49 +153,85 @@ def fpfh(points, normal_radius, feature_radius, viewpoint=(0.0, 0.0, 0.0), norma
     f1, f2, f3, valid, sfrag = pair_features(p32[pi], n32[pi], p32[pj], n32[pj])
     with np.errstate(invalid="ignore"):
         args = bin_args(f1, f2, f3)
-    afrag = np.any(np.abs(args - np.round(args)) <= 1e-5, axis=1)
-    pfrag = ((sfrag | afrag) & valid) | nfrag[pi] | nfrag[pj]
+    # per histogram h: a pair near a bin edge of feature h, near the swap decision or with a fragile normal
+    afrag = np.abs(args - np.round(args)) <= 1e-5
+    pfrag = (((sfrag[:, None] | afrag) & valid[:, None]) | (nfrag[pi] | nfrag[pj])[:, None])
     bins = np.clip(np.floor(np.nan_to_num(args, nan=0.0)).astype(np.int64), 0, BINS - 1)
     counts = np.zeros((n, DIM), dtype=np.int64)
     for h in range(3):
-        np.add.at(counts, (pi[valid], h * BINS + bins[valid, h]), 1)
-    spfh_frag = np.zeros(n, dtype=bool)
-    np.logical_or.at(spfh_frag, pi, pfrag)
-    np.logical_or.at(spfh_frag, ii, bfrag_pair)
-    spfh_frag |= bfrag_out
+        counts[:, h * BINS:(h + 1) * BINS] = np.bincount(
+            pi[valid] * BINS + bins[valid, h], minlength=n * BINS).reshape(n, BINS)
+    # hard: a neighbour near the radius may join or leave (K and the weights change)
+    hard = bfrag_out.copy()
+    np.logical_or.at(hard, ii, bfrag_pair)
+    # soft: a fragile pair of SPFH_j moves one count of a histogram at most
+    nsoft = np.stack([np.bincount(pi, weights=pfrag[:, h], minlength=n) for h in range(3)], axis=1)
     # FPFH: neighbours j != i at distance > 0, weight 1 / d^2 (FP64 of the FP32 distance)
     use = other & (d2 > 0)
     fi, fj = ii[use], jj[use]
     Kj = K[fj]
     w = np.where(Kj > 1, (100.0 / np.maximum(Kj - 1, 1)) / d2[use].astype(np.float64), 0.0)
-    acc = np.zeros((n, DIM))
-    np.add.at(acc, fi, counts[fj].astype(np.float64) * w[:, None])
+    W = sparse.csr_matrix((w, (fi, fj)), shape=(n, n))
+    acc = np.asarray(W @ counts.astype(np.float64))
     out = np.zeros((n, DIM), dtype=np.float32)
+    # moving one count of weight w between two bins of a histogram with sum s moves the output by 200 w / s in L1:
+    # a point is fragile when its soft pairs could move it by more than SOFT_L1 in all, or when a hard flag reaches it
+    wsoft = W @ nsoft
+    moved = np.zeros(n)
     for h in range(3):
         s = acc[:, h * BINS:(h + 1) * BINS].sum(axis=1)
         pos = s > 0
         out[pos, h * BINS:(h + 1) * BINS] = (acc[pos, h * BINS:(h + 1) * BINS] * (100.0 / s[pos])[:, None]).astype(
             np.float32)
-    frag = spfh_frag.copy()
-    np.logical_or.at(frag, fi, spfh_frag[fj])
+        moved += np.where(wsoft[:, h] > 0, 200.0 * wsoft[:, h] / np.maximum(s, 1e-300), 0.0)
+    np.logical_or.at(hard, fi, hard[fj])
+    frag = hard | (moved > SOFT_L1)
+    if bounds:
+        return out, normals, frag, hard, moved
     return out, normals, frag
+
+
+def fma32(a, b, c):
+    """The device's fmaf(a, b, c) on float32 arrays, rounded once: a * b is exact in float64, and s = a * b + c in
+    float64 is exact up to the tail e that TwoSum recovers.  Rounding s to float32 is then correct unless s lies
+    exactly halfway between two float32 values and e != 0 (double rounding): the tail then decides the direction."""
+    a, b, c = (np.asarray(x, dtype=np.float32).astype(np.float64) for x in (a, b, c))
+    with np.errstate(over="ignore", invalid="ignore"):
+        p = a * b
+        s = p + c
+        bb = s - p
+        e = (p - (s - bb)) + (c - bb)
+        r = s.astype(np.float32)
+        lo = np.where(r.astype(np.float64) > s, np.nextafter(r, np.float32(-np.inf)), r)
+        mid = (lo.astype(np.float64) + np.nextafter(lo, np.float32(np.inf)).astype(np.float64)) * 0.5
+        tie = np.isfinite(s) & (s == mid) & (e != 0)
+    if tie.any():
+        r = np.where(tie, np.where(e > 0, np.nextafter(lo, np.float32(np.inf)), lo), r)
+    return r
 
 
 def descriptor_distances(fs, ft):
     """n_s x n_t squared distances as the device forms them: d = a - b in FP32, acc = fma(d, d, acc) for the 33
-    dimensions in order (a float64 product is exact, so fma is one float64 add rounded to float32)."""
+    dimensions in order (fma32)."""
     fs = np.asarray(fs, dtype=np.float32)
     ft = np.asarray(ft, dtype=np.float32)
     acc = np.zeros((fs.shape[0], ft.shape[0]), dtype=np.float32)
     for k in range(DIM):
-        d = (fs[:, k][:, None] - ft[:, k][None, :]).astype(np.float32).astype(np.float64)
-        acc = (acc.astype(np.float64) + d * d).astype(np.float32)
+        d = (fs[:, k][:, None] - ft[:, k][None, :]).astype(np.float32)
+        acc = fma32(d, d, acc)
     return acc
+
+
+def near_tie(best, second):
+    """Best and second-best distances within 1e-6 relative but not equal (descriptor_distances is the device's value
+    bit for bit, and an exact tie goes to the lowest index on both sides); no second-best is no tie."""
+    with np.errstate(invalid="ignore"):
+        return np.isfinite(second) & (second != best) & (second - best <= 1e-6 * np.maximum(second, 1e-30))
 
 
 def nearest_neighbours(fs, ft, block=2048):
     """(nn_src_to_tgt, nn_tgt_to_src, fragile_src, fragile_tgt): ties to the lowest index; fragile = best and
-    second-best within 1e-6 relative."""
+    second-best within 1e-6 relative (near_tie)."""
     fs = np.asarray(fs, dtype=np.float32)
     ft = np.asarray(ft, dtype=np.float32)
     ns, nt = fs.shape[0], ft.shape[0]
@@ -204,7 +245,7 @@ def nearest_neighbours(fs, ft, block=2048):
         nn_t[r0:r0 + block] = np.argmin(D, axis=1)
         if nt > 1:
             part = np.partition(D, 1, axis=1)
-            fr_s[r0:r0 + block] = part[:, 1] - part[:, 0] <= 1e-6 * np.maximum(part[:, 1], 1e-30)
+            fr_s[r0:r0 + block] = near_tie(part[:, 0], part[:, 1])
         # running column minimum and second minimum (ties keep the earlier, i.e. lower, row)
         arg = np.argmin(D, axis=0)
         m = D[arg, np.arange(nt)]
@@ -212,13 +253,12 @@ def nearest_neighbours(fs, ft, block=2048):
             sec = np.partition(D, 1, axis=0)[1]
         else:
             sec = np.full(nt, np.inf)
-        better = m < col_best
+        better = (m < col_best) | (nn_s < 0)          # (an all-inf column still picks its lowest row)
         new_second = np.where(better, np.minimum(col_best, sec), np.minimum(col_second, m))
         nn_s = np.where(better, arg + r0, nn_s)
         col_best = np.where(better, m, col_best)
         col_second = new_second
-    fr_t = col_second - col_best <= 1e-6 * np.maximum(col_second, 1e-30)
-    return nn_t, nn_s, fr_s, fr_t
+    return nn_t, nn_s, fr_s, near_tie(col_best, col_second)
 
 
 def match_list(nn_t, nn_s, crosscheck):
@@ -237,18 +277,34 @@ def match_list(nn_t, nn_s, crosscheck):
     return np.concatenate([first, second]).reshape(-1, 2)
 
 
+def philox_blocks(seed, domain, event, blocks):
+    """Philox4x32-10 (oracle.philox) on an array of block counters at once: [len(blocks), 4] uint32."""
+    blocks = np.asarray(blocks, dtype=np.uint64)
+    m32 = np.uint64(0xFFFFFFFF)
+    c0, c1 = blocks & m32, blocks >> np.uint64(32)
+    c2 = np.full_like(c0, np.uint64(event) & m32)
+    c3 = np.full_like(c0, np.uint64(domain) & m32)
+    k0, k1 = int(seed) & 0xFFFFFFFF, (int(seed) >> 32) & 0xFFFFFFFF
+    for _ in range(10):
+        p0 = np.uint64(0xD2511F53) * c0
+        p1 = np.uint64(0xCD9E8D57) * c2
+        c0, c1, c2, c3 = ((p1 >> np.uint64(32)) ^ c1 ^ np.uint64(k0), p1 & m32,
+                          (p0 >> np.uint64(32)) ^ c3 ^ np.uint64(k1), p0 & m32)
+        k0 = (k0 + 0x9E3779B9) & 0xFFFFFFFF
+        k1 = (k1 + 0xBB67AE85) & 0xFFFFFFFF
+    return np.stack([c0, c1, c2, c3], axis=1).astype(np.uint32)
+
+
 def tuple_draws(seed, first_trial, count, ncorr):
     """List positions of trials [first_trial, first_trial + count): rand31(seed; TUPLE, 0, 3t + k) % ncorr."""
-    from oracle import oracle as O
-
     k0 = 3 * first_trial
     k1 = 3 * (first_trial + count)
-    blocks = np.stack([O.philox(seed, DOMAIN_TUPLE, 0, b) for b in range(k0 >> 2, ((k1 - 1) >> 2) + 1)])
+    blocks = philox_blocks(seed, DOMAIN_TUPLE, 0, np.arange(k0 >> 2, ((k1 - 1) >> 2) + 1, dtype=np.uint64))
     words = blocks.reshape(-1)[k0 - 4 * (k0 >> 2):][:k1 - k0] >> 1
     return (words.astype(np.int64) % ncorr).reshape(count, 3)
 
 
-def tuple_test(src, tgt, corr, scale, seed, chunk=4096):
+def tuple_test(src, tgt, corr, scale, seed, chunk=1 << 16):
     """(pairs (3 * kept, 2), fragile_trial_seen): the first min(#passing, 1000) passing trials in trial order."""
     corr = np.asarray(corr, dtype=np.int64).reshape(-1, 2)
     ncorr = corr.shape[0]
@@ -260,15 +316,22 @@ def tuple_test(src, tgt, corr, scale, seed, chunk=4096):
         r = tuple_draws(seed, t0, cnt, ncorr)
         ok = np.ones(cnt, dtype=bool)
         near = np.zeros(cnt, dtype=bool)
+        could = np.ones(cnt, dtype=bool)   # every edge passes or is near a bound: a near edge may decide the trial
         for e in range(3):
             a, b = r[:, e], r[:, (e + 1) % 3]
             li = np.sqrt(sqdist32(s32[corr[a, 0]], s32[corr[b, 0]]))
             lj = np.sqrt(sqdist32(t32[corr[a, 1]], t32[corr[b, 1]]))
             with np.errstate(invalid="ignore", divide="ignore"):
                 lo, hi = (li * s).astype(np.float32), (li / s).astype(np.float32)
-                ok &= (lo < lj) & (lj < hi)
+                ok_e = (lo < lj) & (lj < hi)
                 tol = 1e-6 * np.maximum(lj.astype(np.float64), 1e-30)
-                near |= (np.abs(lo.astype(np.float64) - lj) <= tol) | (np.abs(hi.astype(np.float64) - lj) <= tol)
+                # (a repeated draw gives li = lj = 0, which fails exactly on both sides)
+                near_e = (lj > 0) & ((np.abs(lo.astype(np.float64) - lj) <= tol) |
+                                     (np.abs(hi.astype(np.float64) - lj) <= tol))
+            ok &= ok_e
+            near |= near_e
+            could &= ok_e | near_e
+        near &= could
         for u in np.flatnonzero(ok | near):
             fragile |= bool(near[u])
             if ok[u]:

@@ -81,22 +81,55 @@ def mask_filter(src, tgt, keep):
     return np.asfortranarray(src[:, idx]), np.asfortranarray(tgt[:, idx]), rm
 
 
-def knn_pca_normals(points, k=20, viewpoint=(0.0, 0.0, 0.0)):
+def knn_sqdist32(Pf, rows):
+    """FP32 squared distances from the points `rows` to all points, as k6_normals.cu forms them:
+    fmaf(dz, dz, fmaf(dy, dy, dx * dx)) with d = p_j - p_i."""
+    from oracle.features import fma32
+
+    d = [(Pf[c][None, :] - Pf[c][rows][:, None]).astype(np.float32) for c in range(3)]
+    return fma32(d[2], d[2], fma32(d[1], d[1], d[0] * d[0]))
+
+
+def knn_pca_normals(points, k=20, viewpoint=(0.0, 0.0, 0.0), return_fragile=False, block=256):
     """Restatement of what PSULVSB.cc:35-85 asks PCL for: for every point the k nearest neighbours (itself
-    included), the eigenvector of the smallest eigenvalue of their covariance, flipped towards the viewpoint."""
+    included), the eigenvector of the smallest eigenvalue of their covariance, flipped towards the viewpoint.
+
+    As the kernel decides it: the fused FP32 distance (knn_sqdist32), ties to the lower index, all n points when
+    n < k, NaN when fewer than 3 points remain.  With return_fragile, also a per-point flag for results that
+    summation order may decide: the k-th and (k+1)-th distances within 1e-6 relative (an exact tie is decided the
+    same way on both sides), the two smallest eigenvalues within 1e-6 relative, or the normal within 1e-7 of
+    perpendicular to the viewpoint direction."""
     P = np.asarray(points, dtype=np.float64)
     n = P.shape[1]
     Pf = P.astype(np.float32)
-    out = np.zeros((3, n))
-    vp = np.asarray(viewpoint, dtype=np.float64)
-    for i in range(n):
-        d = ((Pf - Pf[:, i:i + 1]) ** 2).sum(axis=0)
-        idx = np.argsort(d, kind="stable")[:k]
-        nb = P[:, idx]
-        c = np.cov(nb, bias=True) * nb.shape[1]
-        w, v = np.linalg.eigh(c)
-        nv = v[:, 0]
-        if (vp - P[:, i]) @ nv < 0:
-            nv = -nv
-        out[:, i] = nv
-    return out
+    out = np.full((3, n), np.nan)
+    frag = np.zeros(n, dtype=bool)
+    m = min(k, n)
+    if m >= 3:
+        vp = np.asarray(viewpoint, dtype=np.float64)
+        idx = np.zeros((n, m), dtype=np.int64)
+        for r0 in range(0, n, block):
+            rows = np.arange(r0, min(n, r0 + block))
+            d = knn_sqdist32(Pf, rows)
+            # key = (distance bits, index): non-negative float32 bits keep their order, the index breaks ties
+            key = (d.view(np.uint32).astype(np.uint64) << np.uint64(32)) | np.arange(n, dtype=np.uint64)[None, :]
+            if n > m:
+                key = np.partition(key, m, axis=1)[:, :m + 1]
+            key = np.sort(key, axis=1)
+            idx[rows] = (key[:, :m] & np.uint64(0xFFFFFFFF)).astype(np.int64)
+            if n > m:
+                dk = (key[:, m - 1] >> np.uint64(32)).astype(np.uint32).view(np.float32).astype(np.float64)
+                dk1 = (key[:, m] >> np.uint64(32)).astype(np.uint32).view(np.float32).astype(np.float64)
+                frag[rows] = (dk1 != dk) & (dk1 - dk <= 1e-6 * dk1)
+        nb = P[:, idx].transpose(1, 2, 0)                       # [n, m, 3]
+        dev = nb - nb.mean(axis=1, keepdims=True)
+        cov = np.einsum("nka,nkb->nab", dev, dev)
+        w, v = np.linalg.eigh(cov)
+        nv = v[:, :, 0]
+        side = ((vp[None, :] - P.T) * nv).sum(axis=1)
+        nv[side < 0] *= -1
+        out = np.ascontiguousarray(nv.T)
+        scale = np.maximum(np.abs(w[:, 2]), 1e-300)
+        frag |= (np.abs(w[:, 1] - w[:, 0]) <= 1e-6 * scale)
+        frag |= np.abs(side) <= 1e-7 * np.linalg.norm(vp[None, :] - P.T, axis=1)
+    return (out, frag) if return_fragile else out

@@ -186,3 +186,114 @@ def test_feature_nn_loop_is_packed():
                     ops[op] = ops.get(op, 0) + 1
     assert ops.get("FFMA2", 0) >= 32 and ops.get("FFMA2", 0) > ops.get("FFMA", 0), ops
     assert ops.get("FADD2", 0) >= 32, ops
+
+
+def exact_fma32(a, b, c):
+    """float32(a * b + c) rounded once (round half to even), from exact rationals: the reference for fmaf."""
+    from fractions import Fraction
+
+    x = Fraction(float(a)) * Fraction(float(b)) + Fraction(float(c))
+    if x == 0:
+        return np.float32(0.0)
+    m, e = abs(x), 0
+    while m >= 2:
+        m, e = m / 2, e + 1
+    while m < 1:
+        m, e = m * 2, e - 1
+    q = abs(x) / Fraction(2) ** (e - 23)          # the 24-bit significand, scaled to an integer part
+    r = math.floor(q)
+    if q - r > Fraction(1, 2) or (q - r == Fraction(1, 2) and r % 2):
+        r += 1
+    return np.float32(math.copysign(float(r * Fraction(2) ** (e - 23)), x))
+
+
+def test_fma32_rounds_once():
+    y = 2.0 ** -10
+    # a * b + c lands a quarter float64 ulp off a float32 midpoint: float64 rounding alone would hit the midpoint
+    # and round half-to-even the wrong way
+    cases = [(1 + y, 2.0 ** -24 * (1 - y + y * y), 1.0, 1 + 2.0 ** -23),                   # 1 + 2^-24 + 2^-54
+             (1 - y, 2.0 ** -24 * (1 + y + y * y), 1 + 2.0 ** -23, 1 + 2.0 ** -23),        # 1 + 3 2^-24 - 2^-54
+             (-(1 + y), 2.0 ** -24 * (1 - y + y * y), -1.0, -(1 + 2.0 ** -23))]
+    for a, b, c, want in cases:
+        a, b, c = np.float32(a), np.float32(b), np.float32(c)
+        assert F.fma32(a, b, c) == np.float32(want) == exact_fma32(a, b, c)
+        assert np.float32(float(a) * float(b) + float(c)) != np.float32(want)   # the naive double rounding is wrong
+    rng = np.random.default_rng(0)
+    a = rng.normal(0, 1, 3000).astype(np.float32)
+    b = (rng.normal(0, 1, 3000) * 10.0 ** rng.integers(-8, 8, 3000)).astype(np.float32)
+    c = (rng.normal(0, 1, 3000) * 10.0 ** rng.integers(-8, 8, 3000)).astype(np.float32)
+    got = F.fma32(a, b, c)
+    assert all(got[i] == exact_fma32(a[i], b[i], c[i]) for i in range(3000))
+    # the k-NN normals' distance: fmaf(dz, dz, fmaf(dy, dy, dx * dx))
+    d = rng.normal(0, 1, (3, 500)).astype(np.float32)
+    from oracle import prefilter as OP
+
+    P = np.concatenate([np.zeros((3, 1)), d], axis=1).astype(np.float32)
+    got = OP.knn_sqdist32(P, np.array([0]))[0, 1:]
+    want = [exact_fma32(z, z, exact_fma32(y, y, np.float32(x * x))) for x, y, z in d.T]
+    assert np.array_equal(got, np.array(want, dtype=np.float32))
+    # descriptor distances take the same path; an overflow is inf
+    big = np.full((1, 33), 1e20, np.float32)
+    assert np.isinf(F.descriptor_distances(big, -big)).all()
+
+
+def test_knn_restatement_ties_and_fragile_rule():
+    from oracle import prefilter as OP
+
+    vp = (0.3, 0.2, 5.0)
+    base = np.array([[0.0, 1.0, 0.0, 0.0], [0.0, 0.0, 1.0, 0.0], [0.0, 0.0, 0.0, 1.0]])
+    # point 0's 2nd, 3rd and 4th neighbours tie exactly at d^2 = 1: k = 3 keeps the lower indices 1 and 2, so the
+    # normal is the plane z = 0's; an exact tie is not fragile
+    nv, frag = OP.knn_pca_normals(base, k=3, viewpoint=vp, return_fragile=True)
+    assert np.allclose(nv[:, 0], [0, 0, 1]) and not frag[0]
+    # point 3 a hair further (d^2 = 1 + 2^-22 in FP32, 2.4e-7 relative): the same pick, but fragile
+    near = base.copy()
+    near[2, 3] = 1 + 2.0 ** -23
+    nv, frag = OP.knn_pca_normals(near, k=3, viewpoint=vp, return_fragile=True)
+    assert np.allclose(nv[:, 0], [0, 0, 1]) and frag[0]
+    # 1e-5 relative further: not fragile
+    far = base.copy()
+    far[2, 3] = 1 + 1e-5
+    assert not OP.knn_pca_normals(far, k=3, viewpoint=vp, return_fragile=True)[1][0]
+    # the same cloud in another order: the two lowest tied indices, now (0, 0, 1) and (0, 1, 0), set the plane
+    swapped = base[:, [0, 3, 2, 1]]
+    nv = OP.knn_pca_normals(swapped, k=3, viewpoint=vp)
+    assert np.allclose(nv[:, 0], [1, 0, 0])               # plane x = 0
+    # n < k uses all n points; n < 3 is NaN; the default call returns the normals only
+    assert OP.knn_pca_normals(base, k=20).shape == (3, 4)
+    assert np.isnan(OP.knn_pca_normals(base[:, :2], k=20)).all()
+    assert np.isnan(OP.knn_pca_normals(base[:, :1], k=3)).all()
+
+
+def test_vectorised_philox_matches_the_oracle():
+    rng = np.random.default_rng(2)
+    blocks = np.concatenate([np.arange(0, 1000, dtype=np.uint64), rng.integers(0, 2 ** 62, 1000, dtype=np.uint64),
+                             np.arange(2 ** 30 - 500, 2 ** 30 + 500, dtype=np.uint64),
+                             np.arange(2 ** 32 - 300, 2 ** 32 + 300, dtype=np.uint64),
+                             np.array([2 ** 64 - 1], dtype=np.uint64)])
+    for seed in (0, 11, (7 << 32) | 5):
+        got = F.philox_blocks(seed, F.DOMAIN_TUPLE, 0, blocks)
+        want = np.stack([O.philox(seed, F.DOMAIN_TUPLE, 0, int(b)) for b in blocks])
+        assert np.array_equal(got, want)
+    assert np.array_equal(F.philox_blocks(3, 2, 9, blocks[:50]), np.stack([O.philox(3, 2, 9, int(b))
+                                                                           for b in blocks[:50]]))
+    # draws of trials whose 3t + k crosses 2^32 (blocks above 2^32 / 4)
+    t0 = (2 ** 32) // 3 - 5
+    d = F.tuple_draws(11, t0, 10, 1000)
+    for u in range(10):
+        for k in range(3):
+            assert d[u, k] == O.rand31(11, F.DOMAIN_TUPLE, 0, 3 * (t0 + u) + k) % 1000
+
+
+@pytest.mark.parametrize("offset", [0.0, 1e3])
+def test_neighbours_match_brute_force(offset):
+    """The k-d tree query (radius widened by 1e-4) finds every pair the FP32 distance test accepts."""
+    rng = np.random.default_rng(3)
+    P = rng.uniform(0, 1, (3, 300)) + offset
+    p32 = P.T.astype(np.float32)
+    for r in (0.05, 0.2, 0.6):
+        ii, jj, d2, _, _ = F.neighbours(P, r)
+        d = np.stack([F.sqdist32(np.repeat(p32[i:i + 1], 300, 0), p32) for i in range(300)])
+        bi, bj = np.nonzero(d <= np.float32(r * r))
+        assert np.array_equal(ii, bi) and np.array_equal(jj, bj)
+        assert np.array_equal(d2, d[bi, bj])
