@@ -1,8 +1,11 @@
 // psulvsb_fpfh.cc -- upstream TEASER++'s teaser_cpp_fpfh flow against the B200 library: load a PLY, apply a rigid
 // transform (and optional uniform noise), compute FPFH descriptors of both clouds, match them (crosscheck, no tuple
-// test), solve(src_cloud, tgt_cloud, correspondences) and report the rotation and translation errors.
+// test), solve(src_cloud, tgt_cloud, correspondences) and report the rotation and translation errors.  With
+// icp_distance > 0 the solve's answer is then refined by point-to-point ICP on the two clouds (psulvsb_icp_host, the
+// step upstream's Python example hands to Open3D) and a second line reports the refined errors.
 //
 //   psulvsb_fpfh <file.ply> [vertex_scale = 1] [normal_radius = 0.03] [feature_radius = 0.05] [noise = 0] [seed = 1]
+//                [icp_distance = 0]
 //
 // Differences from the upstream example, on purpose: a seeded generator; the target is the transformed source itself
 // (same points, same order) so that the true correspondences are known; normals and descriptors on the GPU.
@@ -15,16 +18,19 @@
 #include <cstdio>
 #include <cstdlib>
 #include <random>
+#include <vector>
 
 int main(int argc, char** argv) {
   if (argc < 2) {
-    std::fprintf(stderr, "usage: %s file.ply [vertex_scale] [normal_radius] [feature_radius] [noise] [seed]\n", argv[0]);
+    std::fprintf(stderr, "usage: %s file.ply [vertex_scale] [normal_radius] [feature_radius] [noise] [seed] [icp_distance]\n",
+                 argv[0]);
     return 64;
   }
   const double scale = argc > 2 ? std::atof(argv[2]) : 1.0;
   const double rn = argc > 3 ? std::atof(argv[3]) : 0.03, rf = argc > 4 ? std::atof(argv[4]) : 0.05;
   const double noise = argc > 5 ? std::atof(argv[5]) : 0.0;
   const unsigned long long seed = argc > 6 ? std::strtoull(argv[6], nullptr, 10) : 1ull;
+  const double icp_distance = argc > 7 ? std::atof(argv[7]) : 0.0;
 
   teaser::PLYReader reader;
   teaser::PointCloud src;
@@ -100,5 +106,33 @@ int main(int argc, char** argv) {
   std::printf("points=%zu correspondences=%zu true=%d valid=%d rotation_error_deg=%.6f translation_error=%.6g "
               "extent=%.6g\n",
               src.size(), corr.size(), true_pairs, int(sol.valid), rot_err_deg, std::sqrt(terr), extent);
-  return sol.valid ? 0 : 1;
+  if (!sol.valid || icp_distance <= 0) return sol.valid ? 0 : 1;
+
+  std::vector<double> ps, pt;  // column-major 3 x n
+  for (const auto& p : src) ps.insert(ps.end(), {p.x, p.y, p.z});
+  for (const auto& p : tgt) pt.insert(pt.end(), {p.x, p.y, p.z});
+  psulvsb_icp_params_t ip;
+  psulvsb_icp_default_params(&ip);
+  ip.max_correspondence_distance = icp_distance;
+  double R0[9], t0[3];
+  for (int i = 0; i < 3; ++i) {
+    for (int j = 0; j < 3; ++j) R0[3 * j + i] = sol.rotation(i, j);
+    t0[i] = sol.translation(i);
+  }
+  psulvsb_icp_result_t icp;
+  const int rc = psulvsb_icp_host(ps.data(), int(src.size()), pt.data(), int(tgt.size()), nullptr, &ip, R0, t0, &icp,
+                                  nullptr, nullptr);
+  if (rc != PSULVSB_OK) {
+    std::printf("icp failed (status %d): %s\n", rc, psulvsb_last_error());
+    return rc;
+  }
+  double tr2 = 0.0, terr2 = 0.0;
+  for (int i = 0; i < 3; ++i)
+    for (int j = 0; j < 3; ++j) tr2 += icp.rotation[3 * j + i] * R[i][j];
+  for (int r = 0; r < 3; ++r) terr2 += (icp.translation[r] - t[r]) * (icp.translation[r] - t[r]);
+  std::printf("icp: fitness=%.6f inlier_rmse=%.6g iterations=%d status=%d rotation_error_deg=%.6g "
+              "translation_error=%.6g\n",
+              icp.fitness, icp.inlier_rmse, icp.iterations, icp.status,
+              std::acos(std::fmax(-1.0, std::fmin(1.0, (tr2 - 1) / 2))) * 180.0 / M_PI, std::sqrt(terr2));
+  return 0;
 }

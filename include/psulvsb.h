@@ -368,6 +368,70 @@ int psulvsb_match_host(const double* src_pts, int n_src, const double* tgt_pts, 
                        const float* ft, int crosscheck, int tuple_test, double tuple_scale, uint64_t seed, int* pairs,
                        long long capacity, long long* n_pairs);
 
+/* ---- Refinement of a registration on the raw clouds (DESIGN.md section 11): rigid ICP, point-to-point or
+ * point-to-plane, in the loop of Open3D's registration_icp -- evaluate T0; then repeatedly compute the update U from
+ * the current correspondences, set T <- U T and evaluate T; stop when both |d fitness| < relative_fitness and
+ * |d inlier_rmse| < relative_rmse, or after max_iterations updates.  The correspondence of a source point (transformed
+ * from the original P by T in FP64) is the target point at the smallest squared distance <= d^2 (ties: lowest index;
+ * point-to-plane skips targets with a non-finite normal).  Convention q ~ R p + t; R column-major.  Every sum has one
+ * fixed order, so results are bit-identical from call to call.  Parity with Open3D / PCL is unpinned; the tests compare
+ * with a numpy restatement (oracle/icp.py). */
+typedef struct psulvsb_icp_params {
+  double max_correspondence_distance; /* d: finite, > 0                                                  */
+  double relative_fitness;            /* >= 0 (default 1e-6)                                             */
+  double relative_rmse;               /* >= 0 (default 1e-6)                                             */
+  int max_iterations;                 /* updates at most (default 30); 0 = evaluate T0 only             */
+  int point_to_plane;                 /* 0: point-to-point (Umeyama without scale), 1: point-to-plane   */
+} psulvsb_icp_params_t;
+
+enum {
+  PSULVSB_ICP_CONVERGED = 0,     /* the relative rule stopped the loop                                  */
+  PSULVSB_ICP_MAX_ITERATIONS = 1,/* max_iterations updates were applied                                 */
+  PSULVSB_ICP_NO_UPDATE = 2      /* too few correspondences (< 3 point-to-point, < 6 point-to-plane), a non-positive
+                                    pivot or a non-finite solution of the 6x6 system, or an empty cloud: T is the last
+                                    transform evaluated                                                  */
+};
+
+typedef struct psulvsb_icp_result {
+  double rotation[9]; /* column-major                                                                     */
+  double translation[3];
+  double fitness;     /* correspondences / n_s at the final T                                             */
+  double inlier_rmse; /* sqrt(sum d^2 / correspondences), 0 without correspondences                        */
+  int n_correspondences;
+  int iterations;     /* updates applied                                                                   */
+  int status;         /* PSULVSB_ICP_*                                                                     */
+} psulvsb_icp_result_t;
+
+/* Trace record k: the evaluation of T_k (k = 0 .. iterations). */
+typedef struct psulvsb_icp_iteration {
+  double rotation[9];
+  double translation[3];
+  double fitness;
+  double inlier_rmse;
+  int n_correspondences;
+} psulvsb_icp_iteration_t;
+
+/* max_correspondence_distance 0 (invalid: the caller sets it), max_iterations 30, relative criteria 1e-6,
+ * point-to-point. */
+void psulvsb_icp_default_params(psulvsb_icp_params_t* p);
+/* Device scratch of psulvsb_icp (depends on the sizes only); 0 for a negative size. */
+unsigned long long psulvsb_icp_workspace_bytes(int n_s, int n_t);
+/* d_src 3 x n_s, d_tgt 3 x n_t, d_tgt_normals 3 x n_t (required for point-to-plane, else ignored): column-major
+ * doubles on the device.  R0 (column-major) and t0 on the host.  Asynchronous on `stream`: no host round trip inside
+ * the loop.  d_result: one psulvsb_icp_result_t on the device; d_trace (may be NULL): room for max_iterations + 1
+ * records, of which iterations + 1 are written; d_corr (may be NULL): n_s ints, the target index of every source point
+ * at the final T or -1.  An empty cloud returns T0 with fitness 0, 0 iterations and PSULVSB_ICP_NO_UPDATE.  Bad
+ * arguments (negative sizes, a non-finite or non-positive d, max_iterations < 0, negative or NaN relative criteria,
+ * point_to_plane not 0 / 1 or without normals, a required NULL, non-finite R0 / t0) return PSULVSB_ERR_INVALID before
+ * any device work. */
+int psulvsb_icp(void* stream, const double* d_src, int n_s, const double* d_tgt, int n_t, const double* d_tgt_normals,
+                const psulvsb_icp_params_t* params, const double R0[9], const double t0[3], void* d_work,
+                psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr);
+/* The same on host buffers, synchronous (one device-to-host copy at the end). */
+int psulvsb_icp_host(const double* src, int n_s, const double* tgt, int n_t, const double* tgt_normals,
+                     const psulvsb_icp_params_t* params, const double R0[9], const double t0[3],
+                     psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace, int* corr);
+
 /* Clique escalation (registration.cc:1000-1085 -> teaser/src/graph.cc:12-125, PMC exact maximum clique) of the
  * graph with n_vertices vertices and the given edges (uint2 endpoint pairs).  A deterministic greedy maximal
  * clique (most neighbours among the remaining candidates first, ties: lowest index) gives the lower bound;

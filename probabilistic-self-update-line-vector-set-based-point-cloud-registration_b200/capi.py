@@ -32,6 +32,7 @@ SYMBOLS = [
     "psulvsb_comm_allreduce_sum_u32", "psulvsb_comm_allreduce_max_u64", "psulvsb_score_batch_sharded",
     "psulvsb_solve_sharded", "psulvsb_shard_row_range",
     "psulvsb_fpfh_workspace_bytes", "psulvsb_fpfh", "psulvsb_fpfh_host", "psulvsb_feature_nn", "psulvsb_match_host",
+    "psulvsb_icp_default_params", "psulvsb_icp_workspace_bytes", "psulvsb_icp", "psulvsb_icp_host",
 ]
 UNIQUE_ID_BYTES = 128
 
@@ -137,6 +138,41 @@ class Trace(C.Structure):
     ]
 
 
+class IcpParams(C.Structure):
+    """psulvsb_icp_params_t."""
+    _fields_ = [
+        ("max_correspondence_distance", C.c_double),
+        ("relative_fitness", C.c_double),
+        ("relative_rmse", C.c_double),
+        ("max_iterations", C.c_int),
+        ("point_to_plane", C.c_int),
+    ]
+
+
+class IcpResult(C.Structure):
+    """psulvsb_icp_result_t (rotation column-major)."""
+    _fields_ = [
+        ("rotation", C.c_double * 9),
+        ("translation", C.c_double * 3),
+        ("fitness", C.c_double),
+        ("inlier_rmse", C.c_double),
+        ("n_correspondences", C.c_int),
+        ("iterations", C.c_int),
+        ("status", C.c_int),
+    ]
+
+
+class IcpIteration(C.Structure):
+    """psulvsb_icp_iteration_t: the evaluation of T_k."""
+    _fields_ = [
+        ("rotation", C.c_double * 9),
+        ("translation", C.c_double * 3),
+        ("fitness", C.c_double),
+        ("inlier_rmse", C.c_double),
+        ("n_correspondences", C.c_int),
+    ]
+
+
 _lib = None
 _vp = C.c_void_p
 _ull = C.c_ulonglong
@@ -238,6 +274,14 @@ def _declare(L: C.CDLL) -> None:
     L.psulvsb_feature_nn.argtypes = [_vp, _vp, C.c_int, _vp, C.c_int, _vp, _vp]
     L.psulvsb_match_host.argtypes = [_vp, C.c_int, _vp, C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_double, C.c_uint64,
                                      _vp, C.c_longlong, C.POINTER(C.c_longlong)]
+    L.psulvsb_icp_default_params.argtypes = [C.POINTER(IcpParams)]
+    L.psulvsb_icp_default_params.restype = None
+    L.psulvsb_icp_workspace_bytes.argtypes = [C.c_int, C.c_int]
+    L.psulvsb_icp_workspace_bytes.restype = _ull
+    L.psulvsb_icp.argtypes = [_vp, _vp, C.c_int, _vp, C.c_int, _vp, C.POINTER(IcpParams), C.POINTER(C.c_double),
+                              C.POINTER(C.c_double), _vp, _vp, _vp, _vp]
+    L.psulvsb_icp_host.argtypes = [_vp, C.c_int, _vp, C.c_int, _vp, C.POINTER(IcpParams), C.POINTER(C.c_double),
+                                   C.POINTER(C.c_double), _vp, _vp, _vp]
     for name in SYMBOLS:
         getattr(L, name)  # AttributeError here = the library does not export what the header declares
 

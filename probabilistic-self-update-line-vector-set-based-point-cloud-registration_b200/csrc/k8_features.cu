@@ -17,6 +17,7 @@
 
 #include "common.cuh"
 #include "eig3.cuh"
+#include "grid.cuh"
 
 namespace psulvsb {
 
@@ -25,7 +26,6 @@ namespace {
 constexpr int FT_THREADS = 128;
 constexpr int FT_BINS = 11;
 constexpr int FT_DIM = 33;
-constexpr int SCAN_THREADS = 1024;
 
 struct Grid {
   double inv_h;
@@ -35,15 +35,6 @@ struct Grid {
 };
 
 __device__ __forceinline__ long long cell_of(float x, double inv_h) { return (long long)floor((double)x * inv_h); }
-
-__device__ __forceinline__ unsigned int bucket_of(long long cx, long long cy, long long cz, unsigned int mask) {
-  unsigned long long k = (unsigned long long)cx * 0x9E3779B97F4A7C15ull ^ (unsigned long long)cy * 0xC2B2AE3D27D4EB4Full ^
-                         (unsigned long long)cz * 0x165667B19E3779F9ull;
-  k ^= k >> 31;
-  k *= 0xBF58476D1CE4E5B9ull;
-  k ^= k >> 29;
-  return (unsigned int)k & mask;
-}
 
 // FP32 squared distance, left to right and unfused (the restatement evaluates the same expression in numpy float32)
 __device__ __forceinline__ float sqdist(float4 a, float4 b) {
@@ -83,54 +74,6 @@ __global__ void __launch_bounds__(FT_THREADS)
   const unsigned int b = bucket_of(cell_of(x, inv_h), cell_of(y, inv_h), cell_of(z, inv_h), mask);
   pbucket[i] = (int)b;
   atomicAdd(count + b, 1);
-}
-
-// exclusive scan of count[0, m) into start[0, m] (one CTA; m is O(n)), and cursor = start
-__global__ void __launch_bounds__(SCAN_THREADS) k8_scan(const int* __restrict__ count, int m, int* __restrict__ start,
-                                                        int* __restrict__ cursor) {
-  __shared__ int warp_tot[SCAN_THREADS / 32];
-  __shared__ int carry;
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  if (tid == 0) carry = 0;
-  __syncthreads();
-  for (int i0 = 0; i0 < m; i0 += SCAN_THREADS) {
-    const int i = i0 + tid;
-    const int v = i < m ? count[i] : 0;
-    int x = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_tot[wid] = x;
-    __syncthreads();
-    if (wid == 0) {
-      int w = warp_tot[lane];
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int y = __shfl_up_sync(0xffffffffu, w, o);
-        if (lane >= o) w += y;
-      }
-      warp_tot[lane] = w;
-    }
-    __syncthreads();
-    const int excl = carry + (wid ? warp_tot[wid - 1] : 0) + x - v;
-    if (i < m) {
-      start[i] = excl;
-      if (cursor) cursor[i] = excl;
-    }
-    __syncthreads();
-    if (tid == 0) carry += warp_tot[SCAN_THREADS / 32 - 1];
-    __syncthreads();
-  }
-  if (tid == 0) start[m] = carry;
-}
-
-__global__ void __launch_bounds__(FT_THREADS)
-    k8_grid_scatter(int n, const int* __restrict__ pbucket, int* __restrict__ cursor, int* __restrict__ tmp) {
-  const int i = blockIdx.x * FT_THREADS + threadIdx.x;
-  if (i >= n) return;
-  tmp[atomicAdd(cursor + pbucket[i], 1)] = i;
 }
 
 // the scatter's order inside a bucket depends on timing: rank each member by index instead
@@ -481,12 +424,6 @@ __global__ void __launch_bounds__(SCAN_THREADS)
 }
 
 inline size_t up256(size_t x) { return (x + 255) & ~size_t(255); }
-
-unsigned int bucket_count(int n) {
-  unsigned int nb = 1;
-  while (nb < (unsigned int)n) nb <<= 1;
-  return nb;
-}
 
 struct FpfhWork {
   int *pbucket, *count, *start, *cursor, *tmp, *counts, *kcount;

@@ -1,0 +1,124 @@
+"""Refinement of a registration on the raw clouds: rigid ICP, point-to-point or point-to-plane, on the GPU.
+
+What users of TEASER++ run after the global solve (Open3D's registration_icp, PCL's IterativeClosestPoint), through the
+C ABI (include/psulvsb.h, csrc/k9_icp.cu; DESIGN.md section 11).  `icp` takes host arrays; `icp_device` takes CUDA
+tensors [N, 3] float64 (== column-major 3xN) and runs on the current stream.  Convention: q ~ R p + t.
+"""
+from __future__ import annotations
+
+import ctypes as C
+from dataclasses import dataclass
+from typing import Optional
+
+import numpy as np
+
+from . import capi
+
+CONVERGED, MAX_ITERATIONS, NO_UPDATE = 0, 1, 2
+
+
+@dataclass
+class IcpResult:
+    R: np.ndarray                  # 3x3
+    t: np.ndarray                  # 3
+    fitness: float                 # correspondences / n_src at the final T
+    inlier_rmse: float
+    n_correspondences: int
+    iterations: int                # updates applied
+    status: int                    # CONVERGED, MAX_ITERATIONS or NO_UPDATE
+    correspondences: object        # [n_src] int32 target index or -1 (numpy; a CUDA tensor from icp_device)
+    trace: Optional[dict] = None   # per evaluation k = 0 .. iterations: R [K, 3, 3], t, fitness, inlier_rmse, n_corr
+
+
+def _cm(a, what) -> np.ndarray:
+    a = np.asarray(a, dtype=np.float64)
+    if a.ndim != 2 or a.shape[0] != 3:
+        raise ValueError(f"{what}: expected a 3xN matrix, got {a.shape}")
+    return np.asfortranarray(a)
+
+
+def _params(d, point_to_plane, max_iterations, relative_fitness, relative_rmse) -> capi.IcpParams:
+    p = capi.IcpParams()
+    capi.lib().psulvsb_icp_default_params(C.byref(p))
+    p.max_correspondence_distance = float(d)
+    p.point_to_plane = int(bool(point_to_plane))
+    p.max_iterations = int(max_iterations)
+    p.relative_fitness = float(relative_fitness)
+    p.relative_rmse = float(relative_rmse)
+    return p
+
+
+def _transform(R0, t0):
+    R = np.asarray(R0, dtype=np.float64).reshape(3, 3)
+    t = np.asarray(t0, dtype=np.float64).reshape(3)
+    return (C.c_double * 9)(*R.flatten(order="F")), (C.c_double * 3)(*t)
+
+
+def _trace(records, n) -> dict:
+    recs = [records[k] for k in range(n)]
+    return {"R": np.array([np.array(r.rotation[:]).reshape(3, 3, order="F") for r in recs]).reshape(n, 3, 3),
+            "t": np.array([r.translation[:] for r in recs]).reshape(n, 3),
+            "fitness": np.array([r.fitness for r in recs]),
+            "inlier_rmse": np.array([r.inlier_rmse for r in recs]),
+            "n_correspondences": np.array([r.n_correspondences for r in recs], dtype=np.int64)}
+
+
+def _result(res: capi.IcpResult, records, corr) -> IcpResult:
+    return IcpResult(R=np.array(res.rotation[:]).reshape(3, 3, order="F"), t=np.array(res.translation[:]),
+                     fitness=res.fitness, inlier_rmse=res.inlier_rmse, n_correspondences=res.n_correspondences,
+                     iterations=res.iterations, status=res.status, correspondences=corr,
+                     trace=None if records is None else _trace(records, res.iterations + 1))
+
+
+def icp(src, tgt, R0, t0, max_correspondence_distance: float, *, target_normals=None, point_to_plane: bool = False,
+        max_iterations: int = 30, relative_fitness: float = 1e-6, relative_rmse: float = 1e-6,
+        trace: bool = False) -> IcpResult:
+    """psulvsb_icp_host: refine (R0, t0) so that tgt ~ R src + t.  src 3 x n_s, tgt 3 x n_t; target_normals 3 x n_t is
+    required for point-to-plane (a target point with a non-finite normal is then no candidate)."""
+    s, q = _cm(src, "src"), _cm(tgt, "tgt")
+    nrm = None
+    if target_normals is not None:
+        nrm = _cm(target_normals, "target_normals")
+        if nrm.shape != q.shape:
+            raise ValueError("one normal per target point is needed")
+    p = _params(max_correspondence_distance, point_to_plane, max_iterations, relative_fitness, relative_rmse)
+    R, t = _transform(R0, t0)
+    res = capi.IcpResult()
+    records = (capi.IcpIteration * (max(int(max_iterations), 0) + 1))() if trace else None
+    corr = np.empty(s.shape[1], dtype=np.int32)
+    capi.check(capi.lib().psulvsb_icp_host(s.ctypes.data, s.shape[1], q.ctypes.data, q.shape[1],
+                                           None if nrm is None else nrm.ctypes.data, C.byref(p), R, t, C.byref(res),
+                                           records, corr.ctypes.data))
+    return _result(res, records, corr)
+
+
+def icp_device(d_src, d_tgt, R0, t0, max_correspondence_distance: float, *, d_target_normals=None,
+               point_to_plane: bool = False, max_iterations: int = 30, relative_fitness: float = 1e-6,
+               relative_rmse: float = 1e-6, trace: bool = False, work=None) -> IcpResult:
+    """psulvsb_icp on CUDA tensors [n, 3] float64 and the current stream.  The small result (and the trace) are read
+    back, which waits for the stream; the correspondences stay on the device.  `work`: an optional uint8 CUDA tensor
+    of at least psulvsb_icp_workspace_bytes(n_s, n_t) bytes to reuse."""
+    import torch
+
+    from .stages import _dev, _stream
+
+    ns, nt = d_src.shape[0], d_tgt.shape[0]
+    dev = d_src.device
+    if work is None:
+        work = torch.empty(max(1, capi.lib().psulvsb_icp_workspace_bytes(ns, nt)), dtype=torch.uint8, device=dev)
+    elif work.numel() < capi.lib().psulvsb_icp_workspace_bytes(ns, nt):
+        raise ValueError("work is smaller than psulvsb_icp_workspace_bytes(n_s, n_t)")
+    nrec = max(int(max_iterations), 0) + 1
+    out = torch.empty(C.sizeof(capi.IcpResult), dtype=torch.uint8, device=dev)
+    rec = torch.empty(nrec * C.sizeof(capi.IcpIteration) if trace else 1, dtype=torch.uint8, device=dev)
+    corr = torch.empty(max(ns, 1), dtype=torch.int32, device=dev)
+    p = _params(max_correspondence_distance, point_to_plane, max_iterations, relative_fitness, relative_rmse)
+    R, t = _transform(R0, t0)
+    capi.check(capi.lib().psulvsb_icp(_stream(), _dev(d_src) if ns else None, ns, _dev(d_tgt) if nt else None, nt,
+                                      None if d_target_normals is None else _dev(d_target_normals), C.byref(p), R, t,
+                                      _dev(work), _dev(out), _dev(rec) if trace else None, _dev(corr)))
+    res = capi.IcpResult.from_buffer_copy(out.cpu().numpy().tobytes())
+    records = None
+    if trace:
+        records = (capi.IcpIteration * nrec).from_buffer_copy(rec.cpu().numpy().tobytes())
+    return _result(res, records, corr[:ns])
