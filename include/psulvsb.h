@@ -246,6 +246,17 @@ int psulvsb_mask_symmetrize(void* stream, uint32_t* d_mask, int n, int row_strid
 int psulvsb_compact_edges(void* stream, const uint32_t* d_mask, int n, int row_stride_words,
                           const uint32_t* d_row_counts, unsigned long long* d_row_offsets, void* d_edges_uint2,
                           unsigned long long edge_capacity, unsigned long long* d_n_edges);
+/* Unknown-scale stage 1 (estimate_scaling = true, registration.cc:687-752): the length-ratio histogram with the
+ * reference's mid-loop growth of MaxScale, its peak ("the first bin to reach the maximum height") and the reduced set
+ * (bins peak, peak - 1, peak + 1, each in pair order) -- the solve's own code.  Synchronous on `stream`.
+ * d_pair_bin (optional): n (n - 1) / 2 bins, row-major pair order (i < j).  d_edges_uint2 (optional, NULL = count
+ * only): the reduced set as (i, j) pairs; fewer than *n_edges slots is PSULVSB_ERR_CAPACITY with *n_edges set.
+ * Host outputs: *n_edges, *max_scale (the final MaxScale, may be NULL), peak[2] = {max height, peak bin} (may be
+ * NULL).  NULL arrays / n_edges or n < 2: PSULVSB_ERR_INVALID before any device work; an infinite ratio or a final
+ * MaxScale above 2e6: PSULVSB_ERR_UNSUPPORTED, as in psulvsb_solve. */
+int psulvsb_ratio_reduced_set(void* stream, const double* d_src64, const double* d_dst64, int n, uint32_t* d_pair_bin,
+                              void* d_edges_uint2, unsigned long long edge_capacity, unsigned long long* n_edges,
+                              double* max_scale, unsigned int peak[2]);
 
 /* Stage 2 -- replayable sampling without replacement (registration.cc:852-861, :916-932):
  * d_out[r] = r-th distinct value of rand31(seed, domain, event, k) % n, k = 0,1,2,...

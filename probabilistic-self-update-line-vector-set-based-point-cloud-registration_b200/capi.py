@@ -22,7 +22,7 @@ SYMBOLS = [
     "psulvsb_create", "psulvsb_destroy", "psulvsb_solve", "psulvsb_solve_batch", "psulvsb_batch_upload",
     "psulvsb_batch_solve_resident", "psulvsb_batch_submit", "psulvsb_batch_wait", "psulvsb_batch_resident_size", "psulvsb_debug_set", "psulvsb_launch_count", "psulvsb_last_device_ms", "psulvsb_last_stage_ms",
     "psulvsb_last_ticks", "psulvsb_last_chunk_ticks", "psulvsb_set_batching", "psulvsb_set_host_threads", "psulvsb_pack_points", "psulvsb_consistency_mask", "psulvsb_consistency_mask_rows",
-    "psulvsb_mask_symmetrize", "psulvsb_compact_edges", "psulvsb_sample_workspace_bytes",
+    "psulvsb_mask_symmetrize", "psulvsb_compact_edges", "psulvsb_ratio_reduced_set", "psulvsb_sample_workspace_bytes",
     "psulvsb_sample_default_max_draws", "psulvsb_sample", "psulvsb_philox_fill", "psulvsb_gnc_tls_rotation",
     "psulvsb_kabsch_batch", "psulvsb_tls_translation", "psulvsb_score_batch", "psulvsb_score_one",
     "psulvsb_max_clique", "psulvsb_max_clique_scratch_words", "psulvsb_gnc_tls_rotation_batch",
@@ -230,6 +230,8 @@ def _declare(L: C.CDLL) -> None:
                                                 C.c_double, _vp, C.c_int, _vp, _vp]
     L.psulvsb_mask_symmetrize.argtypes = [_vp, _vp, C.c_int, C.c_int]
     L.psulvsb_compact_edges.argtypes = [_vp, _vp, C.c_int, C.c_int, _vp, _vp, _vp, _ull, _vp]
+    L.psulvsb_ratio_reduced_set.argtypes = [_vp, _vp, _vp, C.c_int, _vp, _vp, _ull, C.POINTER(_ull),
+                                            C.POINTER(C.c_double), C.POINTER(C.c_uint)]
     L.psulvsb_sample_workspace_bytes.argtypes = [_ull, _ull, _ull]
     L.psulvsb_sample_workspace_bytes.restype = _ull
     L.psulvsb_sample_default_max_draws.argtypes = [_ull, _ull]

@@ -323,6 +323,89 @@ int psulvsb_compact_edges(void* stream, const uint32_t* d_mask, int n, int row_s
   return launch_compact_edges(st, dj.d, 1, n, true, d_edges_uint2 != nullptr);
 }
 
+int psulvsb_ratio_reduced_set(void* stream, const double* d_src64, const double* d_dst64, int n, uint32_t* d_pair_bin,
+                              void* d_edges_uint2, unsigned long long edge_capacity, unsigned long long* n_edges,
+                              double* max_scale, unsigned int peak[2]) {
+  if (!d_src64 || !d_dst64 || !n_edges || n < 2)
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_ratio_reduced_set: NULL array / n_edges, or n < 2");
+  if (int rc = need_device()) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t L = (size_t)n * (size_t)(n - 1) / 2;
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    const size_t o = (off + 15) & ~(size_t)15;
+    off = o + bytes;
+    return o;
+  };
+  const size_t o_bins = d_pair_bin ? 0 : take(sizeof(uint32_t) * L);
+  const size_t o_rmax = take(sizeof(double) * (size_t)n), o_bpi = take(sizeof(unsigned long long) * RATIO_MAX_GROWTHS),
+               o_bps = take(sizeof(double) * RATIO_MAX_GROWTHS), o_bpn = take(sizeof(unsigned int)),
+               o_fs = take(sizeof(double)), o_bad = take(sizeof(int)), o_peak = take(4 * sizeof(unsigned int)),
+               o_cc = take(sizeof(unsigned int) * 3 * (size_t)n),
+               o_co = take(sizeof(unsigned long long) * (3 * (size_t)n + 1)), o_ne = take(sizeof(unsigned long long));
+  struct Scratch {
+    char* p = nullptr;
+    void* hist = nullptr;
+    cudaStream_t s;
+    ~Scratch() {
+      if (p) cudaFreeAsync(p, s);
+      if (hist) cudaFreeAsync(hist, s);
+    }
+  } scr;
+  scr.s = st;
+  PSU_CUDA(cudaMallocAsync((void**)&scr.p, off, st));
+  std::vector<RatioJob> rj(1);
+  RatioJob& j = rj[0];
+  std::memset(&j, 0, sizeof(j));
+  j.src64 = d_src64;
+  j.dst64 = d_dst64;
+  j.n = n;
+  j.pair_bin = d_pair_bin ? d_pair_bin : reinterpret_cast<uint32_t*>(scr.p + o_bins);
+  j.row_max = reinterpret_cast<double*>(scr.p + o_rmax);
+  j.bp_idx = reinterpret_cast<unsigned long long*>(scr.p + o_bpi);
+  j.bp_scale = reinterpret_cast<double*>(scr.p + o_bps);
+  j.bp_n = reinterpret_cast<unsigned int*>(scr.p + o_bpn);
+  j.final_scale = reinterpret_cast<double*>(scr.p + o_fs);
+  j.bad = reinterpret_cast<int*>(scr.p + o_bad);
+  j.peak = reinterpret_cast<unsigned int*>(scr.p + o_peak);
+  j.class_counts = reinterpret_cast<unsigned int*>(scr.p + o_cc);
+  j.class_offsets = reinterpret_cast<unsigned long long*>(scr.p + o_co);
+  j.n_edges = reinterpret_cast<unsigned long long*>(scr.p + o_ne);
+  j.active = 1;
+  DeviceJob<RatioJob> dj(st);
+  if (int rc = dj.put(j)) return rc;
+  auto arena = [&](size_t bytes) -> void* {
+    const cudaError_t e = cudaMallocAsync(&scr.hist, bytes, st);
+    if (e == cudaSuccess) return scr.hist;
+    scr.hist = nullptr;
+    fail(PSULVSB_ERR_CUDA, std::string("psulvsb_ratio_reduced_set: histogram allocation: ") + cudaGetErrorString(e));
+    return nullptr;
+  };
+  if (int rc = ratio_count(st, rj, dj.d, n, arena, nullptr, nullptr)) return rc;
+  unsigned long long ne = 0;
+  double fs = 0.0;
+  unsigned int pk[2] = {0u, 0u};
+  PSU_CUDA(cudaMemcpyAsync(&ne, j.n_edges, sizeof(ne), cudaMemcpyDeviceToHost, st));
+  PSU_CUDA(cudaMemcpyAsync(&fs, j.final_scale, sizeof(fs), cudaMemcpyDeviceToHost, st));
+  PSU_CUDA(cudaMemcpyAsync(pk, j.peak, sizeof(pk), cudaMemcpyDeviceToHost, st));
+  PSU_CUDA(cudaStreamSynchronize(st));
+  *n_edges = ne;
+  if (max_scale) *max_scale = fs;
+  if (peak) {
+    peak[0] = pk[0];
+    peak[1] = pk[1];
+  }
+  if (!d_edges_uint2) return PSULVSB_OK;
+  if (ne > edge_capacity)
+    return fail(PSULVSB_ERR_CAPACITY, "psulvsb_ratio_reduced_set: " + std::to_string(ne) + " edges, capacity " +
+                                          std::to_string(edge_capacity));
+  j.edges = (uint2*)d_edges_uint2;
+  j.cap = edge_capacity;
+  if (int rc = ratio_emit(st, rj, dj.d, n)) return rc;
+  PSU_CUDA(cudaStreamSynchronize(st));
+  return PSULVSB_OK;
+}
+
 unsigned long long psulvsb_sample_default_max_draws(unsigned long long n, unsigned long long count) {
   return sample_default_max_draws(n, count);
 }

@@ -11,6 +11,9 @@
 #include <math.h>
 #include <stdint.h>
 
+#include <functional>
+#include <vector>
+
 #include "common.cuh"
 
 namespace psulvsb {
@@ -54,8 +57,8 @@ struct CompactJob {
 };
 
 // unknown-scale stage 1 (k1_ratio.cu): ratio histogram and its three-bin reduced set
-constexpr unsigned int RATIO_EXCEED_CAP = 1024;  // growth candidates kept per job
-constexpr double RATIO_MAX_SCALE = 2.0e6;        // largest MaxScale served (a 40 M-bin histogram)
+constexpr double RATIO_MAX_SCALE = 2.0e6;  // largest MaxScale served (a 40 M-bin histogram)
+constexpr int RATIO_MAX_GROWTHS = 8;       // each growth more than doubles MaxScale: the 8th passes RATIO_MAX_SCALE
 struct RatioJob {
   const double* src64;  // column-major 3 x n
   const double* dst64;
@@ -63,10 +66,8 @@ struct RatioJob {
   uint32_t* pair_bin;                 // [n (n - 1) / 2] bin of every pair, row-major pair order
   unsigned int* hist;                 // [final MaxScale * 20], zero on entry (sized after phase 0)
   unsigned long long* last;           // same length, zero on entry
-  unsigned long long* exceed_idx;     // [RATIO_EXCEED_CAP] pairs with X > 10000 (growth candidates)
-  double* exceed_x;
-  unsigned int* exceed_n;             // zero on entry
-  unsigned long long* bp_idx;         // [RATIO_EXCEED_CAP] growth break points: from pair bp_idx[k] on ...
+  double* row_max;                    // [n - 1] largest ratio of each row (NaN ignored)
+  unsigned long long* bp_idx;         // [RATIO_MAX_GROWTHS] growth break points: from pair bp_idx[k] on ...
   double* bp_scale;                   // ... MaxScale == bp_scale[k]
   unsigned int* bp_n;
   double* final_scale;                // MaxScale after the last pair
@@ -76,7 +77,7 @@ struct RatioJob {
   unsigned long long* n_edges;
   uint2* edges;                       // NULL in phase 0
   unsigned long long cap;
-  int* bad;                           // 1: infinite ratio, 2: too many growth candidates, 3: histogram too large
+  int* bad;                           // written by phase 0: 0, 1 an infinite ratio, 3 final MaxScale > RATIO_MAX_SCALE
   int active;
 };
 
@@ -178,7 +179,15 @@ int launch_interleave_points(cudaStream_t st, const float4* in, int n, float4* o
 int launch_consistency_mask(cudaStream_t st, const K1Job* d_jobs, int n_jobs, int max_n, int max_rows, bool row_sectors);
 int launch_symmetrize(cudaStream_t st, uint32_t* mask, int n, int stride);
 int launch_compact_edges(cudaStream_t st, const CompactJob* d_jobs, int n_jobs, int max_n, bool scan, bool emit);
-int launch_ratio_reduced_set(cudaStream_t st, const RatioJob* d_jobs, int n_jobs, int max_n, int phase);
+// The unknown-scale stage 1 of the jobs rj (device copy d_rj) up to the reduced-set sizes: phase 0, then the final
+// MaxScales and refusal flags come back to the host (rj[b].final_scale == rj[0].final_scale + b and rj[b].bad ==
+// rj[0].bad + b; `st` is synchronised).  A refused job ends the call with PSULVSB_ERR_UNSUPPORTED.  hist_arena(bytes)
+// returns that much device memory (NULL: failed, the message is set) for the histograms, zeroed and laid out here;
+// phase 1 runs between the events ev0 and ev1 (either may be NULL) and leaves each size in *rj[b].n_edges.
+int ratio_count(cudaStream_t st, std::vector<RatioJob>& rj, RatioJob* d_rj, int max_n,
+                const std::function<void*(size_t)>& hist_arena, cudaEvent_t ev0, cudaEvent_t ev1);
+// phase 2: every job's reduced set (rj[b].edges, rj[b].cap) in reference order
+int ratio_emit(cudaStream_t st, const std::vector<RatioJob>& rj, RatioJob* d_rj, int max_n);
 
 // Draw budget for `count` distinct values out of n by rejection (mean + 8 sigma; coupon collector
 // tail for count == n).  Same formula on host and device so both agree on the stream window.

@@ -95,6 +95,26 @@ def compact_edges(mask: torch.Tensor, counts: torch.Tensor, n: int, stride: int)
     return edges[:total], offsets
 
 
+def ratio_reduced_set(src, dst, pair_bins: bool = False):
+    """Unknown-scale stage 1 of 3xN FP64 points -> dict(edges [n_edges, 2] int64 in reference order, n_edges,
+    max_scale (final MaxScale), peak_bin, peak_height[, pair_bins: n (n - 1) / 2 uint32, row-major pair order])."""
+    d_src, d_dst = to_device_points(src), to_device_points(dst)
+    n = d_src.shape[0]
+    L = capi.lib()
+    bins = torch.zeros(max(n * (n - 1) // 2, 1), dtype=torch.int32, device="cuda") if pair_bins else None
+    ne, ms, pk = C.c_ulonglong(0), C.c_double(0.0), (C.c_uint * 2)()
+    capi.check(L.psulvsb_ratio_reduced_set(_stream(), _dev(d_src), _dev(d_dst), n, _dev(bins) if pair_bins else None,
+                                           None, 0, C.byref(ne), C.byref(ms), pk))
+    edges = torch.zeros((max(ne.value, 1), 2), dtype=torch.int32, device="cuda")
+    capi.check(L.psulvsb_ratio_reduced_set(_stream(), _dev(d_src), _dev(d_dst), n, None, _dev(edges), ne.value,
+                                           C.byref(ne), C.byref(ms), pk))
+    out = {"edges": edges[:ne.value].cpu().numpy().astype(np.int64), "n_edges": ne.value, "max_scale": ms.value,
+           "peak_height": int(pk[0]), "peak_bin": int(pk[1])}
+    if pair_bins:
+        out["pair_bins"] = bins[:n * (n - 1) // 2].cpu().numpy().view(np.uint32)
+    return out
+
+
 def sample(seed: int, domain: int, event: int, n: int, count: int, max_draws: int = 0):
     out = torch.zeros(max(count, 1), dtype=torch.int32, device="cuda")
     nbytes = capi.lib().psulvsb_sample_workspace_bytes(n, count, max_draws)
