@@ -460,10 +460,16 @@ int psulvsb_max_clique(void* stream, const void* d_edges_uint2, unsigned long lo
  * counts[h] = #{ j : | q_j - s (R_h p_j + t_h) | <= tau } over all n points, evaluated in FP32
  * from float4 tiles with every point inside the FP32 error band re-evaluated in FP64, plus the
  * argmax packed as (count << 32) | (0xFFFFFFFF - h) in *d_best (first best hypothesis wins).
+ * *d_best is combined with atomicMax, not overwritten: zero it before the first call (calls over
+ * parts of one hypothesis set with their hyp_begin may then share it).  d_best and
+ * d_border_count (units re-evaluated in FP64, added to *d_border_count) may be NULL.
  * d_hyp: n_hyp x 12 doubles (R column-major then t).  hyp_begin offsets the ids written into
- * d_best (hypothesis sharding across GPUs).  center_src / center_dst: the (host) centres the
- * float4 tiles were packed with (psulvsb_pack_points), NULL = 0; coord_bound: max |coordinate|
- * of the packed tiles. */
+ * d_best (hypothesis sharding across GPUs); hyp_begin + n_hyp must not exceed 0xFFFFFFFF
+ * (PSULVSB_ERR_UNSUPPORTED).  center_src / center_dst: the (host) centres the float4 tiles were
+ * packed with (psulvsb_pack_points), NULL = 0; coord_bound: max |coordinate| of the packed tiles.
+ * n = 0 zeroes the counts (and *d_best receives the first hypothesis's key); n < 0 is
+ * PSULVSB_ERR_INVALID.  When tau^2 or the error band exceeds the FP32 range, every point is
+ * re-evaluated in FP64: the counts stay exact, at FP64 speed. */
 int psulvsb_score_batch(void* stream, const void* d_src_f4, const void* d_dst_f4, const double* d_src64,
                         const double* d_dst64, int n, const double* d_hyp, unsigned long long n_hyp,
                         unsigned long long hyp_begin, double scale, double tau, double coord_bound,

@@ -59,7 +59,8 @@ __global__ void __launch_bounds__(SB_THREADS)
   // ---- hypotheses -> registers: Rf = s R, tf = s (R c_src + t) - c_dst  (centred coordinates)
   float Rf[SB_HPT][9], tf[SB_HPT][3], eps[SB_HPT], mn[SB_HPT];
   int cnt[SB_HPT];
-  const float tau2 = (float)(a.tau * a.tau);
+  const double tau2d = a.tau * a.tau;
+  const float tau2 = (float)tau2d;
 #pragma unroll
   for (int k = 0; k < SB_HPT; ++k) {
     const unsigned long long h = h0 + k;
@@ -78,9 +79,12 @@ __global__ void __launch_bounds__(SB_THREADS)
         tf[k][r] = (float)tp;
         tmax = fmax(tmax, fabs(tp));
       }
-      // |u - u_c| <= 64 mu tau (G + tau),  G = |t'|_inf + (1 + sqrt3 s) Cmax   (DESIGN.md "K4 error band")
+      // a wrong fast sign has |u| <= 64 mu tau (G + tau) + 640 (mu G)^2,  G = |t'|_inf + (1 + sqrt3 s) Cmax
+      // (DESIGN.md "K4 error band"); tau^2 or the band beyond FP32: eps = inf sends every point to the FP64 fix-up
       const double G = tmax + (1.0 + 1.7320508 * fabs(a.scale)) * (double)a.coord_bound;
-      eps[k] = (float)(64.0 * 5.9604644775390625e-08 * a.tau * (G + a.tau) * 1.0001) + 1e-37f;
+      const double muG = 5.9604644775390625e-08 * G;
+      const double e = (64.0 * 5.9604644775390625e-08 * a.tau * (G + a.tau) + 640.0 * (muG * muG)) * 1.0001;
+      eps[k] = (e < 3.4028234663852886e38 && tau2d < 3.4028234663852886e38) ? (float)e + 1e-37f : __int_as_float(0x7f800000);
     } else {
 #pragma unroll
       for (int i = 0; i < 9; ++i) Rf[k][i] = 0.f;
@@ -232,6 +236,11 @@ __global__ void __launch_bounds__(SB_THREADS)
   }
 }
 
+// n = 0: the key of the first hypothesis (count 0), combined like the batch kernel's
+__global__ void score_empty_best_kernel(unsigned long long* __restrict__ best, unsigned long long key) {
+  if (key) atomicMax(best, key);
+}
+
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
     score_one_kernel(const double* __restrict__ src, const double* __restrict__ dst, int n, double scale,
@@ -308,8 +317,19 @@ int launch_score_batch(cudaStream_t st, const float4* src, const float4* dst, co
                        int n, const double* hyp, unsigned long long n_hyp, unsigned long long hyp_begin, double scale,
                        double tau, double coord_bound, const double* csrc, const double* cdst, uint32_t* counts,
                        unsigned long long* best, unsigned long long* border) {
-  if (n_hyp == 0 || n <= 0) return PSULVSB_OK;
-  if (hyp_begin + n_hyp > 0xFFFFFFFFull) return fail(PSULVSB_ERR_UNSUPPORTED, "score_batch: hypothesis id > 32 bits");
+  if (n < 0) return fail(PSULVSB_ERR_INVALID, "score_batch: n < 0");
+  if (n_hyp == 0) return PSULVSB_OK;
+  // ids hyp_begin .. hyp_begin + n_hyp - 1 must stay below 0xFFFFFFFF (written so that it cannot wrap)
+  if (n_hyp > 0xFFFFFFFFull || hyp_begin > 0xFFFFFFFFull - n_hyp)
+    return fail(PSULVSB_ERR_UNSUPPORTED, "score_batch: hypothesis id > 32 bits");
+  if (n == 0) {  // no points: every count is 0, and the first hypothesis is the best
+    PSU_CUDA(cudaMemsetAsync(counts, 0, sizeof(uint32_t) * n_hyp, st));
+    if (best) {
+      score_empty_best_kernel<<<1, 1, 0, st>>>(best, 0xFFFFFFFFull - hyp_begin);
+      PSU_CHECK_LAUNCH("score_empty_best_kernel");
+    }
+    return PSULVSB_OK;
+  }
   ScoreArgs a;
   a.scale = scale;
   a.tau = tau;
