@@ -198,6 +198,7 @@ int psulvsb_debug_set(const char* name, double value) {
   else if (n == "sample_list_cap_test") k.sample_list_cap_test = (int)value;
   else if (n == "k1_variant") k.k1_variant = (int)value;
   else if (n == "upload_prof") k.upload_prof = (int)value;
+  else if (n == "edge_wide") k.edge_wide = (int)value;
   else if (n == "reset") k = DebugKnobs();
   else return fail(PSULVSB_ERR_INVALID, "psulvsb_debug_set: unknown switch " + n);
   return PSULVSB_OK;
@@ -314,13 +315,13 @@ int psulvsb_compact_edges(void* stream, const uint32_t* d_mask, int n, int row_s
   j.stride = row_stride_words;
   j.row_counts = d_row_counts;
   j.offsets = d_row_offsets;
-  j.edges = (uint2*)d_edges_uint2;
+  j.edges = d_edges_uint2;
   j.cap = edge_capacity;
   j.n_edges = d_n_edges;
   j.active = 1;
   DeviceJob<CompactJob> dj(st);
   if (int rc = dj.put(j)) return rc;
-  return launch_compact_edges(st, dj.d, 1, n, true, d_edges_uint2 != nullptr);
+  return launch_compact_edges(st, dj.d, 1, n, true, d_edges_uint2 != nullptr, false);
 }
 
 int psulvsb_ratio_reduced_set(void* stream, const double* d_src64, const double* d_dst64, int n, uint32_t* d_pair_bin,
@@ -399,9 +400,9 @@ int psulvsb_ratio_reduced_set(void* stream, const double* d_src64, const double*
   if (ne > edge_capacity)
     return fail(PSULVSB_ERR_CAPACITY, "psulvsb_ratio_reduced_set: " + std::to_string(ne) + " edges, capacity " +
                                           std::to_string(edge_capacity));
-  j.edges = (uint2*)d_edges_uint2;
+  j.edges = d_edges_uint2;
   j.cap = edge_capacity;
-  if (int rc = ratio_emit(st, rj, dj.d, n)) return rc;
+  if (int rc = ratio_emit(st, rj, dj.d, n, false)) return rc;
   PSU_CUDA(cudaStreamSynchronize(st));
   return PSULVSB_OK;
 }

@@ -51,6 +51,7 @@ struct DebugKnobs {
   int sample_list_cap_test = 0;   // > 0: caps the sampler's bucket lists (exercises the overflow fallback)
   int k1_variant = 0;             // 1..4: rows per thread of the consistency kernel
   int upload_prof = 0;            // 1: print the upload's phase timings to stderr
+  int edge_wide = 0;              // 1: the engine keeps the reduced set in EdgeWide format whatever the working-set size
 };
 DebugKnobs& debug_knobs();
 

@@ -710,7 +710,7 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
       if (int rc = launch_consistency_mask(st, m.k1, B, maxC, sharded ? row_e - row_b : maxC, true)) return rc;
     PSU_CUDA(cudaEventRecord(ev_m1, st));
     ++launches;
-    if (int rc = launch_compact_edges(st, m.cj, B, maxC, true, false)) return rc;
+    if (int rc = launch_compact_edges(st, m.cj, B, maxC, true, false, false)) return rc;
     ++launches;
   }
   if (int rc = h_small.ensure((sizeof(unsigned long long) + sizeof(int)) * (size_t)B + 64 + 66 * sizeof(unsigned long long)))
@@ -735,7 +735,10 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
     PSU_CUDA(cudaStreamSynchronize(st));
   }
 
-  // ---- edge arena, sized from the measured reduced-set sizes
+  // ---- edge arena, sized from the measured reduced-set sizes.  The reduced set is EdgeNarrow (4 bytes per edge) when
+  // every working set of the chunk fits 16-bit point indices; the sharded exchange moves EdgeWide lists.
+  bool narrow = !sharded && !debug_knobs().edge_wide;
+  for (int b = 0; b < B; ++b) narrow = narrow && edge_narrow_fits(lay[(size_t)(b0 + b)].Ccap);
   const int grid_ctas_max = sm_count() / (B > 0 ? B : 1);  // CTAs per registration the GNC kernel's grid mode may use
   unsigned long long max_cap = 0, max_nred = 0;
   {
@@ -747,7 +750,7 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
         unsigned long long cap = h_nedges[b] + reserve[(size_t)(b0 + b)];
         if (cap < 64) cap = 64;
         J.edge_cap = cap;
-        J.edges = be.take<uint2>((size_t)cap);
+        J.edges = narrow ? (void*)be.take<EdgeNarrow::T>((size_t)cap) : (void*)be.take<EdgeWide::T>((size_t)cap);
         // (the (1.0, 1.0) rate pair draws ALL n values by rejection -- a random order, ~n (ln n + 10.6) draws)
         J.first_words = sample_table_words(cap, sample_default_max_draws(cap, cap));
         J.first = be.take<uint32_t>((size_t)J.first_words);
@@ -778,7 +781,7 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
           rj[(size_t)b].cap = cap;
         }
         // (sharded: this rank's rows land at their place in the global list)
-        cj[(size_t)b].edges = J.edges + (sharded && be.base ? shard_off[(size_t)comm_rank(comm)] : 0ull);
+        cj[(size_t)b].edges = static_cast<EdgeWide::T*>(J.edges) + (sharded && be.base ? shard_off[(size_t)comm_rank(comm)] : 0ull);
         cj[(size_t)b].cap = cap - (sharded ? shard_off[(size_t)comm_rank(comm)] : 0ull);
         max_cap = cap > max_cap ? cap : max_cap;
         max_nred = h_nedges[b] > max_nred ? h_nedges[b] : max_nred;
@@ -792,10 +795,10 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
   if (max_cap >= 0x7FFFFFF0ull) return fail(PSULVSB_ERR_UNSUPPORTED, "reduced set exceeds the 31-bit sample / line-vector indices");
   PSU_CUDA(cudaMemcpyAsync(m.jobs, jobs.data(), sizeof(JobCtl) * (size_t)B, cudaMemcpyHostToDevice, st));
   if (ratio) {
-    if (int rc = ratio_emit(st, rj, m.rj, maxC)) return rc;
+    if (int rc = ratio_emit(st, rj, m.rj, maxC, narrow)) return rc;
   } else {
     PSU_CUDA(cudaMemcpyAsync(m.cj, cj.data(), sizeof(CompactJob) * (size_t)B, cudaMemcpyHostToDevice, st));
-    if (int rc = launch_compact_edges(st, m.cj, B, maxC, false, true)) return rc;
+    if (int rc = launch_compact_edges(st, m.cj, B, maxC, false, true, narrow)) return rc;
     if (sharded) {  // every rank receives every other rank's block of the edge list (8 bytes per edge, over NVLink)
       std::vector<unsigned long long> off32(shard_off);
       for (auto& o : off32) o *= 2ull;
@@ -872,12 +875,11 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
     const double elapsed =
         std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t_begin).count() / 1e6;
     if (round_start_pending) {
-      engine_round_start_kernel<<<B, kCtlThreads, 0, st>>>(m.jobs, m.sl, m.sb, m.gj, m.cq, P, m.n_done);
-      PSU_CHECK_LAUNCH("engine_round_start_kernel");
-      if (int rc = launch_sample(st, m.sl, B, draws_bound, max_cap, true)) return rc;
+      if (int rc = launch_round_start(st, B, m.jobs, m.sl, m.sb, m.gj, m.cq, P, m.n_done, narrow)) return rc;
+      if (int rc = launch_sample(st, m.sl, B, draws_bound, max_cap, max_ccap, narrow)) return rc;
       launches += 5;
     }
-    if (int rc = launch_sample(st, m.sb, B, draws_bound, max_cap)) return rc;
+    if (int rc = launch_sample(st, m.sb, B, draws_bound, max_cap, 0, narrow)) return rc;
     if (ratio) {
       engine_scale_kernel<<<B, kCtlThreads, 0, st>>>(m.jobs, m.gj, m.cq, P);
       PSU_CHECK_LAUNCH("engine_scale_kernel");

@@ -15,6 +15,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "edge_fmt.cuh"
 
 namespace psulvsb {
 
@@ -50,7 +51,7 @@ struct CompactJob {
   int n, stride;
   const uint32_t* row_counts;
   unsigned long long* offsets;  // [n+1]
-  uint2* edges;
+  void* edges;                  // EdgeWide or EdgeNarrow list (edge_fmt.cuh), as the launch says
   unsigned long long cap;
   unsigned long long* n_edges;
   int active;
@@ -75,7 +76,7 @@ struct RatioJob {
   unsigned int* class_counts;         // [3 n]
   unsigned long long* class_offsets;  // [3 n + 1]
   unsigned long long* n_edges;
-  uint2* edges;                       // NULL in phase 0
+  void* edges;                        // NULL in phase 0; EdgeWide or EdgeNarrow list, as ratio_emit says
   unsigned long long cap;
   int* bad;                           // written by phase 0: 0, 1 an infinite ratio, 3 final MaxScale > RATIO_MAX_SCALE
   int active;
@@ -99,15 +100,15 @@ struct SampleJob {
   int identity;                  // 1: out[r] = r (registration.cc:839-847, empty-sample fallback)
   // optional post-processing fused into the emission kernel (batch engine):
   int post;                      // 0 none, 1 endpoint flags of the sampled edges, 2 gather basic edges
-  const uint2* edges;            // post 1/2: the reduced set
+  const void* edges;             // post 1/2: the reduced set, EdgeWide or EdgeNarrow (edge_fmt.cuh), as the launch says
   const uint32_t* via;           // post 2: L_sampled (out[r] indexes it)
-  uint2* gathered;               // post 2: gathered[r] = edges[via[out[r]]]
+  uint2* gathered;               // post 2: gathered[r] = edges[via[out[r]]], unpacked (uint2 whatever the list's format)
   const double* pts8;            // post 2, optional: 64-byte point records (sx sy sz tx ty tz 0 0) ...
   double* lv_out;                // ... then the line vector of gathered[r] goes to lv_out[c * lv_cap + r], c = 0..5
   unsigned long long lv_cap;     //     (r < lv_cap): the GNC-TLS kernel finds its line vectors already formed
   uint8_t* flags;                // post 1: [n_points] endpoint flags
   uint32_t* vbits;               // post 1, optional: [ceil(n / 32)] value bitmap, zero on entry and on exit -- the flags
-                                 // then come from a streaming pass over the edge list (launch_sample(flag_pass = true))
+                                 // then come from a streaming pass over the edge list (launch_sample(flag_points > 0))
   int n_points;
   int active;
 };
@@ -178,7 +179,9 @@ int launch_interleave_points(cudaStream_t st, const float4* in, int n, float4* o
 // row_sectors: EVERY job's mask has stride % 8 == 0 (rows on 32-byte sector boundaries): tiles leave as whole sectors
 int launch_consistency_mask(cudaStream_t st, const K1Job* d_jobs, int n_jobs, int max_n, int max_rows, bool row_sectors);
 int launch_symmetrize(cudaStream_t st, uint32_t* mask, int n, int stride);
-int launch_compact_edges(cudaStream_t st, const CompactJob* d_jobs, int n_jobs, int max_n, bool scan, bool emit);
+// narrow: the jobs' edge lists are EdgeNarrow (every n <= kEdgeNarrowMaxPoints), else EdgeWide
+int launch_compact_edges(cudaStream_t st, const CompactJob* d_jobs, int n_jobs, int max_n, bool scan, bool emit,
+                         bool narrow);
 // The unknown-scale stage 1 of the jobs rj (device copy d_rj) up to the reduced-set sizes: phase 0, then the final
 // MaxScales and refusal flags come back to the host (rj[b].final_scale == rj[0].final_scale + b and rj[b].bad ==
 // rj[0].bad + b; `st` is synchronised).  A refused job ends the call with PSULVSB_ERR_UNSUPPORTED.  hist_arena(bytes)
@@ -186,8 +189,8 @@ int launch_compact_edges(cudaStream_t st, const CompactJob* d_jobs, int n_jobs, 
 // phase 1 runs between the events ev0 and ev1 (either may be NULL) and leaves each size in *rj[b].n_edges.
 int ratio_count(cudaStream_t st, std::vector<RatioJob>& rj, RatioJob* d_rj, int max_n,
                 const std::function<void*(size_t)>& hist_arena, cudaEvent_t ev0, cudaEvent_t ev1);
-// phase 2: every job's reduced set (rj[b].edges, rj[b].cap) in reference order
-int ratio_emit(cudaStream_t st, const std::vector<RatioJob>& rj, RatioJob* d_rj, int max_n);
+// phase 2: every job's reduced set (rj[b].edges, rj[b].cap) in reference order, EdgeNarrow lists if `narrow`
+int ratio_emit(cudaStream_t st, const std::vector<RatioJob>& rj, RatioJob* d_rj, int max_n, bool narrow);
 
 // Draw budget for `count` distinct values out of n by rejection (mean + 8 sigma; coupon collector
 // tail for count == n).  Same formula on host and device so both agree on the stream window.
@@ -213,8 +216,10 @@ unsigned long long sample_chunk_slots(unsigned long long max_draws);
 unsigned long long sample_list_entries(unsigned long long n, unsigned long long max_draws);  // 0: lists not applicable
 unsigned long long sample_list_counters();
 unsigned long long sample_table_words(unsigned long long n, unsigned long long max_draws);
+// flag_points > 0: the post-1 jobs' endpoint flags come from the flag pass (SampleJob::vbits), n_points <= flag_points;
+// narrow: the jobs' SampleJob::edges are EdgeNarrow lists, else EdgeWide
 int launch_sample(cudaStream_t st, const SampleJob* d_jobs, int n_jobs, unsigned long long max_draws_bound,
-                  unsigned long long n_bound, bool flag_pass = false);
+                  unsigned long long n_bound, int flag_points = 0, bool narrow = false);
 int launch_philox_fill(cudaStream_t st, uint64_t seed, uint32_t domain, uint32_t event, unsigned long long first_k,
                        unsigned long long count, uint32_t* out);
 

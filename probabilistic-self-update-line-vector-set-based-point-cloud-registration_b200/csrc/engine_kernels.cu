@@ -244,6 +244,7 @@ __global__ void __launch_bounds__(BLK)
 // round start: self-update append (registration.cc:786-832) and the L-sampled draw set-up
 // (registration.cc:837-863)
 // ------------------------------------------------------------------------------------------
+template <class F>
 __global__ void __launch_bounds__(BLK)
     engine_round_start_kernel(JobCtl* __restrict__ jobs, SampleJob* __restrict__ sl, SampleJob* __restrict__ sb,
                               GncJob* __restrict__ gj, CliqueJob* __restrict__ cq, EngineParams P,
@@ -307,7 +308,7 @@ __global__ void __launch_bounds__(BLK)
       const int cnt = m0 + i;
       for (int j = tid; j < cnt; j += BLK) {
         const int other = (j < m0) ? J.inlier_map[j] : (C + (j - m0));
-        J.edges[off + j] = make_uint2((unsigned)(C + i), (unsigned)other);
+        F::store(J.edges, off + j, (unsigned)(C + i), (unsigned)other);
       }
     }
   }
@@ -360,6 +361,16 @@ __global__ void __launch_bounds__(BLK)
     J.phase = PHASE_LOCAL;
     prepare_local(J, sb[blockIdx.x], gj[blockIdx.x], cq[blockIdx.x], P);
   }
+}
+
+int launch_round_start(cudaStream_t st, int n_jobs, JobCtl* jobs, SampleJob* sl, SampleJob* sb, GncJob* gj, CliqueJob* cq,
+                       const EngineParams& P, int* n_done, bool narrow) {
+  if (narrow)
+    engine_round_start_kernel<EdgeNarrow><<<n_jobs, BLK, 0, st>>>(jobs, sl, sb, gj, cq, P, n_done);
+  else
+    engine_round_start_kernel<EdgeWide><<<n_jobs, BLK, 0, st>>>(jobs, sl, sb, gj, cq, P, n_done);
+  PSU_CHECK_LAUNCH("engine_round_start_kernel");
+  return PSULVSB_OK;
 }
 
 // ------------------------------------------------------------------------------------------

@@ -10,8 +10,9 @@ constexpr int kCtlThreads = 1024;  // block size of every control kernel (== BLK
 
 __global__ void engine_init_kernel(JobCtl* jobs, SampleJob* sl, SampleJob* sb, GncJob* gj, CliqueJob* cq,
                                    const unsigned long long* n_edges, EngineParams P, int* n_done);
-__global__ void engine_round_start_kernel(JobCtl* jobs, SampleJob* sl, SampleJob* sb, GncJob* gj, CliqueJob* cq,
-                                          EngineParams P, int* n_done);
+// the round-start kernel over n_jobs registrations; narrow: JobCtl::edges are EdgeNarrow lists, else EdgeWide
+int launch_round_start(cudaStream_t st, int n_jobs, JobCtl* jobs, SampleJob* sl, SampleJob* sb, GncJob* gj, CliqueJob* cq,
+                       const EngineParams& P, int* n_done, bool narrow);
 __global__ void engine_scale_kernel(JobCtl* jobs, GncJob* gj, CliqueJob* cq, EngineParams P);
 __global__ void engine_local_control_kernel(JobCtl* jobs, SampleJob* sl, SampleJob* sb, GncJob* gj, CliqueJob* cq,
                                             EngineParams P, double elapsed_s, int* n_done);

@@ -72,7 +72,7 @@ struct JobCtl {
   double* xs_sorted;         // [translation_sort_doubles(Ccap)] sorting scratch of the max-stabbing translation
   uint8_t* sampled_flags;    // [Ccap]
   uint8_t* rot_flags;        // [Ccap]
-  uint2* edges;              // reduced set (L_reduced_set) as endpoint pairs
+  void* edges;               // reduced set (L_reduced_set) as endpoint pairs, EdgeNarrow or EdgeWide (edge_fmt.cuh)
   unsigned long long edge_cap;
   uint32_t* vbits;            // sampler value bitmap of the L sample [ceil(edge_cap / 32)], zero between uses
   uint32_t* blist;            // sampler bucket lists [blist_cap]

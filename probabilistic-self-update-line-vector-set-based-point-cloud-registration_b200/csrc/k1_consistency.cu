@@ -571,23 +571,30 @@ __global__ void __launch_bounds__(1024) row_scan_kernel(const CompactJob* __rest
   }
 }
 
-// one warp per row: emit (i, j) for every set bit j > i, ascending j, at offsets[i]
+// one warp per row: emit (i, j) for every set bit j > i, ascending j, at offsets[i], in edge format F
+template <class F>
 __global__ void compact_edges_kernel(const CompactJob* __restrict__ jobs) {
   const CompactJob& job = jobs[blockIdx.y];
   if (!job.active || !job.edges) return;
   const uint32_t* __restrict__ mask = job.mask;
   const int n = job.n, stride = job.stride;
   const unsigned long long cap = job.cap;
-  uint2* __restrict__ edges = job.edges;
+  void* __restrict__ edges = job.edges;
   const int row = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
   const int lane = threadIdx.x & 31;
   if (row >= n) return;
-  if (job.row_counts && job.row_counts[row] == 0u) return;  // nothing to emit (or a row another rank owns: its words are not this rank's)
+  // the row's count, offset and first 32 mask words are loaded together, and each step loads the next 32 words before
+  // it emits: a warp lives for a few steps, so exposed load latency, not bytes, bounded this pass
+  const unsigned int count = job.row_counts ? job.row_counts[row] : 1u;
   const int W = (n + 31) >> 5;
   unsigned long long base = job.offsets[row];
+  const uint32_t* __restrict__ mrow = mask + (size_t)row * stride;
+  uint32_t next = (row >> 5) + lane < W ? mrow[(row >> 5) + lane] : 0u;
+  if (count == 0u) return;  // nothing to emit (or a row another rank owns: its words are not this rank's)
   for (int w0 = row >> 5; w0 < W; w0 += 32) {
     const int w = w0 + lane;
-    uint32_t word = (w < W) ? mask[(size_t)row * stride + w] : 0u;
+    uint32_t word = next;
+    next = (w + 32 < W) ? mrow[w + 32] : 0u;
     const int pc = __popc(word);
     int incl = pc;
 #pragma unroll
@@ -599,7 +606,7 @@ __global__ void compact_edges_kernel(const CompactJob* __restrict__ jobs) {
     while (word) {
       const int b = __ffs(word) - 1;
       word &= word - 1;
-      if (pos < cap) edges[pos] = make_uint2((unsigned)row, (unsigned)(w * 32 + b));
+      if (pos < cap) F::store(edges, pos, (unsigned)row, (unsigned)(w * 32 + b));
       ++pos;
     }
     base += (unsigned long long)__shfl_sync(0xffffffffu, incl, 31);
@@ -710,7 +717,8 @@ int launch_symmetrize(cudaStream_t st, uint32_t* mask, int n, int stride) {
   return PSULVSB_OK;
 }
 
-int launch_compact_edges(cudaStream_t st, const CompactJob* d_jobs, int n_jobs, int max_n, bool scan, bool emit) {
+int launch_compact_edges(cudaStream_t st, const CompactJob* d_jobs, int n_jobs, int max_n, bool scan, bool emit,
+                         bool narrow) {
   if (n_jobs <= 0 || max_n < 1) return PSULVSB_OK;
   if (scan) {
     row_scan_kernel<<<n_jobs, 1024, 0, st>>>(d_jobs);
@@ -719,7 +727,10 @@ int launch_compact_edges(cudaStream_t st, const CompactJob* d_jobs, int n_jobs, 
   if (emit) {
     const long long threads = (long long)max_n * 32;
     dim3 grid((unsigned)((threads + 255) / 256), n_jobs);
-    compact_edges_kernel<<<grid, 256, 0, st>>>(d_jobs);
+    if (narrow)
+      compact_edges_kernel<EdgeNarrow><<<grid, 256, 0, st>>>(d_jobs);
+    else
+      compact_edges_kernel<EdgeWide><<<grid, 256, 0, st>>>(d_jobs);
     PSU_CHECK_LAUNCH("compact_edges_kernel");
   }
   return PSULVSB_OK;

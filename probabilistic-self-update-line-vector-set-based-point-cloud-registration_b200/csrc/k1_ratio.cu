@@ -336,7 +336,8 @@ __global__ void __launch_bounds__(1024) ratio_class_scan_kernel(const RatioJob* 
   }
 }
 
-// one warp per row: emit (i, j) of every member of class c at class_offsets[c * n + i], ascending j
+// one warp per row: emit (i, j) of every member of class c at class_offsets[c * n + i], ascending j, in edge format F
+template <class F>
 __global__ void __launch_bounds__(256) ratio_class_emit_kernel(const RatioJob* __restrict__ jobs) {
   const RatioJob& job = jobs[blockIdx.y];
   if (!job.active || !job.edges) return;
@@ -358,7 +359,7 @@ __global__ void __launch_bounds__(256) ratio_class_emit_kernel(const RatioJob* _
       const unsigned int m = __ballot_sync(0xffffffffu, c == cc);
       if (c == cc) {
         const unsigned long long p = pos[cc] + (unsigned long long)__popc(m & ((1u << lane) - 1u));
-        if (p < job.cap) job.edges[p] = make_uint2((unsigned)row, (unsigned)(row + 1 + k));
+        if (p < job.cap) F::store(job.edges, p, (unsigned)row, (unsigned)(row + 1 + k));
       }
       pos[cc] += (unsigned long long)__popc(m);
     }
@@ -369,7 +370,8 @@ __global__ void __launch_bounds__(256) ratio_class_emit_kernel(const RatioJob* _
 
 // phase 0: row maxima + replay of the growth rule (final MaxScale ready -> host sizes the histogram);
 // phase 1: bins + histogram + peak + class counts + scan (n_edges ready); phase 2: emit edges
-static int launch_ratio_reduced_set(cudaStream_t st, const RatioJob* d_jobs, int n_jobs, int max_n, int phase) {
+static int launch_ratio_reduced_set(cudaStream_t st, const RatioJob* d_jobs, int n_jobs, int max_n, int phase,
+                                    bool narrow = false) {
   if (n_jobs <= 0 || max_n < 2) return PSULVSB_OK;
   const long long row_threads = (long long)max_n * 32;
   const dim3 row_grid((unsigned)((row_threads + 255) / 256), (unsigned)n_jobs);
@@ -396,7 +398,10 @@ static int launch_ratio_reduced_set(cudaStream_t st, const RatioJob* d_jobs, int
     ratio_class_scan_kernel<<<n_jobs, 1024, 0, st>>>(d_jobs);
     PSU_CHECK_LAUNCH("ratio_class_scan_kernel");
   } else {
-    ratio_class_emit_kernel<<<row_grid, 256, 0, st>>>(d_jobs);
+    if (narrow)
+      ratio_class_emit_kernel<EdgeNarrow><<<row_grid, 256, 0, st>>>(d_jobs);
+    else
+      ratio_class_emit_kernel<EdgeWide><<<row_grid, 256, 0, st>>>(d_jobs);
     PSU_CHECK_LAUNCH("ratio_class_emit_kernel");
   }
   return PSULVSB_OK;
@@ -443,9 +448,9 @@ int ratio_count(cudaStream_t st, std::vector<RatioJob>& rj, RatioJob* d_rj, int 
   return PSULVSB_OK;
 }
 
-int ratio_emit(cudaStream_t st, const std::vector<RatioJob>& rj, RatioJob* d_rj, int max_n) {
+int ratio_emit(cudaStream_t st, const std::vector<RatioJob>& rj, RatioJob* d_rj, int max_n, bool narrow) {
   PSU_CUDA(cudaMemcpyAsync(d_rj, rj.data(), sizeof(RatioJob) * rj.size(), cudaMemcpyHostToDevice, st));
-  return launch_ratio_reduced_set(st, d_rj, (int)rj.size(), max_n, 2);
+  return launch_ratio_reduced_set(st, d_rj, (int)rj.size(), max_n, 2, narrow);
 }
 
 }  // namespace psulvsb

@@ -40,6 +40,8 @@ constexpr int SMP_CHUNK = SMP_THREADS * 4;  // draws per chunk (one Philox block
 constexpr int SMB_THREADS = 1024;           // bucket pass (one CTA per SM: the table fills shared memory)
 constexpr int SMP_BW = 49152;               // values per bucket (192 KB of shared memory)
 constexpr int SMP_MAX_LIST_BUCKETS = 512;   // bucket lists are used for 3 .. 512 buckets
+constexpr int SMF_THREADS = 256;            // flag pass
+constexpr int SMF_MAX_POINTS = 65536 * 8;   // flag pass: largest n_points marked in shared memory (a 64 KB bitmap)
 
 // layout of the bucket lists for (n, max_draws).  An entry is ONE 32-bit word where that works, (k << w_bits) | (v - lo): the draw
 // index takes the bits it needs and the rest addresses the value inside its bucket, so the bucket width shrinks
@@ -473,6 +475,7 @@ __global__ void __launch_bounds__(SMB_THREADS, 1) sample_bucket_kernel(const Sam
   if (tid == 0 && carry_s < job.count && job.status) job.status[0] = 0ull;  // draw budget too small
 }
 
+template <class F>
 __global__ void __launch_bounds__(SMP_THREADS) sample_emit_kernel(const SampleJob* __restrict__ jobs) {
   const SampleJob& job = jobs[blockIdx.y];
   if (!job.active) return;
@@ -485,11 +488,11 @@ __global__ void __launch_bounds__(SMP_THREADS) sample_emit_kernel(const SampleJo
          r += (unsigned long long)gridDim.x * SMP_THREADS) {
       out[r] = (uint32_t)r;
       if (job.post == 1) {
-        const uint2 e = job.edges[r];
+        const uint2 e = F::load(job.edges, r);
         job.flags[e.x] = 1;
         job.flags[e.y] = 1;
       } else if (job.post == 2) {
-        job.gathered[r] = job.edges[job.via[r]];
+        job.gathered[r] = F::load(job.edges, job.via[r]);
       }
     }
     if (blockIdx.x == 0 && tid == 0 && job.status) job.status[0] = 1ull;  // nothing drawn; non-zero = success
@@ -540,12 +543,12 @@ __global__ void __launch_bounds__(SMP_THREADS) sample_emit_kernel(const SampleJo
             if (job.post == 1 && !job.vbits) {
               // src_sampled/dst_sampled = unique endpoints of the sampled line vectors
               // (registration.cc:870-894); only the SET matters downstream, kept as per-point flags
-              const uint2 e = job.edges[v];
+              const uint2 e = F::load(job.edges, v);
               job.flags[e.x] = 1;
               job.flags[e.y] = 1;
             } else if (job.post == 2) {
               // basic line vectors (registration.cc:922-925) as endpoint pairs
-              const uint2 e = job.edges[job.via[v]];
+              const uint2 e = F::load(job.edges, job.via[v]);
               job.gathered[rank] = e;
               if (job.lv_out && rank < job.lv_cap) {
                 // the line vector itself, formed here (many warps in flight hide the dependent gathers) instead of in
@@ -578,20 +581,42 @@ __global__ void __launch_bounds__(SMP_THREADS) sample_emit_kernel(const SampleJo
 }
 
 // post 1 with a value bitmap: endpoint flags of the sampled edges (registration.cc:870-894) by STREAMING the edge list in
-// value order -- a warp takes 1024 consecutive values, skips the 32-value rows without a sampled one and reads the
-// others coalesced -- instead of one random 8-byte gather (a 64-byte HBM atom) per sampled edge.  Clears the bitmap.
-__global__ void __launch_bounds__(256) sample_flag_kernel(const SampleJob* __restrict__ jobs) {
+// value order -- a lane takes one 32-value row at a time, skips the rows without a sampled value and reads the others
+// coalesced -- instead of one random gather (a 64-byte HBM atom) per sampled edge.  Clears the bitmap.
+// The endpoints are marked in a shared-memory bitmap of the job's points (n_points <= onchip_points, the bitmap's
+// capacity; larger jobs store their flags directly): cfg-A marks ~30 endpoints per point, so each CTA then writes every marked point's flag
+// once -- 16-byte stores where 16 neighbours are all marked -- instead of two scattered byte stores per sampled edge.
+// Few CTAs per job keep that write-out small.  flags must be 16-byte aligned.
+template <class F>
+__global__ void __launch_bounds__(SMF_THREADS) sample_flag_kernel(const SampleJob* __restrict__ jobs, int onchip_points) {
   const SampleJob& job = jobs[blockIdx.y];
   if (!job.active || job.identity || job.post != 1 || !job.vbits) return;
+  extern __shared__ uint32_t pbits[];  // [ceil(n_points / 32)] endpoint bitmap
+  const int tid = threadIdx.x;
+  const bool onchip = job.n_points <= onchip_points;
+  const int pwords = (job.n_points + 31) >> 5;
+  if (onchip) {
+    for (int i = tid; i < pwords; i += SMF_THREADS) pbits[i] = 0u;
+    __syncthreads();
+  }
+  uint8_t* __restrict__ flags = job.flags;
+  auto mark = [&](uint32_t p) {
+    if (!onchip) {
+      flags[p] = 1;
+      return;
+    }
+    const uint32_t bit = 1u << (p & 31u);
+    if (!(pbits[p >> 5] & bit)) atomicOr(&pbits[p >> 5], bit);  // (most points are marked early on: a read, no atomic)
+  };
   const unsigned long long nwords = (job.n + 31) >> 5;
-  const unsigned long long threads = (unsigned long long)gridDim.x * 256;
-  const uint2* __restrict__ edges = job.edges;
+  const unsigned long long threads = (unsigned long long)gridDim.x * SMF_THREADS;
+  const void* __restrict__ edges = job.edges;
   // a lane owns one 32-value row (its bitmap word) per step and walks the set bits four at a time, loads first
-  for (unsigned long long wi = (unsigned long long)blockIdx.x * 256 + threadIdx.x; wi < nwords; wi += threads) {
+  for (unsigned long long wi = (unsigned long long)blockIdx.x * SMF_THREADS + tid; wi < nwords; wi += threads) {
     uint32_t word = __ldcg(job.vbits + wi);
     if (!word) continue;
     job.vbits[wi] = 0u;  // zero on exit
-    const uint2* __restrict__ row = edges + wi * 32;
+    const unsigned long long row = wi * 32;
     while (word) {
       uint2 e[4];
       int m = 0;
@@ -600,16 +625,44 @@ __global__ void __launch_bounds__(256) sample_flag_kernel(const SampleJob* __res
         if (word) {
           const int bit = __ffs(word) - 1;
           word &= word - 1;
-          e[j] = row[bit];
+          e[j] = F::load(edges, row + bit);
           m = j + 1;
         }
       }
 #pragma unroll
       for (int j = 0; j < 4; ++j)
         if (j < m) {
-          job.flags[e[j].x] = 1;
-          job.flags[e[j].y] = 1;
+          mark(e[j].x);
+          mark(e[j].y);
         }
+    }
+  }
+  if (!onchip) return;
+  __syncthreads();
+  // write-out: a lane takes 32 points (32 bytes of flags); only marked points are written (other CTAs of the job
+  // write theirs, the bucket pass zeroed the flags)
+  for (int w = tid; w < pwords; w += SMF_THREADS) {
+    const uint32_t bits = pbits[w];
+    if (!bits) continue;
+    uint8_t* __restrict__ f = flags + 32 * (size_t)w;
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const uint32_t half = (bits >> (16 * h)) & 0xFFFFu;
+      if (half == 0xFFFFu) {
+        reinterpret_cast<uint4*>(f)[h] = make_uint4(0x01010101u, 0x01010101u, 0x01010101u, 0x01010101u);
+        continue;
+      }
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const uint32_t nib = (half >> (4 * q)) & 0xFu;
+        uint8_t* __restrict__ g = f + 16 * h + 4 * q;
+        if (nib == 0xFu)
+          *reinterpret_cast<uint32_t*>(g) = 0x01010101u;
+        else
+#pragma unroll
+          for (int l = 0; l < 4; ++l)
+            if ((nib >> l) & 1u) g[l] = 1;
+      }
     }
   }
 }
@@ -644,12 +697,15 @@ unsigned long long sample_table_words(unsigned long long n, unsigned long long m
 
 // n_bound: upper bound of SampleJob::n over the jobs (sizes the bucket grid)
 int launch_sample(cudaStream_t st, const SampleJob* d_jobs, int n_jobs, unsigned long long max_draws_bound,
-                  unsigned long long n_bound, bool flag_pass) {
+                  unsigned long long n_bound, int flag_points, bool narrow) {
   if (n_jobs <= 0) return PSULVSB_OK;
   static bool attr_set = false;
   const size_t smem = (size_t)SMP_BW * 4 + (size_t)SMP_BW / 8;  // first-occurrence table + the bucket's value bitmap
+  const int fsmem_max = SMF_MAX_POINTS / 8;
   if (!attr_set) {
     PSU_CUDA(cudaFuncSetAttribute(sample_bucket_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    PSU_CUDA(cudaFuncSetAttribute(sample_flag_kernel<EdgeWide>, cudaFuncAttributeMaxDynamicSharedMemorySize, fsmem_max));
+    PSU_CUDA(cudaFuncSetAttribute(sample_flag_kernel<EdgeNarrow>, cudaFuncAttributeMaxDynamicSharedMemorySize, fsmem_max));
     attr_set = true;
   }
   const unsigned long long nchunks = (max_draws_bound + SMP_CHUNK - 1) / SMP_CHUNK;
@@ -668,14 +724,25 @@ int launch_sample(cudaStream_t st, const SampleJob* d_jobs, int n_jobs, unsigned
   if (bx < 1) bx = 1;
   sample_bucket_kernel<<<dim3((unsigned)bx, (unsigned)n_jobs), SMB_THREADS, smem, st>>>(d_jobs);
   PSU_CHECK_LAUNCH("sample_bucket_kernel");
-  sample_emit_kernel<<<dim3((unsigned)gx, (unsigned)n_jobs), SMP_THREADS, 0, st>>>(d_jobs);
+  if (narrow)
+    sample_emit_kernel<EdgeNarrow><<<dim3((unsigned)gx, (unsigned)n_jobs), SMP_THREADS, 0, st>>>(d_jobs);
+  else
+    sample_emit_kernel<EdgeWide><<<dim3((unsigned)gx, (unsigned)n_jobs), SMP_THREADS, 0, st>>>(d_jobs);
   PSU_CHECK_LAUNCH("sample_emit_kernel");
-  if (flag_pass) {
-    unsigned long long fx = (n_bound + 32ull * 256 - 1) / (32ull * 256);  // CTAs of 256 lanes x one 32-value row each
+  if (flag_points > 0) {
+    // CTAs of 256 lanes x one 32-value row each.  Each writes out the flags of all points it marked (C / 16 stores when
+    // they are dense), so a job gets a few CTAs, not hundreds: 8 per job at 296 jobs (measured on cfg-A: half as many
+    // took 1.92 instead of 1.81 ms per step, the lanes over the list count for more than the write-out)
+    unsigned long long fx = (n_bound + 32ull * SMF_THREADS - 1) / (32ull * SMF_THREADS);
     const unsigned long long fcap = ((unsigned long long)sm_count() * 16 + (unsigned long long)n_jobs - 1) / (unsigned long long)n_jobs;
     if (fx > fcap) fx = fcap;
     if (fx < 1) fx = 1;
-    sample_flag_kernel<<<dim3((unsigned)fx, (unsigned)n_jobs), 256, 0, st>>>(d_jobs);
+    const int onchip_points = flag_points <= SMF_MAX_POINTS ? flag_points : 0;
+    const size_t fsmem = (size_t)(onchip_points + 31) / 32 * 4;
+    if (narrow)
+      sample_flag_kernel<EdgeNarrow><<<dim3((unsigned)fx, (unsigned)n_jobs), SMF_THREADS, fsmem, st>>>(d_jobs, onchip_points);
+    else
+      sample_flag_kernel<EdgeWide><<<dim3((unsigned)fx, (unsigned)n_jobs), SMF_THREADS, fsmem, st>>>(d_jobs, onchip_points);
     PSU_CHECK_LAUNCH("sample_flag_kernel");
   }
   return PSULVSB_OK;
