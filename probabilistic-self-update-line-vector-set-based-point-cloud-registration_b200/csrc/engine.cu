@@ -741,6 +741,11 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
   for (int b = 0; b < B; ++b) narrow = narrow && edge_narrow_fits(lay[(size_t)(b0 + b)].Ccap);
   const int grid_ctas_max = sm_count() / (B > 0 ? B : 1);  // CTAs per registration the GNC kernel's grid mode may use
   unsigned long long max_cap = 0, max_nred = 0;
+  // every sample of the chunk goes to the sampler's on-chip pass except the (1.0, 1.0) escalation, whose window is
+  // longer than the draw cache and the bucket lists cover: neither is ever read, so neither is reserved
+  bool sample_onchip = true;
+  for (int b = 0; b < B; ++b)
+    sample_onchip = sample_onchip && sample_onchip_bound(std::max(h_nedges[b] + reserve[(size_t)(b0 + b)], 64ull));
   {
     Bump be;
     for (int pass = 0; pass < 2; ++pass) {
@@ -754,14 +759,14 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
         // (the (1.0, 1.0) rate pair draws ALL n values by rejection -- a random order, ~n (ln n + 10.6) draws)
         J.first_words = sample_table_words(cap, sample_default_max_draws(cap, cap));
         J.first = be.take<uint32_t>((size_t)J.first_words);
-        J.draws_cap = (cap + 3) & ~3ull;  // covers every rate pair below (1.0, 1.0); longer windows recompute
-        J.draws = be.take<uint32_t>((size_t)J.draws_cap);
+        J.draws_cap = sample_onchip ? 0ull : (cap + 3) & ~3ull;  // covers every rate pair below (1.0, 1.0); longer windows recompute
+        J.draws = J.draws_cap ? be.take<uint32_t>((size_t)J.draws_cap) : nullptr;
         J.chunk_prefix = be.take<unsigned long long>((size_t)sample_chunk_slots(sample_default_max_draws(cap, cap)));
         J.ticket = be.take<unsigned int>(4);
         // bucket lists of the sampler: sized for the L sample at the largest rate below 1.0 (0.5 -> ~0.7 cap draws)
-        J.blist_cap = sample_list_entries(cap, cap) ? sample_list_entries(cap, cap) : 0ull;
+        J.blist_cap = sample_onchip ? 0ull : sample_list_entries(cap, cap);
         J.blist = J.blist_cap ? be.take<uint32_t>((size_t)J.blist_cap) : nullptr;
-        J.bcount = be.take<unsigned int>((size_t)sample_list_counters());
+        J.bcount = J.blist ? be.take<unsigned int>((size_t)sample_list_counters()) : nullptr;
         J.vbits = be.take<uint32_t>((size_t)((cap + 31) / 32 + 32));
         J.L_sampled = be.take<uint32_t>((size_t)cap);
         J.basic_idx = be.take<uint32_t>((size_t)cap);

@@ -216,6 +216,9 @@ unsigned long long sample_chunk_slots(unsigned long long max_draws);
 unsigned long long sample_list_entries(unsigned long long n, unsigned long long max_draws);  // 0: lists not applicable
 unsigned long long sample_list_counters();
 unsigned long long sample_table_words(unsigned long long n, unsigned long long max_draws);
+// true: launch_sample with this n_bound draws its jobs on chip (all but the (1.0, 1.0) escalation's long windows),
+// without the draw cache and bucket lists
+bool sample_onchip_bound(unsigned long long n_bound);
 // flag_points > 0: the post-1 jobs' endpoint flags come from the flag pass (SampleJob::vbits), n_points <= flag_points;
 // narrow: the jobs' SampleJob::edges are EdgeNarrow lists, else EdgeWide
 int launch_sample(cudaStream_t st, const SampleJob* d_jobs, int n_jobs, unsigned long long max_draws_bound,

@@ -174,7 +174,8 @@ __global__ void __launch_bounds__(BLK)
   // arena layout, or the previous solve did not complete)
   if (P.zero_sampler_scratch)
     for (unsigned long long i = tid; i < J.first_words; i += stride) J.first[i] = 0u;  // sampler accept bitmask
-  for (int i = tid; i < P.sampler_counters; i += stride) J.bcount[i] = 0u;  // sampler list counters
+  if (J.bcount)
+    for (int i = tid; i < P.sampler_counters; i += stride) J.bcount[i] = 0u;  // sampler list counters
   if (P.zero_sampler_scratch)
     for (unsigned long long i = tid; i < (J.edge_cap + 31) / 32 + 32; i += stride) J.vbits[i] = 0u;
   if (tid == 0) {
