@@ -444,6 +444,37 @@ int psulvsb_icp_host(const double* src, int n_s, const double* tgt, int n_t, con
                      const psulvsb_icp_params_t* params, const double R0[9], const double t0[3],
                      psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace, int* corr);
 
+/* ---- A batch of B independent ICP problems in one call (DESIGN.md section 11, "Batches"): every pair has its own
+ * clouds, target normals and initial transform; all share one psulvsb_icp_params_t.  Every launch covers all pairs, so
+ * a call issues as many launches as psulvsb_icp whatever B is.  Pair b's result, trace records and correspondences are
+ * bit-identical to what psulvsb_icp_host returns for that pair alone (an empty cloud included). */
+typedef struct psulvsb_icp_pair {
+  const double* src;         /* 3 x n_s, column-major                                                  */
+  int n_s;
+  const double* tgt;         /* 3 x n_t                                                                */
+  int n_t;
+  const double* tgt_normals; /* 3 x n_t, point-to-plane only (else ignored)                            */
+  double R0[9];              /* column-major                                                           */
+  double t0[3];
+} psulvsb_icp_pair_t;
+
+/* Device scratch of psulvsb_icp_batch (depends on the pairs' sizes only); 0 for B <= 0 or a negative size. */
+unsigned long long psulvsb_icp_batch_workspace_bytes(const psulvsb_icp_pair_t* pairs, int B);
+/* pairs: a HOST array whose cloud pointers are device pointers; it is read before the call returns.  Asynchronous on
+ * `stream`.  d_work: psulvsb_icp_batch_workspace_bytes(pairs, B) bytes; d_results[B]; d_trace (may be NULL):
+ * B * (max_iterations + 1) records, pair b's from b * (max_iterations + 1); d_corr (may be NULL): sum of n_s ints, pair
+ * b's from sum_{a<b} n_s(a), target indices local to the pair.  PSULVSB_ERR_INVALID before any device work for B < 0,
+ * the parameters psulvsb_icp refuses, a required NULL, a pair with a negative size, a NULL cloud that is not empty, a
+ * non-finite R0 / t0, or point-to-plane without normals on a pair with n_t > 0; PSULVSB_ERR_UNSUPPORTED when the
+ * pairs' n_s or n_t add up to 2^31 or more.  B = 0 does nothing. */
+int psulvsb_icp_batch(void* stream, const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                      void* d_work, psulvsb_icp_result_t* d_results, psulvsb_icp_iteration_t* d_trace, int* d_corr);
+/* The same on host buffers (pairs' pointers are host pointers), synchronous: one upload of the clouds and one download
+ * of results[B], trace (may be NULL; iterations + 1 records of pair b written from b * (max_iterations + 1)) and corr
+ * (may be NULL). */
+int psulvsb_icp_batch_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                           psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr);
+
 /* Clique escalation (registration.cc:1000-1085 -> teaser/src/graph.cc:12-125, PMC exact maximum clique) of the
  * graph with n_vertices vertices and the given edges (uint2 endpoint pairs).  A deterministic greedy maximal
  * clique (most neighbours among the remaining candidates first, ties: lowest index) gives the lower bound;

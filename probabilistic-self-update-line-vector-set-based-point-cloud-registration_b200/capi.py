@@ -33,6 +33,7 @@ SYMBOLS = [
     "psulvsb_solve_sharded", "psulvsb_shard_row_range",
     "psulvsb_fpfh_workspace_bytes", "psulvsb_fpfh", "psulvsb_fpfh_host", "psulvsb_feature_nn", "psulvsb_match_host",
     "psulvsb_icp_default_params", "psulvsb_icp_workspace_bytes", "psulvsb_icp", "psulvsb_icp_host",
+    "psulvsb_icp_batch_workspace_bytes", "psulvsb_icp_batch", "psulvsb_icp_batch_host",
 ]
 UNIQUE_ID_BYTES = 128
 
@@ -173,6 +174,19 @@ class IcpIteration(C.Structure):
     ]
 
 
+class IcpPair(C.Structure):
+    """psulvsb_icp_pair_t: one problem of a batch (R0 column-major)."""
+    _fields_ = [
+        ("src", C.c_void_p),
+        ("n_s", C.c_int),
+        ("tgt", C.c_void_p),
+        ("n_t", C.c_int),
+        ("tgt_normals", C.c_void_p),
+        ("R0", C.c_double * 9),
+        ("t0", C.c_double * 3),
+    ]
+
+
 _lib = None
 _vp = C.c_void_p
 _ull = C.c_ulonglong
@@ -284,6 +298,10 @@ def _declare(L: C.CDLL) -> None:
                               C.POINTER(C.c_double), _vp, _vp, _vp, _vp]
     L.psulvsb_icp_host.argtypes = [_vp, C.c_int, _vp, C.c_int, _vp, C.POINTER(IcpParams), C.POINTER(C.c_double),
                                    C.POINTER(C.c_double), _vp, _vp, _vp]
+    L.psulvsb_icp_batch_workspace_bytes.argtypes = [C.POINTER(IcpPair), C.c_int]
+    L.psulvsb_icp_batch_workspace_bytes.restype = _ull
+    L.psulvsb_icp_batch.argtypes = [_vp, C.POINTER(IcpPair), C.c_int, C.POINTER(IcpParams), _vp, _vp, _vp, _vp]
+    L.psulvsb_icp_batch_host.argtypes = [C.POINTER(IcpPair), C.c_int, C.POINTER(IcpParams), _vp, _vp, _vp]
     for name in SYMBOLS:
         getattr(L, name)  # AttributeError here = the library does not export what the header declares
 

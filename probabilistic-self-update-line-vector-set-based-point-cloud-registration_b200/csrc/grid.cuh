@@ -1,5 +1,6 @@
 // grid.cuh -- the hashed uniform grid shared by the FPFH stage (k8_features.cu) and ICP (k9_icp.cu): the bucket hash,
-// the one-CTA exclusive scan of the bucket counts and the scatter of point indices into their buckets.  Each user bins
+// the one-CTA exclusive scan of the bucket counts (ICP scans one segment per pair of a batch with it) and the scatter
+// of point indices into their buckets.  Each user bins
 // its own coordinates (FP32 cells for FPFH, FP64 cells relative to the bounding-box corner for ICP) and orders each
 // bucket's members by index itself, so a bucket's points sit in ascending index order whatever the scatter's timing.
 #pragma once
@@ -29,13 +30,13 @@ __device__ __forceinline__ unsigned int bucket_of(long long cx, long long cy, lo
   return (unsigned int)k & mask;
 }
 
-// exclusive scan of count[0, m) into start[0, m] (one CTA; m is O(n)), and cursor = start
-__global__ void __launch_bounds__(SCAN_THREADS) k8_scan(const int* __restrict__ count, int m, int* __restrict__ start,
-                                                        int* __restrict__ cursor) {
+// base + exclusive scan of count[0, m) into start[0, m] by one CTA of SCAN_THREADS threads, and cursor = start
+__device__ __forceinline__ void cta_scan(const int* __restrict__ count, int m, int* __restrict__ start,
+                                         int* __restrict__ cursor, int base) {
   __shared__ int warp_tot[SCAN_THREADS / 32];
   __shared__ int carry;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  if (tid == 0) carry = 0;
+  if (tid == 0) carry = base;
   __syncthreads();
   for (int i0 = 0; i0 < m; i0 += SCAN_THREADS) {
     const int i = i0 + tid;
@@ -68,6 +69,12 @@ __global__ void __launch_bounds__(SCAN_THREADS) k8_scan(const int* __restrict__ 
     __syncthreads();
   }
   if (tid == 0) start[m] = carry;
+}
+
+// exclusive scan of count[0, m) into start[0, m] (one CTA; m is O(n)), and cursor = start
+__global__ void __launch_bounds__(SCAN_THREADS) k8_scan(const int* __restrict__ count, int m, int* __restrict__ start,
+                                                        int* __restrict__ cursor) {
+  cta_scan(count, m, start, cursor, 0);
 }
 
 // tmp[start[b] ..] receives the indices of bucket b's members in arrival order; a point with a negative bucket is left

@@ -2,16 +2,22 @@
 // linearisation), in the loop of Open3D's registration_icp: the refinement users of TEASER++ run after the global
 // solve.  DESIGN.md section 11 is the specification; oracle/icp.py restates it in numpy.
 //
-// The target does not move, so its grid is built once per call: cell size h = d (1 + 1e-6), cells floor((x - c) / h)
-// in FP64 relative to the target's bounding-box corner c (a pair within d is never two cells apart, also far from the
-// origin), hashed into 2^ceil(log2 n_t) buckets (grid.cuh) whose members sit in ascending index order as FP64 records
-// (x, y, z, index).  Every round then evaluates the current transform T_k, which lives in device memory:
-//   k9_icp_correspond  one thread per source point: transform, nearest target within d over the 27 cells, per-CTA sums;
+// A call refines a batch of B independent pairs that share the parameters (one pair for psulvsb_icp); every launch
+// covers all of them.  Each pair's target does not move, so its grid is built once per call: cell size h = d (1 + 1e-6),
+// cells floor((x - c) / h) in FP64 relative to the target's bounding-box corner c (a pair within d is never two cells
+// apart, also far from the origin), hashed into the pair's own table of 2^ceil(log2 n_t) buckets (grid.cuh) whose
+// members sit in ascending index order as FP64 records (x, y, z, index).  Every round then evaluates each pair's
+// current transform T_k, which lives in device memory:
+//   k9_icp_correspond  one thread per source point, one CTA per (pair, 128-point tile): transform, nearest target
+//                      within d over the 27 cells, per-CTA sums;
 //   k9_icp_cross       (point-to-point) the centred cross-covariance H over the correspondences, per-CTA sums;
-//   k9_icp_step        one CTA: the CTA sums in a fixed order, trace record k, the stop rule, the update U, T <- U T.
-// The host issues max_iterations + 1 rounds without looking at the device; once the loop has stopped, the state's
-// `done` flag makes every remaining launch return at once.  No floating-point atomics: every result is bit-identical
-// from call to call.
+//   k9_icp_step        one CTA per pair: the pair's CTA sums in a fixed order, trace record k, the stop rule, the
+//                      update U, T <- U T.
+// A CTA finds its pair by a binary search over the prefix of the pairs' tile counts.  Tiles, bucket tables and the
+// order of every sum depend on the pair's own sizes only, so a pair's results are bit-identical whatever else is in the
+// batch.  The host issues max_iterations + 1 rounds without looking at the device; once a pair's loop has stopped, its
+// state's `done` flag makes its CTAs of every remaining launch return at once.  No floating-point atomics: every result
+// is bit-identical from call to call.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -51,12 +57,33 @@ struct IcpInit {
   double t[3];
 };
 
-struct IcpGrid {
-  const double4* rec;  // [n in the grid] sorted by bucket, ascending index inside a bucket; .w = index
-  const int* start;    // [nb + 1]
-  unsigned int mask;   // nb - 1
-  double inv_h;
+// one pair on the device: the caller's psulvsb_icp_pair_t and where the pair sits in the batch's concatenations
+struct IcpPair {
+  const double* src;
+  const double* tgt;
+  const double* nrm;  // point-to-plane only, else nullptr
+  long long b0;       // first bucket of the pair's table (count, cursor); its start table begins at b0 + pair
+  int ns, nt;         // the caller's sizes
+  int s0;             // first source point (correspondences)
+  int t0;             // first target point in the grid's arrays (an empty pair has none)
+  unsigned int mask;  // nb - 1
+  int live;           // ns > 0 && nt > 0; an empty pair's result is T0 (k9_icp_bounds)
+  IcpInit init;
 };
+
+// the pair of item x: the p with first[p] <= x < first[p + 1] (first[0, B] ascending, first[0] <= x < first[B]; a pair
+// without items is never the answer)
+__device__ __forceinline__ int pair_of(const int* __restrict__ first, int B, int x) {
+  int lo = 0, hi = B;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (first[mid] <= x)
+      lo = mid;
+    else
+      hi = mid;
+  }
+  return lo;
+}
 
 __device__ __forceinline__ long long icp_cell(double x, double c, double inv_h) {
   return (long long)floor(dmul(dsub(x, c), inv_h));
@@ -70,9 +97,11 @@ __device__ __forceinline__ void transform_point(const double* R, const double* t
   oz = dadd(dadd(dadd(dmul(R[6], x), dmul(R[7], y)), dmul(R[8], z)), t[2]);
 }
 
-// per-CTA sums of c[0, NV): a fixed shuffle tree in each warp, then the warps in order; partials is value-major
+// per-CTA sums of c[0, NV) of tile `tile` of a pair with `ntiles` tiles: a fixed shuffle tree in each warp, then the
+// warps in order; the pair's partials are value-major
 template <int NV>
-__device__ __forceinline__ void cta_partials(const double (&c)[NV], double* __restrict__ partials) {
+__device__ __forceinline__ void cta_partials(const double (&c)[NV], double* __restrict__ partials, int ntiles,
+                                             int tile) {
   __shared__ double sh[NV][ICP_THREADS / 32];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
 #pragma unroll
@@ -87,18 +116,33 @@ __device__ __forceinline__ void cta_partials(const double (&c)[NV], double* __re
     double s = sh[threadIdx.x][0];
 #pragma unroll
     for (int w = 1; w < ICP_THREADS / 32; ++w) s += sh[threadIdx.x][w];
-    partials[(size_t)threadIdx.x * gridDim.x + blockIdx.x] = s;
+    partials[(size_t)threadIdx.x * ntiles + tile] = s;
   }
 }
 
-// ---- target grid: corner and state, count, (k8_scan, k8_grid_scatter), order
+__device__ void write_transform(const IcpState* st, double* rotation, double* translation) {
+  for (int r = 0; r < 3; ++r) {
+    for (int c = 0; c < 3; ++c) rotation[3 * c + r] = st->R[3 * r + c];
+    translation[r] = st->t[r];
+  }
+}
+
+// ---- target grids: corner and state, count, (segmented scan, k8_grid_scatter), order
+// one CTA per pair; an empty pair gets its result here: T0, fitness 0, no update, one trace record, every
+// correspondence -1
 __global__ void __launch_bounds__(STEP_THREADS)
-    k9_icp_bounds(const double* __restrict__ tgt, int n, IcpInit init, IcpState* __restrict__ st) {
+    k9_icp_bounds(const IcpPair* __restrict__ pairs, IcpState* __restrict__ states, int nrec, int* __restrict__ corr,
+                  psulvsb_icp_iteration_t* __restrict__ trace, psulvsb_icp_result_t* __restrict__ results) {
   __shared__ double red[3][STEP_THREADS / 32];
+  const IcpPair& pr = pairs[blockIdx.x];
+  IcpState* st = states + blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int n = pr.live ? pr.nt : 0;
+  if (!pr.live)
+    for (int i = tid; i < pr.ns; i += STEP_THREADS) corr[pr.s0 + i] = -1;
   double m[3] = {INFINITY, INFINITY, INFINITY};
   for (int i = tid; i < n; i += STEP_THREADS)
-    for (int r = 0; r < 3; ++r) m[r] = fmin(m[r], tgt[3 * (size_t)i + r]);
+    for (int r = 0; r < 3; ++r) m[r] = fmin(m[r], pr.tgt[3 * (size_t)i + r]);
   for (int r = 0; r < 3; ++r) {
     for (int o = 16; o > 0; o >>= 1) m[r] = fmin(m[r], __shfl_xor_sync(0xffffffffu, m[r], o));
     if (lane == 0) red[r][wid] = m[r];
@@ -109,72 +153,120 @@ __global__ void __launch_bounds__(STEP_THREADS)
     double c = red[r][0];
     for (int w = 1; w < STEP_THREADS / 32; ++w) c = fmin(c, red[r][w]);
     st->corner[r] = c;
-    st->t[r] = init.t[r];
+    st->t[r] = pr.init.t[r];
     st->mu_p[r] = st->mu_q[r] = 0.0;
   }
-  for (int e = 0; e < 9; ++e) st->R[e] = init.R[e];
+  for (int e = 0; e < 9; ++e) st->R[e] = pr.init.R[e];
   st->fitness = st->rmse = 0.0;
   st->n_corr = st->iter = st->done = st->status = 0;
+  if (pr.live) return;
+  st->done = 1;
+  st->status = PSULVSB_ICP_NO_UPDATE;
+  psulvsb_icp_result_t* res = results + blockIdx.x;
+  write_transform(st, res->rotation, res->translation);
+  res->fitness = res->inlier_rmse = 0.0;
+  res->n_correspondences = res->iterations = 0;
+  res->status = PSULVSB_ICP_NO_UPDATE;
+  if (trace) {
+    psulvsb_icp_iteration_t* rec = trace + (size_t)blockIdx.x * nrec;
+    write_transform(st, rec->rotation, rec->translation);
+    rec->fitness = rec->inlier_rmse = 0.0;
+    rec->n_correspondences = 0;
+  }
 }
 
-// a target point with a non-finite normal is no candidate of point-to-plane: it stays out of the grid (bucket -1)
+// one thread per target point of a live pair (tgt_first: prefix of the pairs' binned targets); a target point with a
+// non-finite normal is no candidate of point-to-plane: it stays out of the grid (bucket -1).  pbucket holds the bucket's
+// index in the batch's concatenated tables.
 __global__ void __launch_bounds__(GRID_THREADS)
-    k9_icp_grid_count(const double* __restrict__ tgt, int n, const double* __restrict__ normals,
-                      const IcpState* __restrict__ st, double inv_h, unsigned int mask, int* __restrict__ pbucket,
+    k9_icp_grid_count(const IcpPair* __restrict__ pairs, const int* __restrict__ tgt_first, int B, int n,
+                      const IcpState* __restrict__ states, double inv_h, int* __restrict__ pbucket,
                       int* __restrict__ count) {
   const int i = blockIdx.x * GRID_THREADS + threadIdx.x;
   if (i >= n) return;
-  if (normals && !(isfinite(normals[3 * (size_t)i]) && isfinite(normals[3 * (size_t)i + 1]) &&
-                   isfinite(normals[3 * (size_t)i + 2]))) {
+  const int p = pair_of(tgt_first, B, i);
+  const IcpPair& pr = pairs[p];
+  const double* normals = pr.nrm;
+  const size_t l = (size_t)(i - pr.t0);
+  if (normals && !(isfinite(normals[3 * l]) && isfinite(normals[3 * l + 1]) && isfinite(normals[3 * l + 2]))) {
     pbucket[i] = -1;
     return;
   }
-  const double* q = tgt + 3 * (size_t)i;
-  const unsigned int b = bucket_of(icp_cell(q[0], st->corner[0], inv_h), icp_cell(q[1], st->corner[1], inv_h),
-                                   icp_cell(q[2], st->corner[2], inv_h), mask);
+  const double* q = pr.tgt + 3 * l;
+  const IcpState* st = states + p;
+  const long long b = pr.b0 + bucket_of(icp_cell(q[0], st->corner[0], inv_h), icp_cell(q[1], st->corner[1], inv_h),
+                                        icp_cell(q[2], st->corner[2], inv_h), pr.mask);
   pbucket[i] = (int)b;
   atomicAdd(count + b, 1);
 }
 
-// the scatter's order inside a bucket depends on timing: rank each member by index instead
+// one CTA per pair: its bucket table, positions counted from its first target point
+__global__ void __launch_bounds__(SCAN_THREADS)
+    k9_icp_grid_scan(const IcpPair* __restrict__ pairs, const int* __restrict__ count, int* __restrict__ start,
+                     int* __restrict__ cursor) {
+  const IcpPair& pr = pairs[blockIdx.x];
+  if (!pr.live) return;
+  cta_scan(count + pr.b0, (int)(pr.mask + 1), start + pr.b0 + blockIdx.x, cursor + pr.b0, pr.t0);
+}
+
+// one thread per scatter slot; the scatter's order inside a bucket depends on timing: rank each member by index instead
 __global__ void __launch_bounds__(GRID_THREADS)
-    k9_icp_grid_order(const double* __restrict__ tgt, int n, const int* __restrict__ pbucket,
-                      const int* __restrict__ start, unsigned int nb, const int* __restrict__ tmp,
+    k9_icp_grid_order(const IcpPair* __restrict__ pairs, const int* __restrict__ tgt_first, int B, int n,
+                      const int* __restrict__ pbucket, const int* __restrict__ start, const int* __restrict__ tmp,
                       double4* __restrict__ rec) {
-  const int p = blockIdx.x * GRID_THREADS + threadIdx.x;
-  if (p >= n || p >= start[nb]) return;
-  const int i = tmp[p];
-  const int b = pbucket[i], s0 = start[b], s1 = start[b + 1];
+  const int s = blockIdx.x * GRID_THREADS + threadIdx.x;
+  if (s >= n) return;
+  const int p = pair_of(tgt_first, B, s);
+  const IcpPair& pr = pairs[p];
+  const int* pstart = start + p;  // the pair's table: pstart[pr.b0, pr.b0 + nb]
+  if (s >= pstart[pr.b0 + pr.mask + 1]) return;  // slots of targets left out of the grid
+  const int i = tmp[s];
+  const int b = pbucket[i], s0 = pstart[b], s1 = pstart[b + 1];
   int rank = 0;
   for (int q = s0; q < s1; ++q) rank += tmp[q] < i;
-  rec[s0 + rank] = make_double4(tgt[3 * (size_t)i], tgt[3 * (size_t)i + 1], tgt[3 * (size_t)i + 2], (double)i);
+  const size_t l = (size_t)(i - pr.t0);
+  rec[s0 + rank] = make_double4(pr.tgt[3 * l], pr.tgt[3 * l + 1], pr.tgt[3 * l + 2], (double)(i - pr.t0));
 }
 
 // ---- evaluation of T_k: corr[i] = the target at the smallest d^2 <= dd (ties: lowest index) or -1, and the CTA sums
 // of what the step needs (point-to-point: count, sum d^2, sum p', sum q; point-to-plane: count, sum d^2, J^T J, J^T r)
 template <bool P2L>
 __global__ void __launch_bounds__(ICP_THREADS)
-    k9_icp_correspond(IcpGrid g, const double* __restrict__ src, int ns, const double* __restrict__ normals,
-                      const IcpState* __restrict__ st, double dd, int* __restrict__ corr,
+    k9_icp_correspond(const IcpPair* __restrict__ pairs, const int* __restrict__ tile_first, int B,
+                      const double4* __restrict__ rec, const int* __restrict__ start, double inv_h,
+                      const IcpState* __restrict__ states, double dd, int* __restrict__ corr,
                       double* __restrict__ partials) {
+  // the pair, its bucket mask and its start table are read from shared memory at each use: held in registers across
+  // the 27-cell walk they push the point-to-plane instantiation past 128 registers (4 CTAs per SM) into spills
+  __shared__ volatile int s_pair, s_start;
+  __shared__ volatile unsigned int s_mask;
+  const int p = pair_of(tile_first, B, blockIdx.x);
+  const IcpState* st = states + p;
   if (st->done) return;
+  if (threadIdx.x == 0) {
+    s_pair = p;
+    s_start = (int)(pairs[p].b0 + p);
+    s_mask = pairs[p].mask;
+  }
+  __syncthreads();
   constexpr int NV = P2L ? NV_P2L : NV_P2P;
-  const int i = blockIdx.x * ICP_THREADS + threadIdx.x;
+  const int i = (blockIdx.x - tile_first[p]) * ICP_THREADS + threadIdx.x;
   double c[NV];
 #pragma unroll
   for (int v = 0; v < NV; ++v) c[v] = 0.0;
-  if (i < ns) {
+  if (i < pairs[p].ns) {
+    const double* src = pairs[p].src;
     double px, py, pz;
     transform_point(st->R, st->t, src[3 * (size_t)i], src[3 * (size_t)i + 1], src[3 * (size_t)i + 2], px, py, pz);
-    const long long cx = icp_cell(px, st->corner[0], g.inv_h), cy = icp_cell(py, st->corner[1], g.inv_h),
-                    cz = icp_cell(pz, st->corner[2], g.inv_h);
+    const long long cx = icp_cell(px, st->corner[0], inv_h), cy = icp_cell(py, st->corner[1], inv_h),
+                    cz = icp_cell(pz, st->corner[2], inv_h);
     // the 27 cells in a fixed order (dz, dy, dx), each bucket once: visit bit k = first cell of its bucket
     unsigned int visit = 0;
     {
       unsigned int b[27];
 #pragma unroll
       for (int k = 0; k < 27; ++k) {
-        b[k] = bucket_of(cx + k % 3 - 1, cy + (k / 3) % 3 - 1, cz + k / 9 - 1, g.mask);
+        b[k] = bucket_of(cx + k % 3 - 1, cy + (k / 3) % 3 - 1, cz + k / 9 - 1, s_mask);
         bool dup = false;
 #pragma unroll
         for (int s = 0; s < k; ++s) dup |= b[s] == b[k];
@@ -186,10 +278,10 @@ __global__ void __launch_bounds__(ICP_THREADS)
 #pragma unroll 1
     for (int k = 0; k < 27; ++k) {
       if (!((visit >> k) & 1u)) continue;
-      const unsigned int b = bucket_of(cx + k % 3 - 1, cy + (k / 3) % 3 - 1, cz + k / 9 - 1, g.mask);
-      const int e = g.start[b + 1];
-      for (int u = g.start[b]; u < e; ++u) {
-        const double4 q = g.rec[u];
+      const unsigned int b = bucket_of(cx + k % 3 - 1, cy + (k / 3) % 3 - 1, cz + k / 9 - 1, s_mask);
+      const int e = start[s_start + b + 1];
+      for (int u = start[s_start + b]; u < e; ++u) {
+        const double4 q = rec[u];
         const double dx = dsub(q.x, px), dy = dsub(q.y, py), dz = dsub(q.z, pz);
         const double d2 = dadd(dadd(dmul(dx, dx), dmul(dy, dy)), dmul(dz, dz));
         const int j = (int)q.w;
@@ -202,7 +294,7 @@ __global__ void __launch_bounds__(ICP_THREADS)
         }
       }
     }
-    corr[i] = bj;
+    corr[pairs[s_pair].s0 + i] = bj;
     if (bj >= 0) {
       c[0] = 1.0;
       c[1] = best;
@@ -214,6 +306,7 @@ __global__ void __launch_bounds__(ICP_THREADS)
         c[6] = qy;
         c[7] = qz;
       } else {
+        const double* normals = pairs[s_pair].nrm;
         const double nx = normals[3 * (size_t)bj], ny = normals[3 * (size_t)bj + 1], nz = normals[3 * (size_t)bj + 2];
         // r = (p' - q) . n, J = [p' x n, n] (Open3D TransformationEstimationPointToPlane)
         const double r = dadd(dadd(dmul(dsub(px, qx), nx), dmul(dsub(py, qy), ny)), dmul(dsub(pz, qz), nz));
@@ -229,26 +322,33 @@ __global__ void __launch_bounds__(ICP_THREADS)
       }
     }
   }
-  cta_partials<NV>(c, partials);
+  const int tile0 = tile_first[s_pair];
+  cta_partials<NV>(c, partials + (size_t)NV_P2L * tile0, tile_first[s_pair + 1] - tile0, blockIdx.x - tile0);
 }
 
 // ---- point-to-point: H = sum (p' - mu_p)(q - mu_q)^T over the correspondences of T_k
 __global__ void __launch_bounds__(ICP_THREADS)
-    k9_icp_cross(const double* __restrict__ src, int ns, const double* __restrict__ tgt, const int* __restrict__ corr,
-                 const IcpState* __restrict__ st, double* __restrict__ partials) {
+    k9_icp_cross(const IcpPair* __restrict__ pairs, const int* __restrict__ tile_first, int B,
+                 const int* __restrict__ corr, const IcpState* __restrict__ states, double* __restrict__ partials) {
+  const int p = pair_of(tile_first, B, blockIdx.x);
+  const IcpState* st = states + p;
   if (st->done) return;
-  const int i = blockIdx.x * ICP_THREADS + threadIdx.x;
+  const IcpPair& pr = pairs[p];
+  const int tile0 = tile_first[p], tile = blockIdx.x - tile0;
+  const int i = tile * ICP_THREADS + threadIdx.x;
   double c[NV_CROSS];
 #pragma unroll
   for (int v = 0; v < NV_CROSS; ++v) c[v] = 0.0;
-  const int j = i < ns ? corr[i] : -1;
+  const int j = i < pr.ns ? corr[pr.s0 + i] : -1;
   if (j >= 0) {
-    double p[3];
-    transform_point(st->R, st->t, src[3 * (size_t)i], src[3 * (size_t)i + 1], src[3 * (size_t)i + 2], p[0], p[1], p[2]);
+    const double *src = pr.src, *tgt = pr.tgt;
+    double p3[3];
+    transform_point(st->R, st->t, src[3 * (size_t)i], src[3 * (size_t)i + 1], src[3 * (size_t)i + 2], p3[0], p3[1],
+                    p3[2]);
     double a[3], b[3];
 #pragma unroll
     for (int r = 0; r < 3; ++r) {
-      a[r] = dsub(p[r], st->mu_p[r]);
+      a[r] = dsub(p3[r], st->mu_p[r]);
       b[r] = dsub(tgt[3 * (size_t)j + r], st->mu_q[r]);
     }
 #pragma unroll
@@ -256,7 +356,7 @@ __global__ void __launch_bounds__(ICP_THREADS)
 #pragma unroll
       for (int s = 0; s < 3; ++s) c[3 * r + s] = dmul(a[r], b[s]);
   }
-  cta_partials<NV_CROSS>(c, partials);
+  cta_partials<NV_CROSS>(c, partials + (size_t)NV_P2L * tile0, tile_first[p + 1] - tile0, tile);
 }
 
 // 6x6 Cholesky of the J^T J upper triangle A (21 entries) and solve A x = -g; false on a non-positive pivot or a
@@ -304,28 +404,26 @@ __device__ void compose(IcpState* st, const double Ru[3][3], const double tu[3])
   st->iter += 1;
 }
 
-__device__ void write_transform(const IcpState* st, double* rotation, double* translation) {
-  for (int r = 0; r < 3; ++r) {
-    for (int c = 0; c < 3; ++c) rotation[3 * c + r] = st->R[3 * r + c];
-    translation[r] = st->t[r];
-  }
-}
-
 struct StepParams {
-  int ns, max_iterations;
+  int max_iterations;
   double relative_fitness, relative_rmse;
 };
 
-// phase 0 (after k9_icp_correspond): record k, stop rule, point-to-plane update or point-to-point means;
-// phase 1 (after k9_icp_cross): the point-to-point update
+// one CTA per pair; phase 0 (after k9_icp_correspond): record k, stop rule, point-to-plane update or point-to-point
+// means; phase 1 (after k9_icp_cross): the point-to-point update
 template <bool P2L>
 __global__ void __launch_bounds__(STEP_THREADS)
-    k9_icp_step(int phase, const double* __restrict__ partials, int nblk, StepParams prm, IcpState* __restrict__ st,
-                psulvsb_icp_iteration_t* __restrict__ trace, psulvsb_icp_result_t* __restrict__ result) {
+    k9_icp_step(int phase, const IcpPair* __restrict__ pairs, const int* __restrict__ tile_first,
+                const double* __restrict__ partials, StepParams prm, IcpState* __restrict__ states,
+                psulvsb_icp_iteration_t* __restrict__ trace, psulvsb_icp_result_t* __restrict__ results) {
   __shared__ double run[STEP_RUNS][32];
   __shared__ double S[32];
+  const int p = blockIdx.x;
+  IcpState* st = states + p;
   if (st->done) return;
   const int nv = phase ? NV_CROSS : (P2L ? NV_P2L : NV_P2P);
+  const int tile0 = tile_first[p], nblk = tile_first[p + 1] - tile0;
+  partials += (size_t)NV_P2L * tile0;
   // CTA partials: STEP_RUNS contiguous runs summed in index order, then the runs in order
   const int tid = threadIdx.x, v = tid & 31, run_id = tid >> 5;
   const int len = (nblk + STEP_RUNS - 1) / STEP_RUNS, b0 = run_id * len, b1 = min(nblk, b0 + len);
@@ -352,11 +450,11 @@ __global__ void __launch_bounds__(STEP_THREADS)
     return;
   }
   const int cnt = (int)S[0];
-  const double fitness = (double)cnt / (double)prm.ns;
+  const double fitness = (double)cnt / (double)pairs[p].ns;
   const double rmse = cnt > 0 ? sqrt(S[1] / (double)cnt) : 0.0;
   const int k = st->iter;
   if (trace) {
-    psulvsb_icp_iteration_t* rec = trace + k;
+    psulvsb_icp_iteration_t* rec = trace + (size_t)p * (prm.max_iterations + 1) + k;
     write_transform(st, rec->rotation, rec->translation);
     rec->fitness = fitness;
     rec->inlier_rmse = rmse;
@@ -396,6 +494,7 @@ __global__ void __launch_bounds__(STEP_THREADS)
   if (status >= 0) {
     st->status = status;
     st->done = 1;
+    psulvsb_icp_result_t* result = results + p;
     write_transform(st, result->rotation, result->translation);
     result->fitness = fitness;
     result->inlier_rmse = rmse;
@@ -408,16 +507,43 @@ __global__ void __launch_bounds__(STEP_THREADS)
 inline size_t up256(size_t x) { return (x + 255) & ~size_t(255); }
 inline int blocks(long long n, int t) { return (int)((n + t - 1) / t); }
 
-struct IcpWork {
-  IcpState* state;
-  double4* rec;
-  int *pbucket, *count, *start, *cursor, *tmp, *corr;
-  double* partials;
+bool live(const psulvsb_icp_pair_t& p) { return p.n_s > 0 && p.n_t > 0; }
+
+// what a batch's workspace depends on: B, the source points of all pairs, and the targets, buckets and 128-point
+// source tiles of the pairs that are not empty
+struct IcpSizes {
+  long long ns = 0, nt = 0, nb = 0, tiles = 0;
+  int B = 0;
 };
 
-size_t icp_layout(int ns, int nt, char* base, IcpWork* w) {
-  const size_t NS = (size_t)(ns > 0 ? ns : 0), NT = (size_t)(nt > 0 ? nt : 0), nb = bucket_count(nt);
-  const size_t nblk = (NS + ICP_THREADS - 1) / ICP_THREADS;
+IcpSizes icp_sizes(const psulvsb_icp_pair_t* pairs, int B) {
+  IcpSizes z;
+  z.B = B;
+  for (int b = 0; b < B; ++b) {
+    z.ns += pairs[b].n_s;
+    if (!live(pairs[b])) continue;
+    z.nt += pairs[b].n_t;
+    z.nb += bucket_count(pairs[b].n_t);
+    z.tiles += (pairs[b].n_s + ICP_THREADS - 1) / ICP_THREADS;
+  }
+  return z;
+}
+
+struct IcpWork {
+  IcpPair* pair;                 // [B], followed by tile_first and tgt_first: one copy uploads the three
+  int *tile_first, *tgt_first;   // [B + 1] each: prefix of the pairs' tiles, of their binned targets
+  IcpState* state;               // [B]
+  double4* rec;                  // [nt]
+  int *pbucket, *tmp;            // [nt]
+  int *count, *cursor;           // [nb]
+  int* start;                    // [nb + B]: pair p's table at b0 + p, nb_p + 1 entries
+  int* corr;                     // [ns]
+  double* partials;              // [NV_P2L * tiles]: pair p's at NV_P2L * tile_first[p], value-major
+  size_t table_bytes;            // pair + tile_first + tgt_first
+};
+
+size_t icp_layout(const IcpSizes& z, char* base, IcpWork* w) {
+  const size_t B = (size_t)z.B;
   size_t off = 0;
   auto take = [&](size_t bytes) {
     char* p = base ? base + off : nullptr;
@@ -425,15 +551,19 @@ size_t icp_layout(int ns, int nt, char* base, IcpWork* w) {
     return p;
   };
   IcpWork v;
-  v.state = (IcpState*)take(sizeof(IcpState));
-  v.rec = (double4*)take(32 * NT);
-  v.pbucket = (int*)take(4 * NT);
-  v.count = (int*)take(4 * nb);
-  v.start = (int*)take(4 * (nb + 1));
-  v.cursor = (int*)take(4 * nb);
-  v.tmp = (int*)take(4 * NT);
-  v.corr = (int*)take(4 * NS);
-  v.partials = (double*)take(8 * (size_t)NV_P2L * nblk);
+  v.table_bytes = sizeof(IcpPair) * B + 2 * 4 * (B + 1);
+  v.pair = (IcpPair*)take(v.table_bytes);
+  v.tile_first = (int*)((char*)v.pair + sizeof(IcpPair) * B);
+  v.tgt_first = v.tile_first + (B + 1);
+  v.state = (IcpState*)take(sizeof(IcpState) * B);
+  v.rec = (double4*)take(32 * (size_t)z.nt);
+  v.pbucket = (int*)take(4 * (size_t)z.nt);
+  v.tmp = (int*)take(4 * (size_t)z.nt);
+  v.count = (int*)take(4 * (size_t)z.nb);
+  v.cursor = (int*)take(4 * (size_t)z.nb);
+  v.start = (int*)take(4 * ((size_t)z.nb + B));
+  v.corr = (int*)take(4 * (size_t)z.ns);
+  v.partials = (double*)take(8 * (size_t)NV_P2L * (size_t)z.tiles);
   if (w) *w = v;
   return off;
 }
@@ -453,6 +583,24 @@ bool transform_ok(const double* R0, const double* t0) {
   return true;
 }
 
+// PSULVSB_ERR_INVALID for a bad pair, PSULVSB_ERR_UNSUPPORTED for concatenations past the int range, else OK
+int pairs_check(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params, const char* who) {
+  long long ns = 0, nt = 0;
+  for (int b = 0; b < B; ++b) {
+    const psulvsb_icp_pair_t& p = pairs[b];
+    if (p.n_s < 0 || p.n_t < 0 || (p.n_s > 0 && !p.src) || (p.n_t > 0 && !p.tgt) || !transform_ok(p.R0, p.t0) ||
+        (params->point_to_plane && p.n_t > 0 && !p.tgt_normals))
+      return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad pair " + std::to_string(b));
+    ns += p.n_s;
+    nt += p.n_t;
+  }
+  const IcpSizes z = icp_sizes(pairs, B);
+  // the buckets' start tables are indexed by int
+  if (ns >= (1ll << 31) || nt >= (1ll << 31) || z.nb + B >= (1ll << 31))
+    return fail(PSULVSB_ERR_UNSUPPORTED, std::string(who) + ": the batch's clouds exceed 2^31 - 1 points in all");
+  return PSULVSB_OK;
+}
+
 // an empty cloud: T0, fitness 0, no update (one trace record, every correspondence -1)
 void empty_result(const double* R0, const double* t0, psulvsb_icp_result_t* res, psulvsb_icp_iteration_t* rec) {
   *res = psulvsb_icp_result_t{};
@@ -462,51 +610,167 @@ void empty_result(const double* R0, const double* t0, psulvsb_icp_result_t* res,
   res->status = PSULVSB_ICP_NO_UPDATE;
 }
 
-int run_icp(cudaStream_t st, const double* src, int ns, const double* tgt, int nt, const double* normals,
-            const psulvsb_icp_params_t& prm, const double* R0, const double* t0, void* work,
-            psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr) {
+// the batch on the device (pairs checked, B >= 1): one upload of the pair table, the grids, max_iterations + 1 rounds
+// and one copy of the correspondences; the launch count does not depend on B
+int run_icp(cudaStream_t st, const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t& prm, void* work,
+            psulvsb_icp_result_t* d_results, psulvsb_icp_iteration_t* d_trace, int* d_corr) {
+  const IcpSizes z = icp_sizes(pairs, B);
   IcpWork w;
-  icp_layout(ns, nt, static_cast<char*>(work), &w);
+  icp_layout(z, static_cast<char*>(work), &w);
   const bool p2l = prm.point_to_plane != 0;
   const double d = prm.max_correspondence_distance;
-  const unsigned int nb = bucket_count(nt);
-  IcpInit init;
-  for (int r = 0; r < 3; ++r) {
-    for (int c = 0; c < 3; ++c) init.R[3 * r + c] = R0[3 * c + r];
-    init.t[r] = t0[r];
-  }
-  const IcpGrid g{w.rec, w.start, nb - 1, 1.0 / (d * (1.0 + 1e-6))};
-  k9_icp_bounds<<<1, STEP_THREADS, 0, st>>>(tgt, nt, init, w.state);
-  PSU_CHECK_LAUNCH("k9_icp_bounds");
-  PSU_CUDA(cudaMemsetAsync(w.count, 0, 4 * (size_t)nb, st));
-  k9_icp_grid_count<<<blocks(nt, GRID_THREADS), GRID_THREADS, 0, st>>>(tgt, nt, p2l ? normals : nullptr, w.state,
-                                                                       g.inv_h, g.mask, w.pbucket, w.count);
-  PSU_CHECK_LAUNCH("k9_icp_grid_count");
-  k8_scan<<<1, SCAN_THREADS, 0, st>>>(w.count, (int)nb, w.start, w.cursor);
-  PSU_CHECK_LAUNCH("k8_scan");
-  k8_grid_scatter<<<blocks(nt, GRID_THREADS), GRID_THREADS, 0, st>>>(nt, w.pbucket, w.cursor, w.tmp);
-  PSU_CHECK_LAUNCH("k8_grid_scatter");
-  k9_icp_grid_order<<<blocks(nt, GRID_THREADS), GRID_THREADS, 0, st>>>(tgt, nt, w.pbucket, w.start, nb, w.tmp, w.rec);
-  PSU_CHECK_LAUNCH("k9_icp_grid_order");
-  const int nblk = blocks(ns, ICP_THREADS);
-  const StepParams sp{ns, prm.max_iterations, prm.relative_fitness, prm.relative_rmse};
-  const double dd = d * d;
-  for (int k = 0; k <= prm.max_iterations; ++k) {
-    if (p2l) {
-      k9_icp_correspond<true><<<nblk, ICP_THREADS, 0, st>>>(g, src, ns, normals, w.state, dd, w.corr, w.partials);
-      k9_icp_step<true><<<1, STEP_THREADS, 0, st>>>(0, w.partials, nblk, sp, w.state, d_trace, d_result);
-    } else {
-      k9_icp_correspond<false><<<nblk, ICP_THREADS, 0, st>>>(g, src, ns, nullptr, w.state, dd, w.corr, w.partials);
-      k9_icp_step<false><<<1, STEP_THREADS, 0, st>>>(0, w.partials, nblk, sp, w.state, d_trace, d_result);
-      if (k < prm.max_iterations) {
-        k9_icp_cross<<<nblk, ICP_THREADS, 0, st>>>(src, ns, tgt, w.corr, w.state, w.partials);
-        k9_icp_step<false><<<1, STEP_THREADS, 0, st>>>(1, w.partials, nblk, sp, w.state, d_trace, d_result);
-      }
+  std::vector<char> table(w.table_bytes);
+  IcpPair* hp = reinterpret_cast<IcpPair*>(table.data());
+  int* tile_first = reinterpret_cast<int*>(table.data() + sizeof(IcpPair) * (size_t)B);
+  int* tgt_first = tile_first + (B + 1);
+  long long b0 = 0;
+  int s0 = 0;
+  tile_first[0] = tgt_first[0] = 0;
+  for (int b = 0; b < B; ++b) {
+    const psulvsb_icp_pair_t& q = pairs[b];
+    IcpPair& h = hp[b];
+    h = IcpPair{};
+    h.live = live(q);
+    h.src = q.src;
+    h.tgt = q.tgt;
+    h.nrm = p2l ? q.tgt_normals : nullptr;
+    h.ns = q.n_s;
+    h.nt = q.n_t;
+    h.s0 = s0;
+    h.t0 = tgt_first[b];
+    h.b0 = b0;
+    const unsigned int nb = h.live ? bucket_count(q.n_t) : 0u;
+    h.mask = nb - 1;
+    for (int r = 0; r < 3; ++r) {
+      for (int c = 0; c < 3; ++c) h.init.R[3 * r + c] = q.R0[3 * c + r];
+      h.init.t[r] = q.t0[r];
     }
-    PSU_CHECK_LAUNCH("k9_icp round");
+    s0 += q.n_s;
+    b0 += nb;
+    tile_first[b + 1] = tile_first[b] + (h.live ? blocks(q.n_s, ICP_THREADS) : 0);
+    tgt_first[b + 1] = tgt_first[b] + (h.live ? q.n_t : 0);
   }
-  if (d_corr) PSU_CUDA(cudaMemcpyAsync(d_corr, w.corr, 4 * (size_t)ns, cudaMemcpyDeviceToDevice, st));
+  PSU_CUDA(cudaMemcpyAsync(w.pair, table.data(), table.size(), cudaMemcpyHostToDevice, st));
+  const int nrec = prm.max_iterations + 1;
+  k9_icp_bounds<<<B, STEP_THREADS, 0, st>>>(w.pair, w.state, nrec, w.corr, d_trace, d_results);
+  PSU_CHECK_LAUNCH("k9_icp_bounds");
+  const int nt = (int)z.nt, tiles = (int)z.tiles;
+  if (tiles > 0) {
+    const double inv_h = 1.0 / (d * (1.0 + 1e-6));
+    PSU_CUDA(cudaMemsetAsync(w.count, 0, 4 * (size_t)z.nb, st));
+    k9_icp_grid_count<<<blocks(nt, GRID_THREADS), GRID_THREADS, 0, st>>>(w.pair, w.tgt_first, B, nt, w.state, inv_h,
+                                                                         w.pbucket, w.count);
+    PSU_CHECK_LAUNCH("k9_icp_grid_count");
+    k9_icp_grid_scan<<<B, SCAN_THREADS, 0, st>>>(w.pair, w.count, w.start, w.cursor);
+    PSU_CHECK_LAUNCH("k9_icp_grid_scan");
+    k8_grid_scatter<<<blocks(nt, GRID_THREADS), GRID_THREADS, 0, st>>>(nt, w.pbucket, w.cursor, w.tmp);
+    PSU_CHECK_LAUNCH("k8_grid_scatter");
+    k9_icp_grid_order<<<blocks(nt, GRID_THREADS), GRID_THREADS, 0, st>>>(w.pair, w.tgt_first, B, nt, w.pbucket,
+                                                                         w.start, w.tmp, w.rec);
+    PSU_CHECK_LAUNCH("k9_icp_grid_order");
+    const StepParams sp{prm.max_iterations, prm.relative_fitness, prm.relative_rmse};
+    const double dd = d * d;
+    for (int k = 0; k <= prm.max_iterations; ++k) {
+      if (p2l) {
+        k9_icp_correspond<true><<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.rec, w.start, inv_h,
+                                                               w.state, dd, w.corr, w.partials);
+        k9_icp_step<true><<<B, STEP_THREADS, 0, st>>>(0, w.pair, w.tile_first, w.partials, sp, w.state, d_trace,
+                                                      d_results);
+      } else {
+        k9_icp_correspond<false><<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.rec, w.start, inv_h,
+                                                                w.state, dd, w.corr, w.partials);
+        k9_icp_step<false><<<B, STEP_THREADS, 0, st>>>(0, w.pair, w.tile_first, w.partials, sp, w.state, d_trace,
+                                                       d_results);
+        if (k < prm.max_iterations) {
+          k9_icp_cross<<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.corr, w.state, w.partials);
+          k9_icp_step<false><<<B, STEP_THREADS, 0, st>>>(1, w.pair, w.tile_first, w.partials, sp, w.state, d_trace,
+                                                         d_results);
+        }
+      }
+      PSU_CHECK_LAUNCH("k9_icp round");
+    }
+  }
+  if (d_corr && z.ns > 0)
+    PSU_CUDA(cudaMemcpyAsync(d_corr, w.corr, 4 * (size_t)z.ns, cudaMemcpyDeviceToDevice, st));
   return PSULVSB_OK;
+}
+
+// the batch on host buffers (pairs checked, B >= 1): the live pairs' clouds go up in one copy, results, trace records
+// and correspondences come back in one
+int run_icp_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t& prm,
+                 psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr, const char* who) {
+  const bool p2l = prm.point_to_plane != 0;
+  const IcpSizes z = icp_sizes(pairs, B);
+  const size_t nrec = (size_t)prm.max_iterations + 1, NB = (size_t)B;
+  // outputs first and contiguous, so that one copy brings them back
+  const size_t o_trace = up256(sizeof(psulvsb_icp_result_t) * NB),
+               o_corr = o_trace + (trace ? sizeof(psulvsb_icp_iteration_t) * nrec * NB : 0),
+               o_end = o_corr + (corr ? 4 * (size_t)z.ns : 0), o_in = up256(o_end);
+  const size_t in_bytes = 24 * (size_t)(z.ns + z.nt * (p2l ? 2 : 1));
+  const size_t o_work = up256(o_in + in_bytes);
+  // the live pairs' src, tgt (and normals) in pair order: pair b's src at in_off[b], tgt and normals after it
+  std::vector<char> in(in_bytes);
+  std::vector<size_t> in_off(NB);
+  size_t off = 0;
+  for (int b = 0; b < B; ++b) {
+    const psulvsb_icp_pair_t& q = pairs[b];
+    in_off[b] = off;
+    if (!live(q)) continue;
+    auto put = [&](const double* h, int n) {
+      std::memcpy(in.data() + off, h, 24 * (size_t)n);
+      off += 24 * (size_t)n;
+    };
+    put(q.src, q.n_s);
+    put(q.tgt, q.n_t);
+    if (p2l) put(q.tgt_normals, q.n_t);
+  }
+  void* buf = nullptr;
+  if (cudaMalloc(&buf, o_work + icp_layout(z, nullptr, nullptr)) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(PSULVSB_ERR_CUDA, std::string(who) + ": cudaMalloc failed");
+  }
+  char* base = static_cast<char*>(buf);
+  std::vector<psulvsb_icp_pair_t> dev(pairs, pairs + B);
+  for (int b = 0; b < B; ++b) {
+    psulvsb_icp_pair_t& q = dev[b];
+    const double* src = reinterpret_cast<const double*>(base + o_in + in_off[b]);
+    const bool on = live(q);
+    q.src = on ? src : nullptr;
+    q.tgt = on ? src + 3 * (size_t)q.n_s : nullptr;
+    q.tgt_normals = on && p2l ? src + 3 * ((size_t)q.n_s + q.n_t) : nullptr;
+  }
+  std::vector<char> out(o_end);
+  int rc = PSULVSB_OK;
+  auto step = [&](cudaError_t e, const char* what) {
+    if (!rc && e != cudaSuccess)
+      rc = fail(PSULVSB_ERR_CUDA, std::string(who) + ": " + what + ": " + cudaGetErrorString(e));
+  };
+  if (in_bytes) step(cudaMemcpy(base + o_in, in.data(), in_bytes, cudaMemcpyHostToDevice), "copy in");
+  if (!rc)
+    rc = run_icp(nullptr, dev.data(), B, prm, base + o_work, (psulvsb_icp_result_t*)base,
+                 trace ? (psulvsb_icp_iteration_t*)(base + o_trace) : nullptr, corr ? (int*)(base + o_corr) : nullptr);
+  if (!rc) step(cudaMemcpy(out.data(), base, o_end, cudaMemcpyDeviceToHost), "copy out");
+  cudaFree(buf);
+  if (rc) return rc;
+  std::memcpy(results, out.data(), sizeof(psulvsb_icp_result_t) * NB);
+  for (int b = 0; trace && b < B; ++b)
+    std::memcpy(trace + nrec * b, out.data() + o_trace + sizeof(psulvsb_icp_iteration_t) * nrec * b,
+                sizeof(psulvsb_icp_iteration_t) * (size_t)(results[b].iterations + 1));
+  if (corr) std::memcpy(corr, out.data() + o_corr, 4 * (size_t)z.ns);
+  return PSULVSB_OK;
+}
+
+psulvsb_icp_pair_t one_pair(const double* src, int n_s, const double* tgt, int n_t, const double* normals,
+                            const double* R0, const double* t0) {
+  psulvsb_icp_pair_t p{};
+  p.src = src;
+  p.n_s = n_s;
+  p.tgt = tgt;
+  p.n_t = n_t;
+  p.tgt_normals = normals;
+  std::memcpy(p.R0, R0, sizeof p.R0);
+  std::memcpy(p.t0, t0, sizeof p.t0);
+  return p;
 }
 
 }  // namespace
@@ -527,7 +791,16 @@ void psulvsb_icp_default_params(psulvsb_icp_params_t* p) {
 }
 
 unsigned long long psulvsb_icp_workspace_bytes(int n_s, int n_t) {
-  return (n_s < 0 || n_t < 0) ? 0ull : (unsigned long long)psulvsb::icp_layout(n_s, n_t, nullptr, nullptr);
+  if (n_s < 0 || n_t < 0) return 0ull;
+  const psulvsb_icp_pair_t p{nullptr, n_s, nullptr, n_t, nullptr, {}, {}};
+  return (unsigned long long)psulvsb::icp_layout(psulvsb::icp_sizes(&p, 1), nullptr, nullptr);
+}
+
+unsigned long long psulvsb_icp_batch_workspace_bytes(const psulvsb_icp_pair_t* pairs, int B) {
+  if (B <= 0 || !pairs) return 0ull;
+  for (int b = 0; b < B; ++b)
+    if (pairs[b].n_s < 0 || pairs[b].n_t < 0) return 0ull;
+  return (unsigned long long)psulvsb::icp_layout(psulvsb::icp_sizes(pairs, B), nullptr, nullptr);
 }
 
 int psulvsb_icp(void* stream, const double* d_src, int n_s, const double* d_tgt, int n_t, const double* d_tgt_normals,
@@ -548,8 +821,8 @@ int psulvsb_icp(void* stream, const double* d_src, int n_s, const double* d_tgt,
     if (d_corr && n_s) PSU_CUDA(cudaMemsetAsync(d_corr, 0xFF, 4 * (size_t)n_s, st));
     return PSULVSB_OK;
   }
-  return psulvsb::run_icp(st, d_src, n_s, d_tgt, n_t, d_tgt_normals, *params, R0, t0, d_work, d_result, d_trace,
-                          d_corr);
+  const psulvsb_icp_pair_t p = psulvsb::one_pair(d_src, n_s, d_tgt, n_t, d_tgt_normals, R0, t0);
+  return psulvsb::run_icp(st, &p, 1, *params, d_work, d_result, d_trace, d_corr);
 }
 
 int psulvsb_icp_host(const double* src, int n_s, const double* tgt, int n_t, const double* tgt_normals,
@@ -566,39 +839,28 @@ int psulvsb_icp_host(const double* src, int n_s, const double* tgt, int n_t, con
     for (int i = 0; corr && i < n_s; ++i) corr[i] = -1;
     return PSULVSB_OK;
   }
-  using psulvsb::up256;
-  const bool p2l = params->point_to_plane != 0;
-  const size_t NS = (size_t)n_s, NT = (size_t)n_t, nrec = (size_t)params->max_iterations + 1;
-  // outputs first and contiguous, so that one copy brings them back
-  const size_t o_trace = up256(sizeof(psulvsb_icp_result_t)), o_corr = o_trace + sizeof(psulvsb_icp_iteration_t) * nrec,
-               o_end = o_corr + 4 * NS, o_src = up256(o_end), o_tgt = o_src + up256(24 * NS),
-               o_nrm = o_tgt + up256(24 * NT), o_work = o_nrm + (p2l ? up256(24 * NT) : 0);
-  void* buf = nullptr;
-  if (cudaMalloc(&buf, o_work + psulvsb_icp_workspace_bytes(n_s, n_t)) != cudaSuccess) {
-    cudaGetLastError();
-    return fail(PSULVSB_ERR_CUDA, "psulvsb_icp_host: cudaMalloc failed");
-  }
-  char* b = static_cast<char*>(buf);
-  std::vector<char> out(o_end);
-  int rc = PSULVSB_OK;
-  auto step = [&](cudaError_t e, const char* what) {
-    if (!rc && e != cudaSuccess) rc = fail(PSULVSB_ERR_CUDA, std::string("psulvsb_icp_host: ") + what + ": " +
-                                                                cudaGetErrorString(e));
-  };
-  step(cudaMemcpy(b + o_src, src, 24 * NS, cudaMemcpyHostToDevice), "copy in");
-  step(cudaMemcpy(b + o_tgt, tgt, 24 * NT, cudaMemcpyHostToDevice), "copy in");
-  if (p2l) step(cudaMemcpy(b + o_nrm, tgt_normals, 24 * NT, cudaMemcpyHostToDevice), "copy in");
-  if (!rc)
-    rc = psulvsb::run_icp(nullptr, (const double*)(b + o_src), n_s, (const double*)(b + o_tgt), n_t,
-                          p2l ? (const double*)(b + o_nrm) : nullptr, *params, R0, t0, b + o_work,
-                          (psulvsb_icp_result_t*)b, (psulvsb_icp_iteration_t*)(b + o_trace), (int*)(b + o_corr));
-  if (!rc) step(cudaMemcpy(out.data(), b, o_end, cudaMemcpyDeviceToHost), "copy out");
-  cudaFree(buf);
-  if (rc) return rc;
-  std::memcpy(result, out.data(), sizeof *result);
-  if (trace) std::memcpy(trace, out.data() + o_trace, sizeof(psulvsb_icp_iteration_t) * (size_t)(result->iterations + 1));
-  if (corr) std::memcpy(corr, out.data() + o_corr, 4 * NS);
-  return PSULVSB_OK;
+  const psulvsb_icp_pair_t p = psulvsb::one_pair(src, n_s, tgt, n_t, tgt_normals, R0, t0);
+  return psulvsb::run_icp_host(&p, 1, *params, result, trace, corr, "psulvsb_icp_host");
+}
+
+int psulvsb_icp_batch(void* stream, const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                      void* d_work, psulvsb_icp_result_t* d_results, psulvsb_icp_iteration_t* d_trace, int* d_corr) {
+  if (B < 0 || !psulvsb::icp_params_ok(params) || (B > 0 && (!pairs || !d_work || !d_results)))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_icp_batch: bad argument");
+  if (int rc = psulvsb::pairs_check(pairs, B, params, "psulvsb_icp_batch")) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = psulvsb::need_device()) return rc;
+  return psulvsb::run_icp((cudaStream_t)stream, pairs, B, *params, d_work, d_results, d_trace, d_corr);
+}
+
+int psulvsb_icp_batch_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                           psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr) {
+  if (B < 0 || !psulvsb::icp_params_ok(params) || (B > 0 && (!pairs || !results)))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_icp_batch_host: bad argument");
+  if (int rc = psulvsb::pairs_check(pairs, B, params, "psulvsb_icp_batch_host")) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = psulvsb::need_device()) return rc;
+  return psulvsb::run_icp_host(pairs, B, *params, results, trace, corr, "psulvsb_icp_batch_host");
 }
 
 }  // extern "C"

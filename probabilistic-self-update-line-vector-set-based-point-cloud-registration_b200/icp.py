@@ -2,7 +2,9 @@
 
 What users of TEASER++ run after the global solve (Open3D's registration_icp, PCL's IterativeClosestPoint), through the
 C ABI (include/psulvsb.h, csrc/k9_icp.cu; DESIGN.md section 11).  `icp` takes host arrays; `icp_device` takes CUDA
-tensors [N, 3] float64 (== column-major 3xN) and runs on the current stream.  Convention: q ~ R p + t.
+tensors [N, 3] float64 (== column-major 3xN) and runs on the current stream.  `icp_batch` / `icp_batch_device` refine
+B independent pairs with shared parameters in one call; pair b's result is bit-identical to `icp` on that pair alone.
+Convention: q ~ R p + t.
 """
 from __future__ import annotations
 
@@ -122,3 +124,98 @@ def icp_device(d_src, d_tgt, R0, t0, max_correspondence_distance: float, *, d_ta
     if trace:
         records = (capi.IcpIteration * nrec).from_buffer_copy(rec.cpu().numpy().tobytes())
     return _result(res, records, corr[:ns])
+
+
+def _batch_transforms(R0s, t0s, B):
+    R = np.asarray(R0s, dtype=np.float64).reshape(B, 3, 3)
+    t = np.asarray(t0s, dtype=np.float64).reshape(B, 3)
+    return R, t
+
+
+def _batch_pairs(ptrs, sizes, R, t):
+    """psulvsb_icp_pair_t[B] from (src, tgt, normals) pointers and (n_s, n_t) per pair."""
+    pairs = (capi.IcpPair * max(len(sizes), 1))()
+    for b, ((ps, pt, pn), (ns, nt)) in enumerate(zip(ptrs, sizes)):
+        pairs[b].src, pairs[b].n_s, pairs[b].tgt, pairs[b].n_t, pairs[b].tgt_normals = ps, ns, pt, nt, pn
+        pairs[b].R0[:] = R[b].flatten(order="F").tolist()
+        pairs[b].t0[:] = t[b].tolist()
+    return pairs
+
+
+def _batch_results(res, records, nrec, corr, sizes):
+    out, o = [], 0
+    for b, (ns, _) in enumerate(sizes):
+        recs = None if records is None else records[b * nrec:(b + 1) * nrec]
+        out.append(_result(res[b], recs, corr[o:o + ns]))
+        o += ns
+    return out
+
+
+def icp_batch(srcs, tgts, R0s, t0s, max_correspondence_distance: float, *, target_normals=None,
+              point_to_plane: bool = False, max_iterations: int = 30, relative_fitness: float = 1e-6,
+              relative_rmse: float = 1e-6, trace: bool = False) -> list:
+    """psulvsb_icp_batch_host: refine B pairs in one call with shared parameters.  srcs, tgts (and target_normals, for
+    point-to-plane): sequences of 3 x n arrays; R0s [B, 3, 3], t0s [B, 3].  Returns one IcpResult per pair, each equal bit
+    for bit to `icp` on that pair alone."""
+    s = [_cm(a, "src") for a in srcs]
+    q = [_cm(a, "tgt") for a in tgts]
+    B = len(s)
+    if len(q) != B:
+        raise ValueError(f"{B} sources and {len(q)} targets")
+    nrm = [None] * B
+    if target_normals is not None:                            # None for a pair without target points
+        nrm = [None if a is None else _cm(a, "target_normals") for a in target_normals]
+        if len(nrm) != B or any(n is not None and n.shape != t.shape for n, t in zip(nrm, q)):
+            raise ValueError("one normal per target point is needed")
+    R, t = _batch_transforms(R0s, t0s, B)
+    sizes = [(a.shape[1], b.shape[1]) for a, b in zip(s, q)]
+    pairs = _batch_pairs([(a.ctypes.data, b.ctypes.data, None if n is None else n.ctypes.data)
+                          for a, b, n in zip(s, q, nrm)], sizes, R, t)
+    p = _params(max_correspondence_distance, point_to_plane, max_iterations, relative_fitness, relative_rmse)
+    nrec = max(int(max_iterations), 0) + 1
+    res = (capi.IcpResult * max(B, 1))()
+    records = (capi.IcpIteration * (B * nrec))() if trace and B else None
+    corr = np.empty(sum(ns for ns, _ in sizes), dtype=np.int32)
+    capi.check(capi.lib().psulvsb_icp_batch_host(pairs, B, C.byref(p), res, records, corr.ctypes.data))
+    return _batch_results(res, records, nrec, corr, sizes)
+
+
+def icp_batch_device(d_srcs, d_tgts, R0s, t0s, max_correspondence_distance: float, *, d_target_normals=None,
+                     point_to_plane: bool = False, max_iterations: int = 30, relative_fitness: float = 1e-6,
+                     relative_rmse: float = 1e-6, trace: bool = False, work=None) -> list:
+    """psulvsb_icp_batch on sequences of CUDA tensors [n, 3] float64 and the current stream.  The small results (and the
+    traces) are read back, which waits for the stream; the correspondences stay on the device as views into one tensor.
+    `work`: an optional uint8 CUDA tensor of at least psulvsb_icp_batch_workspace_bytes bytes to reuse."""
+    import torch
+
+    from .stages import _dev, _stream
+
+    B = len(d_srcs)
+    if len(d_tgts) != B:
+        raise ValueError(f"{B} sources and {len(d_tgts)} targets")
+    nrm = [None] * B if d_target_normals is None else list(d_target_normals)
+    if len(nrm) != B:
+        raise ValueError(f"{B} targets and {len(nrm)} normal sets")
+    R, t = _batch_transforms(R0s, t0s, B)
+    sizes = [(a.shape[0], b.shape[0]) for a, b in zip(d_srcs, d_tgts)]
+    pairs = _batch_pairs([(_dev(a) if a.shape[0] else None, _dev(b) if b.shape[0] else None,
+                           None if n is None else _dev(n)) for a, b, n in zip(d_srcs, d_tgts, nrm)], sizes, R, t)
+    L = capi.lib()
+    nbytes = L.psulvsb_icp_batch_workspace_bytes(pairs, B)
+    dev = d_srcs[0].device if B else torch.device("cuda")
+    if work is None:
+        work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=dev)
+    elif work.numel() < nbytes:
+        raise ValueError("work is smaller than psulvsb_icp_batch_workspace_bytes(pairs, B)")
+    nrec = max(int(max_iterations), 0) + 1
+    out = torch.empty(max(B, 1) * C.sizeof(capi.IcpResult), dtype=torch.uint8, device=dev)
+    rec = torch.empty(B * nrec * C.sizeof(capi.IcpIteration) if trace and B else 1, dtype=torch.uint8, device=dev)
+    corr = torch.empty(max(sum(ns for ns, _ in sizes), 1), dtype=torch.int32, device=dev)
+    p = _params(max_correspondence_distance, point_to_plane, max_iterations, relative_fitness, relative_rmse)
+    capi.check(L.psulvsb_icp_batch(_stream(), pairs, B, C.byref(p), _dev(work), _dev(out),
+                                   _dev(rec) if trace else None, _dev(corr)))
+    res = (capi.IcpResult * max(B, 1)).from_buffer_copy(out.cpu().numpy().tobytes())
+    records = None
+    if trace and B:
+        records = (capi.IcpIteration * (B * nrec)).from_buffer_copy(rec.cpu().numpy().tobytes())
+    return _batch_results(res, records, nrec, corr, sizes)
