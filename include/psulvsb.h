@@ -380,6 +380,51 @@ int psulvsb_match_host(const double* src_pts, int n_src, const double* tgt_pts, 
                        const float* ft, int crosscheck, int tuple_test, double tuple_scale, uint64_t seed, int* pairs,
                        long long capacity, long long* n_pairs);
 
+/* ---- Correspondences for a batch in one call (DESIGN.md section 10, "Batches").  The clouds / pairs array is a HOST
+ * array, read before the call returns; its data pointers are device pointers for the asynchronous variants and host
+ * pointers for _host.  The radii and the matcher's flags are shared; the viewpoint and the seed belong to each item.
+ * Every launch covers the whole batch.  Item b's output is bit-identical to what psulvsb_fpfh_host (with its
+ * viewpoint) or psulvsb_match_host (with its seed) returns for it alone, whatever else is in the batch and in which
+ * order.  PSULVSB_ERR_INVALID before any device work for B < 0, radii that are not finite and > 0, a negative size, a
+ * NULL pointer of an item that is not empty, a non-finite tuple_scale with the tuple test, or a required NULL output;
+ * PSULVSB_ERR_UNSUPPORTED when the sizes (n; n_src or n_tgt) add up to 2^31 or more.  B = 0 does nothing. */
+typedef struct psulvsb_fpfh_cloud {
+  const double* pts;  /* 3 x n, column-major                                                              */
+  int n;
+  double viewpoint[3]; /* normals flip towards it; zeros = the origin, as NULL does for psulvsb_fpfh        */
+} psulvsb_fpfh_cloud_t;
+/* Device scratch of psulvsb_fpfh_batch (depends on the sizes only); 0 for B <= 0 or a negative size. */
+unsigned long long psulvsb_fpfh_batch_workspace_bytes(const psulvsb_fpfh_cloud_t* clouds, int B);
+/* Cloud c's descriptors are rows [sum_{a<c} n_a, ...) of the (sum n) x 33 floats d_features, its normals the same rows
+ * of the (sum n) x 3 doubles d_normals (may be NULL).  Asynchronous on `stream`. */
+int psulvsb_fpfh_batch(void* stream, const psulvsb_fpfh_cloud_t* clouds, int B, double normal_radius,
+                       double feature_radius, void* d_work, double* d_normals, float* d_features);
+/* The same on host buffers, synchronous (normals may be NULL). */
+int psulvsb_fpfh_batch_host(const psulvsb_fpfh_cloud_t* clouds, int B, double normal_radius, double feature_radius,
+                            double* normals, float* features);
+
+typedef struct psulvsb_match_pair {
+  const double* src;  /* 3 x n_src, column-major: the tuple test's points                                 */
+  int n_src;
+  const double* tgt;  /* 3 x n_tgt                                                                        */
+  int n_tgt;
+  const float* fs;    /* n_src x 33 descriptors                                                           */
+  const float* ft;    /* n_tgt x 33                                                                       */
+  uint64_t seed;      /* the tuple test's Philox key for this pair                                        */
+} psulvsb_match_pair_t;
+/* Output layout: pair b's (source, target) index pairs (interleaved ints) begin at pair offset sum_{a<b} cap_a with
+ *   cap = 0 when a side is empty, else 3000 with the tuple test, else n_src with crosscheck and n_src + n_tgt without;
+ * counts[b] receives pair b's count (at most cap_b).  Device scratch of psulvsb_match_batch (depends on the sizes and
+ * the flags only); 0 for B <= 0 or a negative size. */
+unsigned long long psulvsb_match_batch_workspace_bytes(const psulvsb_match_pair_t* pairs, int B, int crosscheck,
+                                                       int tuple_test);
+/* Asynchronous on `stream`, without a host round trip: d_pairs holds sum cap pairs, d_counts[B] long longs. */
+int psulvsb_match_batch(void* stream, const psulvsb_match_pair_t* pairs, int B, int crosscheck, int tuple_test,
+                        double tuple_scale, void* d_work, int* d_pairs, long long* d_counts);
+/* The same on host buffers, synchronous; pairs_out holds sum cap pairs (entries past counts[b] are unspecified). */
+int psulvsb_match_batch_host(const psulvsb_match_pair_t* pairs, int B, int crosscheck, int tuple_test,
+                             double tuple_scale, int* pairs_out, long long* counts);
+
 /* ---- Refinement of a registration on the raw clouds (DESIGN.md section 11): rigid ICP, point-to-point or
  * point-to-plane, in the loop of Open3D's registration_icp -- evaluate T0; then repeatedly compute the update U from
  * the current correspondences, set T <- U T and evaluate T; stop when both |d fitness| < relative_fitness and

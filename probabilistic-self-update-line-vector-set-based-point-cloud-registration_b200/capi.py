@@ -34,6 +34,8 @@ SYMBOLS = [
     "psulvsb_fpfh_workspace_bytes", "psulvsb_fpfh", "psulvsb_fpfh_host", "psulvsb_feature_nn", "psulvsb_match_host",
     "psulvsb_icp_default_params", "psulvsb_icp_workspace_bytes", "psulvsb_icp", "psulvsb_icp_host",
     "psulvsb_icp_batch_workspace_bytes", "psulvsb_icp_batch", "psulvsb_icp_batch_host",
+    "psulvsb_fpfh_batch_workspace_bytes", "psulvsb_fpfh_batch", "psulvsb_fpfh_batch_host",
+    "psulvsb_match_batch_workspace_bytes", "psulvsb_match_batch", "psulvsb_match_batch_host",
 ]
 UNIQUE_ID_BYTES = 128
 
@@ -187,6 +189,28 @@ class IcpPair(C.Structure):
     ]
 
 
+class FpfhCloud(C.Structure):
+    """psulvsb_fpfh_cloud_t: one cloud of an FPFH batch."""
+    _fields_ = [
+        ("pts", C.c_void_p),
+        ("n", C.c_int),
+        ("viewpoint", C.c_double * 3),
+    ]
+
+
+class MatchPair(C.Structure):
+    """psulvsb_match_pair_t: one pair of a matcher batch."""
+    _fields_ = [
+        ("src", C.c_void_p),
+        ("n_src", C.c_int),
+        ("tgt", C.c_void_p),
+        ("n_tgt", C.c_int),
+        ("fs", C.c_void_p),
+        ("ft", C.c_void_p),
+        ("seed", C.c_uint64),
+    ]
+
+
 _lib = None
 _vp = C.c_void_p
 _ull = C.c_ulonglong
@@ -302,6 +326,14 @@ def _declare(L: C.CDLL) -> None:
     L.psulvsb_icp_batch_workspace_bytes.restype = _ull
     L.psulvsb_icp_batch.argtypes = [_vp, C.POINTER(IcpPair), C.c_int, C.POINTER(IcpParams), _vp, _vp, _vp, _vp]
     L.psulvsb_icp_batch_host.argtypes = [C.POINTER(IcpPair), C.c_int, C.POINTER(IcpParams), _vp, _vp, _vp]
+    L.psulvsb_fpfh_batch_workspace_bytes.argtypes = [C.POINTER(FpfhCloud), C.c_int]
+    L.psulvsb_fpfh_batch_workspace_bytes.restype = _ull
+    L.psulvsb_fpfh_batch.argtypes = [_vp, C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_double, _vp, _vp, _vp]
+    L.psulvsb_fpfh_batch_host.argtypes = [C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_double, _vp, _vp]
+    L.psulvsb_match_batch_workspace_bytes.argtypes = [C.POINTER(MatchPair), C.c_int, C.c_int, C.c_int]
+    L.psulvsb_match_batch_workspace_bytes.restype = _ull
+    L.psulvsb_match_batch.argtypes = [_vp, C.POINTER(MatchPair), C.c_int, C.c_int, C.c_int, C.c_double, _vp, _vp, _vp]
+    L.psulvsb_match_batch_host.argtypes = [C.POINTER(MatchPair), C.c_int, C.c_int, C.c_int, C.c_double, _vp, _vp]
     for name in SYMBOLS:
         getattr(L, name)  # AttributeError here = the library does not export what the header declares
 

@@ -1,6 +1,6 @@
 // grid.cuh -- the hashed uniform grid shared by the FPFH stage (k8_features.cu) and ICP (k9_icp.cu): the bucket hash,
-// the one-CTA exclusive scan of the bucket counts (ICP scans one segment per pair of a batch with it) and the scatter
-// of point indices into their buckets.  Each user bins
+// the one-CTA exclusive scan of the bucket counts (both scan one segment per cloud of a batch with it), the scatter of
+// point indices into their buckets and the lookup of a batch item by its prefix.  Each user bins
 // its own coordinates (FP32 cells for FPFH, FP64 cells relative to the bounding-box corner for ICP) and orders each
 // bucket's members by index itself, so a bucket's points sit in ascending index order whatever the scatter's timing.
 #pragma once
@@ -71,10 +71,18 @@ __device__ __forceinline__ void cta_scan(const int* __restrict__ count, int m, i
   if (tid == 0) start[m] = carry;
 }
 
-// exclusive scan of count[0, m) into start[0, m] (one CTA; m is O(n)), and cursor = start
-__global__ void __launch_bounds__(SCAN_THREADS) k8_scan(const int* __restrict__ count, int m, int* __restrict__ start,
-                                                        int* __restrict__ cursor) {
-  cta_scan(count, m, start, cursor, 0);
+// the item of x in a batch: the p with first[p] <= x < first[p + 1] (first[0, B] ascending, first[0] <= x < first[B]; an
+// item without entries is never the answer)
+__device__ __forceinline__ int pair_of(const int* __restrict__ first, int B, int x) {
+  int lo = 0, hi = B;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (first[mid] <= x)
+      lo = mid;
+    else
+      hi = mid;
+  }
+  return lo;
 }
 
 // tmp[start[b] ..] receives the indices of bucket b's members in arrival order; a point with a negative bucket is left

@@ -12,8 +12,11 @@
 // add candidates; the distance test removes them.  No neighbour list is stored: each pass walks the cells again.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cmath>
+#include <cstring>
 #include <string>
+#include <vector>
 
 #include "common.cuh"
 #include "eig3.cuh"
@@ -64,39 +67,93 @@ __device__ __forceinline__ void for_neighbours(const Grid& g, float4 p, float r2
       }
 }
 
-// ---- grid build: count, scan, scatter, order (each bucket's members ascending by index)
+// ---- FPFH batches.  Every cloud starts on a 128-point tile, so a CTA belongs to one cloud; it finds it by pair_of over
+// the prefix of the clouds' tiles.  Per-point arrays (spts, nf, pbucket, tmp, counts, kcount, the outputs) are the
+// concatenation of the clouds' (cloud c's from p0); each cloud keeps its own table of bucket_count(n) buckets, whose
+// start entries count positions from the batch's first point.
+struct FtCloud {
+  const double* pts;  // 3 x n, column-major
+  double vp[3];       // normals flip towards it
+  int n;
+  int p0;             // first point in the per-point arrays
+  int b0;             // first bucket (count, cursor); the start table is start[b0 + c, b0 + c + nb] for cloud c
+  unsigned int mask;  // nb - 1
+};
+
+// the CTA's cloud ci and the cloud's index of the CTA's first point.  A batch of one (kBatch false) takes its cloud
+// from the kernel parameter `one`: its fields stay operands of the parameter bank instead of registers.
+template <bool kBatch>
+__device__ __forceinline__ const FtCloud& cloud_tile(const FtCloud* __restrict__ clouds, const FtCloud& one,
+                                              const int* __restrict__ tile_first, int B, int& ci, int& first) {
+  if constexpr (kBatch) {
+    ci = pair_of(tile_first, B, blockIdx.x);
+    first = (blockIdx.x - tile_first[ci]) * FT_THREADS;
+    return clouds[ci];
+  } else {
+    ci = 0;
+    first = blockIdx.x * FT_THREADS;
+    return one;
+  }
+}
+
+// ---- grid build: count, scan (one CTA per cloud), scatter (grid.cuh), order (each bucket's members ascending by index)
+template <bool kBatch>
 __global__ void __launch_bounds__(FT_THREADS)
-    k8_grid_count(const double* __restrict__ pts, int n, double inv_h, unsigned int mask, int* __restrict__ pbucket,
-                  int* __restrict__ count) {
-  const int i = blockIdx.x * FT_THREADS + threadIdx.x;
-  if (i >= n) return;
+    k8_grid_count(const FtCloud* __restrict__ clouds, __grid_constant__ const FtCloud one, const int* __restrict__ tile_first, int B, double inv_h,
+                  int* __restrict__ pbucket, int* __restrict__ count) {
+  int ci, first;
+  const FtCloud& cl = cloud_tile<kBatch>(clouds, one, tile_first, B, ci, first);
+  const int i = first + threadIdx.x;
+  if (i >= cl.n) return;
+  const double* pts = cl.pts;
   const float x = (float)pts[3 * (size_t)i], y = (float)pts[3 * (size_t)i + 1], z = (float)pts[3 * (size_t)i + 2];
-  const unsigned int b = bucket_of(cell_of(x, inv_h), cell_of(y, inv_h), cell_of(z, inv_h), mask);
-  pbucket[i] = (int)b;
+  const int b = cl.b0 + (int)bucket_of(cell_of(x, inv_h), cell_of(y, inv_h), cell_of(z, inv_h), cl.mask);
+  pbucket[cl.p0 + i] = b;
   atomicAdd(count + b, 1);
 }
 
+template <bool kBatch>
+__global__ void __launch_bounds__(SCAN_THREADS)
+    k8_cloud_scan(const FtCloud* __restrict__ clouds, __grid_constant__ const FtCloud one, const int* __restrict__ count,
+                  int* __restrict__ start, int* __restrict__ cursor) {
+  const FtCloud& cl = kBatch ? clouds[blockIdx.x] : one;
+  if (cl.n == 0) return;
+  cta_scan(count + cl.b0, (int)(cl.mask + 1), start + cl.b0 + blockIdx.x, cursor + cl.b0, cl.p0);
+}
+
 // the scatter's order inside a bucket depends on timing: rank each member by index instead
+template <bool kBatch>
 __global__ void __launch_bounds__(FT_THREADS)
-    k8_grid_order(const double* __restrict__ pts, int n, const int* __restrict__ pbucket, const int* __restrict__ start,
-                  const int* __restrict__ tmp, float4* __restrict__ spts) {
-  const int p = blockIdx.x * FT_THREADS + threadIdx.x;
-  if (p >= n) return;
-  const int i = tmp[p];
-  const int b = pbucket[i], s0 = start[b], s1 = start[b + 1];
+    k8_grid_order(const FtCloud* __restrict__ clouds, __grid_constant__ const FtCloud one, const int* __restrict__ tile_first, int B,
+                  const int* __restrict__ pbucket, const int* __restrict__ start, const int* __restrict__ tmp,
+                  float4* __restrict__ spts) {
+  int ci, first;
+  const FtCloud& cl = cloud_tile<kBatch>(clouds, one, tile_first, B, ci, first);
+  const int l = first + threadIdx.x;
+  if (l >= cl.n) return;
+  const int i = tmp[cl.p0 + l];
+  const int b = pbucket[i] + ci, s0 = start[b], s1 = start[b + 1];
   int rank = 0;
   for (int q = s0; q < s1; ++q) rank += tmp[q] < i;
-  spts[s0 + rank] = make_float4((float)pts[3 * (size_t)i], (float)pts[3 * (size_t)i + 1],
-                                (float)pts[3 * (size_t)i + 2], __int_as_float(i));
+  const int j = i - cl.p0;
+  const double* pts = cl.pts;
+  spts[s0 + rank] = make_float4((float)pts[3 * (size_t)j], (float)pts[3 * (size_t)j + 1], (float)pts[3 * (size_t)j + 2],
+                                __int_as_float(j));
 }
 
 // ---- radius normals: FP64 mean and covariance of the r_n neighbourhood, smallest eigenvector, towards the viewpoint
+template <bool kBatch>
 __global__ void __launch_bounds__(FT_THREADS)
-    k8_radius_normals(Grid g, const double* __restrict__ pts, int n, float rn2, double vx, double vy, double vz,
+    k8_radius_normals(const FtCloud* __restrict__ clouds, __grid_constant__ const FtCloud one, const int* __restrict__ tile_first, int B, double inv_h,
+                      const float4* __restrict__ spts, const int* __restrict__ start, float rn2,
                       double* __restrict__ normals, float4* __restrict__ nf) {
-  const int p = blockIdx.x * FT_THREADS + threadIdx.x;
-  if (p >= n) return;
-  const float4 me = g.spts[p];
+  int ci, first;
+  const FtCloud& cl = cloud_tile<kBatch>(clouds, one, tile_first, B, ci, first);
+  const int p = first + threadIdx.x;
+  if (p >= cl.n) return;
+  const Grid g{inv_h, cl.mask, spts, start + cl.b0 + ci};
+  const double* pts = cl.pts;
+  const float4 me = spts[cl.p0 + p];
   const int i = __float_as_int(me.w);
   double mean[3] = {0, 0, 0};
   int cnt = 0;
@@ -118,15 +175,17 @@ __global__ void __launch_bounds__(FT_THREADS)
     });
     smallest_eigenvector(cov, nv);
     const double px = pts[3 * (size_t)i], py = pts[3 * (size_t)i + 1], pz = pts[3 * (size_t)i + 2];
+    const double vx = cl.vp[0], vy = cl.vp[1], vz = cl.vp[2];
     if ((vx - px) * nv[0] + (vy - py) * nv[1] + (vz - pz) * nv[2] < 0.0) {  // flipNormalTowardsViewpoint
       nv[0] = -nv[0];
       nv[1] = -nv[1];
       nv[2] = -nv[2];
     }
   }
+  const size_t o = (size_t)cl.p0 + i;
   if (normals)
-    for (int r = 0; r < 3; ++r) normals[3 * (size_t)i + r] = nv[r];
-  nf[i] = make_float4((float)nv[0], (float)nv[1], (float)nv[2], 0.f);
+    for (int r = 0; r < 3; ++r) normals[3 * o + r] = nv[r];
+  nf[o] = make_float4((float)nv[0], (float)nv[1], (float)nv[2], 0.f);
 }
 
 __device__ __forceinline__ float dot3(float ax, float ay, float az, float bx, float by, float bz) {
@@ -176,40 +235,68 @@ __device__ __forceinline__ bool pair_features(float4 p, float4 np, float4 q, flo
 }
 
 // ---- SPFH: integer counts of the 3 x 11 bins over the pairs (i, j != i) of the r_f neighbourhood, and K_i
+template <bool kBatch>
 __global__ void __launch_bounds__(FT_THREADS)
-    k8_spfh(Grid g, int n, float rf2, const float4* __restrict__ nf, int* __restrict__ counts, int* __restrict__ kcount) {
+    k8_spfh(const FtCloud* __restrict__ clouds, __grid_constant__ const FtCloud one, const int* __restrict__ tile_first, int B, double inv_h,
+            const float4* __restrict__ spts, const int* __restrict__ start, float rf2, const float4* __restrict__ nf,
+            int* __restrict__ counts, int* __restrict__ kcount) {
   __shared__ int hist[FT_DIM][FT_THREADS];
-  const int p = blockIdx.x * FT_THREADS + threadIdx.x;
-  if (p >= n) return;
+  // a batch's grid and first point are read from shared memory at each use: held in registers across the walk they
+  // push the kernel into spills
+  __shared__ Grid s_grid;
+  __shared__ volatile int s_p0;
+  int ci, first;
+  const FtCloud& cl = cloud_tile<kBatch>(clouds, one, tile_first, B, ci, first);
+  const int p = first + threadIdx.x;
+  const Grid one_grid{inv_h, cl.mask, spts, start};
+  if constexpr (kBatch) {
+    if (threadIdx.x == 0) {
+      s_grid = Grid{inv_h, cl.mask, spts, start + cl.b0 + ci};
+      s_p0 = cl.p0;
+    }
+    __syncthreads();
+  }
+  const Grid& g = kBatch ? s_grid : one_grid;
+  auto p0 = [&]() { return kBatch ? (int)s_p0 : 0; };
+  if (p >= cl.n) return;
   const int tid = threadIdx.x;
   for (int b = 0; b < FT_DIM; ++b) hist[b][tid] = 0;
-  const float4 me = g.spts[p];
+  const float4 me = spts[p0() + p];
   const int i = __float_as_int(me.w);
-  const float4 ni = nf[i];
+  const float4 ni = nf[p0() + i];
   int K = 0;
   constexpr double kPi = 3.14159265358979323846;
   for_neighbours(g, me, rf2, [&](float4 q, int j) {
     ++K;
     float f1, f2, f3;
-    if (j == i || !pair_features(me, ni, q, nf[j], f1, f2, f3)) return;
+    if (j == i || !pair_features(me, ni, q, nf[p0() + j], f1, f2, f3)) return;
     hist[feature_bin(11.0 * ((double)f1 + kPi) / (2.0 * kPi))][tid] += 1;
     hist[FT_BINS + feature_bin(11.0 * ((double)f2 + 1.0) / 2.0)][tid] += 1;
     hist[2 * FT_BINS + feature_bin(11.0 * ((double)f3 + 1.0) / 2.0)][tid] += 1;
   });
-  for (int b = 0; b < FT_DIM; ++b) counts[(size_t)i * FT_DIM + b] = hist[b][tid];
-  kcount[i] = K;
+  const size_t o = (size_t)p0() + i;
+  for (int b = 0; b < FT_DIM; ++b) counts[o * FT_DIM + b] = hist[b][tid];
+  kcount[o] = K;
 }
 
 // ---- FPFH: sum over neighbours j != i at distance > 0 of SPFH_j / |p_j - p_i|^2 (FP64), each 11 bins scaled to 100
+template <bool kBatch>
 __global__ void __launch_bounds__(FT_THREADS)
-    k8_fpfh(Grid g, int n, float rf2, const int* __restrict__ counts, const int* __restrict__ kcount,
-            float* __restrict__ out) {
+    k8_fpfh(const FtCloud* __restrict__ clouds, __grid_constant__ const FtCloud one, const int* __restrict__ tile_first, int B, double inv_h,
+            const float4* __restrict__ spts, const int* __restrict__ start, float rf2, const int* __restrict__ counts,
+            const int* __restrict__ kcount, float* __restrict__ out) {
   __shared__ double acc[FT_DIM][FT_THREADS];
-  const int p = blockIdx.x * FT_THREADS + threadIdx.x;
-  if (p >= n) return;
+  int ci, first;
+  const FtCloud& cl = cloud_tile<kBatch>(clouds, one, tile_first, B, ci, first);
+  const int p = first + threadIdx.x;
+  if (p >= cl.n) return;
+  const Grid g{inv_h, cl.mask, spts, start + cl.b0 + ci};
+  counts += (size_t)cl.p0 * FT_DIM;
+  kcount += cl.p0;
+  out += (size_t)cl.p0 * FT_DIM;
   const int tid = threadIdx.x;
   for (int b = 0; b < FT_DIM; ++b) acc[b][tid] = 0.0;
-  const float4 me = g.spts[p];
+  const float4 me = spts[cl.p0 + p];
   const int i = __float_as_int(me.w);
   for_neighbours(g, me, rf2, [&](float4 q, int j) {
     const float d2 = sqdist(me, q);
@@ -225,26 +312,59 @@ __global__ void __launch_bounds__(FT_THREADS)
   }
 }
 
-// ---- two-way nearest neighbour over the n_s x n_t matrix of squared L2 distances (difference form, FP32).
+// ---- matcher batches: one pair on the device, the caller's psulvsb_match_pair_t and where it sits in the
+// concatenations.  A pair with an empty side has ns = nt = 0: it takes no CTA, no list entry and no output.
+struct FtPair {
+  const double* src;
+  const double* tgt;
+  const float* fs;
+  const float* ft;
+  uint64_t seed;
+  long long list0;  // first entry of its list (in the tuple test's workspace, else in the output)
+  long long out0;   // first output pair: the caps of the pairs before it
+  int ns, nt;
+  int s0, t0;       // first source / target in the concatenations (row keys, nn_t, flags; column keys, nn_s)
+  int rblocks;      // the NN's 256-row CTAs
+};
+
+// ---- two-way nearest neighbour over each pair's n_s x n_t matrix of squared L2 distances (difference form, FP32).
+// A flat CTA index maps to (pair, 256-row block, 2048-column range) through the prefix of the pairs' CTA counts.
 // A thread owns NN_ROWS source rows (in registers); a CTA walks one column range in tiles of 2 * NN_PAIRS target
 // descriptors staged in shared memory as negated {column c, column c + 1} float2 pairs, so every dimension costs one
 // FADD2 (the two differences) and one FFMA2 (the two squares into the two sums) per row.  Row minima stay in the
 // thread (ascending columns, strict <: ties keep the lower column) and meet the other column ranges in a packed 64-bit
 // atomicMin; column minima go warp -> CTA (shared memory) -> one packed atomicMin per column and CTA.  Key =
-// (distance bits << 32) | index: non-negative float bits keep their order and the low word breaks ties.
+// (distance bits << 32) | index: non-negative float bits keep their order and the low word breaks ties.  Row keys and
+// column keys are the concatenations over the pairs.
 constexpr int NN_THREADS = 128;
 constexpr int NN_ROWS = 2;
 constexpr int NN_PAIRS = 32;
 constexpr int NN_DP = 34;  // 33 dimensions padded to an even count (the pad is 0 on both sides)
 constexpr int NN_COLS_PER_CTA = 2048;
 
+template <bool kBatch>
 __global__ void __launch_bounds__(NN_THREADS)
-    k8_feature_nn(const float* __restrict__ fs, int ns, const float* __restrict__ ft, int nt,
+    k8_feature_nn(const FtPair* __restrict__ pairs, __grid_constant__ const FtPair one, const int* __restrict__ cta_first, int B,
                   unsigned long long* __restrict__ row_key, unsigned long long* __restrict__ col_key) {
   __shared__ __align__(16) float2 tile[NN_PAIRS][NN_DP];
   __shared__ unsigned long long wcol[NN_THREADS / 32][2 * NN_PAIRS];
+  // a batch of one (kBatch false) takes its pair from the parameter `one` and a (row block, column range) grid
+  int rblock = blockIdx.x, crange = blockIdx.y;
+  FtPair pq = one;
+  if constexpr (kBatch) {
+    const int pi = pair_of(cta_first, B, blockIdx.x);
+    pq = pairs[pi];
+    const int cta = blockIdx.x - cta_first[pi];
+    rblock = cta % pq.rblocks;
+    crange = cta / pq.rblocks;
+  }
+  const float* __restrict__ fs = pq.fs;
+  const float* __restrict__ ft = pq.ft;
+  const int ns = pq.ns, nt = pq.nt;
+  row_key += pq.s0;
+  col_key += pq.t0;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const int row0 = (blockIdx.x * NN_THREADS + tid) * NN_ROWS;  // lane-contiguous rows: lower lane = lower rows
+  const int row0 = (rblock * NN_THREADS + tid) * NN_ROWS;  // lane-contiguous rows: lower lane = lower rows
   float a[NN_ROWS][NN_DP];
 #pragma unroll
   for (int r = 0; r < NN_ROWS; ++r)
@@ -254,7 +374,7 @@ __global__ void __launch_bounds__(NN_THREADS)
   unsigned long long best[NN_ROWS];
 #pragma unroll
   for (int r = 0; r < NN_ROWS; ++r) best[r] = ~0ull;
-  const int c_begin = blockIdx.y * NN_COLS_PER_CTA, c_end = min(nt, c_begin + NN_COLS_PER_CTA);
+  const int c_begin = crange * NN_COLS_PER_CTA, c_end = min(nt, c_begin + NN_COLS_PER_CTA);
   for (int c0 = c_begin; c0 < c_end; c0 += 2 * NN_PAIRS) {
     __syncthreads();
     for (int e = tid; e < NN_PAIRS * NN_DP; e += NN_THREADS) {
@@ -328,39 +448,74 @@ __global__ void k8_nn_finish(const unsigned long long* __restrict__ key, int n, 
   if (i < n) out[i] = key[i] == ~0ull ? -1 : (int)(unsigned int)key[i];
 }
 
-// ---- matcher list (FGR AdvancedMatching): flag[i] for the first part, then one scan places the pairs
-// crosscheck: flag[i] = nn_s(nn_t(i)) == i.  one-way: flag[i] = i is nn_s(j) for some j (mark pass below).
-__global__ void k8_match_flags(const int* __restrict__ nn_t, int ns, const int* __restrict__ nn_s, int crosscheck,
+// ---- matcher list (FGR AdvancedMatching) over the concatenations: flag[i] for the first part, then one scan per pair
+// places the pairs.  crosscheck: flag[i] = nn_s(nn_t(i)) == i.  one-way: flag[i] = i is nn_s(j) for some j (mark pass).
+// nn_t[x] / nn_s[y] hold indices local to the pair.
+__global__ void k8_match_flags(const FtPair* __restrict__ pairs, const int* __restrict__ s_first, int B, int NS,
+                               const int* __restrict__ nn_t, const int* __restrict__ nn_s, int crosscheck,
                                const int* __restrict__ marked, int* __restrict__ flag) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= ns) return;
-  const int j = nn_t[i];
-  flag[i] = crosscheck ? (j >= 0 && nn_s[j] == i) : (marked[i] != 0 && j >= 0);
+  const int x = blockIdx.x * blockDim.x + threadIdx.x;
+  if (x >= NS) return;
+  const FtPair& pr = pairs[pair_of(s_first, B, x)];
+  const int j = nn_t[x];
+  flag[x] = crosscheck ? (j >= 0 && nn_s[pr.t0 + j] == x - pr.s0) : (marked[x] != 0 && j >= 0);
 }
 
-__global__ void k8_match_mark(const int* __restrict__ nn_s, int nt, int* __restrict__ marked) {
-  const int j = blockIdx.x * blockDim.x + threadIdx.x;
-  if (j < nt && nn_s[j] >= 0) marked[nn_s[j]] = 1;
+__global__ void k8_match_mark(const FtPair* __restrict__ pairs, const int* __restrict__ t_first, int B, int NT,
+                              const int* __restrict__ nn_s, int* __restrict__ marked) {
+  const int y = blockIdx.x * blockDim.x + threadIdx.x;
+  if (y < NT && nn_s[y] >= 0) marked[pairs[pair_of(t_first, B, y)].s0 + nn_s[y]] = 1;
 }
 
-// pairs[2k] = source index, pairs[2k + 1] = target index; one-way lists append (nn_s(j), j) for every j after the scan
-__global__ void k8_match_place(const int* __restrict__ nn_t, int ns, const int* __restrict__ nn_s, int nt,
-                               int crosscheck, const int* __restrict__ flag, const int* __restrict__ pos,
-                               int* __restrict__ pairs) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < ns && flag[i]) {
-    pairs[2 * (size_t)pos[i]] = i;
-    pairs[2 * (size_t)pos[i] + 1] = nn_t[i];
+// one CTA per pair: pos[s0 + pair, s0 + pair + ns] = exclusive scan of the pair's flags; ncorr = the list's length.
+// counts (may be NULL) receives ncorr, or 0 ahead of the tuple test.
+__global__ void __launch_bounds__(SCAN_THREADS)
+    k8_match_scan(const FtPair* __restrict__ pairs, const int* __restrict__ flag, int crosscheck, int tuple_test,
+                  int* __restrict__ pos, int* __restrict__ ncorr, long long* __restrict__ counts) {
+  const FtPair& pr = pairs[blockIdx.x];
+  int* p = pos + pr.s0 + blockIdx.x;
+  cta_scan(flag + pr.s0, pr.ns, p, nullptr, 0);
+  if (threadIdx.x == 0) {
+    const int n = p[pr.ns] + (crosscheck ? 0 : pr.nt);
+    ncorr[blockIdx.x] = n;
+    counts[blockIdx.x] = tuple_test ? 0 : n;
   }
-  if (!crosscheck && i < nt) {
-    const size_t k = (size_t)pos[ns] + i;
-    pairs[2 * k] = nn_s[i];
-    pairs[2 * k + 1] = i;
+}
+
+// list[2k] = source index, list[2k + 1] = target index from the pair's list0; one thread per source of every pair,
+// then (one-way lists) one per target: (nn_s(j), j) for every j after the flagged part
+__global__ void k8_match_place(const FtPair* __restrict__ pairs, const int* __restrict__ s_first,
+                               const int* __restrict__ t_first, int B, int NS, int NT, const int* __restrict__ nn_t,
+                               const int* __restrict__ nn_s, int crosscheck, const int* __restrict__ flag,
+                               const int* __restrict__ pos, int* __restrict__ list) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x;
+  if (x < NS) {
+    if (!flag[x]) return;
+    const int p = pair_of(s_first, B, x);
+    const FtPair& pr = pairs[p];
+    const size_t k = (size_t)pr.list0 + pos[x + p];
+    list[2 * k] = x - pr.s0;
+    list[2 * k + 1] = nn_t[x];
+  } else if (!crosscheck && x < NS + NT) {
+    const int y = x - NS, p = pair_of(t_first, B, y);
+    const FtPair& pr = pairs[p];
+    const size_t k = (size_t)pr.list0 + pos[pr.s0 + p + pr.ns] + (y - pr.t0);
+    list[2 * k] = nn_s[y];
+    list[2 * k + 1] = y - pr.t0;
   }
 }
 
 // ---- tuple test: trial t draws list positions rand31(seed; TUPLE, 0, 3t + k) % ncorr, k = 0, 1, 2, and passes iff
-// every source / target edge length ratio of the triangle lies strictly inside (s, 1/s) (FP32, FGR's expression)
+// every source / target edge length ratio of the triangle lies strictly inside (s, 1/s) (FP32, FGR's expression).
+// The kept set is the first 1000 passing trials among the first 100 ncorr, so the rounds' chunking cannot change it.
+// Round r evaluates trials [r span, (r + 1) span) of every pair that is not done.
+constexpr int TUPLE_THREADS = 256;
+
+struct TupleState {
+  int kept;
+  int done;
+};
+
 __device__ __forceinline__ float len3(const double* __restrict__ P, int a, int b) {
   const float dx = (float)P[3 * (size_t)a] - (float)P[3 * (size_t)b];
   const float dy = (float)P[3 * (size_t)a + 1] - (float)P[3 * (size_t)b + 1];
@@ -368,33 +523,55 @@ __device__ __forceinline__ float len3(const double* __restrict__ P, int a, int b
   return __fsqrt_rn(dot3(dx, dy, dz, dx, dy, dz));
 }
 
-__global__ void k8_tuple_trials(const double* __restrict__ src, const double* __restrict__ tgt,
-                                const int* __restrict__ list, int ncorr, float s, uint64_t seed,
-                                unsigned long long t0, int nt, int* __restrict__ pass) {
-  const int u = blockIdx.x * blockDim.x + threadIdx.x;
-  if (u >= nt) return;
+// one thread per (pair, trial of the round), `bpp` CTAs per pair: pass[pair * span + u]
+__global__ void __launch_bounds__(TUPLE_THREADS)
+    k8_tuple_trials(const FtPair* __restrict__ pairs, int bpp, int span, unsigned long long t0,
+                    const TupleState* __restrict__ state, const int* __restrict__ ncorr, const int* __restrict__ lists,
+                    float s, unsigned char* __restrict__ pass) {
+  const int p = blockIdx.x / bpp, u = (blockIdx.x % bpp) * TUPLE_THREADS + threadIdx.x;
+  if (u >= span) return;
+  const size_t x = (size_t)p * span + u;
+  const int n = ncorr[p];
   const unsigned long long t = t0 + u;
+  if (state[p].done || t >= 100ull * (unsigned long long)n) return;
+  const uint64_t seed = pairs[p].seed;
+  const double *src = pairs[p].src, *tgt = pairs[p].tgt;
+  const int* list = lists + 2 * pairs[p].list0;
   int r[3];
-  for (int k = 0; k < 3; ++k)
-    r[k] = (int)(philox_rand31(seed, PSULVSB_DOMAIN_TUPLE, 0u, 3 * t + k) % (uint32_t)ncorr);
+#pragma unroll
+  for (int k = 0; k < 3; ++k) r[k] = (int)(philox_rand31(seed, PSULVSB_DOMAIN_TUPLE, 0u, 3 * t + k) % (uint32_t)n);
   bool ok = true;
+#pragma unroll
   for (int e = 0; e < 3; ++e) {
-    const int a = r[e], b = r[(e + 1) % 3];
+    const int a = r[e], b = r[e == 2 ? 0 : e + 1];
     const float li = len3(src, list[2 * a], list[2 * b]);
     const float lj = len3(tgt, list[2 * a + 1], list[2 * b + 1]);
     ok = ok && (__fmul_rn(li, s) < lj) && (lj < __fdiv_rn(li, s));
   }
-  pass[u] = ok ? 1 : 0;
+  pass[x] = ok ? 1 : 0;
 }
 
-// appends the passing trials of one chunk, in trial order, while fewer than max_tuples have been kept (one CTA)
+// one CTA per pair: appends the passing trials of the round, in trial order, while fewer than max_tuples have been
+// kept; a pair is done once it holds max_tuples or has run its 100 ncorr trials: counts[pair] = 3 kept, ndone += 1
 __global__ void __launch_bounds__(SCAN_THREADS)
-    k8_tuple_keep(const int* __restrict__ pass, int nt, unsigned long long t0, const int* __restrict__ list,
-                  int ncorr, uint64_t seed, int max_tuples, int* __restrict__ kept, int* __restrict__ out) {
+    k8_tuple_keep(const FtPair* __restrict__ pairs, int span, unsigned long long t0,
+                  const unsigned char* __restrict__ pass, const int* __restrict__ ncorr, const int* __restrict__ lists,
+                  int max_tuples, TupleState* __restrict__ state, int* __restrict__ ndone, int* __restrict__ outs,
+                  long long* __restrict__ counts) {
   __shared__ int warp_tot[SCAN_THREADS / 32];
   __shared__ int base;
+  const int p = blockIdx.x;
+  TupleState* st = state + p;
+  if (st->done) return;
+  const FtPair& pr = pairs[p];
+  const int n = ncorr[p];
+  const unsigned long long trials = 100ull * (unsigned long long)n;
+  const int nt = t0 >= trials ? 0 : (int)(trials - t0 < (unsigned long long)span ? trials - t0 : span);
+  const int* list = lists + 2 * pr.list0;
+  int* out = outs + 2 * pr.out0;
+  pass += (size_t)p * span;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  if (tid == 0) base = *kept;
+  if (tid == 0) base = st->kept;
   __syncthreads();
   for (int u0 = 0; u0 < nt && base < max_tuples; u0 += SCAN_THREADS) {
     const int u = u0 + tid;
@@ -411,7 +588,7 @@ __global__ void __launch_bounds__(SCAN_THREADS)
     if (f && slot < max_tuples) {
       const unsigned long long t = t0 + u;
       for (int k = 0; k < 3; ++k) {
-        const int r = (int)(philox_rand31(seed, PSULVSB_DOMAIN_TUPLE, 0u, 3 * t + k) % (uint32_t)ncorr);
+        const int r = (int)(philox_rand31(pr.seed, PSULVSB_DOMAIN_TUPLE, 0u, 3 * t + k) % (uint32_t)n);
         out[2 * (3 * (size_t)slot + k)] = list[2 * r];
         out[2 * (3 * (size_t)slot + k) + 1] = list[2 * r + 1];
       }
@@ -420,37 +597,16 @@ __global__ void __launch_bounds__(SCAN_THREADS)
     if (tid == 0) base = min(max_tuples, base + total);
     __syncthreads();
   }
-  if (tid == 0) *kept = base;
+  if (tid != 0) return;
+  st->kept = base;
+  if (base >= max_tuples || t0 + nt >= trials) {
+    st->done = 1;
+    counts[p] = 3ll * base;
+    atomicAdd(ndone, 1);
+  }
 }
 
 inline size_t up256(size_t x) { return (x + 255) & ~size_t(255); }
-
-struct FpfhWork {
-  int *pbucket, *count, *start, *cursor, *tmp, *counts, *kcount;
-  float4 *spts, *nf;
-};
-
-size_t fpfh_layout(int n, char* base, FpfhWork* w) {
-  const size_t nn = (size_t)(n > 0 ? n : 0), nb = bucket_count(n);
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    char* p = base ? base + off : nullptr;
-    off += up256(bytes);
-    return p;
-  };
-  FpfhWork v;
-  v.spts = (float4*)take(16 * nn);
-  v.nf = (float4*)take(16 * nn);
-  v.pbucket = (int*)take(4 * nn);
-  v.count = (int*)take(4 * nb);
-  v.start = (int*)take(4 * (nb + 1));
-  v.cursor = (int*)take(4 * nb);
-  v.tmp = (int*)take(4 * nn);
-  v.counts = (int*)take(4 * FT_DIM * nn);
-  v.kcount = (int*)take(4 * nn);
-  if (w) *w = v;
-  return off;
-}
 
 struct DevBuf {
   void* p = nullptr;
@@ -471,137 +627,387 @@ bool radius_ok(double r) { return std::isfinite(r) && r > 0.0; }
 
 inline int blocks(long long n, int t) { return (int)((n + t - 1) / t); }
 
-int run_fpfh(cudaStream_t st, const double* pts, int n, double rn, double rf, const double* viewpoint, void* work,
+// ---- FPFH batch on the host side
+struct FpfhSizes {
+  long long n = 0, nb = 0, tiles = 0;
+  int B = 0;
+};
+
+FpfhSizes fpfh_sizes(const psulvsb_fpfh_cloud_t* clouds, int B) {
+  FpfhSizes z;
+  z.B = B;
+  for (int c = 0; c < B; ++c) {
+    const int n = clouds[c].n;
+    if (n <= 0) continue;
+    z.n += n;
+    z.nb += bucket_count(n);
+    z.tiles += (n + FT_THREADS - 1) / FT_THREADS;
+  }
+  return z;
+}
+
+struct FpfhWork {
+  FtCloud* cloud;   // [B], followed by tile_first [B + 1]: one copy uploads both
+  int* tile_first;
+  size_t table_bytes;
+  float4 *spts, *nf;  // [n]: spts sorted by bucket, ascending index inside a bucket; .w = index in the cloud
+  int *pbucket, *tmp, *kcount;  // [n]
+  int *count, *cursor;          // [nb]
+  int* start;                   // [nb + B]
+  int* counts;                  // [33 n]
+};
+
+size_t fpfh_layout(const FpfhSizes& z, char* base, FpfhWork* w) {
+  const size_t nn = (size_t)z.n, nb = (size_t)z.nb, B = (size_t)z.B;
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    char* p = base ? base + off : nullptr;
+    off += up256(bytes);
+    return p;
+  };
+  FpfhWork v;
+  v.table_bytes = sizeof(FtCloud) * B + 4 * (B + 1);
+  v.cloud = (FtCloud*)take(v.table_bytes);
+  v.tile_first = (int*)((char*)v.cloud + sizeof(FtCloud) * B);
+  v.spts = (float4*)take(16 * nn);
+  v.nf = (float4*)take(16 * nn);
+  v.pbucket = (int*)take(4 * nn);
+  v.count = (int*)take(4 * nb);
+  v.start = (int*)take(4 * (nb + B));
+  v.cursor = (int*)take(4 * nb);
+  v.tmp = (int*)take(4 * nn);
+  v.counts = (int*)take(4 * FT_DIM * nn);
+  v.kcount = (int*)take(4 * nn);
+  if (w) *w = v;
+  return off;
+}
+
+// PSULVSB_ERR_INVALID for a bad cloud, PSULVSB_ERR_UNSUPPORTED for concatenations past the int range, else OK
+int clouds_check(const psulvsb_fpfh_cloud_t* clouds, int B, const char* who) {
+  for (int c = 0; c < B; ++c)
+    if (clouds[c].n < 0 || (clouds[c].n > 0 && !clouds[c].pts))
+      return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad cloud " + std::to_string(c));
+  const FpfhSizes z = fpfh_sizes(clouds, B);
+  if (z.n >= (1ll << 31) || z.nb + B >= (1ll << 31))
+    return fail(PSULVSB_ERR_UNSUPPORTED, std::string(who) + ": the batch's clouds exceed 2^31 - 1 points in all");
+  return PSULVSB_OK;
+}
+
+template <bool kBatch>
+void launch_fpfh(cudaStream_t st, const FpfhWork& w, const FtCloud& one, int B, int tiles, int n, double inv_h, float rn2,
+                 float rf2, double* normals, float* features) {
+  k8_grid_count<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, inv_h, w.pbucket, w.count);
+  k8_cloud_scan<kBatch><<<B, SCAN_THREADS, 0, st>>>(w.cloud, one, w.count, w.start, w.cursor);
+  k8_grid_scatter<<<blocks(n, GRID_THREADS), GRID_THREADS, 0, st>>>(n, w.pbucket, w.cursor, w.tmp);
+  k8_grid_order<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, w.pbucket, w.start, w.tmp, w.spts);
+  k8_radius_normals<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, inv_h, w.spts, w.start, rn2,
+                                                          normals, w.nf);
+  k8_spfh<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, inv_h, w.spts, w.start, rf2, w.nf,
+                                                w.counts, w.kcount);
+  k8_fpfh<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, inv_h, w.spts, w.start, rf2, w.counts,
+                                                w.kcount, features);
+}
+
+// the batch on the device (clouds checked, B >= 1): one upload of the cloud table, then seven launches over all clouds
+int run_fpfh(cudaStream_t st, const psulvsb_fpfh_cloud_t* clouds, int B, double rn, double rf, void* work,
              double* normals, float* features) {
-  if (n == 0) return PSULVSB_OK;
+  const FpfhSizes z = fpfh_sizes(clouds, B);
+  if (z.tiles == 0) return PSULVSB_OK;
   FpfhWork w;
-  fpfh_layout(n, static_cast<char*>(work), &w);
-  const unsigned int nb = bucket_count(n);
-  const double h = (rn > rf ? rn : rf) * (1.0 + 1e-5);
-  Grid g{1.0 / h, nb - 1, w.spts, w.start};
-  PSU_CUDA(cudaMemsetAsync(w.count, 0, 4 * (size_t)nb, st));
-  k8_grid_count<<<blocks(n, FT_THREADS), FT_THREADS, 0, st>>>(pts, n, g.inv_h, g.mask, w.pbucket, w.count);
-  PSU_CHECK_LAUNCH("k8_grid_count");
-  k8_scan<<<1, SCAN_THREADS, 0, st>>>(w.count, (int)nb, w.start, w.cursor);
-  PSU_CHECK_LAUNCH("k8_scan");
-  k8_grid_scatter<<<blocks(n, FT_THREADS), FT_THREADS, 0, st>>>(n, w.pbucket, w.cursor, w.tmp);
-  PSU_CHECK_LAUNCH("k8_grid_scatter");
-  k8_grid_order<<<blocks(n, FT_THREADS), FT_THREADS, 0, st>>>(pts, n, w.pbucket, w.start, w.tmp, w.spts);
-  PSU_CHECK_LAUNCH("k8_grid_order");
-  const double vx = viewpoint ? viewpoint[0] : 0.0, vy = viewpoint ? viewpoint[1] : 0.0,
-               vz = viewpoint ? viewpoint[2] : 0.0;
-  k8_radius_normals<<<blocks(n, FT_THREADS), FT_THREADS, 0, st>>>(g, pts, n, (float)(rn * rn), vx, vy, vz, normals,
-                                                                   w.nf);
-  PSU_CHECK_LAUNCH("k8_radius_normals");
-  k8_spfh<<<blocks(n, FT_THREADS), FT_THREADS, 0, st>>>(g, n, (float)(rf * rf), w.nf, w.counts, w.kcount);
-  PSU_CHECK_LAUNCH("k8_spfh");
-  k8_fpfh<<<blocks(n, FT_THREADS), FT_THREADS, 0, st>>>(g, n, (float)(rf * rf), w.counts, w.kcount, features);
+  fpfh_layout(z, static_cast<char*>(work), &w);
+  std::vector<char> table(w.table_bytes);
+  FtCloud* hc = reinterpret_cast<FtCloud*>(table.data());
+  int* tile_first = reinterpret_cast<int*>(table.data() + sizeof(FtCloud) * (size_t)B);
+  tile_first[0] = 0;
+  long long p0 = 0, b0 = 0;
+  for (int c = 0; c < B; ++c) {
+    const psulvsb_fpfh_cloud_t& q = clouds[c];
+    FtCloud& h = hc[c];
+    const unsigned int nb = q.n > 0 ? bucket_count(q.n) : 0u;
+    h.pts = q.pts;
+    for (int r = 0; r < 3; ++r) h.vp[r] = q.viewpoint[r];
+    h.n = q.n;
+    h.p0 = (int)p0;
+    h.b0 = (int)b0;
+    h.mask = nb - 1;
+    p0 += q.n;
+    b0 += nb;
+    tile_first[c + 1] = tile_first[c] + blocks(q.n, FT_THREADS);
+  }
+  if (B > 1) PSU_CUDA(cudaMemcpyAsync(w.cloud, table.data(), table.size(), cudaMemcpyHostToDevice, st));
+  const double h = (rn > rf ? rn : rf) * (1.0 + 1e-5), inv_h = 1.0 / h;
+  const int tiles = (int)z.tiles, n = (int)z.n;
+  const float rn2 = (float)(rn * rn), rf2 = (float)(rf * rf);
+  PSU_CUDA(cudaMemsetAsync(w.count, 0, 4 * (size_t)z.nb, st));
+  if (B == 1)
+    launch_fpfh<false>(st, w, hc[0], 1, tiles, n, inv_h, rn2, rf2, normals, features);
+  else
+    launch_fpfh<true>(st, w, hc[0], B, tiles, n, inv_h, rn2, rf2, normals, features);
   PSU_CHECK_LAUNCH("k8_fpfh");
   return PSULVSB_OK;
 }
 
-int run_feature_nn(cudaStream_t st, const float* fs, int ns, const float* ft, int nt, int* nn_s2t, int* nn_t2s) {
-  if (ns == 0 && nt == 0) return PSULVSB_OK;
-  if (ns == 0 || nt == 0) {  // nothing to be near to
-    if (ns) PSU_CUDA(cudaMemsetAsync(nn_s2t, 0xFF, 4 * (size_t)ns, st));
-    if (nt) PSU_CUDA(cudaMemsetAsync(nn_t2s, 0xFF, 4 * (size_t)nt, st));
-    return PSULVSB_OK;
+// the batch on host buffers (clouds checked, B >= 1): the clouds go up in one copy, features and normals come back
+int run_fpfh_host(const psulvsb_fpfh_cloud_t* clouds, int B, double rn, double rf, double* normals, float* features,
+                  const char* who) {
+  const FpfhSizes z = fpfh_sizes(clouds, B);
+  if (z.n == 0) return PSULVSB_OK;
+  const size_t N = (size_t)z.n, o_n = up256(4 * FT_DIM * N), o_in = o_n + up256(normals ? 24 * N : 0),
+               o_w = o_in + up256(24 * N);
+  std::vector<char> in(B > 1 ? 24 * N : 0);
+  std::vector<psulvsb_fpfh_cloud_t> dev(clouds, clouds + B);
+  DevBuf buf;
+  if (int rc = buf.alloc(o_w + fpfh_layout(z, nullptr, nullptr), who)) return rc;
+  char* b = static_cast<char*>(buf.p);
+  // a single cloud goes up straight from the caller's buffer: packing it first would only add a host copy
+  size_t off = 0;
+  for (int c = 0; c < B; ++c) {
+    if (dev[c].n <= 0) continue;
+    const size_t bytes = 24 * (size_t)dev[c].n;
+    if (B > 1) std::memcpy(in.data() + off, dev[c].pts, bytes);
+    dev[c].pts = reinterpret_cast<const double*>(b + o_in + off);
+    off += bytes;
   }
-  unsigned long long* keys = nullptr;
-  const size_t nk = (size_t)ns + (size_t)nt;
-  PSU_CUDA(cudaMallocAsync((void**)&keys, 8 * nk, st));
-  int rc = PSULVSB_OK;
-  if (cudaMemsetAsync(keys, 0xFF, 8 * nk, st) != cudaSuccess) rc = fail(PSULVSB_ERR_CUDA, "feature nn: memset failed");
-  if (!rc) {
-    const dim3 grid(blocks(ns, NN_THREADS * NN_ROWS), blocks(nt, NN_COLS_PER_CTA));
-    k8_feature_nn<<<grid, NN_THREADS, 0, st>>>(fs, ns, ft, nt, keys, keys + ns);
-    if (cudaGetLastError() != cudaSuccess) rc = fail(PSULVSB_ERR_CUDA, "k8_feature_nn launch failed");
-  }
-  if (!rc) {
-    k8_nn_finish<<<blocks(ns, 256), 256, 0, st>>>(keys, ns, nn_s2t);
-    k8_nn_finish<<<blocks(nt, 256), 256, 0, st>>>(keys + ns, nt, nn_t2s);
-    if (cudaGetLastError() != cudaSuccess) rc = fail(PSULVSB_ERR_CUDA, "k8_nn_finish launch failed");
-  }
-  cudaFreeAsync(keys, st);
-  return rc;
+  PSU_CUDA(cudaMemcpyAsync(b + o_in, B > 1 ? in.data() : (const void*)clouds[0].pts, 24 * N, cudaMemcpyHostToDevice,
+                           nullptr));
+  if (int rc = run_fpfh(nullptr, dev.data(), B, rn, rf, b + o_w, normals ? (double*)(b + o_n) : nullptr, (float*)b))
+    return rc;
+  PSU_CUDA(cudaMemcpyAsync(features, b, 4 * FT_DIM * N, cudaMemcpyDeviceToHost, nullptr));
+  if (normals) PSU_CUDA(cudaMemcpyAsync(normals, b + o_n, 24 * N, cudaMemcpyDeviceToHost, nullptr));
+  PSU_CUDA(cudaStreamSynchronize(nullptr));
+  return PSULVSB_OK;
 }
 
+// ---- matcher batch on the host side
 constexpr int MAX_TUPLES = 1000;
-constexpr int TUPLE_CHUNK = 1 << 20;
+// trials of one tuple round over the whole batch, and the bounds of a pair's share: a single pair evaluates 2^20
+// trials per round, a batch of 592 pairs 2^16 each
+constexpr long long TUPLE_ROUND = 1ll << 26;
+constexpr int TUPLE_CHUNK_MIN = 1 << 16, TUPLE_CHUNK_MAX = 1 << 20;
 
-// host buffers in: descriptors -> two-way NN -> list -> tuple test; pairs out
-int run_match_host(const double* src, int ns, const double* tgt, int nt, const float* fs, const float* ft,
-                   int crosscheck, int tuple_test, double tuple_scale, uint64_t seed, int* pairs, long long capacity,
-                   long long* n_pairs) {
-  *n_pairs = 0;
-  cudaStream_t st = nullptr;
-  const size_t NS = (size_t)ns, NT = (size_t)nt, NL = NS + NT;
+bool live(const psulvsb_match_pair_t& p) { return p.n_src > 0 && p.n_tgt > 0; }
+
+long long list_cap(const psulvsb_match_pair_t& p, int crosscheck) {
+  return live(p) ? (crosscheck ? p.n_src : (long long)p.n_src + p.n_tgt) : 0;
+}
+
+long long out_cap(const psulvsb_match_pair_t& p, int crosscheck, int tuple_test) {
+  return !live(p) ? 0 : (tuple_test ? 3ll * MAX_TUPLES : list_cap(p, crosscheck));
+}
+
+struct MatchSizes {
+  long long ns = 0, nt = 0, ctas = 0, list = 0, out = 0, max_list = 0;
+  int B = 0, span = 0;  // span: trials per pair and tuple round (0 without the tuple test)
+};
+
+MatchSizes match_sizes(const psulvsb_match_pair_t* pairs, int B, int crosscheck, int tuple_test) {
+  MatchSizes z;
+  z.B = B;
+  for (int b = 0; b < B; ++b) {
+    const psulvsb_match_pair_t& p = pairs[b];
+    z.out += out_cap(p, crosscheck, tuple_test);
+    if (!live(p)) continue;
+    z.ns += p.n_src;
+    z.nt += p.n_tgt;
+    z.ctas += (long long)blocks(p.n_src, NN_THREADS * NN_ROWS) * blocks(p.n_tgt, NN_COLS_PER_CTA);
+    z.list += list_cap(p, crosscheck);
+    z.max_list = std::max(z.max_list, list_cap(p, crosscheck));
+  }
+  if (tuple_test && z.max_list > 0) {
+    long long chunk = TUPLE_CHUNK_MAX;
+    while (chunk > TUPLE_CHUNK_MIN && chunk * B > TUPLE_ROUND) chunk >>= 1;
+    z.span = (int)std::min(chunk, 100 * z.max_list);
+  }
+  return z;
+}
+
+struct MatchWork {
+  FtPair* pair;  // [B], followed by cta_first, s_first, t_first [B + 1] each: one copy uploads the four
+  int *cta_first, *s_first, *t_first;
+  size_t table_bytes;
+  unsigned long long* key;  // [ns + nt]: row keys, then column keys
+  int* nn;                  // [ns + nt]: nn_t (source -> target), then nn_s
+  int *mark, *flag;         // [ns]
+  int* pos;                 // [ns + B]: pair p's scan at s0 + p, ns + 1 entries
+  int* ncorr;               // [B]
+  TupleState* state;        // [B], followed by ndone: one memset clears both
+  int* ndone;
+  int* list;                // [2 list] (tuple test)
+  unsigned char* pass;      // [B span] (tuple test)
+};
+
+size_t match_layout(const MatchSizes& z, char* base, MatchWork* w) {
+  const size_t B = (size_t)z.B, NS = (size_t)z.ns, NT = (size_t)z.nt;
   size_t off = 0;
   auto take = [&](size_t bytes) {
-    const size_t o = off;
+    char* p = base ? base + off : nullptr;
     off += up256(bytes);
-    return o;
+    return p;
   };
-  const size_t o_src = take(24 * NS), o_tgt = take(24 * NT), o_fs = take(4 * FT_DIM * NS), o_ft = take(4 * FT_DIM * NT);
-  const size_t o_nnt = take(4 * NS), o_nns = take(4 * NT), o_mark = take(4 * NS), o_flag = take(4 * NS),
-               o_pos = take(4 * (NS + 1)), o_list = take(8 * NL), o_pass = take(4 * (size_t)TUPLE_CHUNK),
-               o_kept = take(4), o_out = take(8 * 3 * (size_t)MAX_TUPLES);
-  DevBuf buf;
-  if (int rc = buf.alloc(off, "psulvsb_match_host")) return rc;
-  char* b = static_cast<char*>(buf.p);
-  double* d_src = (double*)(b + o_src);
-  double* d_tgt = (double*)(b + o_tgt);
-  float* d_fs = (float*)(b + o_fs);
-  float* d_ft = (float*)(b + o_ft);
-  int *nn_t = (int*)(b + o_nnt), *nn_s = (int*)(b + o_nns), *mark = (int*)(b + o_mark), *flag = (int*)(b + o_flag),
-      *pos = (int*)(b + o_pos), *list = (int*)(b + o_list), *pass = (int*)(b + o_pass), *kept = (int*)(b + o_kept),
-      *out = (int*)(b + o_out);
-  PSU_CUDA(cudaMemcpyAsync(d_src, src, 24 * NS, cudaMemcpyHostToDevice, st));
-  PSU_CUDA(cudaMemcpyAsync(d_tgt, tgt, 24 * NT, cudaMemcpyHostToDevice, st));
-  PSU_CUDA(cudaMemcpyAsync(d_fs, fs, 4 * FT_DIM * NS, cudaMemcpyHostToDevice, st));
-  PSU_CUDA(cudaMemcpyAsync(d_ft, ft, 4 * FT_DIM * NT, cudaMemcpyHostToDevice, st));
-  if (int rc = run_feature_nn(st, d_fs, ns, d_ft, nt, nn_t, nn_s)) return rc;
-  PSU_CUDA(cudaMemsetAsync(mark, 0, 4 * NS, st));
-  k8_match_mark<<<blocks(nt, 256), 256, 0, st>>>(nn_s, nt, mark);
-  PSU_CHECK_LAUNCH("k8_match_mark");
-  k8_match_flags<<<blocks(ns, 256), 256, 0, st>>>(nn_t, ns, nn_s, crosscheck, mark, flag);
-  PSU_CHECK_LAUNCH("k8_match_flags");
-  k8_scan<<<1, SCAN_THREADS, 0, st>>>(flag, ns, pos, nullptr);
-  PSU_CHECK_LAUNCH("k8_scan");
-  const int nplace = ns > nt ? ns : nt;
-  k8_match_place<<<blocks(nplace, 256), 256, 0, st>>>(nn_t, ns, nn_s, nt, crosscheck, flag, pos, list);
-  PSU_CHECK_LAUNCH("k8_match_place");
-  int first = 0;
-  PSU_CUDA(cudaMemcpyAsync(&first, pos + ns, 4, cudaMemcpyDeviceToHost, st));
-  PSU_CUDA(cudaStreamSynchronize(st));
-  const long long ncorr = (long long)first + (crosscheck ? 0 : nt);
-  const int* result = list;
-  long long count = ncorr;
-  if (tuple_test) {
-    count = 0;
-    PSU_CUDA(cudaMemsetAsync(kept, 0, 4, st));
-    const unsigned long long trials = 100ull * (unsigned long long)ncorr;
-    int got = 0;
-    for (unsigned long long t0 = 0; t0 < trials && got < MAX_TUPLES; t0 += TUPLE_CHUNK) {
-      const int chunk = (int)(trials - t0 < (unsigned long long)TUPLE_CHUNK ? trials - t0 : TUPLE_CHUNK);
-      k8_tuple_trials<<<blocks(chunk, 256), 256, 0, st>>>(d_src, d_tgt, list, (int)ncorr, (float)tuple_scale, seed, t0,
-                                                          chunk, pass);
-      PSU_CHECK_LAUNCH("k8_tuple_trials");
-      k8_tuple_keep<<<1, SCAN_THREADS, 0, st>>>(pass, chunk, t0, list, (int)ncorr, seed, MAX_TUPLES, kept, out);
-      PSU_CHECK_LAUNCH("k8_tuple_keep");
-      PSU_CUDA(cudaMemcpyAsync(&got, kept, 4, cudaMemcpyDeviceToHost, st));
-      PSU_CUDA(cudaStreamSynchronize(st));
-    }
-    count = 3ll * got;
-    result = out;
+  MatchWork v;
+  v.table_bytes = sizeof(FtPair) * B + 3 * 4 * (B + 1);
+  v.pair = (FtPair*)take(v.table_bytes);
+  v.cta_first = (int*)((char*)v.pair + sizeof(FtPair) * B);
+  v.s_first = v.cta_first + (B + 1);
+  v.t_first = v.s_first + (B + 1);
+  v.key = (unsigned long long*)take(8 * (NS + NT));
+  v.nn = (int*)take(4 * (NS + NT));
+  v.mark = (int*)take(4 * NS);
+  v.flag = (int*)take(4 * NS);
+  v.pos = (int*)take(4 * (NS + B));
+  v.ncorr = (int*)take(4 * B);
+  v.state = (TupleState*)take(sizeof(TupleState) * B + 4);
+  v.ndone = (int*)(v.state + B);
+  v.list = (int*)take(z.span ? 8 * (size_t)z.list : 0);
+  v.pass = (unsigned char*)take((size_t)z.span * B);
+  if (w) *w = v;
+  return off;
+}
+
+int match_check(const psulvsb_match_pair_t* pairs, int B, const char* who) {
+  long long ns = 0, nt = 0;
+  for (int b = 0; b < B; ++b) {
+    const psulvsb_match_pair_t& p = pairs[b];
+    if (p.n_src < 0 || p.n_tgt < 0 || (p.n_src > 0 && (!p.src || !p.fs)) || (p.n_tgt > 0 && (!p.tgt || !p.ft)))
+      return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad pair " + std::to_string(b));
+    ns += p.n_src;
+    nt += p.n_tgt;
   }
-  *n_pairs = count;
-  if (count > capacity)
-    return fail(PSULVSB_ERR_CAPACITY, "psulvsb_match_host: " + std::to_string(count) + " pairs, capacity " +
-                                          std::to_string(capacity));
-  if (count) PSU_CUDA(cudaMemcpyAsync(pairs, result, 8 * (size_t)count, cudaMemcpyDeviceToHost, st));
-  PSU_CUDA(cudaStreamSynchronize(st));
+  if (ns >= (1ll << 31) || nt >= (1ll << 31))
+    return fail(PSULVSB_ERR_UNSUPPORTED, std::string(who) + ": the batch's clouds exceed 2^31 - 1 points in all");
   return PSULVSB_OK;
+}
+
+// the batch on the device (pairs checked, B >= 1): one upload of the pair table, the NN, the list and the tuple rounds.
+// poll: wait for the stream after every tuple round and stop once every pair is done (the host variants); otherwise
+// all ceil(100 max_list / span) rounds are issued without a host round trip.
+int run_match(cudaStream_t st, const psulvsb_match_pair_t* pairs, int B, int crosscheck, int tuple_test,
+              double tuple_scale, void* work, int* d_pairs, long long* d_counts, bool poll) {
+  const MatchSizes z = match_sizes(pairs, B, crosscheck, tuple_test);
+  MatchWork w;
+  match_layout(z, static_cast<char*>(work), &w);
+  std::vector<char> table(w.table_bytes);
+  FtPair* hp = reinterpret_cast<FtPair*>(table.data());
+  int* cta_first = reinterpret_cast<int*>(table.data() + sizeof(FtPair) * (size_t)B);
+  int *s_first = cta_first + (B + 1), *t_first = s_first + (B + 1);
+  cta_first[0] = s_first[0] = t_first[0] = 0;
+  long long list0 = 0, out0 = 0;
+  for (int b = 0; b < B; ++b) {
+    const psulvsb_match_pair_t& q = pairs[b];
+    FtPair& h = hp[b];
+    h = FtPair{};
+    const bool on = live(q);
+    h.src = q.src;
+    h.tgt = q.tgt;
+    h.fs = q.fs;
+    h.ft = q.ft;
+    h.seed = q.seed;
+    h.ns = on ? q.n_src : 0;
+    h.nt = on ? q.n_tgt : 0;
+    h.s0 = s_first[b];
+    h.t0 = t_first[b];
+    h.rblocks = on ? blocks(q.n_src, NN_THREADS * NN_ROWS) : 1;
+    h.out0 = out0;
+    h.list0 = tuple_test ? list0 : out0;
+    out0 += out_cap(q, crosscheck, tuple_test);
+    list0 += list_cap(q, crosscheck);
+    cta_first[b + 1] = cta_first[b] + (on ? h.rblocks * blocks(q.n_tgt, NN_COLS_PER_CTA) : 0);
+    s_first[b + 1] = s_first[b] + h.ns;
+    t_first[b + 1] = t_first[b] + h.nt;
+  }
+  PSU_CUDA(cudaMemcpyAsync(w.pair, table.data(), table.size(), cudaMemcpyHostToDevice, st));
+  const int NS = (int)z.ns, NT = (int)z.nt;
+  int *nn_t = w.nn, *nn_s = w.nn + NS;
+  if (z.ctas > 0) {
+    PSU_CUDA(cudaMemsetAsync(w.key, 0xFF, 8 * ((size_t)NS + NT), st));
+    if (B == 1)
+      k8_feature_nn<false><<<dim3(hp[0].rblocks, blocks(NT, NN_COLS_PER_CTA)), NN_THREADS, 0, st>>>(
+          w.pair, hp[0], w.cta_first, 1, w.key, w.key + NS);
+    else
+      k8_feature_nn<true><<<(int)z.ctas, NN_THREADS, 0, st>>>(w.pair, hp[0], w.cta_first, B, w.key, w.key + NS);
+    PSU_CHECK_LAUNCH("k8_feature_nn");
+    k8_nn_finish<<<blocks((long long)NS + NT, 256), 256, 0, st>>>(w.key, NS + NT, w.nn);
+    PSU_CHECK_LAUNCH("k8_nn_finish");
+    if (!crosscheck) {
+      PSU_CUDA(cudaMemsetAsync(w.mark, 0, 4 * (size_t)NS, st));
+      k8_match_mark<<<blocks(NT, 256), 256, 0, st>>>(w.pair, w.t_first, B, NT, nn_s, w.mark);
+      PSU_CHECK_LAUNCH("k8_match_mark");
+    }
+    k8_match_flags<<<blocks(NS, 256), 256, 0, st>>>(w.pair, w.s_first, B, NS, nn_t, nn_s, crosscheck, w.mark, w.flag);
+    PSU_CHECK_LAUNCH("k8_match_flags");
+  }
+  k8_match_scan<<<B, SCAN_THREADS, 0, st>>>(w.pair, w.flag, crosscheck, tuple_test, w.pos, w.ncorr, d_counts);
+  PSU_CHECK_LAUNCH("k8_match_scan");
+  if (z.ctas == 0) return PSULVSB_OK;
+  int* list = tuple_test ? w.list : d_pairs;
+  const long long nplace = (long long)NS + (crosscheck ? 0 : NT);
+  k8_match_place<<<blocks(nplace, 256), 256, 0, st>>>(w.pair, w.s_first, w.t_first, B, NS, NT, nn_t, nn_s, crosscheck,
+                                                      w.flag, w.pos, list);
+  PSU_CHECK_LAUNCH("k8_match_place");
+  if (!tuple_test) return PSULVSB_OK;
+  PSU_CUDA(cudaMemsetAsync(w.state, 0, sizeof(TupleState) * (size_t)B + 4, st));
+  const long long span = z.span, rounds = (100 * z.max_list + span - 1) / span;
+  const int bpp = blocks(span, TUPLE_THREADS);
+  for (long long r = 0; r < rounds; ++r) {
+    const unsigned long long t0 = (unsigned long long)(r * span);
+    k8_tuple_trials<<<bpp * B, TUPLE_THREADS, 0, st>>>(w.pair, bpp, (int)span, t0, w.state, w.ncorr, w.list,
+                                                       (float)tuple_scale, w.pass);
+    PSU_CHECK_LAUNCH("k8_tuple_trials");
+    k8_tuple_keep<<<B, SCAN_THREADS, 0, st>>>(w.pair, (int)span, t0, w.pass, w.ncorr, w.list, MAX_TUPLES, w.state,
+                                              w.ndone, d_pairs, d_counts);
+    PSU_CHECK_LAUNCH("k8_tuple_keep");
+    if (poll) {
+      int done = 0;
+      PSU_CUDA(cudaMemcpyAsync(&done, w.ndone, 4, cudaMemcpyDeviceToHost, st));
+      PSU_CUDA(cudaStreamSynchronize(st));
+      if (done == B) break;
+    }
+  }
+  return PSULVSB_OK;
+}
+
+// the batch on host buffers (pairs checked, B >= 1): the live pairs' points and descriptors go up in one copy into
+// `buf`, which then holds counts [B] (long long) and the pairs (Σ cap) from offset 0, ready to come back
+int run_match_host(const psulvsb_match_pair_t* pairs, int B, int crosscheck, int tuple_test, double tuple_scale,
+                   DevBuf& buf, const char* who) {
+  const MatchSizes z = match_sizes(pairs, B, crosscheck, tuple_test);
+  const size_t o_pairs = 8 * (size_t)B, o_in = up256(o_pairs + 8 * (size_t)z.out);
+  // the live pairs' src, tgt, fs, ft in pair order, each pair's block 8-byte aligned
+  std::vector<psulvsb_match_pair_t> dev(pairs, pairs + B);
+  std::vector<size_t> in_off(B);
+  size_t in_bytes = 0;
+  for (int b = 0; b < B; ++b) {
+    in_off[b] = in_bytes;
+    if (live(dev[b])) in_bytes += ((24 + 4 * FT_DIM) * ((size_t)dev[b].n_src + dev[b].n_tgt) + 7) & ~size_t(7);
+  }
+  const size_t o_work = up256(o_in + in_bytes);
+  if (int rc = buf.alloc(o_work + match_layout(z, nullptr, nullptr), who)) return rc;
+  char* base = static_cast<char*>(buf.p);
+  // a single pair's four arrays go up straight from the caller's buffers: packing them first would only add a host copy
+  std::vector<char> in(B > 1 ? in_bytes : 0);
+  for (int b = 0; b < B; ++b) {
+    psulvsb_match_pair_t& q = dev[b];
+    if (!live(q)) continue;
+    size_t off = in_off[b];
+    auto put = [&](const void* h, size_t bytes) -> const char* {
+      char* d = base + o_in + off;
+      if (B > 1)
+        std::memcpy(in.data() + off, h, bytes);
+      else if (cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, nullptr) != cudaSuccess)
+        return nullptr;
+      off += bytes;
+      return d;
+    };
+    const size_t ns = (size_t)q.n_src, nt = (size_t)q.n_tgt;
+    q.src = (const double*)put(q.src, 24 * ns);
+    q.tgt = (const double*)put(q.tgt, 24 * nt);
+    q.fs = (const float*)put(q.fs, 4 * FT_DIM * ns);
+    q.ft = (const float*)put(q.ft, 4 * FT_DIM * nt);
+    if (!q.src || !q.tgt || !q.fs || !q.ft) return fail(PSULVSB_ERR_CUDA, std::string(who) + ": copy in failed");
+  }
+  if (B > 1 && in_bytes) PSU_CUDA(cudaMemcpyAsync(base + o_in, in.data(), in_bytes, cudaMemcpyHostToDevice, nullptr));
+  return run_match(nullptr, dev.data(), B, crosscheck, tuple_test, tuple_scale, base + o_work, (int*)(base + o_pairs),
+                   (long long*)base, true);
 }
 
 }  // namespace
@@ -613,7 +1019,23 @@ using psulvsb::fail;
 extern "C" {
 
 unsigned long long psulvsb_fpfh_workspace_bytes(int n) {
-  return n < 0 ? 0ull : (unsigned long long)psulvsb::fpfh_layout(n, nullptr, nullptr);
+  if (n < 0) return 0ull;
+  const psulvsb_fpfh_cloud_t c{nullptr, n, {0.0, 0.0, 0.0}};
+  return (unsigned long long)psulvsb::fpfh_layout(psulvsb::fpfh_sizes(&c, 1), nullptr, nullptr);
+}
+
+unsigned long long psulvsb_fpfh_batch_workspace_bytes(const psulvsb_fpfh_cloud_t* clouds, int B) {
+  if (B <= 0 || !clouds) return 0ull;
+  for (int c = 0; c < B; ++c)
+    if (clouds[c].n < 0) return 0ull;
+  return (unsigned long long)psulvsb::fpfh_layout(psulvsb::fpfh_sizes(clouds, B), nullptr, nullptr);
+}
+
+static psulvsb_fpfh_cloud_t one_cloud(const double* pts, int n, const double viewpoint[3]) {
+  psulvsb_fpfh_cloud_t c{pts, n, {0.0, 0.0, 0.0}};
+  if (viewpoint)
+    for (int r = 0; r < 3; ++r) c.viewpoint[r] = viewpoint[r];
+  return c;
 }
 
 int psulvsb_fpfh(void* stream, const double* d_pts, int n, double normal_radius, double feature_radius,
@@ -622,8 +1044,8 @@ int psulvsb_fpfh(void* stream, const double* d_pts, int n, double normal_radius,
       (n > 0 && (!d_pts || !d_work || !d_features)))
     return fail(PSULVSB_ERR_INVALID, "psulvsb_fpfh: bad argument (radii must be finite and > 0)");
   if (int rc = psulvsb::need_device()) return rc;
-  return psulvsb::run_fpfh((cudaStream_t)stream, d_pts, n, normal_radius, feature_radius, viewpoint, d_work, d_normals,
-                           d_features);
+  const psulvsb_fpfh_cloud_t c = one_cloud(d_pts, n, viewpoint);
+  return psulvsb::run_fpfh((cudaStream_t)stream, &c, 1, normal_radius, feature_radius, d_work, d_normals, d_features);
 }
 
 int psulvsb_fpfh_host(const double* pts, int n, double normal_radius, double feature_radius, const double viewpoint[3],
@@ -632,19 +1054,31 @@ int psulvsb_fpfh_host(const double* pts, int n, double normal_radius, double fea
       (n > 0 && (!pts || !features)))
     return fail(PSULVSB_ERR_INVALID, "psulvsb_fpfh_host: bad argument (radii must be finite and > 0)");
   if (int rc = psulvsb::need_device()) return rc;
-  if (n == 0) return PSULVSB_OK;
-  const size_t nn = (size_t)n, o_f = psulvsb::up256(24 * nn), o_n = o_f + psulvsb::up256(4 * 33 * nn),
-               o_w = o_n + psulvsb::up256(24 * nn);
-  psulvsb::DevBuf buf;
-  if (int rc = buf.alloc(o_w + psulvsb_fpfh_workspace_bytes(n), "psulvsb_fpfh_host")) return rc;
-  char* b = static_cast<char*>(buf.p);
-  PSU_CUDA(cudaMemcpy(b, pts, 24 * nn, cudaMemcpyHostToDevice));
-  if (int rc = psulvsb::run_fpfh(nullptr, (double*)b, n, normal_radius, feature_radius, viewpoint, b + o_w,
-                                 normals ? (double*)(b + o_n) : nullptr, (float*)(b + o_f)))
-    return rc;
-  PSU_CUDA(cudaMemcpy(features, b + o_f, 4 * 33 * nn, cudaMemcpyDeviceToHost));
-  if (normals) PSU_CUDA(cudaMemcpy(normals, b + o_n, 24 * nn, cudaMemcpyDeviceToHost));
-  return PSULVSB_OK;
+  const psulvsb_fpfh_cloud_t c = one_cloud(pts, n, viewpoint);
+  return psulvsb::run_fpfh_host(&c, 1, normal_radius, feature_radius, normals, features, "psulvsb_fpfh_host");
+}
+
+int psulvsb_fpfh_batch(void* stream, const psulvsb_fpfh_cloud_t* clouds, int B, double normal_radius,
+                       double feature_radius, void* d_work, double* d_normals, float* d_features) {
+  if (B < 0 || !psulvsb::radius_ok(normal_radius) || !psulvsb::radius_ok(feature_radius) ||
+      (B > 0 && (!clouds || !d_work || !d_features)))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_fpfh_batch: bad argument (radii must be finite and > 0)");
+  if (int rc = psulvsb::clouds_check(clouds, B, "psulvsb_fpfh_batch")) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = psulvsb::need_device()) return rc;
+  return psulvsb::run_fpfh((cudaStream_t)stream, clouds, B, normal_radius, feature_radius, d_work, d_normals,
+                           d_features);
+}
+
+int psulvsb_fpfh_batch_host(const psulvsb_fpfh_cloud_t* clouds, int B, double normal_radius, double feature_radius,
+                            double* normals, float* features) {
+  if (B < 0 || !psulvsb::radius_ok(normal_radius) || !psulvsb::radius_ok(feature_radius) ||
+      (B > 0 && (!clouds || !features)))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_fpfh_batch_host: bad argument (radii must be finite and > 0)");
+  if (int rc = psulvsb::clouds_check(clouds, B, "psulvsb_fpfh_batch_host")) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = psulvsb::need_device()) return rc;
+  return psulvsb::run_fpfh_host(clouds, B, normal_radius, feature_radius, normals, features, "psulvsb_fpfh_batch_host");
 }
 
 int psulvsb_feature_nn(void* stream, const float* d_fs, int n_src, const float* d_ft, int n_tgt, int* d_nn_src_to_tgt,
@@ -652,7 +1086,38 @@ int psulvsb_feature_nn(void* stream, const float* d_fs, int n_src, const float* 
   if (n_src < 0 || n_tgt < 0 || (n_src > 0 && (!d_fs || !d_nn_src_to_tgt)) || (n_tgt > 0 && (!d_ft || !d_nn_tgt_to_src)))
     return fail(PSULVSB_ERR_INVALID, "psulvsb_feature_nn: bad argument");
   if (int rc = psulvsb::need_device()) return rc;
-  return psulvsb::run_feature_nn((cudaStream_t)stream, d_fs, n_src, d_ft, n_tgt, d_nn_src_to_tgt, d_nn_tgt_to_src);
+  using namespace psulvsb;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (n_src == 0 && n_tgt == 0) return PSULVSB_OK;
+  if (n_src == 0 || n_tgt == 0) {  // nothing to be near to
+    if (n_src) PSU_CUDA(cudaMemsetAsync(d_nn_src_to_tgt, 0xFF, 4 * (size_t)n_src, st));
+    if (n_tgt) PSU_CUDA(cudaMemsetAsync(d_nn_tgt_to_src, 0xFF, 4 * (size_t)n_tgt, st));
+    return PSULVSB_OK;
+  }
+  // a batch of one: the pair travels as a kernel parameter, the keys in the call's own allocation
+  FtPair one{};
+  one.fs = d_fs;
+  one.ft = d_ft;
+  one.ns = n_src;
+  one.nt = n_tgt;
+  one.rblocks = blocks(n_src, NN_THREADS * NN_ROWS);
+  const size_t nk = (size_t)n_src + (size_t)n_tgt;
+  unsigned long long* keys = nullptr;
+  PSU_CUDA(cudaMallocAsync((void**)&keys, 8 * nk, st));
+  int rc = PSULVSB_OK;
+  if (cudaMemsetAsync(keys, 0xFF, 8 * nk, st) != cudaSuccess) rc = fail(PSULVSB_ERR_CUDA, "feature nn: memset failed");
+  if (!rc) {
+    k8_feature_nn<false><<<dim3(one.rblocks, blocks(n_tgt, NN_COLS_PER_CTA)), NN_THREADS, 0, st>>>(nullptr, one, nullptr,
+                                                                                                  1, keys, keys + n_src);
+    if (cudaGetLastError() != cudaSuccess) rc = fail(PSULVSB_ERR_CUDA, "k8_feature_nn launch failed");
+  }
+  if (!rc) {
+    k8_nn_finish<<<blocks(n_src, 256), 256, 0, st>>>(keys, n_src, d_nn_src_to_tgt);
+    k8_nn_finish<<<blocks(n_tgt, 256), 256, 0, st>>>(keys + n_src, n_tgt, d_nn_tgt_to_src);
+    if (cudaGetLastError() != cudaSuccess) rc = fail(PSULVSB_ERR_CUDA, "k8_nn_finish launch failed");
+  }
+  cudaFreeAsync(keys, st);
+  return rc;
 }
 
 int psulvsb_match_host(const double* src_pts, int n_src, const double* tgt_pts, int n_tgt, const float* fs,
@@ -664,8 +1129,57 @@ int psulvsb_match_host(const double* src_pts, int n_src, const double* tgt_pts, 
   *n_pairs = 0;
   if (int rc = psulvsb::need_device()) return rc;
   if (n_src == 0 || n_tgt == 0) return PSULVSB_OK;
-  return psulvsb::run_match_host(src_pts, n_src, tgt_pts, n_tgt, fs, ft, crosscheck, tuple_test, tuple_scale, seed,
-                                 pairs, capacity, n_pairs);
+  const psulvsb_match_pair_t p{src_pts, n_src, tgt_pts, n_tgt, fs, ft, seed};
+  psulvsb::DevBuf buf;
+  if (int rc = psulvsb::run_match_host(&p, 1, crosscheck, tuple_test, tuple_scale, buf, "psulvsb_match_host")) return rc;
+  long long count = 0;
+  PSU_CUDA(cudaMemcpyAsync(&count, buf.p, 8, cudaMemcpyDeviceToHost, nullptr));
+  PSU_CUDA(cudaStreamSynchronize(nullptr));
+  *n_pairs = count;
+  if (count > capacity)
+    return fail(PSULVSB_ERR_CAPACITY, "psulvsb_match_host: " + std::to_string(count) + " pairs, capacity " +
+                                          std::to_string(capacity));
+  if (count) PSU_CUDA(cudaMemcpyAsync(pairs, (char*)buf.p + 8, 8 * (size_t)count, cudaMemcpyDeviceToHost, nullptr));
+  PSU_CUDA(cudaStreamSynchronize(nullptr));
+  return PSULVSB_OK;
+}
+
+unsigned long long psulvsb_match_batch_workspace_bytes(const psulvsb_match_pair_t* pairs, int B, int crosscheck,
+                                                       int tuple_test) {
+  if (B <= 0 || !pairs) return 0ull;
+  for (int b = 0; b < B; ++b)
+    if (pairs[b].n_src < 0 || pairs[b].n_tgt < 0) return 0ull;
+  return (unsigned long long)psulvsb::match_layout(psulvsb::match_sizes(pairs, B, crosscheck, tuple_test), nullptr,
+                                                   nullptr);
+}
+
+int psulvsb_match_batch(void* stream, const psulvsb_match_pair_t* pairs, int B, int crosscheck, int tuple_test,
+                        double tuple_scale, void* d_work, int* d_pairs, long long* d_counts) {
+  if (B < 0 || (tuple_test && !std::isfinite(tuple_scale)) || (B > 0 && (!pairs || !d_work || !d_pairs || !d_counts)))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_match_batch: bad argument");
+  if (int rc = psulvsb::match_check(pairs, B, "psulvsb_match_batch")) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = psulvsb::need_device()) return rc;
+  return psulvsb::run_match((cudaStream_t)stream, pairs, B, crosscheck, tuple_test, tuple_scale, d_work, d_pairs,
+                            d_counts, false);
+}
+
+int psulvsb_match_batch_host(const psulvsb_match_pair_t* pairs, int B, int crosscheck, int tuple_test,
+                             double tuple_scale, int* pairs_out, long long* counts) {
+  if (B < 0 || (tuple_test && !std::isfinite(tuple_scale)) || (B > 0 && (!pairs || !pairs_out || !counts)))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_match_batch_host: bad argument");
+  if (int rc = psulvsb::match_check(pairs, B, "psulvsb_match_batch_host")) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = psulvsb::need_device()) return rc;
+  psulvsb::DevBuf buf;
+  if (int rc = psulvsb::run_match_host(pairs, B, crosscheck, tuple_test, tuple_scale, buf, "psulvsb_match_batch_host"))
+    return rc;
+  const psulvsb::MatchSizes z = psulvsb::match_sizes(pairs, B, crosscheck, tuple_test);
+  PSU_CUDA(cudaMemcpyAsync(counts, buf.p, 8 * (size_t)B, cudaMemcpyDeviceToHost, nullptr));
+  if (z.out) PSU_CUDA(cudaMemcpyAsync(pairs_out, (char*)buf.p + 8 * (size_t)B, 8 * (size_t)z.out, cudaMemcpyDeviceToHost,
+                                      nullptr));
+  PSU_CUDA(cudaStreamSynchronize(nullptr));
+  return PSULVSB_OK;
 }
 
 }  // extern "C"

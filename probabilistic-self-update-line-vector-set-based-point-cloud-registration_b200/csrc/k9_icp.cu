@@ -71,20 +71,6 @@ struct IcpPair {
   IcpInit init;
 };
 
-// the pair of item x: the p with first[p] <= x < first[p + 1] (first[0, B] ascending, first[0] <= x < first[B]; a pair
-// without items is never the answer)
-__device__ __forceinline__ int pair_of(const int* __restrict__ first, int B, int x) {
-  int lo = 0, hi = B;
-  while (hi - lo > 1) {
-    const int mid = (lo + hi) >> 1;
-    if (first[mid] <= x)
-      lo = mid;
-    else
-      hi = mid;
-  }
-  return lo;
-}
-
 __device__ __forceinline__ long long icp_cell(double x, double c, double inv_h) {
   return (long long)floor(dmul(dsub(x, c), inv_h));
 }
