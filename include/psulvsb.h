@@ -520,6 +520,48 @@ int psulvsb_icp_batch(void* stream, const psulvsb_icp_pair_t* pairs, int B, cons
 int psulvsb_icp_batch_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
                            psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr);
 
+/* ---- Generalized ICP (plane-to-plane, Segal et al.; Open3D's registration_generalized_icp), DESIGN.md section 11
+ * "Generalized ICP": the loop, stop rule, correspondences (every target point is a candidate), trace, results and
+ * statuses of psulvsb_icp; only the update differs.  Each point's covariance is I - (1 - epsilon) n n^T for its unit
+ * normal n (normalised in FP64; a non-finite or zero normal gives I); the update solves the Gauss-Newton system of
+ * sum d^T (Sigma_t + R Sigma_s R^T)^-1 d with Open3D's Jacobian by the 6x6 Cholesky of point-to-plane, and needs 3
+ * correspondences.  params->point_to_plane must be 0 (the entry point is the mode); epsilon: finite, 0 < epsilon <= 1
+ * (Open3D's default 1e-3; 1 gives the linearised point-to-point step).  The sign of a normal does not matter.  The
+ * tests compare with a numpy restatement (tests/gicp_restatement.py). */
+typedef struct psulvsb_gicp_pair {
+  const double* src;         /* 3 x n_s, column-major                                                  */
+  int n_s;
+  const double* tgt;         /* 3 x n_t                                                                */
+  int n_t;
+  const double* src_normals; /* 3 x n_s, required when n_s > 0 and n_t > 0                             */
+  const double* tgt_normals; /* 3 x n_t, required when n_s > 0 and n_t > 0                             */
+  double R0[9];              /* column-major                                                           */
+  double t0[3];
+} psulvsb_gicp_pair_t;
+
+/* psulvsb_icp with generalized ICP's update.  Workspace: psulvsb_icp_workspace_bytes(n_s, n_t).  PSULVSB_ERR_INVALID
+ * before any device work for every argument psulvsb_icp refuses, an epsilon outside (0, 1] or NaN, point_to_plane != 0,
+ * or a NULL normal array when n_s > 0 and n_t > 0. */
+int psulvsb_gicp(void* stream, const double* d_src, int n_s, const double* d_src_normals, const double* d_tgt, int n_t,
+                 const double* d_tgt_normals, const psulvsb_icp_params_t* params, double epsilon, const double R0[9],
+                 const double t0[3], void* d_work, psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace,
+                 int* d_corr);
+/* The same on host buffers, synchronous: clouds and normals go up in one copy, one device-to-host copy at the end. */
+int psulvsb_gicp_host(const double* src, int n_s, const double* src_normals, const double* tgt, int n_t,
+                      const double* tgt_normals, const psulvsb_icp_params_t* params, double epsilon,
+                      const double R0[9], const double t0[3], psulvsb_icp_result_t* result,
+                      psulvsb_icp_iteration_t* trace, int* corr);
+/* Device scratch of psulvsb_gicp_batch: psulvsb_icp_batch_workspace_bytes of the same sizes. */
+unsigned long long psulvsb_gicp_batch_workspace_bytes(const psulvsb_gicp_pair_t* pairs, int B);
+/* psulvsb_icp_batch with generalized ICP's update: the layouts, refusals and the guarantee that pair b's outputs are
+ * bit-identical to psulvsb_gicp_host on that pair alone are psulvsb_icp_batch's, plus psulvsb_gicp's refusals. */
+int psulvsb_gicp_batch(void* stream, const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                       double epsilon, void* d_work, psulvsb_icp_result_t* d_results, psulvsb_icp_iteration_t* d_trace,
+                       int* d_corr);
+/* The same on host buffers, synchronous: one upload of the clouds and normals, one download (psulvsb_icp_batch_host). */
+int psulvsb_gicp_batch_host(const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                            double epsilon, psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr);
+
 /* Clique escalation (registration.cc:1000-1085 -> teaser/src/graph.cc:12-125, PMC exact maximum clique) of the
  * graph with n_vertices vertices and the given edges (uint2 endpoint pairs).  A deterministic greedy maximal
  * clique (most neighbours among the remaining candidates first, ties: lowest index) gives the lower bound;

@@ -36,6 +36,8 @@ SYMBOLS = [
     "psulvsb_icp_batch_workspace_bytes", "psulvsb_icp_batch", "psulvsb_icp_batch_host",
     "psulvsb_fpfh_batch_workspace_bytes", "psulvsb_fpfh_batch", "psulvsb_fpfh_batch_host",
     "psulvsb_match_batch_workspace_bytes", "psulvsb_match_batch", "psulvsb_match_batch_host",
+    "psulvsb_gicp", "psulvsb_gicp_host", "psulvsb_gicp_batch_workspace_bytes", "psulvsb_gicp_batch",
+    "psulvsb_gicp_batch_host",
 ]
 UNIQUE_ID_BYTES = 128
 
@@ -189,6 +191,20 @@ class IcpPair(C.Structure):
     ]
 
 
+class GicpPair(C.Structure):
+    """psulvsb_gicp_pair_t: one generalized-ICP problem of a batch (R0 column-major)."""
+    _fields_ = [
+        ("src", C.c_void_p),
+        ("n_s", C.c_int),
+        ("tgt", C.c_void_p),
+        ("n_t", C.c_int),
+        ("src_normals", C.c_void_p),
+        ("tgt_normals", C.c_void_p),
+        ("R0", C.c_double * 9),
+        ("t0", C.c_double * 3),
+    ]
+
+
 class FpfhCloud(C.Structure):
     """psulvsb_fpfh_cloud_t: one cloud of an FPFH batch."""
     _fields_ = [
@@ -326,6 +342,16 @@ def _declare(L: C.CDLL) -> None:
     L.psulvsb_icp_batch_workspace_bytes.restype = _ull
     L.psulvsb_icp_batch.argtypes = [_vp, C.POINTER(IcpPair), C.c_int, C.POINTER(IcpParams), _vp, _vp, _vp, _vp]
     L.psulvsb_icp_batch_host.argtypes = [C.POINTER(IcpPair), C.c_int, C.POINTER(IcpParams), _vp, _vp, _vp]
+    L.psulvsb_gicp.argtypes = [_vp, _vp, C.c_int, _vp, _vp, C.c_int, _vp, C.POINTER(IcpParams), C.c_double,
+                               C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]
+    L.psulvsb_gicp_host.argtypes = [_vp, C.c_int, _vp, _vp, C.c_int, _vp, C.POINTER(IcpParams), C.c_double,
+                                    C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp]
+    L.psulvsb_gicp_batch_workspace_bytes.argtypes = [C.POINTER(GicpPair), C.c_int]
+    L.psulvsb_gicp_batch_workspace_bytes.restype = _ull
+    L.psulvsb_gicp_batch.argtypes = [_vp, C.POINTER(GicpPair), C.c_int, C.POINTER(IcpParams), C.c_double, _vp, _vp,
+                                     _vp, _vp]
+    L.psulvsb_gicp_batch_host.argtypes = [C.POINTER(GicpPair), C.c_int, C.POINTER(IcpParams), C.c_double, _vp, _vp,
+                                          _vp]
     L.psulvsb_fpfh_batch_workspace_bytes.argtypes = [C.POINTER(FpfhCloud), C.c_int]
     L.psulvsb_fpfh_batch_workspace_bytes.restype = _ull
     L.psulvsb_fpfh_batch.argtypes = [_vp, C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_double, _vp, _vp, _vp]
