@@ -403,6 +403,33 @@ int psulvsb_fpfh_batch(void* stream, const psulvsb_fpfh_cloud_t* clouds, int B, 
 int psulvsb_fpfh_batch_host(const psulvsb_fpfh_cloud_t* clouds, int B, double normal_radius, double feature_radius,
                             double* normals, float* features);
 
+/* ---- Surface normals alone (DESIGN.md section 10, "Normals alone"), on FPFH's grid: O(n * neighbourhood) instead of
+ * the O(n^2) psulvsb_estimate_normals.  Points and normals are column-major 3xn doubles.
+ *   max_nn = 0:      radius neighbourhood, every point within `radius` (FP32 distance test, the point included): the
+ *                    normals psulvsb_fpfh returns with normal_radius = radius, bit for bit, for any feature_radius <=
+ *                    radius.
+ *   3 <= max_nn <= 32: hybrid neighbourhood (Open3D's KDTreeSearchParamHybrid), the max_nn nearest points within
+ *                    `radius`, ranked by (FP32 squared distance, index): ties go to the lower index.  A neighbourhood
+ *                    of at most max_nn points gives the radius mode's normal bit for bit.
+ * FP64 mean and covariance, smallest eigenvector, flipped towards the viewpoint (NULL: origin); fewer than 3 points:
+ * NaN.  Results are bit-identical from call to call.  d_work: psulvsb_normals_workspace_bytes(n) bytes of device
+ * scratch (depends on n only, never more than psulvsb_fpfh_workspace_bytes(n)).  PSULVSB_ERR_INVALID before any
+ * device work for a radius that is not finite and > 0, another max_nn, a negative size or a required NULL; the batch
+ * variants take the FPFH batch's items and return its errors, PSULVSB_ERR_UNSUPPORTED included.  n = 0 or B = 0 does
+ * nothing.  Batch: cloud c's normals are rows [sum_{a<c} n_a, ...) of the (sum n) x 3 doubles, bit-identical to the
+ * single call on cloud c alone (with its viewpoint).  The _host variants take host buffers and are synchronous. */
+unsigned long long psulvsb_normals_workspace_bytes(int n);
+int psulvsb_normals(void* stream, const double* d_pts, int n, double radius, int max_nn, const double viewpoint[3],
+                    void* d_work, double* d_normals);
+int psulvsb_normals_host(const double* pts, int n, double radius, int max_nn, const double viewpoint[3],
+                         double* normals);
+/* Device scratch of psulvsb_normals_batch (depends on the sizes only); 0 for B <= 0 or a negative size. */
+unsigned long long psulvsb_normals_batch_workspace_bytes(const psulvsb_fpfh_cloud_t* clouds, int B);
+int psulvsb_normals_batch(void* stream, const psulvsb_fpfh_cloud_t* clouds, int B, double radius, int max_nn,
+                          void* d_work, double* d_normals);
+int psulvsb_normals_batch_host(const psulvsb_fpfh_cloud_t* clouds, int B, double radius, int max_nn,
+                               double* normals);
+
 typedef struct psulvsb_match_pair {
   const double* src;  /* 3 x n_src, column-major: the tuple test's points                                 */
   int n_src;

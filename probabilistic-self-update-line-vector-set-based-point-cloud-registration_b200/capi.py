@@ -38,6 +38,8 @@ SYMBOLS = [
     "psulvsb_match_batch_workspace_bytes", "psulvsb_match_batch", "psulvsb_match_batch_host",
     "psulvsb_gicp", "psulvsb_gicp_host", "psulvsb_gicp_batch_workspace_bytes", "psulvsb_gicp_batch",
     "psulvsb_gicp_batch_host",
+    "psulvsb_normals_workspace_bytes", "psulvsb_normals", "psulvsb_normals_host",
+    "psulvsb_normals_batch_workspace_bytes", "psulvsb_normals_batch", "psulvsb_normals_batch_host",
 ]
 UNIQUE_ID_BYTES = 128
 
@@ -356,6 +358,14 @@ def _declare(L: C.CDLL) -> None:
     L.psulvsb_fpfh_batch_workspace_bytes.restype = _ull
     L.psulvsb_fpfh_batch.argtypes = [_vp, C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_double, _vp, _vp, _vp]
     L.psulvsb_fpfh_batch_host.argtypes = [C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_double, _vp, _vp]
+    L.psulvsb_normals_workspace_bytes.argtypes = [C.c_int]
+    L.psulvsb_normals_workspace_bytes.restype = _ull
+    L.psulvsb_normals.argtypes = [_vp, _vp, C.c_int, C.c_double, C.c_int, C.POINTER(C.c_double), _vp, _vp]
+    L.psulvsb_normals_host.argtypes = [_vp, C.c_int, C.c_double, C.c_int, C.POINTER(C.c_double), _vp]
+    L.psulvsb_normals_batch_workspace_bytes.argtypes = [C.POINTER(FpfhCloud), C.c_int]
+    L.psulvsb_normals_batch_workspace_bytes.restype = _ull
+    L.psulvsb_normals_batch.argtypes = [_vp, C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_int, _vp, _vp]
+    L.psulvsb_normals_batch_host.argtypes = [C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_int, _vp]
     L.psulvsb_match_batch_workspace_bytes.argtypes = [C.POINTER(MatchPair), C.c_int, C.c_int, C.c_int]
     L.psulvsb_match_batch_workspace_bytes.restype = _ull
     L.psulvsb_match_batch.argtypes = [_vp, C.POINTER(MatchPair), C.c_int, C.c_int, C.c_int, C.c_double, _vp, _vp, _vp]

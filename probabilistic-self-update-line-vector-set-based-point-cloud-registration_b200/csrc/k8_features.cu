@@ -141,12 +141,23 @@ __global__ void __launch_bounds__(FT_THREADS)
                                 __int_as_float(j));
 }
 
-// ---- radius normals: FP64 mean and covariance of the r_n neighbourhood, smallest eigenvector, towards the viewpoint
-template <bool kBatch>
+// hybrid normals: candidate j of point p ranks by (FP32 |p_j - p|^2 bits, j); d^2 >= 0, so the bits keep its order
+constexpr int FT_MAX_NN = 32;
+
+__device__ __forceinline__ unsigned long long nn_key(float4 p, float4 q, int j) {
+  return ((unsigned long long)__float_as_uint(sqdist(p, q)) << 32) | (unsigned int)j;
+}
+
+// ---- radius normals: FP64 mean and covariance of the r_n neighbourhood, smallest eigenvector, towards the viewpoint.
+// kCap (hybrid): only the max_nn smallest keys of the neighbourhood count.  A first walk keeps them in shared memory
+// ([slot][thread]: a warp's slot s is 32 consecutive words) and yields the threshold K* = the max_nn-th smallest key
+// (all keys when the neighbourhood is no larger); the mean and covariance walks then skip keys above K*, so the sums
+// run over the kept points in the radius mode's order.
+template <bool kBatch, bool kCap = false>
 __global__ void __launch_bounds__(FT_THREADS)
     k8_radius_normals(const FtCloud* __restrict__ clouds, __grid_constant__ const FtCloud one, const int* __restrict__ tile_first, int B, double inv_h,
                       const float4* __restrict__ spts, const int* __restrict__ start, float rn2,
-                      double* __restrict__ normals, float4* __restrict__ nf) {
+                      double* __restrict__ normals, float4* __restrict__ nf, int max_nn = 0) {
   int ci, first;
   const FtCloud& cl = cloud_tile<kBatch>(clouds, one, tile_first, B, ci, first);
   const int p = first + threadIdx.x;
@@ -155,9 +166,40 @@ __global__ void __launch_bounds__(FT_THREADS)
   const double* pts = cl.pts;
   const float4 me = spts[cl.p0 + p];
   const int i = __float_as_int(me.w);
+  unsigned long long kstar = ~0ull;
+  if constexpr (kCap) {
+    __shared__ unsigned long long kept[FT_MAX_NN][FT_THREADS];
+    const int tid = threadIdx.x;
+    int nk = 0, top = 0;                 // candidates seen; the slot of the largest kept key
+    unsigned long long kmax = 0;
+    for_neighbours(g, me, rn2, [&](float4 q, int j) {
+      const unsigned long long k = nn_key(me, q, j);
+      if (nk < max_nn) {
+        kept[nk][tid] = k;
+        if (k > kmax) {
+          kmax = k;
+          top = nk;
+        }
+      } else if (k < kmax) {             // replace the largest, then find the new largest
+        kept[top][tid] = k;
+        kmax = 0;
+        for (int s = 0; s < max_nn; ++s) {
+          const unsigned long long v = kept[s][tid];
+          if (v > kmax) {
+            kmax = v;
+            top = s;
+          }
+        }
+      }
+      ++nk;
+    });
+    if (nk > max_nn) kstar = kmax;
+  }
   double mean[3] = {0, 0, 0};
   int cnt = 0;
-  for_neighbours(g, me, rn2, [&](float4, int j) {
+  for_neighbours(g, me, rn2, [&](float4 q, int j) {
+    if constexpr (kCap)
+      if (nn_key(me, q, j) > kstar) return;
     for (int r = 0; r < 3; ++r) mean[r] += pts[3 * (size_t)j + r];
     ++cnt;
   });
@@ -167,7 +209,9 @@ __global__ void __launch_bounds__(FT_THREADS)
   } else {
     for (int r = 0; r < 3; ++r) mean[r] /= (double)cnt;
     double cov[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
-    for_neighbours(g, me, rn2, [&](float4, int j) {
+    for_neighbours(g, me, rn2, [&](float4 q, int j) {
+      if constexpr (kCap)
+        if (nn_key(me, q, j) > kstar) return;
       double d[3];
       for (int r = 0; r < 3; ++r) d[r] = pts[3 * (size_t)j + r] - mean[r];
       for (int r = 0; r < 3; ++r)
@@ -657,7 +701,8 @@ struct FpfhWork {
   int* counts;                  // [33 n]
 };
 
-size_t fpfh_layout(const FpfhSizes& z, char* base, FpfhWork* w) {
+// the FPFH workspace; without descriptors (the normals stage alone) counts and kcount take no room
+size_t fpfh_layout(const FpfhSizes& z, char* base, FpfhWork* w, bool descriptors = true) {
   const size_t nn = (size_t)z.n, nb = (size_t)z.nb, B = (size_t)z.B;
   size_t off = 0;
   auto take = [&](size_t bytes) {
@@ -676,8 +721,8 @@ size_t fpfh_layout(const FpfhSizes& z, char* base, FpfhWork* w) {
   v.start = (int*)take(4 * (nb + B));
   v.cursor = (int*)take(4 * nb);
   v.tmp = (int*)take(4 * nn);
-  v.counts = (int*)take(4 * FT_DIM * nn);
-  v.kcount = (int*)take(4 * nn);
+  v.counts = (int*)take(descriptors ? 4 * FT_DIM * nn : 0);
+  v.kcount = (int*)take(descriptors ? 4 * nn : 0);
   if (w) *w = v;
   return off;
 }
@@ -693,28 +738,37 @@ int clouds_check(const psulvsb_fpfh_cloud_t* clouds, int B, const char* who) {
   return PSULVSB_OK;
 }
 
+// features NULL: the normals stage alone, the first five launches (max_nn > 0: the hybrid neighbourhood)
 template <bool kBatch>
 void launch_fpfh(cudaStream_t st, const FpfhWork& w, const FtCloud& one, int B, int tiles, int n, double inv_h, float rn2,
-                 float rf2, double* normals, float* features) {
+                 float rf2, int max_nn, double* normals, float* features) {
   k8_grid_count<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, inv_h, w.pbucket, w.count);
   k8_cloud_scan<kBatch><<<B, SCAN_THREADS, 0, st>>>(w.cloud, one, w.count, w.start, w.cursor);
   k8_grid_scatter<<<blocks(n, GRID_THREADS), GRID_THREADS, 0, st>>>(n, w.pbucket, w.cursor, w.tmp);
   k8_grid_order<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, w.pbucket, w.start, w.tmp, w.spts);
+  if (max_nn > 0) {
+    k8_radius_normals<kBatch, true><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, inv_h, w.spts,
+                                                                  w.start, rn2, normals, w.nf, max_nn);
+    return;
+  }
   k8_radius_normals<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, inv_h, w.spts, w.start, rn2,
                                                           normals, w.nf);
+  if (!features) return;
   k8_spfh<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, inv_h, w.spts, w.start, rf2, w.nf,
                                                 w.counts, w.kcount);
   k8_fpfh<kBatch><<<tiles, FT_THREADS, 0, st>>>(w.cloud, one, w.tile_first, B, inv_h, w.spts, w.start, rf2, w.counts,
                                                 w.kcount, features);
 }
 
-// the batch on the device (clouds checked, B >= 1): one upload of the cloud table, then seven launches over all clouds
-int run_fpfh(cudaStream_t st, const psulvsb_fpfh_cloud_t* clouds, int B, double rn, double rf, void* work,
+// the batch on the device (clouds checked, B >= 1): one upload of the cloud table, then seven launches over all clouds.
+// features NULL: the normals stage alone on the grid of cell size r_n (FPFH's grid whenever r_f <= r_n), five
+// launches; max_nn: 0 for the radius neighbourhood, else the hybrid cap (normals only)
+int run_fpfh(cudaStream_t st, const psulvsb_fpfh_cloud_t* clouds, int B, double rn, double rf, int max_nn, void* work,
              double* normals, float* features) {
   const FpfhSizes z = fpfh_sizes(clouds, B);
   if (z.tiles == 0) return PSULVSB_OK;
   FpfhWork w;
-  fpfh_layout(z, static_cast<char*>(work), &w);
+  fpfh_layout(z, static_cast<char*>(work), &w, features != nullptr);
   std::vector<char> table(w.table_bytes);
   FtCloud* hc = reinterpret_cast<FtCloud*>(table.data());
   int* tile_first = reinterpret_cast<int*>(table.data() + sizeof(FtCloud) * (size_t)B);
@@ -740,24 +794,25 @@ int run_fpfh(cudaStream_t st, const psulvsb_fpfh_cloud_t* clouds, int B, double 
   const float rn2 = (float)(rn * rn), rf2 = (float)(rf * rf);
   PSU_CUDA(cudaMemsetAsync(w.count, 0, 4 * (size_t)z.nb, st));
   if (B == 1)
-    launch_fpfh<false>(st, w, hc[0], 1, tiles, n, inv_h, rn2, rf2, normals, features);
+    launch_fpfh<false>(st, w, hc[0], 1, tiles, n, inv_h, rn2, rf2, max_nn, normals, features);
   else
-    launch_fpfh<true>(st, w, hc[0], B, tiles, n, inv_h, rn2, rf2, normals, features);
-  PSU_CHECK_LAUNCH("k8_fpfh");
+    launch_fpfh<true>(st, w, hc[0], B, tiles, n, inv_h, rn2, rf2, max_nn, normals, features);
+  PSU_CHECK_LAUNCH(features ? "k8_fpfh" : "k8_radius_normals");
   return PSULVSB_OK;
 }
 
-// the batch on host buffers (clouds checked, B >= 1): the clouds go up in one copy, features and normals come back
-int run_fpfh_host(const psulvsb_fpfh_cloud_t* clouds, int B, double rn, double rf, double* normals, float* features,
-                  const char* who) {
+// the batch on host buffers (clouds checked, B >= 1): the clouds go up in one copy, features and normals come back.
+// features NULL: the normals stage alone (as run_fpfh)
+int run_fpfh_host(const psulvsb_fpfh_cloud_t* clouds, int B, double rn, double rf, int max_nn, double* normals,
+                  float* features, const char* who) {
   const FpfhSizes z = fpfh_sizes(clouds, B);
   if (z.n == 0) return PSULVSB_OK;
-  const size_t N = (size_t)z.n, o_n = up256(4 * FT_DIM * N), o_in = o_n + up256(normals ? 24 * N : 0),
-               o_w = o_in + up256(24 * N);
+  const size_t N = (size_t)z.n, o_n = up256(features ? 4 * FT_DIM * N : 0),
+               o_in = o_n + up256(normals ? 24 * N : 0), o_w = o_in + up256(24 * N);
   std::vector<char> in(B > 1 ? 24 * N : 0);
   std::vector<psulvsb_fpfh_cloud_t> dev(clouds, clouds + B);
   DevBuf buf;
-  if (int rc = buf.alloc(o_w + fpfh_layout(z, nullptr, nullptr), who)) return rc;
+  if (int rc = buf.alloc(o_w + fpfh_layout(z, nullptr, nullptr, features != nullptr), who)) return rc;
   char* b = static_cast<char*>(buf.p);
   // a single cloud goes up straight from the caller's buffer: packing it first would only add a host copy
   size_t off = 0;
@@ -770,9 +825,10 @@ int run_fpfh_host(const psulvsb_fpfh_cloud_t* clouds, int B, double rn, double r
   }
   PSU_CUDA(cudaMemcpyAsync(b + o_in, B > 1 ? in.data() : (const void*)clouds[0].pts, 24 * N, cudaMemcpyHostToDevice,
                            nullptr));
-  if (int rc = run_fpfh(nullptr, dev.data(), B, rn, rf, b + o_w, normals ? (double*)(b + o_n) : nullptr, (float*)b))
+  if (int rc = run_fpfh(nullptr, dev.data(), B, rn, rf, max_nn, b + o_w, normals ? (double*)(b + o_n) : nullptr,
+                        features ? (float*)b : nullptr))
     return rc;
-  PSU_CUDA(cudaMemcpyAsync(features, b, 4 * FT_DIM * N, cudaMemcpyDeviceToHost, nullptr));
+  if (features) PSU_CUDA(cudaMemcpyAsync(features, b, 4 * FT_DIM * N, cudaMemcpyDeviceToHost, nullptr));
   if (normals) PSU_CUDA(cudaMemcpyAsync(normals, b + o_n, 24 * N, cudaMemcpyDeviceToHost, nullptr));
   PSU_CUDA(cudaStreamSynchronize(nullptr));
   return PSULVSB_OK;
@@ -1045,7 +1101,8 @@ int psulvsb_fpfh(void* stream, const double* d_pts, int n, double normal_radius,
     return fail(PSULVSB_ERR_INVALID, "psulvsb_fpfh: bad argument (radii must be finite and > 0)");
   if (int rc = psulvsb::need_device()) return rc;
   const psulvsb_fpfh_cloud_t c = one_cloud(d_pts, n, viewpoint);
-  return psulvsb::run_fpfh((cudaStream_t)stream, &c, 1, normal_radius, feature_radius, d_work, d_normals, d_features);
+  return psulvsb::run_fpfh((cudaStream_t)stream, &c, 1, normal_radius, feature_radius, 0, d_work, d_normals,
+                           d_features);
 }
 
 int psulvsb_fpfh_host(const double* pts, int n, double normal_radius, double feature_radius, const double viewpoint[3],
@@ -1055,7 +1112,7 @@ int psulvsb_fpfh_host(const double* pts, int n, double normal_radius, double fea
     return fail(PSULVSB_ERR_INVALID, "psulvsb_fpfh_host: bad argument (radii must be finite and > 0)");
   if (int rc = psulvsb::need_device()) return rc;
   const psulvsb_fpfh_cloud_t c = one_cloud(pts, n, viewpoint);
-  return psulvsb::run_fpfh_host(&c, 1, normal_radius, feature_radius, normals, features, "psulvsb_fpfh_host");
+  return psulvsb::run_fpfh_host(&c, 1, normal_radius, feature_radius, 0, normals, features, "psulvsb_fpfh_host");
 }
 
 int psulvsb_fpfh_batch(void* stream, const psulvsb_fpfh_cloud_t* clouds, int B, double normal_radius,
@@ -1066,7 +1123,7 @@ int psulvsb_fpfh_batch(void* stream, const psulvsb_fpfh_cloud_t* clouds, int B, 
   if (int rc = psulvsb::clouds_check(clouds, B, "psulvsb_fpfh_batch")) return rc;
   if (B == 0) return PSULVSB_OK;
   if (int rc = psulvsb::need_device()) return rc;
-  return psulvsb::run_fpfh((cudaStream_t)stream, clouds, B, normal_radius, feature_radius, d_work, d_normals,
+  return psulvsb::run_fpfh((cudaStream_t)stream, clouds, B, normal_radius, feature_radius, 0, d_work, d_normals,
                            d_features);
 }
 
@@ -1078,7 +1135,65 @@ int psulvsb_fpfh_batch_host(const psulvsb_fpfh_cloud_t* clouds, int B, double no
   if (int rc = psulvsb::clouds_check(clouds, B, "psulvsb_fpfh_batch_host")) return rc;
   if (B == 0) return PSULVSB_OK;
   if (int rc = psulvsb::need_device()) return rc;
-  return psulvsb::run_fpfh_host(clouds, B, normal_radius, feature_radius, normals, features, "psulvsb_fpfh_batch_host");
+  return psulvsb::run_fpfh_host(clouds, B, normal_radius, feature_radius, 0, normals, features,
+                                "psulvsb_fpfh_batch_host");
+}
+
+// ---- normals alone (DESIGN.md section 10, "Normals alone"): FPFH's grid and normals kernel, nothing after them
+static bool max_nn_ok(int max_nn) { return max_nn == 0 || (max_nn >= 3 && max_nn <= psulvsb::FT_MAX_NN); }
+
+unsigned long long psulvsb_normals_workspace_bytes(int n) {
+  if (n < 0) return 0ull;
+  const psulvsb_fpfh_cloud_t c{nullptr, n, {0.0, 0.0, 0.0}};
+  return (unsigned long long)psulvsb::fpfh_layout(psulvsb::fpfh_sizes(&c, 1), nullptr, nullptr, false);
+}
+
+unsigned long long psulvsb_normals_batch_workspace_bytes(const psulvsb_fpfh_cloud_t* clouds, int B) {
+  if (B <= 0 || !clouds) return 0ull;
+  for (int c = 0; c < B; ++c)
+    if (clouds[c].n < 0) return 0ull;
+  return (unsigned long long)psulvsb::fpfh_layout(psulvsb::fpfh_sizes(clouds, B), nullptr, nullptr, false);
+}
+
+int psulvsb_normals(void* stream, const double* d_pts, int n, double radius, int max_nn, const double viewpoint[3],
+                    void* d_work, double* d_normals) {
+  if (n < 0 || !psulvsb::radius_ok(radius) || !max_nn_ok(max_nn) || (n > 0 && (!d_pts || !d_work || !d_normals)))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_normals: bad argument (radius finite and > 0, max_nn 0 or 3..32)");
+  const psulvsb_fpfh_cloud_t c = one_cloud(d_pts, n, viewpoint);
+  if (int rc = psulvsb::clouds_check(&c, 1, "psulvsb_normals")) return rc;
+  if (int rc = psulvsb::need_device()) return rc;
+  return psulvsb::run_fpfh((cudaStream_t)stream, &c, 1, radius, radius, max_nn, d_work, d_normals, nullptr);
+}
+
+int psulvsb_normals_host(const double* pts, int n, double radius, int max_nn, const double viewpoint[3],
+                         double* normals) {
+  if (n < 0 || !psulvsb::radius_ok(radius) || !max_nn_ok(max_nn) || (n > 0 && (!pts || !normals)))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_normals_host: bad argument (radius finite and > 0, max_nn 0 or 3..32)");
+  const psulvsb_fpfh_cloud_t c = one_cloud(pts, n, viewpoint);
+  if (int rc = psulvsb::clouds_check(&c, 1, "psulvsb_normals_host")) return rc;
+  if (int rc = psulvsb::need_device()) return rc;
+  return psulvsb::run_fpfh_host(&c, 1, radius, radius, max_nn, normals, nullptr, "psulvsb_normals_host");
+}
+
+int psulvsb_normals_batch(void* stream, const psulvsb_fpfh_cloud_t* clouds, int B, double radius, int max_nn,
+                          void* d_work, double* d_normals) {
+  if (B < 0 || !psulvsb::radius_ok(radius) || !max_nn_ok(max_nn) || (B > 0 && (!clouds || !d_work || !d_normals)))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_normals_batch: bad argument (radius finite and > 0, max_nn 0 or 3..32)");
+  if (int rc = psulvsb::clouds_check(clouds, B, "psulvsb_normals_batch")) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = psulvsb::need_device()) return rc;
+  return psulvsb::run_fpfh((cudaStream_t)stream, clouds, B, radius, radius, max_nn, d_work, d_normals, nullptr);
+}
+
+int psulvsb_normals_batch_host(const psulvsb_fpfh_cloud_t* clouds, int B, double radius, int max_nn,
+                               double* normals) {
+  if (B < 0 || !psulvsb::radius_ok(radius) || !max_nn_ok(max_nn) || (B > 0 && (!clouds || !normals)))
+    return fail(PSULVSB_ERR_INVALID,
+                "psulvsb_normals_batch_host: bad argument (radius finite and > 0, max_nn 0 or 3..32)");
+  if (int rc = psulvsb::clouds_check(clouds, B, "psulvsb_normals_batch_host")) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = psulvsb::need_device()) return rc;
+  return psulvsb::run_fpfh_host(clouds, B, radius, radius, max_nn, normals, nullptr, "psulvsb_normals_batch_host");
 }
 
 int psulvsb_feature_nn(void* stream, const float* d_fs, int n_src, const float* d_ft, int n_tgt, int* d_nn_src_to_tgt,

@@ -1,9 +1,10 @@
-"""Correspondences from two raw clouds: FPFH descriptors, the two-way descriptor nearest neighbour and FGR's matcher.
+"""Correspondences from two raw clouds: FPFH descriptors, the two-way descriptor nearest neighbour and FGR's matcher;
+and surface normals alone (radius or hybrid neighbourhood) on the same grid.
 
 What upstream TEASER++ gets from teaser::FPFHEstimation and teaser::Matcher (over PCL and FLANN), on the GPU through
 the C ABI (include/psulvsb.h, csrc/k8_features.cu).  Host arrays in, host arrays out, except fpfh_device /
-nearest_neighbours_device / fpfh_batch_device / match_batch_device, which take and return CUDA tensors on the current
-stream.  The _batch functions compute B clouds or B pairs in one call; each item's result is bit-identical to the
+nearest_neighbours_device / fpfh_batch_device / match_batch_device / normals_device / normals_batch_device, which take
+and return CUDA tensors on the current stream.  The _batch functions compute B clouds or B pairs in one call; each item's result is bit-identical to the
 single call on it alone.
 """
 from __future__ import annotations
@@ -163,6 +164,81 @@ def fpfh_batch_device(d_clouds, normal_radius: float, feature_radius: float, vie
         views.append((feats[o:o + n], normals[o:o + n]))
         o += n
     return feats[:N], normals[:N], views
+
+
+def normals(points, radius: float, max_nn: int = 0, viewpoint=(0.0, 0.0, 0.0)) -> np.ndarray:
+    """psulvsb_normals_host: 3xN points -> 3xN float64 normals (NaN below 3 neighbours), flipped towards `viewpoint`.
+    max_nn = 0: every point within `radius` (the normals of `fpfh` with normal_radius = radius, bit for bit); 3 ... 32:
+    the max_nn nearest of them (Open3D's KDTreeSearchParamHybrid(radius, max_nn)), ties to the lower index."""
+    p = _cm(points)
+    n = p.shape[1]
+    out = np.zeros((3, n), dtype=np.float64, order="F")
+    capi.check(capi.lib().psulvsb_normals_host(p.ctypes.data, n, float(radius), int(max_nn), _vp(viewpoint),
+                                               out.ctypes.data))
+    return out
+
+
+def normals_device(d_pts, radius: float, max_nn: int = 0, viewpoint=(0.0, 0.0, 0.0), work=None):
+    """psulvsb_normals on a CUDA tensor [N, 3] float64 (== column-major 3xN) and the current stream: normals [N, 3].
+    `work`: an optional uint8 CUDA tensor of at least psulvsb_normals_workspace_bytes(N) bytes to reuse."""
+    import torch
+
+    from .stages import _dev, _stream
+
+    n = d_pts.shape[0]
+    nbytes = capi.lib().psulvsb_normals_workspace_bytes(n)
+    if work is None:
+        work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=d_pts.device)
+    elif work.numel() < nbytes:
+        raise ValueError("work is smaller than psulvsb_normals_workspace_bytes(n)")
+    out = torch.empty((max(n, 1), 3), dtype=torch.float64, device=d_pts.device)
+    capi.check(capi.lib().psulvsb_normals(_stream(), _dev(d_pts) if n else None, n, float(radius), int(max_nn),
+                                          _vp(viewpoint), _dev(work), _dev(out)))
+    return out[:n]
+
+
+def normals_batch(clouds, radius: float, max_nn: int = 0, viewpoints=None) -> list:
+    """psulvsb_normals_batch_host: B clouds (3 x n_c each) with a shared radius and max_nn in one call.  Returns one
+    3 x n_c float64 normal array per cloud, each equal bit for bit to `normals` on that cloud alone."""
+    ps = [_cm(p) for p in clouds]
+    B = len(ps)
+    sizes = [p.shape[1] for p in ps]
+    arr = _clouds([p.ctypes.data if p.shape[1] else None for p in ps], sizes, _viewpoints(viewpoints, B))
+    out = np.zeros((max(sum(sizes), 1), 3), dtype=np.float64)
+    capi.check(capi.lib().psulvsb_normals_batch_host(arr, B, float(radius), int(max_nn), out.ctypes.data))
+    res, o = [], 0
+    for n in sizes:
+        res.append(np.asfortranarray(out[o:o + n].T))
+        o += n
+    return res
+
+
+def normals_batch_device(d_clouds, radius: float, max_nn: int = 0, viewpoints=None, work=None):
+    """psulvsb_normals_batch on CUDA tensors [n_c, 3] float64 and the current stream.  Returns (normals [sum n, 3],
+    views): views[c] = cloud c's rows.  `work`: an optional uint8 CUDA tensor of at least
+    psulvsb_normals_batch_workspace_bytes bytes to reuse."""
+    import torch
+
+    from .stages import _dev, _stream
+
+    B = len(d_clouds)
+    sizes = [int(p.shape[0]) for p in d_clouds]
+    arr = _clouds([_dev(p) if n else None for p, n in zip(d_clouds, sizes)], sizes, _viewpoints(viewpoints, B))
+    L = capi.lib()
+    dev = d_clouds[0].device if B else torch.device("cuda")
+    nbytes = L.psulvsb_normals_batch_workspace_bytes(arr, B)
+    if work is None:
+        work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=dev)
+    elif work.numel() < nbytes:
+        raise ValueError("work is smaller than psulvsb_normals_batch_workspace_bytes(clouds, B)")
+    N = sum(sizes)
+    out = torch.empty((max(N, 1), 3), dtype=torch.float64, device=dev)
+    capi.check(L.psulvsb_normals_batch(_stream(), arr, B, float(radius), int(max_nn), _dev(work), _dev(out)))
+    views, o = [], 0
+    for n in sizes:
+        views.append(out[o:o + n])
+        o += n
+    return out[:N], views
 
 
 def match_caps(n_srcs, n_tgts, crosscheck: bool = True, tuple_test: bool = False) -> list:

@@ -7,6 +7,7 @@ tensors [N, 3] float64 (== column-major 3xN) and runs on the current stream.  `i
 B independent pairs with shared parameters in one call; pair b's result is bit-identical to `icp` on that pair alone.
 `gicp`, `gicp_device`, `gicp_batch` and `gicp_batch_device` are the same four calls with generalized ICP's update
 (plane-to-plane; Open3D's registration_generalized_icp); they need the normals of both clouds, for instance the radius
+or hybrid normals of `features.normals` / `features.normals_batch` (on the grid, without descriptors), the radius
 normals `features.fpfh` returns or the k-NN normals of `stages.estimate_normals`.
 Convention: q ~ R p + t.
 """
