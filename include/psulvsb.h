@@ -430,6 +430,35 @@ int psulvsb_normals_batch(void* stream, const psulvsb_fpfh_cloud_t* clouds, int 
 int psulvsb_normals_batch_host(const psulvsb_fpfh_cloud_t* clouds, int B, double radius, int max_nn,
                                double* normals);
 
+/* ---- Voxel downsampling (DESIGN.md section 10, "Voxel downsampling"): Open3D's PointCloud::VoxelDownSample on the
+ * GPU.  Points and voxels are column-major 3xn doubles.  A point with a non-finite coordinate is dropped; lo = the
+ * minimum of the finite points per coordinate, origin = lo - voxel_size * 0.5, and a point's cell is
+ * floor((p - origin) / voxel_size) per coordinate in FP64, converted to int64 with saturation.  Two points share a
+ * voxel iff their three cells are equal.  Each voxel gives the mean of its members (FP64 sums in ascending input
+ * index, then one division by the count); voxels come out in ascending order of their lowest input index, so a cloud
+ * with at most one point per voxel comes back in input order.  Results are bit-identical from call to call.
+ * Capacity = input size: d_out holds 3 x n doubles, of which the first *d_count columns are voxels (the rest is
+ * unspecified).  d_work: psulvsb_voxel_down_sample_workspace_bytes(n) bytes of device scratch (depends on n only; 0
+ * for n < 0).  The device variants are asynchronous on `stream` and leave the count on the device.
+ * PSULVSB_ERR_INVALID before any device work for a voxel_size that is not finite and > 0, a negative size, a NULL
+ * points pointer of a non-empty cloud, a required NULL output or B < 0; PSULVSB_ERR_UNSUPPORTED when the sizes add up
+ * to 2^31 or more (the FPFH batch's rule).  n = 0 or B = 0 does nothing beyond writing zero counts: the _host
+ * variants write them on the host and need no device when every cloud is empty; the device variants write them on the
+ * device, so an empty single call still needs one (B = 0 writes nothing and needs none).  Batch: items are
+ * psulvsb_fpfh_cloud_t (the viewpoint is ignored); cloud c's voxels are columns [sum_{a<c} n_a, ... + counts[c]) of
+ * the 3 x (sum n) doubles, bit-identical to the single call on cloud c alone.  The _host variants take host buffers
+ * and are synchronous. */
+unsigned long long psulvsb_voxel_down_sample_workspace_bytes(int n);
+int psulvsb_voxel_down_sample(void* stream, const double* d_pts, int n, double voxel_size, void* d_work,
+                              double* d_out /* 3 x n capacity */, int* d_count);
+int psulvsb_voxel_down_sample_host(const double* pts, int n, double voxel_size, double* out /* 3 x n */, int* n_out);
+/* Device scratch of psulvsb_voxel_down_sample_batch (depends on the sizes only); 0 for B <= 0 or a negative size. */
+unsigned long long psulvsb_voxel_down_sample_batch_workspace_bytes(const psulvsb_fpfh_cloud_t* clouds, int B);
+int psulvsb_voxel_down_sample_batch(void* stream, const psulvsb_fpfh_cloud_t* clouds, int B, double voxel_size,
+                                    void* d_work, double* d_out, int* d_counts);
+int psulvsb_voxel_down_sample_batch_host(const psulvsb_fpfh_cloud_t* clouds, int B, double voxel_size,
+                                         double* out, int* counts);
+
 typedef struct psulvsb_match_pair {
   const double* src;  /* 3 x n_src, column-major: the tuple test's points                                 */
   int n_src;

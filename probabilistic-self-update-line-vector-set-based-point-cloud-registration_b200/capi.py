@@ -40,6 +40,9 @@ SYMBOLS = [
     "psulvsb_gicp_batch_host",
     "psulvsb_normals_workspace_bytes", "psulvsb_normals", "psulvsb_normals_host",
     "psulvsb_normals_batch_workspace_bytes", "psulvsb_normals_batch", "psulvsb_normals_batch_host",
+    "psulvsb_voxel_down_sample_workspace_bytes", "psulvsb_voxel_down_sample", "psulvsb_voxel_down_sample_host",
+    "psulvsb_voxel_down_sample_batch_workspace_bytes", "psulvsb_voxel_down_sample_batch",
+    "psulvsb_voxel_down_sample_batch_host",
 ]
 UNIQUE_ID_BYTES = 128
 
@@ -366,6 +369,14 @@ def _declare(L: C.CDLL) -> None:
     L.psulvsb_normals_batch_workspace_bytes.restype = _ull
     L.psulvsb_normals_batch.argtypes = [_vp, C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_int, _vp, _vp]
     L.psulvsb_normals_batch_host.argtypes = [C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_int, _vp]
+    L.psulvsb_voxel_down_sample_workspace_bytes.argtypes = [C.c_int]
+    L.psulvsb_voxel_down_sample_workspace_bytes.restype = _ull
+    L.psulvsb_voxel_down_sample.argtypes = [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp]
+    L.psulvsb_voxel_down_sample_host.argtypes = [_vp, C.c_int, C.c_double, _vp, _vp]
+    L.psulvsb_voxel_down_sample_batch_workspace_bytes.argtypes = [C.POINTER(FpfhCloud), C.c_int]
+    L.psulvsb_voxel_down_sample_batch_workspace_bytes.restype = _ull
+    L.psulvsb_voxel_down_sample_batch.argtypes = [_vp, C.POINTER(FpfhCloud), C.c_int, C.c_double, _vp, _vp, _vp]
+    L.psulvsb_voxel_down_sample_batch_host.argtypes = [C.POINTER(FpfhCloud), C.c_int, C.c_double, _vp, _vp]
     L.psulvsb_match_batch_workspace_bytes.argtypes = [C.POINTER(MatchPair), C.c_int, C.c_int, C.c_int]
     L.psulvsb_match_batch_workspace_bytes.restype = _ull
     L.psulvsb_match_batch.argtypes = [_vp, C.POINTER(MatchPair), C.c_int, C.c_int, C.c_int, C.c_double, _vp, _vp, _vp]

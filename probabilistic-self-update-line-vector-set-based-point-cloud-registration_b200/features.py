@@ -1,11 +1,12 @@
 """Correspondences from two raw clouds: FPFH descriptors, the two-way descriptor nearest neighbour and FGR's matcher;
-and surface normals alone (radius or hybrid neighbourhood) on the same grid.
+surface normals alone (radius or hybrid neighbourhood) on the same grid; and the voxel-grid filter that comes first.
 
 What upstream TEASER++ gets from teaser::FPFHEstimation and teaser::Matcher (over PCL and FLANN), on the GPU through
 the C ABI (include/psulvsb.h, csrc/k8_features.cu).  Host arrays in, host arrays out, except fpfh_device /
-nearest_neighbours_device / fpfh_batch_device / match_batch_device / normals_device / normals_batch_device, which take
-and return CUDA tensors on the current stream.  The _batch functions compute B clouds or B pairs in one call; each item's result is bit-identical to the
-single call on it alone.
+nearest_neighbours_device / fpfh_batch_device / match_batch_device / normals_device / normals_batch_device /
+voxel_down_sample_device / voxel_down_sample_batch_device, which take and return CUDA tensors on the current stream.
+The _batch functions compute B clouds or B pairs in one call; each item's result is bit-identical to the single call
+on it alone.
 """
 from __future__ import annotations
 
@@ -239,6 +240,86 @@ def normals_batch_device(d_clouds, radius: float, max_nn: int = 0, viewpoints=No
         views.append(out[o:o + n])
         o += n
     return out[:N], views
+
+
+def voxel_down_sample(points, voxel_size: float) -> np.ndarray:
+    """psulvsb_voxel_down_sample_host (Open3D's voxel_down_sample): 3xN points -> 3xM float64 voxel means, in ascending
+    order of each voxel's lowest input index.  Points with a non-finite coordinate are dropped."""
+    p = _cm(points)
+    n = p.shape[1]
+    out = np.zeros((3, max(n, 1)), dtype=np.float64, order="F")
+    m = C.c_int(0)
+    capi.check(capi.lib().psulvsb_voxel_down_sample_host(p.ctypes.data if n else None, n, float(voxel_size),
+                                                         out.ctypes.data, C.byref(m)))
+    return out[:, :m.value].copy(order="F")
+
+
+def voxel_down_sample_device(d_pts, voxel_size: float, work=None):
+    """psulvsb_voxel_down_sample on a CUDA tensor [N, 3] float64 (== column-major 3xN) and the current stream, without
+    a host round trip.  Returns (voxels [N, 3], count [1] int32): the first count[0] rows are the voxels, the rest is
+    unspecified.  `work`: an optional uint8 CUDA tensor of at least psulvsb_voxel_down_sample_workspace_bytes(N) bytes
+    to reuse."""
+    import torch
+
+    from .stages import _dev, _stream
+
+    n = d_pts.shape[0]
+    nbytes = capi.lib().psulvsb_voxel_down_sample_workspace_bytes(n)
+    if work is None:
+        work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=d_pts.device)
+    elif work.numel() < nbytes:
+        raise ValueError("work is smaller than psulvsb_voxel_down_sample_workspace_bytes(n)")
+    out = torch.empty((max(n, 1), 3), dtype=torch.float64, device=d_pts.device)
+    count = torch.empty(1, dtype=torch.int32, device=d_pts.device)
+    capi.check(capi.lib().psulvsb_voxel_down_sample(_stream(), _dev(d_pts) if n else None, n, float(voxel_size),
+                                                    _dev(work), _dev(out), _dev(count)))
+    return out[:n], count
+
+
+def voxel_down_sample_batch(clouds, voxel_size: float) -> list:
+    """psulvsb_voxel_down_sample_batch_host: B clouds (3 x n_c each) with a shared voxel size in one call.  Returns one
+    3 x m_c float64 array per cloud, each equal bit for bit to `voxel_down_sample` on that cloud alone."""
+    ps = [_cm(p) for p in clouds]
+    B = len(ps)
+    sizes = [p.shape[1] for p in ps]
+    arr = _clouds([p.ctypes.data if p.shape[1] else None for p in ps], sizes, _viewpoints(None, B))
+    out = np.zeros((max(sum(sizes), 1), 3), dtype=np.float64)
+    counts = np.zeros(max(B, 1), dtype=np.int32)
+    capi.check(capi.lib().psulvsb_voxel_down_sample_batch_host(arr, B, float(voxel_size), out.ctypes.data,
+                                                               counts.ctypes.data))
+    res, o = [], 0
+    for c, n in enumerate(sizes):
+        res.append(np.asfortranarray(out[o:o + int(counts[c])].T))
+        o += n
+    return res
+
+
+def voxel_down_sample_batch_device(d_clouds, voxel_size: float, work=None):
+    """psulvsb_voxel_down_sample_batch on CUDA tensors [n_c, 3] float64 and the current stream, without a host round
+    trip.  Returns (voxels [sum n, 3] float64, counts [B] int32, offsets): cloud c's voxels are
+    voxels[offsets[c]:offsets[c] + counts[c]], offsets[c] = sum of the sizes before it.  `work`: an optional uint8 CUDA
+    tensor of at least psulvsb_voxel_down_sample_batch_workspace_bytes bytes to reuse."""
+    import torch
+
+    from .stages import _dev, _stream
+
+    B = len(d_clouds)
+    sizes = [int(p.shape[0]) for p in d_clouds]
+    arr = _clouds([_dev(p) if n else None for p, n in zip(d_clouds, sizes)], sizes, _viewpoints(None, B))
+    L = capi.lib()
+    dev = d_clouds[0].device if B else torch.device("cuda")
+    nbytes = L.psulvsb_voxel_down_sample_batch_workspace_bytes(arr, B)
+    if work is None:
+        work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=dev)
+    elif work.numel() < nbytes:
+        raise ValueError("work is smaller than psulvsb_voxel_down_sample_batch_workspace_bytes(clouds, B)")
+    offsets = np.concatenate([[0], np.cumsum(sizes, dtype=np.int64)]).astype(np.int64)
+    N = int(offsets[-1])
+    out = torch.empty((max(N, 1), 3), dtype=torch.float64, device=dev)
+    counts = torch.empty(max(B, 1), dtype=torch.int32, device=dev)
+    capi.check(L.psulvsb_voxel_down_sample_batch(_stream(), arr, B, float(voxel_size), _dev(work), _dev(out),
+                                                 _dev(counts)))
+    return out[:N], counts[:B], offsets[:B]
 
 
 def match_caps(n_srcs, n_tgts, crosscheck: bool = True, tuple_test: bool = False) -> list:
