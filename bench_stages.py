@@ -33,7 +33,7 @@ def main():
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--debug", action="append", default=[], metavar="NAME=VALUE",
-                    help="psulvsb_debug_set switch (equivalent code paths, e.g. k4_variant=1); repeatable")
+                    help="psulvsb_debug_set switch (equivalent code paths, e.g. edge_wide=1); repeatable")
     args = ap.parse_args()
 
     import torch

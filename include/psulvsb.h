@@ -164,11 +164,9 @@ int psulvsb_set_batching(psulvsb_handle_t h, int chunk, int lanes);
  * the process (its affinity mask).  On a multi-GPU node give every rank its share (cores / ranks). */
 int psulvsb_set_host_threads(psulvsb_handle_t h, int n);
 /* Debug / test switches (process-wide; the library reads NO environment variable).  They select among code paths
- * that produce identical results: "gnc_deep_margin" (rad), "gnc_prefetch", "gnc_cluster" (1 / 2 / 4 / 8 CTAs per
- * registration), "gnc_cps", "gnc_park_pct", "gnc_grid_lv" (line vectors per CTA above which GNC-TLS spreads one
- * registration over the grid), "sample_list_cap_test", "k1_variant" (1..4 rows per thread), "upload_prof" (1: phase
- * timings on stderr), "edge_wide" (1: 8-byte reduced-set edges even where 4-byte ones fit), "reset" (all back to
- * defaults). */
+ * that produce identical results: "gnc_deep_margin" (rad), "sample_list_cap_test", "k1_variant" (1 / 2 / 4 rows per
+ * thread, 0 = automatic; any other value is refused), "edge_wide" (1: 8-byte reduced-set edges even where 4-byte ones
+ * fit), "reset" (all back to defaults).  An unknown name is refused with PSULVSB_ERR_INVALID. */
 int psulvsb_debug_set(const char* name, double value);
 int psulvsb_destroy(psulvsb_handle_t h);
 

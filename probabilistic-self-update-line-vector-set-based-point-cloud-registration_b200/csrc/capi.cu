@@ -190,15 +190,12 @@ int psulvsb_debug_set(const char* name, double value) {
   DebugKnobs& k = debug_knobs();
   const std::string n(name);
   if (n == "gnc_deep_margin") k.gnc_deep_margin = value;
-  else if (n == "gnc_prefetch") k.gnc_prefetch = (int)value;
-  else if (n == "gnc_cluster") k.gnc_cluster = (int)value;
-  else if (n == "gnc_park_pct") k.gnc_park_pct = (int)value;
-  else if (n == "gnc_cps") k.gnc_cps = (int)value;
-  else if (n == "gnc_grid_lv") k.gnc_grid_lv = (int)value;
   else if (n == "sample_list_cap_test") k.sample_list_cap_test = (int)value;
-  else if (n == "k1_variant") k.k1_variant = (int)value;
-  else if (n == "upload_prof") k.upload_prof = (int)value;
-  else if (n == "edge_wide") k.edge_wide = (int)value;
+  else if (n == "k1_variant") {
+    if (value != 0 && value != 1 && value != 2 && value != 4)
+      return fail(PSULVSB_ERR_INVALID, "psulvsb_debug_set: k1_variant must be 0 (automatic), 1, 2 or 4");
+    k.k1_variant = (int)value;
+  } else if (n == "edge_wide") k.edge_wide = (int)value;
   else if (n == "reset") k = DebugKnobs();
   else return fail(PSULVSB_ERR_INVALID, "psulvsb_debug_set: unknown switch " + n);
   return PSULVSB_OK;

@@ -43,14 +43,8 @@ int sm_count();
 // equivalent code paths runs; production callers leave them alone.  No environment variable is read anywhere.
 struct DebugKnobs {
   double gnc_deep_margin = 0.0;   // > 0: overrides the remaining-margin threshold (rad) for parking sleeping line vectors
-  int gnc_cluster = 0;            // 1, 2, 4, 8: CTAs per registration of the GNC-TLS kernel (512 threads, one CTA per SM)
-  int gnc_prefetch = -1;          // >= 0: look-ahead (double-steps) of the L2 prefetch in the streamed GNC pass
-  int gnc_grid_lv = 0;            // > 0: line vectors per CTA above which GNC-TLS goes to grid mode (default 4096)
-  int gnc_cps = 0;                // 1, 2, 4: CTAs per SM (512 / 256 / 128 threads) of one-CTA-per-registration GNC-TLS launches
-  int gnc_park_pct = 0;           // > 0: share (%) of deep sleepers that arms a parking pass of the GNC-TLS kernel
   int sample_list_cap_test = 0;   // > 0: caps the sampler's bucket lists and its on-chip duplicate table (exercises both fallbacks)
-  int k1_variant = 0;             // 1..4: rows per thread of the consistency kernel
-  int upload_prof = 0;            // 1: print the upload's phase timings to stderr
+  int k1_variant = 0;             // 1, 2, 4: rows per thread of the consistency kernel
   int edge_wide = 0;              // 1: the engine keeps the reduced set in EdgeWide format whatever the working-set size
 };
 DebugKnobs& debug_knobs();

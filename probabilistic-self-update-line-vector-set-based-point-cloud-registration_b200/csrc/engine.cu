@@ -271,10 +271,6 @@ int Engine::upload(const psulvsb_problem_t* problems, int nb) {
   // size paired with a half-overwritten layout / input arena)
   B = 0;
   reserve.clear();
-  const bool prof = debug_knobs().upload_prof != 0;
-  const auto t_up0 = std::chrono::steady_clock::now();
-  auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_up0).count(); };
-  double t_layout = 0, t_staged = 0;
   PSU_CUDA(cudaSetDevice(device));
   lay.assign((size_t)nb, ProbLayout());
   size_t od = 0, oi = 0;
@@ -305,7 +301,6 @@ int Engine::upload(const psulvsb_problem_t* problems, int nb) {
   int* hi = reinterpret_cast<int*>(reinterpret_cast<char*>(h_stage.p) + align_up(bytes_d, 256));
   // staging copy + centres / coordinate bound of the FP32 tiles, split over a few host threads (33 MB for a
   // batch of 64 cfg-A pairs: a single-threaded memcpy would cost more than the H2D copy that follows)
-  t_layout = since();
   std::atomic<int> bad_problem(-1), bad_map(-1), copy_error(0);
   // a staged group of problems goes to the device at once (its H2D copy overlaps the staging of the next group)
   auto push_group = [&](int g0, int g1) {
@@ -396,16 +391,9 @@ int Engine::upload(const psulvsb_problem_t* problems, int nb) {
       for (auto& th : pool) th.join();
     }
   }
-  t_staged = since();
   // The tail of the H2D copies is NOT waited for: everything that consumes the inputs is launched on the same stream,
   // and the host-side set-up of the solve overlaps it.  (The staging buffer is reused by the next upload only, which
   // begins with a stream synchronisation.)
-  if (prof) {
-    const double t_issue = since();
-    cudaStreamSynchronize(st);
-    fprintf(stderr, "upload: layout %.3f ms, staged+issued %.3f ms (%.3f), copies done %.3f ms\n", t_layout, t_staged,
-            t_issue, since());
-  }
   if (bad_problem.load() >= 0) {
     cudaStreamSynchronize(st);
     return fail(PSULVSB_ERR_INVALID, "upload: problem " + std::to_string(bad_problem.load()) + " has non-finite coordinates");
@@ -905,8 +893,7 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
     // give each a few thousand line vectors and as the SMs allow
     if (gnc_cluster == 8 && grid_ctas_max >= 16) {
       const long long k_est = (long long)(0.03 * (double)max_nred);
-      const int lv_per_cta = debug_knobs().gnc_grid_lv > 0 ? debug_knobs().gnc_grid_lv : 4096;
-      const long long g = std::min<long long>(grid_ctas_max, k_est / lv_per_cta);
+      const long long g = std::min<long long>(grid_ctas_max, k_est / 4096);
       if (g >= 16) gnc_cluster = (int)g;
     }
     int gnc_cap = (int)((0.03 * (double)max_nred) / (double)gnc_cluster) + 64;
@@ -933,11 +920,6 @@ int Engine::solve_once(const psulvsb_params_t* params, const uint64_t* seeds, ps
       if (cudaEventElapsedTime(&g, ev_g0, ev_g1) == cudaSuccess) gnc_ms += g;  // (the tick's poll already synchronised)
       float a = 0.f;
       if (origin && cudaEventElapsedTime(&a, origin, ev_g0) == cudaSuccess) gnc_iv.emplace_back(a, a + g);
-    }
-    if (debug_knobs().upload_prof) {
-      const double now = std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t_begin).count() / 1e3;
-      std::fprintf(stderr, "tick %d: ends %.3f ms after the solve began; done %d of %d, waiting for a round start %d, clique %d\n",
-                   ticks, now, h_done[0], B, h_done[1], h_done[2]);
     }
     if (h_done[0] >= B) break;
     n_running = B - h_done[0];
@@ -1200,19 +1182,12 @@ class EnginePool {
       if (!skip) {
         const int b0 = call->begin[(size_t)c], nb = call->begin[(size_t)c + 1] - b0;
         e->origin = call->origin;
-        const bool prof = debug_knobs().upload_prof != 0;
-        auto now_ms = [] {
-          return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
-        };
-        double t0, t1;
         {
           // one upload at a time: it has all the staging threads and the whole PCIe link
           std::lock_guard<std::mutex> up(upload_mu);
-          t0 = prof ? now_ms() : 0.0;
           rc = e->upload(call->problems + b0, nb);
           if (!rc && cudaStreamSynchronize(e->st) != cudaSuccess)  // (the copies too: the link is the next upload's now)
             rc = fail(PSULVSB_ERR_CUDA, "upload: copy failed");
-          t1 = prof ? now_ms() : 0.0;
         }
         if (!rc) {
           // at most lane_count() chunks are being solved at a time; the extra worker has the next chunk uploaded by
@@ -1230,10 +1205,6 @@ class EnginePool {
           }
           q_solve.notify_one();
         }
-        if (prof)
-          std::fprintf(stderr, "lane %d: batch %llu chunk %d: upload %.2f .. %.2f, solve .. %.2f ms\n", w,
-                       (unsigned long long)call->id, c, std::fmod(t0, 100000.0), std::fmod(t1, 100000.0),
-                       std::fmod(now_ms(), 100000.0));
         if (rc) msg = psulvsb_last_error();
         else call->recs[(size_t)c] = record_of(e);
       }

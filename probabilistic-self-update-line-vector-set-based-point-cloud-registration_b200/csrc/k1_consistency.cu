@@ -42,12 +42,8 @@ namespace psulvsb {
 namespace {
 
 constexpr int K1_THREADS = 256;
-#ifndef K1_COLPAIR_UNROLL
-#define K1_COLPAIR_UNROLL 4  // column pairs per unrolled step of the word loop (8 columns, as before)
-#endif
-#ifndef K1_R4_CTAS
-#define K1_R4_CTAS 2  // measured with the packed fast path: 3 CTAs per SM (80 registers, 36 B of spills) 2.19 ms vs 2.05 ms
-#endif
+constexpr int K1_COLPAIR_UNROLL = 4;  // column pairs per unrolled step of the word loop (8 columns)
+constexpr int K1_R4_CTAS = 2;  // measured with the packed fast path: 3 CTAs per SM (80 registers, 36 B of spills) 2.19 ms vs 2.05 ms
 
 // exact FP64 test, reference operation order (registration.cc:425-433, SURVEY appendix A.2)
 __device__ __forceinline__ bool exact_consistent(const double* __restrict__ s64, const double* __restrict__ t64, int i,
@@ -203,19 +199,15 @@ __device__ __forceinline__ void eval_word_masked(const float4* __restrict__ cs, 
   }
 }
 
-// Position (in units of 32 rows) of warp w's rows inside row group r of the CTA's row block.  Along the
-// diagonal a warp's work in the tile where group r is partially live is 8 - pos words per tile, so the
-// positions are permuted per group to give every warp (nearly) the same total over the diagonal tiles of a
-// chunk: pos0 + pos1 = 7 for R <= 2, pos0 + pos1 + pos2 in {10, 11} for R >= 3 (identity positions leave
-// warp 0 with 8 + 16 + 24 words against 1 + 9 + 17 for warp 7).
+// Position (in units of 32 rows) of warp w's rows inside row group r of the CTA's row block (R = 1, 2; R = 4 lays
+// its rows out in strips instead).  Along the diagonal a warp's work in the tile where group r is partially live is
+// 8 - pos words per tile, so the second group's positions are reversed to give every warp the same total over the
+// diagonal tiles of a chunk: pos0 + pos1 = 7.
 template <int R>
 __device__ __forceinline__ int k1_warp_pos(int r, int w) {
   static_assert(K1_THREADS == 256, "the position tables are for 8 warps per CTA");
-  if (r == 0) return w;
-  if (R <= 2) return 7 - w;
-  if (r == 1) return (w < 4 ? 7 : 14) - 2 * w;  // 7 5 3 1 6 4 2 0
-  if (r == 2) return (w + 4) & 7;               // 4 5 6 7 0 1 2 3
-  return 7 - ((w + 4) & 7);
+  static_assert(R == 1 || R == 2 || R == 4, "rows per thread are 1, 2 or 4");
+  return r == 0 ? w : 7 - w;
 }
 
 // One CTA = a block of TI = 256 R rows x a chunk of `tiles_per_cta` column tiles (TJ columns each),
@@ -402,14 +394,8 @@ __global__ void __launch_bounds__(K1_THREADS, (R >= 4 ? K1_R4_CTAS : (R >= 2 ? 3
         eval_word_masked<R>(cw, tw, ms, mt, two_beta2, lm, acc, mv);
       } else if (n_live == R)
         eval_word<R, R>(cw, tw, ms, mt, two_beta2, beta4, acc, mv);
-      else if (R == 4)  // (strips of adjacent rows: a pair is live or dead as a whole)
+      else  // only group 0 (R = 2) or the first strip (R = 4: adjacent rows, a pair is live or dead as a whole) is live
         eval_word<(R == 4 ? 2 : 1), R>(cw, tw, ms, mt, two_beta2, beta4, acc, mv);
-      else if (R > 1 && n_live == 1)
-        eval_word<1, R>(cw, tw, ms, mt, two_beta2, beta4, acc, mv);
-      else if (R > 2 && n_live == 2)
-        eval_word<(R > 2 ? 2 : 1), R>(cw, tw, ms, mt, two_beta2, beta4, acc, mv);
-      else
-        eval_word<(R > 3 ? 3 : 1), R>(cw, tw, ms, mt, two_beta2, beta4, acc, mv);
       // the word's epilogue.  FULL: every column of the word is right of every row of the CTA and inside the arrays (all
       // tiles but the block's diagonal ones and the last): no triangle / tail masks
       auto finish = [&](auto full_tag) {
@@ -679,15 +665,13 @@ int launch_consistency_mask(cudaStream_t st, const K1Job* d_jobs, int n_jobs, in
   // measured on B200 (256-column tiles, dead row groups skipped): R = 4 wins once there is enough work
   // (N = 100k: 0.68-0.72 of the FP32-pipe peak vs 0.63; 256 x 5k-point problems: 0.59 vs 0.57; 64: 0.56 vs 0.55)
   int variant = pairs >= 5.0e8 ? 4 : (pairs >= 1.0e8 ? 2 : 1);
-  if (debug_knobs().k1_variant >= 1 && debug_knobs().k1_variant <= 4) variant = debug_knobs().k1_variant;
+  if (debug_knobs().k1_variant != 0) variant = debug_knobs().k1_variant;  // (1, 2 or 4: psulvsb_debug_set checks it)
   // 256-column tiles (measured: half the barrier stalls of 128-column tiles; 512 is no better)
   if (row_sectors) {
-    if (variant == 3) return launch_k1_variant<3, 256, true>(st, d_jobs, n_jobs, max_n, max_rows);
     if (variant == 4) return launch_k1_variant<4, 256, true>(st, d_jobs, n_jobs, max_n, max_rows);
     if (variant == 2) return launch_k1_variant<2, 256, true>(st, d_jobs, n_jobs, max_n, max_rows);
     return launch_k1_variant<1, 256, true>(st, d_jobs, n_jobs, max_n, max_rows);
   }
-  if (variant == 3) return launch_k1_variant<3, 256, false>(st, d_jobs, n_jobs, max_n, max_rows);
   if (variant == 4) return launch_k1_variant<4, 256, false>(st, d_jobs, n_jobs, max_n, max_rows);
   if (variant == 2) return launch_k1_variant<2, 256, false>(st, d_jobs, n_jobs, max_n, max_rows);
   return launch_k1_variant<1, 256, false>(st, d_jobs, n_jobs, max_n, max_rows);

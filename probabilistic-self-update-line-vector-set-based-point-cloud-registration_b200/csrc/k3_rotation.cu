@@ -55,9 +55,7 @@ namespace {
 // threads per CTA is a template parameter T: 256 (two CTAs per SM, so that one hypothesis' serial rotation update
 // overlaps another's pass) for clustered launches, 512 (one CTA per SM, twice the shared-memory cache) when
 // every hypothesis runs on a single CTA (large batches)
-#ifndef GNC_CTAS_PER_SM
-#define GNC_CTAS_PER_SM 2
-#endif
+constexpr int GNC_CTAS_PER_SM = 2;
 
 __device__ __forceinline__ void load_lv(const double* __restrict__ src, const double* __restrict__ dst, uint2 e,
                                         double inv_scale, double sv[3], double tv[3]) {
@@ -95,6 +93,8 @@ constexpr int RED_DEEP = 10;  // deep sleepers left inside the warps' ranges
 constexpr int RED_LEFT = 11;  // positions left inside the warps' ranges
 constexpr int RED_MAX = 15;   // reduced with max: max r^2 (first pass) / -(smallest wake-up drift parked in this pass)
 constexpr double GNC_DEEP_MARGIN_DEFAULT = 0.005;  // remaining margin (rad) from which a sleeping line vector is parked
+constexpr int GNC_PF_STEPS = 1;   // look-ahead (double-steps) of the L2 prefetch in the streamed pass (1, 2, 4 measured equal)
+constexpr int GNC_PARK_PCT = 45;  // share (%) of a CTA's positions that must sleep deeply before a pass is armed
 
 // what thread 0 decides between two passes; everyone reads it after ONE barrier
 struct GncCtl {
@@ -120,8 +120,6 @@ struct GncSmem {
   long long t_stream, t_svd, sum_act, t_prologue, t_start;
   int n_armed, first_armed;
 };
-
-constexpr int GNC_PARK_PCT_DEFAULT = 45;
 
 // 1 / sqrt(x) for a finite x > 0 (x = 0 gives inf, selected away by the caller): the 20-bit seed of MUFU.RSQ64H and
 // two Newton steps with a correction term -- within an ulp of the correctly rounded value, without the special-case
@@ -416,8 +414,7 @@ __device__ __forceinline__ void block_reduce16(GncSmem* sm, double (&v)[GNC_NRED
 
 template <int NC, int T, int CPS>
 __global__ void __launch_bounds__(T, CPS)
-    gnc_tls_kernel(const GncJob* __restrict__ jobs, int cap_per_cta, const double GNC_DEEP_MARGIN, const int pf_steps,
-                   const int park_pct) {
+    gnc_tls_kernel(const GncJob* __restrict__ jobs, int cap_per_cta, const double GNC_DEEP_MARGIN) {
   constexpr int NW = T / 32;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   GncSmem* sm = reinterpret_cast<GncSmem*>(smem_raw);
@@ -527,8 +524,8 @@ __global__ void __launch_bounds__(T, CPS)
 #pragma unroll
           for (int c = 0; c < 3; ++c) acc[r * 3 + c] = fma(sv[r], tv[c], acc[r * 3 + c]);
       };
-      if (ready && pf_steps > 0 && (lane & 3) == 0) {
-        const int pa = la + 64 * pf_steps, pb = lb + 64 * pf_steps;
+      if (ready && (lane & 3) == 0) {
+        const int pa = la + 64 * GNC_PF_STEPS, pb = lb + 64 * GNC_PF_STEPS;
 #pragma unroll
         for (int r = 0; r < 6; ++r) {
           if (pa < gh) asm volatile("prefetch.global.L2 [%0];" ::"l"(g0 + r * st + PH(pa)));
@@ -623,8 +620,8 @@ __global__ void __launch_bounds__(T, CPS)
           const int la = base + lane, lb = la + 32;
           double sa[3], ta[3], sb[3], tb[3], w_ = 0.0;
           uint32_t i_ = 0;
-          if (pf_steps > 0 && (lane & 3) == 0) {
-            const int pa = la + 64 * pf_steps, pb = lb + 64 * pf_steps;
+          if ((lane & 3) == 0) {
+            const int pa = la + 64 * GNC_PF_STEPS, pb = lb + 64 * GNC_PF_STEPS;
 #pragma unroll
             for (int r = 0; r < 6; ++r) {
               if (pa >= cs && pa < gh) asm volatile("prefetch.global.L2 [%0];" ::"l"(g0 + r * st + PH(pa)));
@@ -730,16 +727,16 @@ __global__ void __launch_bounds__(T, CPS)
           const double* __restrict__ ga = g0 + p0;
           // register-free look-ahead: the sectors this warp reads in a later step are pulled into L2 (one lane per
           // 32-byte sector issues the prefetch), so that the loads below see L2 latency instead of HBM's
-          if (pf_steps > 0 && (lane & 3) == 0 && base + 64 * pf_steps + 64 <= n_w) {
-            const double* __restrict__ gp = ga + (size_t)(pf_steps * NW * 64);
+          if ((lane & 3) == 0 && base + 64 * GNC_PF_STEPS + 64 <= n_w) {
+            const double* __restrict__ gp = ga + (size_t)(GNC_PF_STEPS * NW * 64);
 #pragma unroll
             for (int r = 0; r < 6; ++r) {
               asm volatile("prefetch.global.L2 [%0];" ::"l"(gp + r * st));
               asm volatile("prefetch.global.L2 [%0];" ::"l"(gp + r * st + 32));
             }
             if (!unit) {
-              asm volatile("prefetch.global.L2 [%0];" ::"l"(gwl + p0 + pf_steps * NW * 64));
-              asm volatile("prefetch.global.L2 [%0];" ::"l"(gwl + p0 + pf_steps * NW * 64 + 32));
+              asm volatile("prefetch.global.L2 [%0];" ::"l"(gwl + p0 + GNC_PF_STEPS * NW * 64));
+              asm volatile("prefetch.global.L2 [%0];" ::"l"(gwl + p0 + GNC_PF_STEPS * NW * 64 + 32));
             }
           }
 #pragma unroll
@@ -855,7 +852,7 @@ __global__ void __launch_bounds__(T, CPS)
           c.sqrt_th1_up = sqrtf((float)c.th1) * 1.000001f;
           // park when enough of this CTA's positions sleep deeply (its own counts, before the cluster combined them)
           const double deep = sm->part[(red_no - 1) & 1][RED_DEEP], left = sm->part[(red_no - 1) & 1][RED_LEFT];
-          c.armed = (sleeping && !c.reopen && left >= 256.0 && deep * 100.0 >= left * (double)park_pct) ? 1 : 0;
+          c.armed = (sleeping && !c.reopen && left >= 256.0 && deep * 100.0 >= left * (double)GNC_PARK_PCT) ? 1 : 0;
         }
         sm->ctl = c;
       }
@@ -1043,13 +1040,9 @@ int launch_gnc_nc(cudaStream_t st, const GncJob* d_jobs, int n_jobs, int cap_per
   }
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  // (performance knobs only -- any value gives the same results; the tests shrink the margin to force wake-ups)
+  // (a performance knob only -- any value gives the same results; the tests shrink the margin to force wake-ups)
   const double deep_margin = debug_knobs().gnc_deep_margin > 0.0 ? debug_knobs().gnc_deep_margin : GNC_DEEP_MARGIN_DEFAULT;
-  // look-ahead of the L2 prefetch in the streamed pass (0 = off)
-  const int pf_steps = debug_knobs().gnc_prefetch >= 0 ? debug_knobs().gnc_prefetch : 1;
-  // share (%) of a CTA's positions that must sleep deeply before a pass is armed
-  const int park_pct = debug_knobs().gnc_park_pct > 0 ? debug_knobs().gnc_park_pct : GNC_PARK_PCT_DEFAULT;
-  PSU_CUDA(cudaLaunchKernelEx(&cfg, gnc_tls_kernel<NC, T, CPS>, d_jobs, cap_per_cta, deep_margin, pf_steps, park_pct));
+  PSU_CUDA(cudaLaunchKernelEx(&cfg, gnc_tls_kernel<NC, T, CPS>, d_jobs, cap_per_cta, deep_margin));
   return PSULVSB_OK;
 }
 
@@ -1071,8 +1064,6 @@ int gnc_default_capacity() { return gnc_capacity_for(1, 16); }
 
 // CTAs per hypothesis for a batch of n_jobs: as many SMs per job as keeps the whole batch resident
 int gnc_cluster_for(int n_jobs) {
-  const int forced = debug_knobs().gnc_cluster;
-  if (forced == 1 || forced == 2 || forced == 4 || forced == 8) return forced;
   const int slots = sm_count() * GNC_CTAS_PER_SM;
   if (n_jobs * 8 <= slots) return 8;
   if (n_jobs * 4 <= slots) return 4;
@@ -1091,14 +1082,6 @@ int launch_gnc_tls(cudaStream_t st, const GncJob* d_jobs, int n_jobs, int cap_pe
       return fail(PSULVSB_ERR_INVALID, "launch_gnc_tls: grid mode needs CTAs per registration x registrations <= SMs");
     return launch_gnc_nc<0, 512, 1>(st, d_jobs, n_jobs, cap_per_cta, cluster);
   }
-  if (debug_knobs().gnc_cluster > 0) {
-    switch (cluster) {
-      case 8: return launch_gnc_nc<8, 512, 1>(st, d_jobs, n_jobs, cap_per_cta);
-      case 4: return launch_gnc_nc<4, 512, 1>(st, d_jobs, n_jobs, cap_per_cta);
-      case 2: return launch_gnc_nc<2, 512, 1>(st, d_jobs, n_jobs, cap_per_cta);
-      default: return launch_gnc_nc<1, 512, 1>(st, d_jobs, n_jobs, cap_per_cta);
-    }
-  }
   switch (cluster) {
     // (measured: 512 threads x 2 CTAs per SM = 64 registers spills 1.3 KB per thread and loses 25 %)
     case 8:
@@ -1115,10 +1098,8 @@ int launch_gnc_tls(cudaStream_t st, const GncJob* d_jobs, int n_jobs, int cap_pe
       // wave whose stragglers run alone.  Measured on 592 cfg-A pairs per step: 38.8 ms against 41.8 ms with
       // 512-thread CTAs in two waves.  (Caching the points instead of the line vectors was measured and dropped:
       // shared-memory gathers of 96 bytes per line vector cost more than the coalesced stream.)
-      int cps = debug_knobs().gnc_cps;
-      if (cps <= 0) cps = n_active > 2 * sm_count() ? 4 : (n_active > sm_count() ? 2 : 1);
-      if (cps >= 4) return launch_gnc_nc<1, 128, 4>(st, d_jobs, n_jobs, cap_per_cta);
-      if (cps >= 2) return launch_gnc_nc<1, 256, 2>(st, d_jobs, n_jobs, cap_per_cta);
+      if (n_active > 2 * sm_count()) return launch_gnc_nc<1, 128, 4>(st, d_jobs, n_jobs, cap_per_cta);
+      if (n_active > sm_count()) return launch_gnc_nc<1, 256, 2>(st, d_jobs, n_jobs, cap_per_cta);
       return launch_gnc_nc<1, 512, 1>(st, d_jobs, n_jobs, cap_per_cta);
     }
     default: return fail(PSULVSB_ERR_INVALID, "launch_gnc_tls: cluster must be 1, 2, 4, 8 or (grid mode) more");

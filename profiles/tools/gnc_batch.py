@@ -1,6 +1,6 @@
 """GNC-TLS micro-benchmark in the shape of one engine tick of the bench workload: B registrations, one basic subset of
 K line vectors each (cfg-A with FPFH-style outliers: K ~ 22 000), all solved by one launch.
-    python profiles/tools/gnc_batch.py [B] [K]
+    python profiles/tools/gnc_batch.py [B] [K] [line-vector scratch 0|1] [parking 0|1]
 Prints, per cluster size, the launch time and thread 0's cycle split (line-vector passes / SVD / rest) per iteration."""
 import sys
 
@@ -17,10 +17,6 @@ def main():
     K = int(sys.argv[2]) if len(sys.argv) > 2 else 22000
     use_lv = (sys.argv[3] != "0") if len(sys.argv) > 3 else True
     use_perm = (sys.argv[4] != "0") if len(sys.argv) > 4 else True
-    force = (sys.argv[5] != "0") if len(sys.argv) > 5 else False  # 512-thread CTAs, one per SM, at every cluster size
-    for kv in sys.argv[6:]:  # debug switches, e.g. gnc_prefetch=2 gnc_park_pct=40
-        k, v = kv.split("=")
-        capi.debug_set(k, float(v))
     pair = synth.make_pair(5000, 0.95, 3, outliers="fpfh")
     r = stages.consistency_mask(pair["src"], pair["dst"], 0.1)  # the reduced set from the product's own stage 1
     e_all, _ = stages.compact_edges(r["mask"], r["row_counts"], r["n"], r["stride"])
@@ -44,10 +40,8 @@ def main():
     print(f"B={B} K={K} reduced set {len(pi)} lv scratch {'on' if use_lv else 'off'} parking {'on' if perm is not None else 'off'}")
     Rs = {}
     for cluster in (0, 1, 2, 4, 8):
-        if cluster * B > 148 * 2 and cluster > 1 and not force:
+        if cluster * B > 148 * 2 and cluster > 1:
             continue
-        if force:
-            capi.debug_set("gnc_cluster", cluster)
 
         def run():
             capi.check(L.psulvsb_gnc_tls_rotation_batch(torch.cuda.current_stream().cuda_stream, d_src.data_ptr(),

@@ -103,6 +103,23 @@ def test_argument_validation_without_device():
     assert b"cannot open" in L.psulvsb_last_error()
 
 
+def test_debug_switches_accept_only_the_coverage_switches():
+    """psulvsb_debug_set (no device needed) knows four switches and "reset"; the launch-shape tuning switches are gone
+    and are refused like any unknown name, as is a k1_variant the launcher has no kernel for."""
+    L = capi.lib()
+    try:
+        for name in ("gnc_cluster", "gnc_cps", "gnc_prefetch", "gnc_park_pct", "gnc_grid_lv", "upload_prof"):
+            assert L.psulvsb_debug_set(name.encode(), 1.0) == capi.ERR_INVALID, name
+            assert b"unknown switch" in L.psulvsb_last_error()
+        for value in (3.0, 5.0, -1.0, 1.5):
+            assert L.psulvsb_debug_set(b"k1_variant", value) == capi.ERR_INVALID, value
+        for name, value in (("gnc_deep_margin", 1e-4), ("sample_list_cap_test", 4.0), ("edge_wide", 1.0),
+                            ("k1_variant", 0.0), ("k1_variant", 1.0), ("k1_variant", 2.0), ("k1_variant", 4.0)):
+            assert L.psulvsb_debug_set(name.encode(), value) == capi.OK, (name, value)
+    finally:
+        assert L.psulvsb_debug_set(b"reset", 0.0) == capi.OK
+
+
 def test_fp32_pipe_kernels_are_packed_and_tma_staged():
     """The SASS of the consistency-mask and scoring kernels carries what DESIGN.md section 6 says they are built on:
     packed FP32 (FFMA2) in the pair / score loops, their 64-bit operand kept in the operand-reuse cache, and 1-D TMA
