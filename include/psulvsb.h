@@ -198,6 +198,16 @@ int psulvsb_batch_upload(psulvsb_handle_t h, const psulvsb_problem_t* problems, 
  * every upload / psulvsb_solve / psulvsb_solve_batch on the handle replaces -- a mismatch is PSULVSB_ERR_INVALID. */
 int psulvsb_batch_solve_resident(psulvsb_handle_t h, const psulvsb_params_t* params, const uint64_t* seeds,
                                  psulvsb_solution_t* solutions, int n_solutions);
+/* Device-buffer variant of psulvsb_batch_upload: every array pointer in problems[b] (src, dst, ori_src, ori_dst,
+ * keep_mask, reduce_map) is DEVICE memory on the handle's device; the problems array itself, C and M are on the host.
+ * The copy is ordered after the work already queued on `stream` (a cudaStream_t, may be NULL).  When the call
+ * returns, the inputs are resident and the caller's buffers are no longer read.  Then psulvsb_batch_solve_resident
+ * solves the batch, with the solutions of psulvsb_solve_batch on the same arrays from the host.
+ * Accepts and refuses what psulvsb_batch_upload does, with the same codes and messages (the same aliasing rule:
+ * ori_src == src && ori_dst == dst && M == C uploads the points once).  An array that is not device or managed memory
+ * of the handle's device is PSULVSB_ERR_INVALID before any device work; that each array holds 3*C, 3*M or M elements
+ * cannot be checked and is the caller's responsibility.  A refused upload leaves nothing resident. */
+int psulvsb_batch_upload_device(psulvsb_handle_t h, void* stream, const psulvsb_problem_t* problems, int B);
 /* Problems currently resident on the handle (0: nothing uploaded, or the last upload failed). */
 int psulvsb_batch_resident_size(psulvsb_handle_t h);
 /* Kernel launches issued by the handle since creation / device time (ms) of the last solve call: CUDA events,

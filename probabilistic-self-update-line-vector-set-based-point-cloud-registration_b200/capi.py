@@ -20,6 +20,7 @@ DOMAIN_L_SAMPLED, DOMAIN_BASIC, DOMAIN_UNIFORM, DOMAIN_SCALE, DOMAIN_TUPLE = 1, 
 SYMBOLS = [
     "psulvsb_version", "psulvsb_last_error", "psulvsb_default_params", "psulvsb_device_count",
     "psulvsb_create", "psulvsb_destroy", "psulvsb_solve", "psulvsb_solve_batch", "psulvsb_batch_upload",
+    "psulvsb_batch_upload_device",
     "psulvsb_batch_solve_resident", "psulvsb_batch_submit", "psulvsb_batch_wait", "psulvsb_batch_resident_size", "psulvsb_debug_set", "psulvsb_launch_count", "psulvsb_last_device_ms", "psulvsb_last_stage_ms",
     "psulvsb_last_ticks", "psulvsb_last_chunk_ticks", "psulvsb_set_batching", "psulvsb_set_host_threads", "psulvsb_pack_points", "psulvsb_consistency_mask", "psulvsb_consistency_mask_rows",
     "psulvsb_mask_symmetrize", "psulvsb_compact_edges", "psulvsb_ratio_reduced_set", "psulvsb_sample_workspace_bytes",
@@ -265,6 +266,7 @@ def _declare(L: C.CDLL) -> None:
                                        C.POINTER(Solution), C.POINTER(C.c_uint64)]
     L.psulvsb_batch_wait.argtypes = [_vp, C.c_uint64]
     L.psulvsb_batch_upload.argtypes = [_vp, C.POINTER(Problem), C.c_int]
+    L.psulvsb_batch_upload_device.argtypes = [_vp, _vp, C.POINTER(Problem), C.c_int]
     L.psulvsb_batch_solve_resident.argtypes = [_vp, C.POINTER(Params), C.POINTER(C.c_uint64), C.POINTER(Solution),
                                                C.c_int]
     L.psulvsb_debug_set.argtypes = [C.c_char_p, C.c_double]
@@ -473,6 +475,105 @@ class HostProblem:
                        self.keep_mask.ctypes.data_as(_ip), self.reduce_map.ctypes.data_as(_ip))
 
 
+def _tensor(name, t, dtype, shape):
+    """A contiguous tensor of `dtype` and `shape` (None: any extent), else ValueError."""
+    import torch
+
+    if not isinstance(t, torch.Tensor):
+        raise ValueError(f"{name} must be a torch tensor, got {type(t).__name__}")
+    if t.dtype != dtype:
+        raise ValueError(f"{name} must be {dtype}, got {t.dtype}")
+    if t.dim() != len(shape) or any(want is not None and got != want for got, want in zip(t.shape, shape)):
+        raise ValueError(f"{name} must have shape {['*' if w is None else w for w in shape]}, got {list(t.shape)}")
+    if not t.is_contiguous():
+        raise ValueError(f"{name} must be contiguous")
+    return t
+
+
+def _on_one_device(named) -> None:
+    """Every tensor of `named` (name -> tensor) on the same CUDA device, else ValueError."""
+    for name, t in named.items():
+        if not t.is_cuda:
+            raise ValueError(f"{name} must be a CUDA tensor (got one on {t.device})")
+    devices = {t.device for t in named.values()}
+    if len(devices) != 1:
+        raise ValueError(f"the arrays must be on one device, got {sorted(map(str, devices))}")
+
+
+class DeviceProblem:
+    """One registration problem whose arrays are CUDA tensors (Handle.upload_device / solve_batch_device): src, dst
+    [C, 3] and ori_src, ori_dst [M, 3] contiguous float64 (row-major [N, 3] is the C ABI's column-major 3xN, the layout
+    of the other device functions), keep_mask and reduce_map [M] int32.  The defaults are HostProblem's: ori_* alias
+    src / dst, keep_mask is all ones and reduce_map arange(M), made on the device."""
+
+    def __init__(self, src, dst, ori_src=None, ori_dst=None, keep_mask=None, reduce_map=None):
+        import torch
+
+        self.src = _tensor("src", src, torch.float64, (None, 3))
+        self.dst = _tensor("dst", dst, torch.float64, (self.src.shape[0], 3))
+        if (ori_src is None) != (ori_dst is None):
+            raise ValueError("ori_src and ori_dst go together")
+        if ori_src is None:
+            ori_src, ori_dst = self.src, self.dst
+        self.ori_src = _tensor("ori_src", ori_src, torch.float64, (None, 3))
+        M = self.ori_src.shape[0]
+        self.ori_dst = _tensor("ori_dst", ori_dst, torch.float64, (M, 3))
+        if (keep_mask is None) != (reduce_map is None):
+            raise ValueError("keep_mask and reduce_map go together")
+        if keep_mask is None:
+            if self.src.shape[0] != M:
+                raise ValueError("keep_mask / reduce_map are required when C != M")
+            keep_mask = torch.ones(M, dtype=torch.int32, device=self.src.device)
+            reduce_map = torch.arange(M, dtype=torch.int32, device=self.src.device)
+        self.keep_mask = _tensor("keep_mask", keep_mask, torch.int32, (M,))
+        self.reduce_map = _tensor("reduce_map", reduce_map, torch.int32, (M,))
+        _on_one_device({"src": self.src, "dst": self.dst, "ori_src": self.ori_src, "ori_dst": self.ori_dst,
+                        "keep_mask": self.keep_mask, "reduce_map": self.reduce_map})
+        self.device = self.src.device
+
+    @classmethod
+    def from_matches(cls, d_src_cloud, d_tgt_cloud, pairs):
+        """The problem of one pair's correspondences: pairs is that pair's [K, 2] int32 slice of match_batch_device's
+        output (source index, target index), the clouds its [n, 3] float64 CUDA tensors; the points are gathered on
+        the device, in the current stream."""
+        import torch
+
+        _tensor("d_src_cloud", d_src_cloud, torch.float64, (None, 3))
+        _tensor("d_tgt_cloud", d_tgt_cloud, torch.float64, (None, 3))
+        if not isinstance(pairs, torch.Tensor) or pairs.dtype != torch.int32 or pairs.dim() != 2 or pairs.shape[1] != 2:
+            raise ValueError("pairs must be a [K, 2] int32 tensor")
+        _on_one_device({"d_src_cloud": d_src_cloud, "d_tgt_cloud": d_tgt_cloud, "pairs": pairs})
+        return cls(d_src_cloud.index_select(0, pairs[:, 0]), d_tgt_cloud.index_select(0, pairs[:, 1]))
+
+    @property
+    def aliased(self) -> bool:
+        """ori_* are src / dst themselves: the library uploads the points once."""
+        return (self.ori_src.data_ptr() == self.src.data_ptr() and self.ori_dst.data_ptr() == self.dst.data_ptr()
+                and self.ori_src.shape == self.src.shape)
+
+    def c_struct(self) -> Problem:
+        # built on every call: the view follows whatever tensors the attributes hold now
+        ptr = lambda t, ty: C.cast(C.c_void_p(t.data_ptr()), ty)  # noqa: E731
+        return Problem(ptr(self.src, _dp), ptr(self.dst, _dp), self.src.shape[0], ptr(self.ori_src, _dp),
+                       ptr(self.ori_dst, _dp), self.ori_src.shape[0], ptr(self.keep_mask, _ip),
+                       ptr(self.reduce_map, _ip))
+
+
+def _device_problem_array(problems):
+    """psulvsb_problem_t[len(problems)] of DeviceProblems, the same records c_struct() builds, written column by column
+    through a 64-bit view of the array (six ctypes casts per problem cost more than the upload of a 592-problem
+    batch).  Every field sits in its own 8-byte slot (C and M with zero padding above them, little-endian)."""
+    n = len(problems)
+    arr = (Problem * max(n, 1))()
+    if n:
+        words = np.frombuffer(arr, dtype=np.uint64).reshape(max(n, 1), C.sizeof(Problem) // 8)
+        for name in ("src", "dst", "ori_src", "ori_dst", "keep_mask", "reduce_map"):
+            words[:, getattr(Problem, name).offset // 8] = [getattr(p, name).data_ptr() for p in problems]
+        words[:, Problem.C.offset // 8] = [p.src.shape[0] for p in problems]
+        words[:, Problem.M.offset // 8] = [p.ori_src.shape[0] for p in problems]
+    return arr
+
+
 class Handle:
     """psulvsb_handle_t: one device, one stream, private arenas."""
 
@@ -548,6 +649,22 @@ class Handle:
         self._problems = list(problems)  # keep the host arrays alive
         arr = self._problem_array(self._problems)
         check(lib().psulvsb_batch_upload(self._h, arr, len(self._problems)))
+
+    def upload_device(self, problems) -> None:
+        """psulvsb_batch_upload_device: DeviceProblems (one device, this handle's) become the resident batch.  The copy
+        follows the work queued on the current torch stream; when the call returns the tensors may be reused."""
+        import torch
+
+        problems = list(problems)
+        arr = _device_problem_array(problems)
+        dev = problems[0].device if problems else None
+        stream = torch.cuda.current_stream(dev).cuda_stream if dev is not None else None
+        check(lib().psulvsb_batch_upload_device(self._h, stream, arr, len(problems)))
+
+    def solve_batch_device(self, params: Params, problems, seeds=None):
+        """upload_device, then solve_resident: the solutions solve_batch gives on the same arrays from the host."""
+        self.upload_device(problems)
+        return self.solve_resident(params, seeds)
 
     @property
     def resident_size(self) -> int:

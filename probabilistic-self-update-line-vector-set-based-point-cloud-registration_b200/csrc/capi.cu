@@ -174,6 +174,13 @@ int psulvsb_batch_upload(psulvsb_handle_t h, const psulvsb_problem_t* problems, 
   return pool_upload(h->pool, problems, B);
 }
 
+int psulvsb_batch_upload_device(psulvsb_handle_t h, void* stream, const psulvsb_problem_t* problems, int B) {
+  if (int rc = need_device()) return rc;
+  if (!h || !problems || B <= 0)
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_batch_upload_device: NULL argument or B <= 0");
+  return pool_upload_device(h->pool, stream, problems, B);
+}
+
 int psulvsb_batch_solve_resident(psulvsb_handle_t h, const psulvsb_params_t* params, const uint64_t* seeds,
                                  psulvsb_solution_t* solutions, int n_solutions) {
   if (!h || !params || !solutions) return fail(PSULVSB_ERR_INVALID, "psulvsb_batch_solve_resident: NULL argument");

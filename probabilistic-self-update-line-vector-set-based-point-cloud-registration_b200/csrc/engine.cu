@@ -131,6 +131,137 @@ struct ProbLayout {
   int stride;  // mask row stride in words
 };
 
+// ---- device-buffer upload (psulvsb_batch_upload_device) -------------------------------------------------------------
+// One problem of the engine's part: the caller's device arrays, where they go in the input arena, and its tiles.
+struct UploadJob {
+  const double* src;
+  const double* dst;
+  const double* ori_src;  // unused when alias
+  const double* ori_dst;
+  const int* keep_mask;
+  const int* reduce_map;
+  unsigned long long in_dbl, in_int;  // ProbLayout::in_dbl / in_int
+  int C, M;
+  int alias;
+  int tile_first;  // first block of this problem (prefix over the part of max(C, M) / UPLOAD_THREADS tiles)
+};
+// What the upload learns about one problem on the way.  Every field is zero before the launch (one memset) and only
+// grows by exact reductions (max, or, add), so the result does not depend on the order of the atomics.
+struct UploadSummary {
+  unsigned long long lo[2][3];  // min_key of the per-coordinate minimum of src (0) / dst (1)
+  unsigned long long hi[2][3];  // max_key of the maximum
+  unsigned int nonfinite;       // some coordinate of src, dst or a non-aliased ori_* is NaN or infinite
+  unsigned int zeros;           // keep_mask[j] == 0 count
+  unsigned int bad_map;         // some keep_mask[j] == 1 has reduce_map[j] outside [0, C)
+  unsigned int pad;
+};
+constexpr int UPLOAD_THREADS = 256;  // points per tile (256 % 3 == 1: see the kernel)
+
+// order-preserving unsigned images of a double (not NaN): max_key orders like the value, min_key is its complement,
+// so the maximum of either key gives the minimum / maximum and a zeroed slot is the identity
+__host__ __device__ inline unsigned long long max_key_bits(unsigned long long b) {
+  return (b >> 63) ? ~b : b | 0x8000000000000000ull;
+}
+__host__ __device__ inline unsigned long long key_bits_back(unsigned long long k) {
+  return (k >> 63) ? k & 0x7FFFFFFFFFFFFFFFull : ~k;
+}
+
+__global__ void __launch_bounds__(UPLOAD_THREADS)
+    engine_upload_device_kernel(const UploadJob* __restrict__ jobs, int nb, double* __restrict__ in_dbl,
+                                int* __restrict__ in_int, UploadSummary* __restrict__ sum) {
+  __shared__ unsigned long long part[12][UPLOAD_THREADS / 32];
+  int b = 0;
+  for (int hi = nb; hi - b > 1;) {  // the problem whose tiles hold this block
+    const int mid = (b + hi) >> 1;
+    if (jobs[mid].tile_first <= (int)blockIdx.x) b = mid;
+    else hi = mid;
+  }
+  const UploadJob& J = jobs[b];
+  const int t = threadIdx.x, lane = t & 31, wid = t >> 5;
+  const long long p0 = (long long)((int)blockIdx.x - J.tile_first) * UPLOAD_THREADS;  // first point of the tile
+  // The tile's 3 x 256 doubles of an array are read at 3 p0 + t + 256 r, r = 0..2: coalesced, and since 256 % 3 == 1
+  // thread t meets coordinate (t + r) % 3 in its r-th load, i.e. each coordinate exactly once.
+  const int t3 = t % 3;
+  const size_t n3 = (size_t)3 * (size_t)J.C;
+  double* a = in_dbl + J.in_dbl;
+  bool bad = false;
+  unsigned long long key[12];  // [min 0 / max 1][side][coordinate]
+#pragma unroll
+  for (int s = 0; s < 2; ++s) {
+    const double* x = s ? J.dst : J.src;
+    double* out = a + (s ? n3 : 0);
+    unsigned long long lo_r[3], hi_r[3];  // by load r
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+      const size_t i = (size_t)(3 * p0) + (size_t)(t + UPLOAD_THREADS * r);
+      lo_r[r] = hi_r[r] = 0ull;
+      if (i < n3) {
+        const double v = x[i];
+        out[i] = v;
+        bad |= !isfinite(v);
+        const unsigned long long k = max_key_bits((unsigned long long)__double_as_longlong(v));
+        lo_r[r] = ~k;
+        hi_r[r] = k;
+      }
+    }
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {  // coordinate c came with load (c - t) mod 3
+      const int r = (c - t3 + 3) % 3;
+      key[3 * s + c] = r == 0 ? lo_r[0] : (r == 1 ? lo_r[1] : lo_r[2]);
+      key[6 + 3 * s + c] = r == 0 ? hi_r[0] : (r == 1 ? hi_r[1] : hi_r[2]);
+    }
+  }
+  if (!J.alias) {
+    const size_t m3 = (size_t)3 * (size_t)J.M;
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+      const double* x = s ? J.ori_dst : J.ori_src;
+      double* out = a + 2 * n3 + (s ? m3 : 0);
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {
+        const size_t i = (size_t)(3 * p0) + (size_t)(t + UPLOAD_THREADS * r);
+        if (i < m3) {
+          const double v = x[i];
+          out[i] = v;
+          bad |= !isfinite(v);
+        }
+      }
+    }
+  }
+  bool zero = false, bad_map = false;
+  {
+    const long long j = p0 + t;
+    if (j < J.M) {
+      const int k = J.keep_mask[j], m = J.reduce_map[j];
+      int* o = in_int + J.in_int;
+      o[j] = k;
+      o[J.M + j] = m;
+      zero = (k == 0);
+      // a kept correspondence's reduced column becomes a line-vector endpoint: it must name a column of src / dst
+      bad_map = (k == 1 && (m < 0 || m >= J.C));
+    }
+  }
+#pragma unroll
+  for (int q = 0; q < 12; ++q) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) key[q] = max(key[q], __shfl_xor_sync(0xffffffffu, key[q], o));
+    if (lane == 0) part[q][wid] = key[q];
+  }
+  const int any_bad = __syncthreads_or(bad);
+  const int n_zero = __syncthreads_count(zero);
+  const int any_bad_map = __syncthreads_or(bad_map);
+  UploadSummary& S = sum[b];
+  if (t < 12) {
+    unsigned long long m = 0ull;
+    for (int w = 0; w < UPLOAD_THREADS / 32; ++w) m = max(m, part[t][w]);
+    if (m) atomicMax(t < 6 ? &S.lo[t / 3][t % 3] : &S.hi[(t - 6) / 3][t % 3], m);
+  } else if (t == 32) {
+    if (any_bad) atomicOr(&S.nonfinite, 1u);
+    if (n_zero) atomicAdd(&S.zeros, (unsigned int)n_zero);
+    if (any_bad_map) atomicOr(&S.bad_map, 1u);
+  }
+}
+
 }  // namespace
 
 class Engine {
@@ -144,6 +275,7 @@ class Engine {
   std::vector<unsigned long long> reserve;  // self-update edge head-room per job
   size_t in_dbl_total = 0, in_int_total = 0;
   DevBuf d_in_dbl, d_in_int, d_work, d_mask, d_edge, d_jobs, d_misc, d_hist;
+  DevBuf d_upload;  // problem table and summaries of upload_device
   unsigned long long sampler_scratch_sig = 0;  // arena layout of the sampler scratch at the last solve
   bool sampler_scratch_clean = false;          // ... and whether that solve ran to completion
   PinBuf h_stage, h_small;
@@ -173,6 +305,7 @@ class Engine {
     d_jobs.release();
     d_misc.release();
     d_hist.release();
+    d_upload.release();
     h_stage.release();
     h_small.release();
     if (ev_begin) cudaEventDestroy(ev_begin);
@@ -210,10 +343,18 @@ class Engine {
   }
 
   int upload(const psulvsb_problem_t* problems, int nb);
+  // Device-buffer upload in two halves, so that the pool can have every engine's copy in flight at once: `begin`
+  // queues the copy and reductions behind `ready` (an event on the caller's stream), `finish` waits for them and
+  // completes the layouts.  The arrays must have passed check_problem and check_device_pointers; `first` is the
+  // index of problems[0] in the caller's batch (error messages name problems by that index).
+  int upload_device_begin(const psulvsb_problem_t* problems, int nb, cudaEvent_t ready);
+  int upload_device_finish(int first);
   int solve(const psulvsb_params_t* params, const uint64_t* seeds, psulvsb_solution_t* solutions,
             psulvsb_trace_t* trace_first);
 
  private:
+  int plan_layout(const psulvsb_problem_t* problems, int nb);
+  void make_resident(int nb);
   int solve_once(const psulvsb_params_t* params, const uint64_t* seeds, psulvsb_solution_t* solutions,
                  psulvsb_trace_t* trace_first);
 };
@@ -262,26 +403,60 @@ inline void stage_points(double* dst, const double* src, size_t n_doubles, doubl
     poison += v * 0.0;
   }
 }
+
+// The argument check of both uploads; the message names the problem by b.
+int check_problem(const psulvsb_problem_t& p, int b) {
+  if (!p.src || !p.dst || !p.ori_src || !p.ori_dst || !p.keep_mask || !p.reduce_map || p.C < 2 || p.M < 1)
+    return fail(PSULVSB_ERR_INVALID, "upload: problem " + std::to_string(b) + " has a null array, C < 2 or M < 1");
+  return PSULVSB_OK;
+}
+
+// The last step of both uploads: the keep_mask zeros give the working-set capacity, the per-side extrema (lo[s] / hi[s]:
+// per-coordinate minimum / maximum of src (s = 0) and dst (s = 1)) the centres and the coordinate bound of the FP32
+// tiles.  False: a centre or the bound is not finite.
+bool finish_layout(ProbLayout& L, int zeros, const double lo[2][3], const double hi[2][3]) {
+  L.Ccap = L.C0 + zeros;  // every original correspondence can be appended at most once (registration.cc:828)
+  // (differences are translation invariant: each cloud is centred on its own bounding box)
+  for (int s = 0; s < 2; ++s) {
+    double* c = s ? L.cdst : L.csrc;
+    double bound = 0.0;
+    for (int r = 0; r < 3; ++r) {
+      c[r] = 0.5 * (lo[s][r] + hi[s][r]);
+      const double h = 0.5 * (hi[s][r] - lo[s][r]);
+      bound = h > bound ? h : bound;
+    }
+    if (s == 0)
+      L.coord_bound = bound;
+    else
+      L.coord_bound = bound > L.coord_bound ? bound : L.coord_bound;
+  }
+  L.coord_bound = L.coord_bound * (1.0 + 1e-6) + 1e-30;
+  for (int r = 0; r < 3; ++r)
+    if (!std::isfinite(L.csrc[r]) || !std::isfinite(L.cdst[r]) || !std::isfinite(L.coord_bound)) return false;
+  return true;
+}
+
+// the data refusals of both uploads
+int refuse_non_finite(int b) {
+  return fail(PSULVSB_ERR_INVALID, "upload: problem " + std::to_string(b) + " has non-finite coordinates");
+}
+int refuse_bad_map(int b) {
+  return fail(PSULVSB_ERR_INVALID,
+              "upload: problem " + std::to_string(b) + " has keep_mask[j] == 1 with reduce_map[j] outside [0, C)");
+}
 }  // namespace
 
-int Engine::upload(const psulvsb_problem_t* problems, int nb) {
-  if (!problems || nb <= 0) return fail(PSULVSB_ERR_INVALID, "upload: no problems");
-  if (st) cudaStreamSynchronize(st);  // earlier copies out of the staging buffer (and solves on its contents) are done
-  // nothing is resident until this upload has fully succeeded (a failed re-upload must not leave the previous batch
-  // size paired with a half-overwritten layout / input arena)
-  B = 0;
-  reserve.clear();
-  PSU_CUDA(cudaSetDevice(device));
+// Offsets of every problem in the input arenas, mask strides and aliasing (both uploads).
+int Engine::plan_layout(const psulvsb_problem_t* problems, int nb) {
   lay.assign((size_t)nb, ProbLayout());
   size_t od = 0, oi = 0;
   for (int b = 0; b < nb; ++b) {
     const psulvsb_problem_t& p = problems[b];
-    if (!p.src || !p.dst || !p.ori_src || !p.ori_dst || !p.keep_mask || !p.reduce_map || p.C < 2 || p.M < 1)
-      return fail(PSULVSB_ERR_INVALID, "upload: problem " + std::to_string(b) + " has a null array, C < 2 or M < 1");
+    if (int rc = check_problem(p, b)) return rc;
     ProbLayout& L = lay[(size_t)b];
     L.C0 = p.C;
     L.M = p.M;
-    L.Ccap = p.C;  // + the keep_mask zeros, counted by the staging threads below
+    L.Ccap = p.C;  // + the keep_mask zeros (finish_layout)
     L.stride = (int)align_up((size_t)(p.C + 31) / 32, 8);  // whole 32-byte sectors per row and column tile (K1 stores them as such)
     od = align_up(od, 16);
     L.in_dbl = od;
@@ -293,6 +468,28 @@ int Engine::upload(const psulvsb_problem_t* problems, int nb) {
   }
   in_dbl_total = od;
   in_int_total = oi;
+  return PSULVSB_OK;
+}
+
+void Engine::make_resident(int nb) {
+  B = nb;
+  reserve.assign((size_t)nb, 0ull);
+  for (int b = 0; b < nb; ++b) {
+    const ProbLayout& L = lay[(size_t)b];
+    if (L.Ccap > L.C0) reserve[(size_t)b] = 65536ull;
+  }
+}
+
+int Engine::upload(const psulvsb_problem_t* problems, int nb) {
+  if (!problems || nb <= 0) return fail(PSULVSB_ERR_INVALID, "upload: no problems");
+  if (st) cudaStreamSynchronize(st);  // earlier copies out of the staging buffer (and solves on its contents) are done
+  // nothing is resident until this upload has fully succeeded (a failed re-upload must not leave the previous batch
+  // size paired with a half-overwritten layout / input arena)
+  B = 0;
+  reserve.clear();
+  PSU_CUDA(cudaSetDevice(device));
+  if (int rc = plan_layout(problems, nb)) return rc;
+  const size_t od = in_dbl_total, oi = in_int_total;
   const size_t bytes_d = od * sizeof(double), bytes_i = oi * sizeof(int);
   if (int rc = h_stage.ensure(align_up(bytes_d, 256) + bytes_i)) return rc;
   if (int rc = d_in_dbl.ensure(bytes_d)) return rc;
@@ -325,25 +522,21 @@ int Engine::upload(const psulvsb_problem_t* problems, int nb) {
       }
       std::memcpy(hi + L.in_int, p.keep_mask, sizeof(int) * (size_t)p.M);
       std::memcpy(hi + L.in_int + p.M, p.reduce_map, sizeof(int) * (size_t)p.M);
-      {
-        int zeros = 0;
-        for (int j = 0; j < p.M; ++j) {
-          zeros += (p.keep_mask[j] == 0) ? 1 : 0;
-          // a kept correspondence's reduced column becomes a line-vector endpoint on the device (inlier_map,
-          // registration.cc:1432-1434): it must name a column of src / dst
-          if (p.keep_mask[j] == 1 && (p.reduce_map[j] < 0 || p.reduce_map[j] >= p.C)) bad_map.store(b);
-        }
-        L.Ccap = p.C + zeros;  // every original correspondence can be appended at most once (registration.cc:828)
+      int zeros = 0;
+      for (int j = 0; j < p.M; ++j) {
+        zeros += (p.keep_mask[j] == 0) ? 1 : 0;
+        // a kept correspondence's reduced column becomes a line-vector endpoint on the device (inlier_map,
+        // registration.cc:1432-1434): it must name a column of src / dst
+        if (p.keep_mask[j] == 1 && (p.reduce_map[j] < 0 || p.reduce_map[j] >= p.C)) bad_map.store(b);
       }
-      // (differences are translation invariant: each cloud is centred on its own bounding box)
+      double lo[2][3], hi3[2][3];
       for (int s = 0; s < 2; ++s) {
         const double* pts = s ? p.dst : p.src;
         double lo6[6], hi6[6], poison = 0.0;
         stage_points(d + (s ? 3 * (size_t)p.C : 0), pts, (size_t)3 * p.C, lo6, hi6, poison);
-        double lo[3], hi3[3];
         for (int r = 0; r < 3; ++r) {
-          lo[r] = lo6[r] < lo6[r + 3] ? lo6[r] : lo6[r + 3];
-          hi3[r] = hi6[r] > hi6[r + 3] ? hi6[r] : hi6[r + 3];
+          lo[s][r] = lo6[r] < lo6[r + 3] ? lo6[r] : lo6[r + 3];
+          hi3[s][r] = hi6[r] > hi6[r + 3] ? hi6[r] : hi6[r + 3];
         }
         if (!L.alias_ori) {
           const double* ori = s ? p.ori_dst : p.ori_src;
@@ -356,21 +549,8 @@ int Engine::upload(const psulvsb_problem_t* problems, int nb) {
         }
         const bool finite = (poison == 0.0);
         if (!finite) bad_problem.store(b);
-        double* c = s ? L.cdst : L.csrc;
-        double bound = 0.0;
-        for (int r = 0; r < 3; ++r) {
-          c[r] = 0.5 * (lo[r] + hi3[r]);
-          const double h = 0.5 * (hi3[r] - lo[r]);
-          bound = h > bound ? h : bound;
-        }
-        if (s == 0)
-          L.coord_bound = bound;
-        else
-          L.coord_bound = bound > L.coord_bound ? bound : L.coord_bound;
       }
-      L.coord_bound = L.coord_bound * (1.0 + 1e-6) + 1e-30;
-      for (int r = 0; r < 3; ++r)
-        if (!std::isfinite(L.csrc[r]) || !std::isfinite(L.cdst[r]) || !std::isfinite(L.coord_bound)) bad_problem.store(b);
+      if (!finish_layout(L, zeros, lo, hi3)) bad_problem.store(b);
       if (b + 1 - group_begin >= 8 || b + 1 == b1) {  // (measured: groups of 2 finish 0.6 ms later, 13 the same)
         push_group(group_begin, b + 1);
         group_begin = b + 1;
@@ -396,23 +576,90 @@ int Engine::upload(const psulvsb_problem_t* problems, int nb) {
   // begins with a stream synchronisation.)
   if (bad_problem.load() >= 0) {
     cudaStreamSynchronize(st);
-    return fail(PSULVSB_ERR_INVALID, "upload: problem " + std::to_string(bad_problem.load()) + " has non-finite coordinates");
+    return refuse_non_finite(bad_problem.load());
   }
   if (bad_map.load() >= 0) {
     cudaStreamSynchronize(st);
-    return fail(PSULVSB_ERR_INVALID, "upload: problem " + std::to_string(bad_map.load()) +
-                                         " has keep_mask[j] == 1 with reduce_map[j] outside [0, C)");
+    return refuse_bad_map(bad_map.load());
   }
   if (copy_error.load()) {
     cudaStreamSynchronize(st);
     return fail(PSULVSB_ERR_CUDA, "upload: host-to-device copy failed");
   }
-  B = nb;
-  reserve.assign((size_t)nb, 0ull);
+  make_resident(nb);
+  return PSULVSB_OK;
+}
+
+int Engine::upload_device_begin(const psulvsb_problem_t* problems, int nb, cudaEvent_t ready) {
+  if (st) cudaStreamSynchronize(st);  // (as upload: the solves on the previous inputs are done)
+  B = 0;
+  reserve.clear();
+  PSU_CUDA(cudaSetDevice(device));
+  if (int rc = plan_layout(problems, nb)) return rc;
+  if (int rc = d_in_dbl.ensure(in_dbl_total * sizeof(double))) return rc;
+  if (int rc = d_in_int.ensure(in_int_total * sizeof(int))) return rc;
+  const size_t table = align_up(sizeof(UploadJob) * (size_t)nb, 256), bytes = table + sizeof(UploadSummary) * (size_t)nb;
+  if (int rc = h_small.ensure(bytes)) return rc;
+  if (int rc = d_upload.ensure(bytes)) return rc;
+  UploadJob* jobs = reinterpret_cast<UploadJob*>(h_small.p);
+  long long tiles = 0;
   for (int b = 0; b < nb; ++b) {
+    const psulvsb_problem_t& p = problems[b];
     const ProbLayout& L = lay[(size_t)b];
-    if (L.Ccap > L.C0) reserve[(size_t)b] = 65536ull;
+    UploadJob& J = jobs[b];
+    J.src = p.src;
+    J.dst = p.dst;
+    J.ori_src = p.ori_src;
+    J.ori_dst = p.ori_dst;
+    J.keep_mask = p.keep_mask;
+    J.reduce_map = p.reduce_map;
+    J.in_dbl = L.in_dbl;
+    J.in_int = L.in_int;
+    J.C = p.C;
+    J.M = p.M;
+    J.alias = L.alias_ori ? 1 : 0;
+    J.tile_first = (int)tiles;
+    tiles += ((long long)(p.C > p.M ? p.C : p.M) + UPLOAD_THREADS - 1) / UPLOAD_THREADS;
   }
+  if (tiles > 0x7FFFFFFFll) return fail(PSULVSB_ERR_UNSUPPORTED, "upload_device: more than 2^31 - 1 tiles of 256 points");
+  char* d = reinterpret_cast<char*>(d_upload.p);
+  PSU_CUDA(cudaStreamWaitEvent(st, ready, 0));  // the caller's work on its inputs comes first
+  PSU_CUDA(cudaMemcpyAsync(d, jobs, sizeof(UploadJob) * (size_t)nb, cudaMemcpyHostToDevice, st));
+  PSU_CUDA(cudaMemsetAsync(d + table, 0, sizeof(UploadSummary) * (size_t)nb, st));
+  engine_upload_device_kernel<<<(unsigned)tiles, UPLOAD_THREADS, 0, st>>>(
+      reinterpret_cast<const UploadJob*>(d), nb, reinterpret_cast<double*>(d_in_dbl.p),
+      reinterpret_cast<int*>(d_in_int.p), reinterpret_cast<UploadSummary*>(d + table));
+  ++launches;
+  PSU_CUDA(cudaGetLastError());
+  PSU_CUDA(cudaMemcpyAsync(reinterpret_cast<char*>(h_small.p) + table, d + table, sizeof(UploadSummary) * (size_t)nb,
+                           cudaMemcpyDeviceToHost, st));
+  return PSULVSB_OK;
+}
+
+int Engine::upload_device_finish(int first) {
+  PSU_CUDA(cudaStreamSynchronize(st));
+  const int nb = (int)lay.size();
+  const UploadSummary* sum = reinterpret_cast<const UploadSummary*>(
+      reinterpret_cast<const char*>(h_small.p) + align_up(sizeof(UploadJob) * (size_t)nb, 256));
+  auto value = [](unsigned long long key) {
+    const unsigned long long bits = key_bits_back(key);
+    double v;
+    std::memcpy(&v, &bits, sizeof(v));
+    return v;
+  };
+  for (int b = 0; b < nb; ++b) {
+    double lo[2][3], hi[2][3];
+    for (int s = 0; s < 2; ++s)
+      for (int r = 0; r < 3; ++r) {
+        lo[s][r] = value(~sum[b].lo[s][r]);
+        hi[s][r] = value(sum[b].hi[s][r]);
+      }
+    // (the host path's order: non-finite data or centres first, then the reduce_map check)
+    if (sum[b].nonfinite || !finish_layout(lay[(size_t)b], (int)sum[b].zeros, lo, hi)) return refuse_non_finite(first + b);
+  }
+  for (int b = 0; b < nb; ++b)
+    if (sum[b].bad_map) return refuse_bad_map(first + b);
+  make_resident(nb);
   return PSULVSB_OK;
 }
 
@@ -1034,6 +1281,7 @@ class EnginePool {
   int host_threads = 0;  // host threads for staging (0: the CPUs available to the process)
   std::vector<Engine*> eng;
   cudaEvent_t origin = nullptr;
+  cudaEvent_t ready = nullptr;  // upload_device: recorded on the caller's stream
   std::vector<int> res_begin;  // resident partition: engine e holds problems [res_begin[e], res_begin[e + 1])
   int resident_B = 0;
   double last_ms = 0.0;
@@ -1046,6 +1294,7 @@ class EnginePool {
     stop_workers();
     for (Engine* e : eng) delete e;
     if (origin) cudaEventDestroy(origin);
+    if (ready) cudaEventDestroy(ready);
     if (mark_st) cudaStreamDestroy(mark_st);
   }
   int init(int dev) {
@@ -1408,6 +1657,60 @@ class EnginePool {
     return PSULVSB_OK;
   }
 
+  // Every array of the batch must be device (or managed) memory of this handle's device: a kernel reading a host
+  // address would fault the device, so anything else is refused before any device work.
+  int check_device_pointers(const psulvsb_problem_t* problems, int B) {
+    for (int b = 0; b < B; ++b) {
+      const psulvsb_problem_t& p = problems[b];
+      const void* arr[6] = {p.src, p.dst, p.ori_src, p.ori_dst, p.keep_mask, p.reduce_map};
+      static const char* const names[6] = {"src", "dst", "ori_src", "ori_dst", "keep_mask", "reduce_map"};
+      for (int k = 0; k < 6; ++k) {
+        cudaPointerAttributes a;
+        const cudaError_t e = cudaPointerGetAttributes(&a, arr[k]);
+        if (e != cudaSuccess) cudaGetLastError();
+        const bool ok = e == cudaSuccess && (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) &&
+                        a.device == device;
+        if (!ok)
+          return fail(PSULVSB_ERR_INVALID, "upload_device: problem " + std::to_string(b) + ": " + names[k] +
+                                               " is not device memory of device " + std::to_string(device));
+      }
+    }
+    return PSULVSB_OK;
+  }
+
+  // psulvsb_batch_upload_device: the split of upload, each engine's copy ordered after the caller's stream
+  int upload_device(cudaStream_t caller, const psulvsb_problem_t* problems, int B) {
+    drain();
+    resident_B = 0;
+    for (int b = 0; b < B; ++b)
+      if (int rc = check_problem(problems[b], b)) return rc;
+    PSU_CUDA(cudaSetDevice(device));
+    if (int rc = check_device_pointers(problems, B)) return rc;
+    const int ch = chunk_size();
+    int parts = (B + ch - 1) / ch;
+    if (parts > lane_count()) parts = lane_count();
+    if (int rc = ensure_engines(parts)) return rc;
+    partition(B, parts, res_begin);
+    if (!ready) PSU_CUDA(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
+    PSU_CUDA(cudaEventRecord(ready, caller));
+    int rc = PSULVSB_OK;
+    for (int e = 0; e < parts && !rc; ++e)
+      rc = eng[(size_t)e]->upload_device_begin(problems + res_begin[(size_t)e],
+                                               res_begin[(size_t)e + 1] - res_begin[(size_t)e], ready);
+    if (rc) {
+      // (the caller's buffers are not read after the call returns, whatever it returns)
+      for (int e = 0; e < parts; ++e) cudaStreamSynchronize(eng[(size_t)e]->st);
+      return rc;
+    }
+    for (int e = 0; e < parts; ++e)
+      if (int r = eng[(size_t)e]->upload_device_finish(res_begin[(size_t)e])) {
+        for (int f = e + 1; f < parts; ++f) cudaStreamSynchronize(eng[(size_t)f]->st);
+        return r;
+      }
+    resident_B = B;
+    return PSULVSB_OK;
+  }
+
   int solve_resident(const psulvsb_params_t* params, const uint64_t* seeds, psulvsb_solution_t* solutions,
                      psulvsb_trace_t* trace_first) {
     drain();
@@ -1486,6 +1789,9 @@ int pool_solve_sharded(EnginePool* p, Comm* comm, const psulvsb_params_t* params
   return p->solve_sharded(comm, params, problem, solution, trace);
 }
 int pool_upload(EnginePool* p, const psulvsb_problem_t* problems, int B) { return p->upload(problems, B); }
+int pool_upload_device(EnginePool* p, void* stream, const psulvsb_problem_t* problems, int B) {
+  return p->upload_device(static_cast<cudaStream_t>(stream), problems, B);
+}
 int pool_solve_resident(EnginePool* p, const psulvsb_params_t* params, const uint64_t* seeds,
                         psulvsb_solution_t* solutions, psulvsb_trace_t* trace_first) {
   return p->solve_resident(params, seeds, solutions, trace_first);

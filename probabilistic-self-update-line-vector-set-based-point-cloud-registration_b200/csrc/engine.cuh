@@ -270,6 +270,8 @@ int pool_submit(EnginePool* p, const psulvsb_params_t* params, const psulvsb_pro
                 const uint64_t* seeds, psulvsb_solution_t* solutions, uint64_t* ticket);
 int pool_wait(EnginePool* p, uint64_t ticket);
 int pool_upload(EnginePool* p, const psulvsb_problem_t* problems, int B);
+// every array pointer of problems[b] is device memory (psulvsb_batch_upload_device)
+int pool_upload_device(EnginePool* p, void* stream, const psulvsb_problem_t* problems, int B);
 // ONE registration whose consistency rows are sharded over the ranks of `comm` (every rank passes the same problem and
 // gets the same solution)
 int pool_solve_sharded(EnginePool* p, Comm* comm, const psulvsb_params_t* params, const psulvsb_problem_t* problem,
