@@ -626,6 +626,67 @@ int psulvsb_gicp_batch(void* stream, const psulvsb_gicp_pair_t* pairs, int B, co
 int psulvsb_gicp_batch_host(const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
                             double epsilon, psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr);
 
+/* ---- Robust kernels for point-to-plane ICP and generalized ICP (DESIGN.md section 11, "Robust kernels"; Open3D's
+ * TransformationEstimationPointToPlane(loss) and TransformationEstimationForGeneralizedICP(epsilon, kernel)).  The
+ * loop, stop rule, correspondences, fitness, the unweighted inlier_rmse, trace, statuses and minimum counts (6 for
+ * point-to-plane, 3 for GICP) are those of the plain calls; only the update changes.  A residual r gets the weight
+ * rho(r), FP64, every operation rounded in the order written:
+ *   L2      1 (k ignored)                 HUBER  k / max(|r|, k)          CAUCHY  1 / (1 + (r / k)^2)
+ *   GM      k / (k + r^2)^2               TUKEY  (1 - min(1, |r| / k)^2)^2
+ * Point-to-plane weights r = (p' - q).n; with the L2 loss the robust call is bit-identical to psulvsb_icp in
+ * point-to-plane mode.  GICP whitens d = p' - q with W = C^-1/2 (C = 2 I - (1 - epsilon)(m m^T + n n^T)) and weights
+ * each of the three rows r_i = W_i . d on its own, as Open3D does; W's rows are world-frame directions, so the weights
+ * depend on the world frame.  With the L2 loss the objective is psulvsb_gicp's, summed in another order. */
+enum {
+  PSULVSB_LOSS_L2 = 0,
+  PSULVSB_LOSS_HUBER = 1,
+  PSULVSB_LOSS_CAUCHY = 2,
+  PSULVSB_LOSS_GM = 3,    /* Geman-McClure */
+  PSULVSB_LOSS_TUKEY = 4
+};
+
+typedef struct psulvsb_robust_kernel {
+  int type;  /* PSULVSB_LOSS_*                                                                              */
+  double k;  /* the kernel's scale: finite and > 0 (ignored by PSULVSB_LOSS_L2)                             */
+} psulvsb_robust_kernel_t;
+
+/* psulvsb_icp / psulvsb_icp_host / psulvsb_icp_batch / psulvsb_icp_batch_host in point-to-plane mode with the robust
+ * kernel *loss (read before the call returns).  Workspaces are psulvsb_icp[_batch]_workspace_bytes.
+ * PSULVSB_ERR_INVALID before any device work for everything the plain call refuses, a NULL loss, an unknown type, a k
+ * that is not finite and > 0 (types other than L2), or point_to_plane != 1 (Open3D has no robust point-to-point). */
+int psulvsb_icp_robust(void* stream, const double* d_src, int n_s, const double* d_tgt, int n_t,
+                       const double* d_tgt_normals, const psulvsb_icp_params_t* params,
+                       const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3], void* d_work,
+                       psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr);
+int psulvsb_icp_robust_host(const double* src, int n_s, const double* tgt, int n_t, const double* tgt_normals,
+                            const psulvsb_icp_params_t* params, const psulvsb_robust_kernel_t* loss, const double R0[9],
+                            const double t0[3], psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace,
+                            int* corr);
+int psulvsb_icp_robust_batch(void* stream, const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                             const psulvsb_robust_kernel_t* loss, void* d_work, psulvsb_icp_result_t* d_results,
+                             psulvsb_icp_iteration_t* d_trace, int* d_corr);
+int psulvsb_icp_robust_batch_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                                  const psulvsb_robust_kernel_t* loss, psulvsb_icp_result_t* results,
+                                  psulvsb_icp_iteration_t* trace, int* corr);
+/* psulvsb_gicp / psulvsb_gicp_host / psulvsb_gicp_batch / psulvsb_gicp_batch_host with the robust kernel *loss.
+ * Workspaces are psulvsb_icp_workspace_bytes / psulvsb_gicp_batch_workspace_bytes.  PSULVSB_ERR_INVALID before any
+ * device work for everything the plain call refuses and the loss refusals of psulvsb_icp_robust. */
+int psulvsb_gicp_robust(void* stream, const double* d_src, int n_s, const double* d_src_normals, const double* d_tgt,
+                        int n_t, const double* d_tgt_normals, const psulvsb_icp_params_t* params, double epsilon,
+                        const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3], void* d_work,
+                        psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr);
+int psulvsb_gicp_robust_host(const double* src, int n_s, const double* src_normals, const double* tgt, int n_t,
+                             const double* tgt_normals, const psulvsb_icp_params_t* params, double epsilon,
+                             const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3],
+                             psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace, int* corr);
+int psulvsb_gicp_robust_batch(void* stream, const psulvsb_gicp_pair_t* pairs, int B,
+                              const psulvsb_icp_params_t* params, double epsilon, const psulvsb_robust_kernel_t* loss,
+                              void* d_work, psulvsb_icp_result_t* d_results, psulvsb_icp_iteration_t* d_trace,
+                              int* d_corr);
+int psulvsb_gicp_robust_batch_host(const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                                   double epsilon, const psulvsb_robust_kernel_t* loss, psulvsb_icp_result_t* results,
+                                   psulvsb_icp_iteration_t* trace, int* corr);
+
 /* Clique escalation (registration.cc:1000-1085 -> teaser/src/graph.cc:12-125, PMC exact maximum clique) of the
  * graph with n_vertices vertices and the given edges (uint2 endpoint pairs).  A deterministic greedy maximal
  * clique (most neighbours among the remaining candidates first, ties: lowest index) gives the lower bound;

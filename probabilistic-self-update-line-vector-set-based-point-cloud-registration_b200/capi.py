@@ -39,6 +39,8 @@ SYMBOLS = [
     "psulvsb_match_batch_workspace_bytes", "psulvsb_match_batch", "psulvsb_match_batch_host",
     "psulvsb_gicp", "psulvsb_gicp_host", "psulvsb_gicp_batch_workspace_bytes", "psulvsb_gicp_batch",
     "psulvsb_gicp_batch_host",
+    "psulvsb_icp_robust", "psulvsb_icp_robust_host", "psulvsb_icp_robust_batch", "psulvsb_icp_robust_batch_host",
+    "psulvsb_gicp_robust", "psulvsb_gicp_robust_host", "psulvsb_gicp_robust_batch", "psulvsb_gicp_robust_batch_host",
     "psulvsb_normals_workspace_bytes", "psulvsb_normals", "psulvsb_normals_host",
     "psulvsb_normals_batch_workspace_bytes", "psulvsb_normals_batch", "psulvsb_normals_batch_host",
     "psulvsb_voxel_down_sample_workspace_bytes", "psulvsb_voxel_down_sample", "psulvsb_voxel_down_sample_host",
@@ -211,6 +213,17 @@ class GicpPair(C.Structure):
     ]
 
 
+LOSS_L2, LOSS_HUBER, LOSS_CAUCHY, LOSS_GM, LOSS_TUKEY = range(5)
+
+
+class RobustKernel(C.Structure):
+    """psulvsb_robust_kernel_t: a PSULVSB_LOSS_* type and its scale k."""
+    _fields_ = [
+        ("type", C.c_int),
+        ("k", C.c_double),
+    ]
+
+
 class FpfhCloud(C.Structure):
     """psulvsb_fpfh_cloud_t: one cloud of an FPFH batch."""
     _fields_ = [
@@ -359,6 +372,22 @@ def _declare(L: C.CDLL) -> None:
                                      _vp, _vp]
     L.psulvsb_gicp_batch_host.argtypes = [C.POINTER(GicpPair), C.c_int, C.POINTER(IcpParams), C.c_double, _vp, _vp,
                                           _vp]
+    _rk = C.POINTER(RobustKernel)
+    L.psulvsb_icp_robust.argtypes = [_vp, _vp, C.c_int, _vp, C.c_int, _vp, C.POINTER(IcpParams), _rk,
+                                     C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]
+    L.psulvsb_icp_robust_host.argtypes = [_vp, C.c_int, _vp, C.c_int, _vp, C.POINTER(IcpParams), _rk,
+                                          C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp]
+    L.psulvsb_icp_robust_batch.argtypes = [_vp, C.POINTER(IcpPair), C.c_int, C.POINTER(IcpParams), _rk, _vp, _vp, _vp,
+                                           _vp]
+    L.psulvsb_icp_robust_batch_host.argtypes = [C.POINTER(IcpPair), C.c_int, C.POINTER(IcpParams), _rk, _vp, _vp, _vp]
+    L.psulvsb_gicp_robust.argtypes = [_vp, _vp, C.c_int, _vp, _vp, C.c_int, _vp, C.POINTER(IcpParams), C.c_double, _rk,
+                                      C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]
+    L.psulvsb_gicp_robust_host.argtypes = [_vp, C.c_int, _vp, _vp, C.c_int, _vp, C.POINTER(IcpParams), C.c_double,
+                                           _rk, C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp]
+    L.psulvsb_gicp_robust_batch.argtypes = [_vp, C.POINTER(GicpPair), C.c_int, C.POINTER(IcpParams), C.c_double, _rk,
+                                            _vp, _vp, _vp, _vp]
+    L.psulvsb_gicp_robust_batch_host.argtypes = [C.POINTER(GicpPair), C.c_int, C.POINTER(IcpParams), C.c_double, _rk,
+                                                 _vp, _vp, _vp]
     L.psulvsb_fpfh_batch_workspace_bytes.argtypes = [C.POINTER(FpfhCloud), C.c_int]
     L.psulvsb_fpfh_batch_workspace_bytes.restype = _ull
     L.psulvsb_fpfh_batch.argtypes = [_vp, C.POINTER(FpfhCloud), C.c_int, C.c_double, C.c_double, _vp, _vp, _vp]

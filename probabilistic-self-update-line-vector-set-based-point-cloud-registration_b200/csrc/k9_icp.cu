@@ -12,6 +12,9 @@
 //   k9_icp_correspond  one thread per source point, one CTA per (pair, 128-point tile): transform, nearest target
 //                      within d over the 27 cells, per-CTA sums (point-to-plane: the 6x6 system's terms);
 //   k9_gicp_correspond the same pass for generalized ICP, whose per-CTA sums are its 6x6 system's terms;
+//   k9_robust_p2l_correspond, k9_robust_gicp_correspond
+//                      the same passes with a robust kernel: each point-to-plane row, and each row of GICP's whitened
+//                      residual, weighted by rho(r) (tests/robust_icp_restatement.py);
 //   k9_icp_cross       (point-to-point) the centred cross-covariance H over the correspondences, per-CTA sums;
 //   k9_icp_step        one CTA per pair: the pair's CTA sums in a fixed order, trace record k, the stop rule, the
 //                      update U, T <- U T.
@@ -304,14 +307,108 @@ __device__ __forceinline__ void gicp_terms(const double p[3], const double q[3],
   }
 }
 
+// ---- robust kernels (DESIGN.md section 11, "Robust kernels"); every operation in the order written, which
+// tests/robust_icp_restatement.py repeats elementwise in numpy
+
+// the weight rho(r) of a residual under the call's loss (type and k checked by the entry points)
+__device__ __forceinline__ double robust_weight(const psulvsb_robust_kernel_t& loss, double r) {
+  const double k = loss.k;
+  switch (loss.type) {
+    case PSULVSB_LOSS_HUBER:
+      return __ddiv_rn(k, fmax(fabs(r), k));
+    case PSULVSB_LOSS_CAUCHY: {
+      const double q = __ddiv_rn(r, k);
+      return __ddiv_rn(1.0, dadd(1.0, dmul(q, q)));
+    }
+    case PSULVSB_LOSS_GM: {
+      const double s = dadd(k, dmul(r, r));
+      return __ddiv_rn(k, dmul(s, s));
+    }
+    case PSULVSB_LOSS_TUKEY: {
+      const double t = fmin(1.0, __ddiv_rn(fabs(r), k));
+      const double u = dsub(1.0, dmul(t, t));
+      return dmul(u, u);
+    }
+    default:
+      return 1.0;
+  }
+}
+
+// c[0, 27) of one weighted point-to-plane row: r = d . o, J = [p' x o, o], u = rho(r) J; J^T J (upper triangle row by
+// row) as u_a J_e and J^T r as u_a r.  ACC adds them to c, else they are written.  With rho = 1 the terms are exactly
+// the point-to-plane pass's.
+template <bool ACC>
+__device__ __forceinline__ void robust_row_terms(double px, double py, double pz, const double d[3], double ox,
+                                                 double oy, double oz, const psulvsb_robust_kernel_t& loss,
+                                                 double* __restrict__ c) {
+  const double r = dadd(dadd(dmul(d[0], ox), dmul(d[1], oy)), dmul(d[2], oz));
+  const double J[6] = {dsub(dmul(py, oz), dmul(pz, oy)), dsub(dmul(pz, ox), dmul(px, oz)),
+                       dsub(dmul(px, oy), dmul(py, ox)), ox, oy, oz};
+  const double rho = robust_weight(loss, r);
+  double u[6];
+#pragma unroll
+  for (int a = 0; a < 6; ++a) u[a] = dmul(rho, J[a]);
+  int v = 0;
+#pragma unroll
+  for (int a = 0; a < 6; ++a)
+#pragma unroll
+    for (int e = a; e < 6; ++e, ++v) c[v] = ACC ? dadd(c[v], dmul(u[a], J[e])) : dmul(u[a], J[e]);
+#pragma unroll
+  for (int a = 0; a < 6; ++a) c[21 + a] = ACC ? dadd(c[21 + a], dmul(u[a], r)) : dmul(u[a], r);
+}
+
+// beta(lambda) = w / ((2 sqrt2 a)(sqrt2 + a)), a = sqrt(2 - w lambda): the coefficient of v v^T in C^-1/2 for the
+// eigenvalue w lambda of w (m m^T + n n^T) along v, |v|^2 = 2 lambda
+__device__ __forceinline__ double whiten_beta(double w, double lambda) {
+  constexpr double SQRT2 = 1.4142135623730951, TWO_SQRT2 = 2.8284271247461903;
+  const double a = __dsqrt_rn(dsub(2.0, dmul(w, lambda)));
+  return __ddiv_rn(w, dmul(dmul(TWO_SQRT2, a), dadd(SQRT2, a)));
+}
+
+// W = C^-1/2 for C = 2 I - w (m m^T + n n^T) in closed form, as (W00, W01, W02, W11, W12, W22); m or n = 0 (a side
+// whose covariance is I) drops that normal.  W = I / sqrt2 + b1 v1 v1^T + b2 v2 v2^T, entry (i, j) as (b v_i) v_j:
+// both normals: v1,2 = m +- s n with s = sign(m . n) (+1 at 0), b_k = beta(|v_k|^2 / 2); one normal v: b1 = 2 beta(1),
+// b2 = 0; neither: I / sqrt2.  Orthogonal v1, v2 avoid the cancellation of an eigensolver as m -> +-n.
+__device__ __forceinline__ void whitening(const double m[3], const double n[3], double w, double W[6]) {
+  const bool hm = m[0] != 0.0 || m[1] != 0.0 || m[2] != 0.0, hn = n[0] != 0.0 || n[1] != 0.0 || n[2] != 0.0;
+  double v1[3], v2[3], b1 = 0.0, b2 = 0.0;
+  if (hm && hn) {
+    const bool neg = dadd(dadd(dmul(m[0], n[0]), dmul(m[1], n[1])), dmul(m[2], n[2])) < 0.0;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+      v1[r] = neg ? dsub(m[r], n[r]) : dadd(m[r], n[r]);
+      v2[r] = neg ? dadd(m[r], n[r]) : dsub(m[r], n[r]);
+    }
+    b1 = whiten_beta(w, dmul(dadd(dadd(dmul(v1[0], v1[0]), dmul(v1[1], v1[1])), dmul(v1[2], v1[2])), 0.5));
+    b2 = whiten_beta(w, dmul(dadd(dadd(dmul(v2[0], v2[0]), dmul(v2[1], v2[1])), dmul(v2[2], v2[2])), 0.5));
+  } else {
+    const double* v = hm ? m : n;  // zeros when neither
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+      v1[r] = v[r];
+      v2[r] = 0.0;
+    }
+    if (hm || hn) b1 = dmul(2.0, whiten_beta(w, 1.0));
+  }
+  constexpr double INV_SQRT2 = 0.7071067811865476;
+  int e = 0;
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int j = i; j < 3; ++j)
+      W[e++] = dadd(dadd(i == j ? INV_SQRT2 : 0.0, dmul(dmul(b1, v1[i]), v1[j])), dmul(dmul(b2, v2[i]), v2[j]));
+}
+
 // ---- evaluation of T_k: corr[i] = the target at the smallest d^2 <= dd (ties: lowest index) or -1, and the CTA sums
 // of what the step needs (point-to-point: count, sum d^2, sum p', sum q; point-to-plane: count, sum d^2, J^T J, J^T r;
-// GICP: count, sum d^2, A^T M A, A^T M d with w = 1 - epsilon); the body of k9_icp_correspond and k9_gicp_correspond
-template <int MODE>
+// GICP: count, sum d^2, A^T M A, A^T M d with w = 1 - epsilon; ROBUST: the same layout, the terms weighted by `loss`);
+// the body of k9_icp_correspond, k9_gicp_correspond and the robust passes
+template <int MODE, bool ROBUST = false>
 __device__ __forceinline__ void correspond(const IcpPair* __restrict__ pairs, const int* __restrict__ tile_first, int B,
                                            const double4* __restrict__ rec, const int* __restrict__ start,
                                            double inv_h, const IcpState* __restrict__ states, double dd, double w,
-                                           int* __restrict__ corr, double* __restrict__ partials) {
+                                           psulvsb_robust_kernel_t loss, int* __restrict__ corr,
+                                           double* __restrict__ partials) {
   // the pair, its bucket mask and its start table are read from shared memory at each use: held in registers across
   // the 27-cell walk they push the point-to-plane instantiation past 128 registers (4 CTAs per SM) into spills
   __shared__ volatile int s_pair, s_start;
@@ -381,6 +478,26 @@ __device__ __forceinline__ void correspond(const IcpPair* __restrict__ pairs, co
         c[5] = qx;
         c[6] = qy;
         c[7] = qz;
+      } else if constexpr (ROBUST) {
+        const double d[3] = {dsub(px, qx), dsub(py, qy), dsub(pz, qz)};
+        if constexpr (MODE == P2L) {
+          const double* normals = pairs[s_pair].nrm;
+          robust_row_terms<false>(px, py, pz, d, normals[3 * (size_t)bj], normals[3 * (size_t)bj + 1],
+                                  normals[3 * (size_t)bj + 2], loss, c + 2);
+        } else {
+          // GICP whitened by W = C^-1/2: its three rows, each a point-to-plane row, added in order
+          double a[3], n[3], m[3], W[6];
+          unit_normal(pairs[s_pair].snrm + 3 * (size_t)i, a);
+          unit_normal(pairs[s_pair].nrm + 3 * (size_t)bj, n);
+          const double* R = st->R;
+#pragma unroll
+          for (int r = 0; r < 3; ++r)
+            m[r] = dadd(dadd(dmul(R[3 * r], a[0]), dmul(R[3 * r + 1], a[1])), dmul(R[3 * r + 2], a[2]));
+          whitening(m, n, w, W);
+          robust_row_terms<false>(px, py, pz, d, W[0], W[1], W[2], loss, c + 2);
+          robust_row_terms<true>(px, py, pz, d, W[1], W[3], W[4], loss, c + 2);
+          robust_row_terms<true>(px, py, pz, d, W[2], W[4], W[5], loss, c + 2);
+        }
       } else if constexpr (MODE == P2L) {
         const double* normals = pairs[s_pair].nrm;
         const double nx = normals[3 * (size_t)bj], ny = normals[3 * (size_t)bj + 1], nz = normals[3 * (size_t)bj + 2];
@@ -419,7 +536,8 @@ __global__ void __launch_bounds__(ICP_THREADS)
                       const double4* __restrict__ rec, const int* __restrict__ start, double inv_h,
                       const IcpState* __restrict__ states, double dd, int* __restrict__ corr,
                       double* __restrict__ partials) {
-  correspond<MODE>(pairs, tile_first, B, rec, start, inv_h, states, dd, 0.0, corr, partials);
+  correspond<MODE>(pairs, tile_first, B, rec, start, inv_h, states, dd, 0.0, psulvsb_robust_kernel_t{}, corr,
+                   partials);
 }
 
 // generalized ICP, w = 1 - epsilon: the same pass under its own name
@@ -428,7 +546,25 @@ __global__ void __launch_bounds__(ICP_THREADS)
                        const double4* __restrict__ rec, const int* __restrict__ start, double inv_h,
                        const IcpState* __restrict__ states, double dd, double w, int* __restrict__ corr,
                        double* __restrict__ partials) {
-  correspond<GICP>(pairs, tile_first, B, rec, start, inv_h, states, dd, w, corr, partials);
+  correspond<GICP>(pairs, tile_first, B, rec, start, inv_h, states, dd, w, psulvsb_robust_kernel_t{}, corr, partials);
+}
+
+// point-to-plane with a robust kernel: the partials of k9_icp_correspond<P2L>, weighted
+__global__ void __launch_bounds__(ICP_THREADS)
+    k9_robust_p2l_correspond(const IcpPair* __restrict__ pairs, const int* __restrict__ tile_first, int B,
+                             const double4* __restrict__ rec, const int* __restrict__ start, double inv_h,
+                             const IcpState* __restrict__ states, double dd, psulvsb_robust_kernel_t loss,
+                             int* __restrict__ corr, double* __restrict__ partials) {
+  correspond<P2L, true>(pairs, tile_first, B, rec, start, inv_h, states, dd, 0.0, loss, corr, partials);
+}
+
+// generalized ICP with a robust kernel, w = 1 - epsilon: the whitened rows, weighted, in GICP's partials layout
+__global__ void __launch_bounds__(ICP_THREADS)
+    k9_robust_gicp_correspond(const IcpPair* __restrict__ pairs, const int* __restrict__ tile_first, int B,
+                              const double4* __restrict__ rec, const int* __restrict__ start, double inv_h,
+                              const IcpState* __restrict__ states, double dd, double w, psulvsb_robust_kernel_t loss,
+                              int* __restrict__ corr, double* __restrict__ partials) {
+  correspond<GICP, true>(pairs, tile_first, B, rec, start, inv_h, states, dd, w, loss, corr, partials);
 }
 
 // ---- point-to-point: H = sum (p' - mu_p)(q - mu_q)^T over the correspondences of T_k
@@ -715,11 +851,13 @@ void empty_result(const double* R0, const double* t0, psulvsb_icp_result_t* res,
   res->status = PSULVSB_ICP_NO_UPDATE;
 }
 
-// what a call minimises: the mode, GICP's source normals (one pointer per pair, else nullptr) and w = 1 - epsilon
+// what a call minimises: the mode, GICP's source normals (one pointer per pair, else nullptr), w = 1 - epsilon and
+// the robust kernel of point-to-plane / GICP (nullptr: none)
 struct Objective {
   Mode mode;
   const double* const* src_normals;
   double w;
+  const psulvsb_robust_kernel_t* loss = nullptr;
 };
 
 Objective icp_objective(const psulvsb_icp_params_t& prm) {
@@ -787,13 +925,21 @@ int run_icp(cudaStream_t st, const psulvsb_icp_pair_t* pairs, int B, const psulv
     const double dd = d * d;
     for (int k = 0; k <= prm.max_iterations; ++k) {
       if (obj.mode == P2L) {
-        k9_icp_correspond<P2L><<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.rec, w.start, inv_h,
-                                                              w.state, dd, w.corr, w.partials);
+        if (obj.loss)
+          k9_robust_p2l_correspond<<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.rec, w.start, inv_h,
+                                                                  w.state, dd, *obj.loss, w.corr, w.partials);
+        else
+          k9_icp_correspond<P2L><<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.rec, w.start, inv_h,
+                                                                w.state, dd, w.corr, w.partials);
         k9_icp_step<P2L><<<B, STEP_THREADS, 0, st>>>(0, w.pair, w.tile_first, w.partials, sp, w.state, d_trace,
                                                      d_results);
       } else if (obj.mode == GICP) {
-        k9_gicp_correspond<<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.rec, w.start, inv_h, w.state,
-                                                          dd, obj.w, w.corr, w.partials);
+        if (obj.loss)
+          k9_robust_gicp_correspond<<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.rec, w.start, inv_h,
+                                                                   w.state, dd, obj.w, *obj.loss, w.corr, w.partials);
+        else
+          k9_gicp_correspond<<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.rec, w.start, inv_h, w.state,
+                                                            dd, obj.w, w.corr, w.partials);
         k9_icp_step<GICP><<<B, STEP_THREADS, 0, st>>>(0, w.pair, w.tile_first, w.partials, sp, w.state, d_trace,
                                                       d_results);
       } else {
@@ -949,6 +1095,140 @@ psulvsb_icp_pair_t one_pair(const double* src, int n_s, const double* tgt, int n
   return p;
 }
 
+bool loss_ok(const psulvsb_robust_kernel_t* loss) {
+  if (!loss || loss->type < PSULVSB_LOSS_L2 || loss->type > PSULVSB_LOSS_TUKEY) return false;
+  return loss->type == PSULVSB_LOSS_L2 || (std::isfinite(loss->k) && loss->k > 0.0);
+}
+
+// the robust ICP entry points are point-to-plane: Open3D has no robust point-to-point
+bool icp_loss_ok(const psulvsb_icp_params_t* params, const psulvsb_robust_kernel_t* loss) {
+  return loss_ok(loss) && params && params->point_to_plane == 1;
+}
+
+// the entry points of ICP and GICP, plain (loss nullptr) or robust; `who` names the entry point in errors
+int icp_single(void* stream, const double* d_src, int n_s, const double* d_tgt, int n_t, const double* d_tgt_normals,
+               const psulvsb_icp_params_t* params, const psulvsb_robust_kernel_t* loss, const double R0[9],
+               const double t0[3], void* d_work, psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace,
+               int* d_corr, const char* who) {
+  if (n_s < 0 || n_t < 0 || !icp_params_ok(params) || !transform_ok(R0, t0) || !d_result ||
+      (params->point_to_plane && !d_tgt_normals) || (n_s > 0 && !d_src) || (n_t > 0 && !d_tgt) ||
+      (n_s > 0 && n_t > 0 && !d_work))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  if (int rc = need_device()) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (n_s == 0 || n_t == 0) return empty_device(st, n_s, R0, t0, d_result, d_trace, d_corr);
+  const psulvsb_icp_pair_t p = one_pair(d_src, n_s, d_tgt, n_t, d_tgt_normals, R0, t0);
+  Objective obj = icp_objective(*params);
+  obj.loss = loss;
+  return run_icp(st, &p, 1, *params, obj, d_work, d_result, d_trace, d_corr);
+}
+
+int icp_single_host(const double* src, int n_s, const double* tgt, int n_t, const double* tgt_normals,
+                    const psulvsb_icp_params_t* params, const psulvsb_robust_kernel_t* loss, const double R0[9],
+                    const double t0[3], psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace, int* corr,
+                    const char* who) {
+  if (n_s < 0 || n_t < 0 || !icp_params_ok(params) || !transform_ok(R0, t0) || !result ||
+      (params->point_to_plane && !tgt_normals) || (n_s > 0 && !src) || (n_t > 0 && !tgt))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  if (int rc = need_device()) return rc;
+  if (n_s == 0 || n_t == 0) {
+    empty_host(n_s, R0, t0, result, trace, corr);
+    return PSULVSB_OK;
+  }
+  const psulvsb_icp_pair_t p = one_pair(src, n_s, tgt, n_t, tgt_normals, R0, t0);
+  Objective obj = icp_objective(*params);
+  obj.loss = loss;
+  return run_icp_host(&p, 1, *params, obj, result, trace, corr, who);
+}
+
+int icp_batch(void* stream, const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+              const psulvsb_robust_kernel_t* loss, void* d_work, psulvsb_icp_result_t* d_results,
+              psulvsb_icp_iteration_t* d_trace, int* d_corr, const char* who) {
+  if (B < 0 || !icp_params_ok(params) || (B > 0 && (!pairs || !d_work || !d_results)))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  if (int rc = pairs_check(pairs, B, params, who)) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = need_device()) return rc;
+  Objective obj = icp_objective(*params);
+  obj.loss = loss;
+  return run_icp((cudaStream_t)stream, pairs, B, *params, obj, d_work, d_results, d_trace, d_corr);
+}
+
+int icp_batch_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                   const psulvsb_robust_kernel_t* loss, psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace,
+                   int* corr, const char* who) {
+  if (B < 0 || !icp_params_ok(params) || (B > 0 && (!pairs || !results)))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  if (int rc = pairs_check(pairs, B, params, who)) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = need_device()) return rc;
+  Objective obj = icp_objective(*params);
+  obj.loss = loss;
+  return run_icp_host(pairs, B, *params, obj, results, trace, corr, who);
+}
+
+int gicp_single(void* stream, const double* d_src, int n_s, const double* d_src_normals, const double* d_tgt, int n_t,
+                const double* d_tgt_normals, const psulvsb_icp_params_t* params, double epsilon,
+                const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3], void* d_work,
+                psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr, const char* who) {
+  const bool both = n_s > 0 && n_t > 0;
+  if (n_s < 0 || n_t < 0 || !gicp_params_ok(params, epsilon) || !transform_ok(R0, t0) || !d_result ||
+      (n_s > 0 && !d_src) || (n_t > 0 && !d_tgt) || (both && (!d_work || !d_src_normals || !d_tgt_normals)))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  if (int rc = need_device()) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!both) return empty_device(st, n_s, R0, t0, d_result, d_trace, d_corr);
+  const psulvsb_icp_pair_t p = one_pair(d_src, n_s, d_tgt, n_t, d_tgt_normals, R0, t0);
+  const Objective obj{GICP, &d_src_normals, 1.0 - epsilon, loss};
+  return run_icp(st, &p, 1, *params, obj, d_work, d_result, d_trace, d_corr);
+}
+
+int gicp_single_host(const double* src, int n_s, const double* src_normals, const double* tgt, int n_t,
+                     const double* tgt_normals, const psulvsb_icp_params_t* params, double epsilon,
+                     const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3],
+                     psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace, int* corr, const char* who) {
+  const bool both = n_s > 0 && n_t > 0;
+  if (n_s < 0 || n_t < 0 || !gicp_params_ok(params, epsilon) || !transform_ok(R0, t0) || !result ||
+      (n_s > 0 && !src) || (n_t > 0 && !tgt) || (both && (!src_normals || !tgt_normals)))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  if (int rc = need_device()) return rc;
+  if (!both) {
+    empty_host(n_s, R0, t0, result, trace, corr);
+    return PSULVSB_OK;
+  }
+  const psulvsb_icp_pair_t p = one_pair(src, n_s, tgt, n_t, tgt_normals, R0, t0);
+  const Objective obj{GICP, &src_normals, 1.0 - epsilon, loss};
+  return run_icp_host(&p, 1, *params, obj, result, trace, corr, who);
+}
+
+int gicp_batch(void* stream, const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+               double epsilon, const psulvsb_robust_kernel_t* loss, void* d_work, psulvsb_icp_result_t* d_results,
+               psulvsb_icp_iteration_t* d_trace, int* d_corr, const char* who) {
+  if (B < 0 || !gicp_params_ok(params, epsilon) || (B > 0 && (!pairs || !d_work || !d_results)))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  std::vector<psulvsb_icp_pair_t> icp;
+  std::vector<const double*> snrm;
+  if (int rc = gicp_pairs(pairs, B, params, icp, snrm, who)) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = need_device()) return rc;
+  const Objective obj{GICP, snrm.data(), 1.0 - epsilon, loss};
+  return run_icp((cudaStream_t)stream, icp.data(), B, *params, obj, d_work, d_results, d_trace, d_corr);
+}
+
+int gicp_batch_host(const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_params_t* params, double epsilon,
+                    const psulvsb_robust_kernel_t* loss, psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace,
+                    int* corr, const char* who) {
+  if (B < 0 || !gicp_params_ok(params, epsilon) || (B > 0 && (!pairs || !results)))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  std::vector<psulvsb_icp_pair_t> icp;
+  std::vector<const double*> snrm;
+  if (int rc = gicp_pairs(pairs, B, params, icp, snrm, who)) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = need_device()) return rc;
+  const Objective obj{GICP, snrm.data(), 1.0 - epsilon, loss};
+  return run_icp_host(icp.data(), B, *params, obj, results, trace, corr, who);
+}
+
 }  // namespace
 
 }  // namespace psulvsb
@@ -982,88 +1262,41 @@ unsigned long long psulvsb_icp_batch_workspace_bytes(const psulvsb_icp_pair_t* p
 int psulvsb_icp(void* stream, const double* d_src, int n_s, const double* d_tgt, int n_t, const double* d_tgt_normals,
                 const psulvsb_icp_params_t* params, const double R0[9], const double t0[3], void* d_work,
                 psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr) {
-  if (n_s < 0 || n_t < 0 || !psulvsb::icp_params_ok(params) || !psulvsb::transform_ok(R0, t0) || !d_result ||
-      (params->point_to_plane && !d_tgt_normals) || (n_s > 0 && !d_src) || (n_t > 0 && !d_tgt) ||
-      (n_s > 0 && n_t > 0 && !d_work))
-    return fail(PSULVSB_ERR_INVALID, "psulvsb_icp: bad argument");
-  if (int rc = psulvsb::need_device()) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (n_s == 0 || n_t == 0) return psulvsb::empty_device(st, n_s, R0, t0, d_result, d_trace, d_corr);
-  const psulvsb_icp_pair_t p = psulvsb::one_pair(d_src, n_s, d_tgt, n_t, d_tgt_normals, R0, t0);
-  return psulvsb::run_icp(st, &p, 1, *params, psulvsb::icp_objective(*params), d_work, d_result, d_trace, d_corr);
+  return psulvsb::icp_single(stream, d_src, n_s, d_tgt, n_t, d_tgt_normals, params, nullptr, R0, t0, d_work, d_result,
+                             d_trace, d_corr, "psulvsb_icp");
 }
 
 int psulvsb_icp_host(const double* src, int n_s, const double* tgt, int n_t, const double* tgt_normals,
                      const psulvsb_icp_params_t* params, const double R0[9], const double t0[3],
                      psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace, int* corr) {
-  if (n_s < 0 || n_t < 0 || !psulvsb::icp_params_ok(params) || !psulvsb::transform_ok(R0, t0) || !result ||
-      (params->point_to_plane && !tgt_normals) || (n_s > 0 && !src) || (n_t > 0 && !tgt))
-    return fail(PSULVSB_ERR_INVALID, "psulvsb_icp_host: bad argument");
-  if (int rc = psulvsb::need_device()) return rc;
-  if (n_s == 0 || n_t == 0) {
-    psulvsb::empty_host(n_s, R0, t0, result, trace, corr);
-    return PSULVSB_OK;
-  }
-  const psulvsb_icp_pair_t p = psulvsb::one_pair(src, n_s, tgt, n_t, tgt_normals, R0, t0);
-  return psulvsb::run_icp_host(&p, 1, *params, psulvsb::icp_objective(*params), result, trace, corr,
-                               "psulvsb_icp_host");
+  return psulvsb::icp_single_host(src, n_s, tgt, n_t, tgt_normals, params, nullptr, R0, t0, result, trace, corr,
+                                  "psulvsb_icp_host");
 }
 
 int psulvsb_icp_batch(void* stream, const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
                       void* d_work, psulvsb_icp_result_t* d_results, psulvsb_icp_iteration_t* d_trace, int* d_corr) {
-  if (B < 0 || !psulvsb::icp_params_ok(params) || (B > 0 && (!pairs || !d_work || !d_results)))
-    return fail(PSULVSB_ERR_INVALID, "psulvsb_icp_batch: bad argument");
-  if (int rc = psulvsb::pairs_check(pairs, B, params, "psulvsb_icp_batch")) return rc;
-  if (B == 0) return PSULVSB_OK;
-  if (int rc = psulvsb::need_device()) return rc;
-  return psulvsb::run_icp((cudaStream_t)stream, pairs, B, *params, psulvsb::icp_objective(*params), d_work, d_results,
-                          d_trace, d_corr);
+  return psulvsb::icp_batch(stream, pairs, B, params, nullptr, d_work, d_results, d_trace, d_corr, "psulvsb_icp_batch");
 }
 
 int psulvsb_icp_batch_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
                            psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr) {
-  if (B < 0 || !psulvsb::icp_params_ok(params) || (B > 0 && (!pairs || !results)))
-    return fail(PSULVSB_ERR_INVALID, "psulvsb_icp_batch_host: bad argument");
-  if (int rc = psulvsb::pairs_check(pairs, B, params, "psulvsb_icp_batch_host")) return rc;
-  if (B == 0) return PSULVSB_OK;
-  if (int rc = psulvsb::need_device()) return rc;
-  return psulvsb::run_icp_host(pairs, B, *params, psulvsb::icp_objective(*params), results, trace, corr,
-                               "psulvsb_icp_batch_host");
+  return psulvsb::icp_batch_host(pairs, B, params, nullptr, results, trace, corr, "psulvsb_icp_batch_host");
 }
 
 int psulvsb_gicp(void* stream, const double* d_src, int n_s, const double* d_src_normals, const double* d_tgt, int n_t,
                  const double* d_tgt_normals, const psulvsb_icp_params_t* params, double epsilon, const double R0[9],
                  const double t0[3], void* d_work, psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace,
                  int* d_corr) {
-  const bool both = n_s > 0 && n_t > 0;
-  if (n_s < 0 || n_t < 0 || !psulvsb::gicp_params_ok(params, epsilon) || !psulvsb::transform_ok(R0, t0) ||
-      !d_result || (n_s > 0 && !d_src) || (n_t > 0 && !d_tgt) ||
-      (both && (!d_work || !d_src_normals || !d_tgt_normals)))
-    return fail(PSULVSB_ERR_INVALID, "psulvsb_gicp: bad argument");
-  if (int rc = psulvsb::need_device()) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (!both) return psulvsb::empty_device(st, n_s, R0, t0, d_result, d_trace, d_corr);
-  const psulvsb_icp_pair_t p = psulvsb::one_pair(d_src, n_s, d_tgt, n_t, d_tgt_normals, R0, t0);
-  const psulvsb::Objective obj{psulvsb::GICP, &d_src_normals, 1.0 - epsilon};
-  return psulvsb::run_icp(st, &p, 1, *params, obj, d_work, d_result, d_trace, d_corr);
+  return psulvsb::gicp_single(stream, d_src, n_s, d_src_normals, d_tgt, n_t, d_tgt_normals, params, epsilon, nullptr,
+                              R0, t0, d_work, d_result, d_trace, d_corr, "psulvsb_gicp");
 }
 
 int psulvsb_gicp_host(const double* src, int n_s, const double* src_normals, const double* tgt, int n_t,
                       const double* tgt_normals, const psulvsb_icp_params_t* params, double epsilon,
                       const double R0[9], const double t0[3], psulvsb_icp_result_t* result,
                       psulvsb_icp_iteration_t* trace, int* corr) {
-  const bool both = n_s > 0 && n_t > 0;
-  if (n_s < 0 || n_t < 0 || !psulvsb::gicp_params_ok(params, epsilon) || !psulvsb::transform_ok(R0, t0) || !result ||
-      (n_s > 0 && !src) || (n_t > 0 && !tgt) || (both && (!src_normals || !tgt_normals)))
-    return fail(PSULVSB_ERR_INVALID, "psulvsb_gicp_host: bad argument");
-  if (int rc = psulvsb::need_device()) return rc;
-  if (!both) {
-    psulvsb::empty_host(n_s, R0, t0, result, trace, corr);
-    return PSULVSB_OK;
-  }
-  const psulvsb_icp_pair_t p = psulvsb::one_pair(src, n_s, tgt, n_t, tgt_normals, R0, t0);
-  const psulvsb::Objective obj{psulvsb::GICP, &src_normals, 1.0 - epsilon};
-  return psulvsb::run_icp_host(&p, 1, *params, obj, result, trace, corr, "psulvsb_gicp_host");
+  return psulvsb::gicp_single_host(src, n_s, src_normals, tgt, n_t, tgt_normals, params, epsilon, nullptr, R0, t0,
+                                   result, trace, corr, "psulvsb_gicp_host");
 }
 
 unsigned long long psulvsb_gicp_batch_workspace_bytes(const psulvsb_gicp_pair_t* pairs, int B) {
@@ -1080,28 +1313,82 @@ unsigned long long psulvsb_gicp_batch_workspace_bytes(const psulvsb_gicp_pair_t*
 int psulvsb_gicp_batch(void* stream, const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
                        double epsilon, void* d_work, psulvsb_icp_result_t* d_results, psulvsb_icp_iteration_t* d_trace,
                        int* d_corr) {
-  if (B < 0 || !psulvsb::gicp_params_ok(params, epsilon) || (B > 0 && (!pairs || !d_work || !d_results)))
-    return fail(PSULVSB_ERR_INVALID, "psulvsb_gicp_batch: bad argument");
-  std::vector<psulvsb_icp_pair_t> icp;
-  std::vector<const double*> snrm;
-  if (int rc = psulvsb::gicp_pairs(pairs, B, params, icp, snrm, "psulvsb_gicp_batch")) return rc;
-  if (B == 0) return PSULVSB_OK;
-  if (int rc = psulvsb::need_device()) return rc;
-  const psulvsb::Objective obj{psulvsb::GICP, snrm.data(), 1.0 - epsilon};
-  return psulvsb::run_icp((cudaStream_t)stream, icp.data(), B, *params, obj, d_work, d_results, d_trace, d_corr);
+  return psulvsb::gicp_batch(stream, pairs, B, params, epsilon, nullptr, d_work, d_results, d_trace, d_corr,
+                             "psulvsb_gicp_batch");
 }
 
 int psulvsb_gicp_batch_host(const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
                             double epsilon, psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr) {
-  if (B < 0 || !psulvsb::gicp_params_ok(params, epsilon) || (B > 0 && (!pairs || !results)))
-    return fail(PSULVSB_ERR_INVALID, "psulvsb_gicp_batch_host: bad argument");
-  std::vector<psulvsb_icp_pair_t> icp;
-  std::vector<const double*> snrm;
-  if (int rc = psulvsb::gicp_pairs(pairs, B, params, icp, snrm, "psulvsb_gicp_batch_host")) return rc;
-  if (B == 0) return PSULVSB_OK;
-  if (int rc = psulvsb::need_device()) return rc;
-  const psulvsb::Objective obj{psulvsb::GICP, snrm.data(), 1.0 - epsilon};
-  return psulvsb::run_icp_host(icp.data(), B, *params, obj, results, trace, corr, "psulvsb_gicp_batch_host");
+  return psulvsb::gicp_batch_host(pairs, B, params, epsilon, nullptr, results, trace, corr, "psulvsb_gicp_batch_host");
+}
+
+int psulvsb_icp_robust(void* stream, const double* d_src, int n_s, const double* d_tgt, int n_t,
+                       const double* d_tgt_normals, const psulvsb_icp_params_t* params,
+                       const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3], void* d_work,
+                       psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr) {
+  if (!psulvsb::icp_loss_ok(params, loss)) return fail(PSULVSB_ERR_INVALID, "psulvsb_icp_robust: bad argument");
+  return psulvsb::icp_single(stream, d_src, n_s, d_tgt, n_t, d_tgt_normals, params, loss, R0, t0, d_work, d_result,
+                             d_trace, d_corr, "psulvsb_icp_robust");
+}
+
+int psulvsb_icp_robust_host(const double* src, int n_s, const double* tgt, int n_t, const double* tgt_normals,
+                            const psulvsb_icp_params_t* params, const psulvsb_robust_kernel_t* loss, const double R0[9],
+                            const double t0[3], psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace,
+                            int* corr) {
+  if (!psulvsb::icp_loss_ok(params, loss)) return fail(PSULVSB_ERR_INVALID, "psulvsb_icp_robust_host: bad argument");
+  return psulvsb::icp_single_host(src, n_s, tgt, n_t, tgt_normals, params, loss, R0, t0, result, trace, corr,
+                                  "psulvsb_icp_robust_host");
+}
+
+int psulvsb_icp_robust_batch(void* stream, const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                             const psulvsb_robust_kernel_t* loss, void* d_work, psulvsb_icp_result_t* d_results,
+                             psulvsb_icp_iteration_t* d_trace, int* d_corr) {
+  if (!psulvsb::icp_loss_ok(params, loss)) return fail(PSULVSB_ERR_INVALID, "psulvsb_icp_robust_batch: bad argument");
+  return psulvsb::icp_batch(stream, pairs, B, params, loss, d_work, d_results, d_trace, d_corr,
+                            "psulvsb_icp_robust_batch");
+}
+
+int psulvsb_icp_robust_batch_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                                  const psulvsb_robust_kernel_t* loss, psulvsb_icp_result_t* results,
+                                  psulvsb_icp_iteration_t* trace, int* corr) {
+  if (!psulvsb::icp_loss_ok(params, loss))
+    return fail(PSULVSB_ERR_INVALID, "psulvsb_icp_robust_batch_host: bad argument");
+  return psulvsb::icp_batch_host(pairs, B, params, loss, results, trace, corr, "psulvsb_icp_robust_batch_host");
+}
+
+int psulvsb_gicp_robust(void* stream, const double* d_src, int n_s, const double* d_src_normals, const double* d_tgt,
+                        int n_t, const double* d_tgt_normals, const psulvsb_icp_params_t* params, double epsilon,
+                        const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3], void* d_work,
+                        psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr) {
+  if (!psulvsb::loss_ok(loss)) return fail(PSULVSB_ERR_INVALID, "psulvsb_gicp_robust: bad argument");
+  return psulvsb::gicp_single(stream, d_src, n_s, d_src_normals, d_tgt, n_t, d_tgt_normals, params, epsilon, loss, R0,
+                              t0, d_work, d_result, d_trace, d_corr, "psulvsb_gicp_robust");
+}
+
+int psulvsb_gicp_robust_host(const double* src, int n_s, const double* src_normals, const double* tgt, int n_t,
+                             const double* tgt_normals, const psulvsb_icp_params_t* params, double epsilon,
+                             const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3],
+                             psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace, int* corr) {
+  if (!psulvsb::loss_ok(loss)) return fail(PSULVSB_ERR_INVALID, "psulvsb_gicp_robust_host: bad argument");
+  return psulvsb::gicp_single_host(src, n_s, src_normals, tgt, n_t, tgt_normals, params, epsilon, loss, R0, t0, result,
+                                   trace, corr, "psulvsb_gicp_robust_host");
+}
+
+int psulvsb_gicp_robust_batch(void* stream, const psulvsb_gicp_pair_t* pairs, int B,
+                              const psulvsb_icp_params_t* params, double epsilon, const psulvsb_robust_kernel_t* loss,
+                              void* d_work, psulvsb_icp_result_t* d_results, psulvsb_icp_iteration_t* d_trace,
+                              int* d_corr) {
+  if (!psulvsb::loss_ok(loss)) return fail(PSULVSB_ERR_INVALID, "psulvsb_gicp_robust_batch: bad argument");
+  return psulvsb::gicp_batch(stream, pairs, B, params, epsilon, loss, d_work, d_results, d_trace, d_corr,
+                             "psulvsb_gicp_robust_batch");
+}
+
+int psulvsb_gicp_robust_batch_host(const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                                   double epsilon, const psulvsb_robust_kernel_t* loss, psulvsb_icp_result_t* results,
+                                   psulvsb_icp_iteration_t* trace, int* corr) {
+  if (!psulvsb::loss_ok(loss)) return fail(PSULVSB_ERR_INVALID, "psulvsb_gicp_robust_batch_host: bad argument");
+  return psulvsb::gicp_batch_host(pairs, B, params, epsilon, loss, results, trace, corr,
+                                  "psulvsb_gicp_robust_batch_host");
 }
 
 }  // extern "C"

@@ -9,6 +9,8 @@ B independent pairs with shared parameters in one call; pair b's result is bit-i
 (plane-to-plane; Open3D's registration_generalized_icp); they need the normals of both clouds, for instance the radius
 or hybrid normals of `features.normals` / `features.normals_batch` (on the grid, without descriptors), the radius
 normals `features.fpfh` returns or the k-NN normals of `stages.estimate_normals`.
+Every call takes `loss=`, a robust kernel of the point-to-plane or generalized-ICP update under Open3D's names
+(`L2Loss`, `HuberLoss`, `CauchyLoss`, `GMLoss`, `TukeyLoss`; DESIGN.md section 11, "Robust kernels").
 Convention: q ~ R p + t.
 """
 from __future__ import annotations
@@ -35,6 +37,55 @@ class IcpResult:
     status: int                    # CONVERGED, MAX_ITERATIONS or NO_UPDATE
     correspondences: object        # [n_src] int32 target index or -1 (numpy; a CUDA tensor from icp_device)
     trace: Optional[dict] = None   # per evaluation k = 0 .. iterations: R [K, 3, 3], t, fitness, inlier_rmse, n_corr
+
+
+class RobustKernel:
+    """psulvsb_robust_kernel_t: the weight rho(r) of a residual in the point-to-plane and generalized-ICP updates."""
+    type = capi.LOSS_L2
+
+    def __init__(self, k: float = 1.0):
+        self.k = float(k)
+
+    def __repr__(self):
+        return f"{type(self).__name__}(k={self.k})"
+
+    def _c(self):
+        return C.byref(capi.RobustKernel(self.type, self.k))
+
+
+class L2Loss(RobustKernel):
+    """rho = 1: the plain update through the robust entry points."""
+    type = capi.LOSS_L2
+
+    def __init__(self):
+        super().__init__(1.0)
+
+
+class HuberLoss(RobustKernel):
+    """rho = k / max(|r|, k)."""
+    type = capi.LOSS_HUBER
+
+
+class CauchyLoss(RobustKernel):
+    """rho = 1 / (1 + (r / k)^2)."""
+    type = capi.LOSS_CAUCHY
+
+
+class GMLoss(RobustKernel):
+    """Geman-McClure, rho = k / (k + r^2)^2."""
+    type = capi.LOSS_GM
+
+
+class TukeyLoss(RobustKernel):
+    """rho = (1 - min(1, |r| / k)^2)^2: 0 beyond k."""
+    type = capi.LOSS_TUKEY
+
+
+def _icp_loss(loss, point_to_plane):
+    """The robust kernel of an ICP call: point-to-plane only, as in Open3D."""
+    if not point_to_plane:
+        raise ValueError("a robust kernel needs point_to_plane=True (Open3D has no robust point-to-point)")
+    return loss._c()
 
 
 def _cm(a, what) -> np.ndarray:
@@ -79,9 +130,10 @@ def _result(res: capi.IcpResult, records, corr) -> IcpResult:
 
 def icp(src, tgt, R0, t0, max_correspondence_distance: float, *, target_normals=None, point_to_plane: bool = False,
         max_iterations: int = 30, relative_fitness: float = 1e-6, relative_rmse: float = 1e-6,
-        trace: bool = False) -> IcpResult:
+        trace: bool = False, loss: Optional[RobustKernel] = None) -> IcpResult:
     """psulvsb_icp_host: refine (R0, t0) so that tgt ~ R src + t.  src 3 x n_s, tgt 3 x n_t; target_normals 3 x n_t is
-    required for point-to-plane (a target point with a non-finite normal is then no candidate)."""
+    required for point-to-plane (a target point with a non-finite normal is then no candidate).  loss: a robust kernel
+    (point-to-plane only; psulvsb_icp_robust_host)."""
     s, q = _cm(src, "src"), _cm(tgt, "tgt")
     nrm = None
     if target_normals is not None:
@@ -93,18 +145,22 @@ def icp(src, tgt, R0, t0, max_correspondence_distance: float, *, target_normals=
     res = capi.IcpResult()
     records = (capi.IcpIteration * (max(int(max_iterations), 0) + 1))() if trace else None
     corr = np.empty(s.shape[1], dtype=np.int32)
-    capi.check(capi.lib().psulvsb_icp_host(s.ctypes.data, s.shape[1], q.ctypes.data, q.shape[1],
-                                           None if nrm is None else nrm.ctypes.data, C.byref(p), R, t, C.byref(res),
-                                           records, corr.ctypes.data))
+    head = (s.ctypes.data, s.shape[1], q.ctypes.data, q.shape[1], None if nrm is None else nrm.ctypes.data, C.byref(p))
+    tail = (R, t, C.byref(res), records, corr.ctypes.data)
+    if loss is None:
+        capi.check(capi.lib().psulvsb_icp_host(*head, *tail))
+    else:
+        capi.check(capi.lib().psulvsb_icp_robust_host(*head, _icp_loss(loss, point_to_plane), *tail))
     return _result(res, records, corr)
 
 
 def icp_device(d_src, d_tgt, R0, t0, max_correspondence_distance: float, *, d_target_normals=None,
                point_to_plane: bool = False, max_iterations: int = 30, relative_fitness: float = 1e-6,
-               relative_rmse: float = 1e-6, trace: bool = False, work=None) -> IcpResult:
+               relative_rmse: float = 1e-6, trace: bool = False, work=None,
+               loss: Optional[RobustKernel] = None) -> IcpResult:
     """psulvsb_icp on CUDA tensors [n, 3] float64 and the current stream.  The small result (and the trace) are read
     back, which waits for the stream; the correspondences stay on the device.  `work`: an optional uint8 CUDA tensor
-    of at least psulvsb_icp_workspace_bytes(n_s, n_t) bytes to reuse."""
+    of at least psulvsb_icp_workspace_bytes(n_s, n_t) bytes to reuse.  loss: as `icp` (psulvsb_icp_robust)."""
     import torch
 
     from .stages import _dev, _stream
@@ -121,9 +177,13 @@ def icp_device(d_src, d_tgt, R0, t0, max_correspondence_distance: float, *, d_ta
     corr = torch.empty(max(ns, 1), dtype=torch.int32, device=dev)
     p = _params(max_correspondence_distance, point_to_plane, max_iterations, relative_fitness, relative_rmse)
     R, t = _transform(R0, t0)
-    capi.check(capi.lib().psulvsb_icp(_stream(), _dev(d_src) if ns else None, ns, _dev(d_tgt) if nt else None, nt,
-                                      None if d_target_normals is None else _dev(d_target_normals), C.byref(p), R, t,
-                                      _dev(work), _dev(out), _dev(rec) if trace else None, _dev(corr)))
+    head = (_stream(), _dev(d_src) if ns else None, ns, _dev(d_tgt) if nt else None, nt,
+            None if d_target_normals is None else _dev(d_target_normals), C.byref(p))
+    tail = (R, t, _dev(work), _dev(out), _dev(rec) if trace else None, _dev(corr))
+    if loss is None:
+        capi.check(capi.lib().psulvsb_icp(*head, *tail))
+    else:
+        capi.check(capi.lib().psulvsb_icp_robust(*head, _icp_loss(loss, point_to_plane), *tail))
     res = capi.IcpResult.from_buffer_copy(out.cpu().numpy().tobytes())
     records = None
     if trace:
@@ -158,10 +218,10 @@ def _batch_results(res, records, nrec, corr, sizes):
 
 def icp_batch(srcs, tgts, R0s, t0s, max_correspondence_distance: float, *, target_normals=None,
               point_to_plane: bool = False, max_iterations: int = 30, relative_fitness: float = 1e-6,
-              relative_rmse: float = 1e-6, trace: bool = False) -> list:
+              relative_rmse: float = 1e-6, trace: bool = False, loss: Optional[RobustKernel] = None) -> list:
     """psulvsb_icp_batch_host: refine B pairs in one call with shared parameters.  srcs, tgts (and target_normals, for
     point-to-plane): sequences of 3 x n arrays; R0s [B, 3, 3], t0s [B, 3].  Returns one IcpResult per pair, each equal bit
-    for bit to `icp` on that pair alone."""
+    for bit to `icp` on that pair alone.  loss: as `icp` (psulvsb_icp_robust_batch_host)."""
     s = [_cm(a, "src") for a in srcs]
     q = [_cm(a, "tgt") for a in tgts]
     B = len(s)
@@ -181,16 +241,22 @@ def icp_batch(srcs, tgts, R0s, t0s, max_correspondence_distance: float, *, targe
     res = (capi.IcpResult * max(B, 1))()
     records = (capi.IcpIteration * (B * nrec))() if trace and B else None
     corr = np.empty(sum(ns for ns, _ in sizes), dtype=np.int32)
-    capi.check(capi.lib().psulvsb_icp_batch_host(pairs, B, C.byref(p), res, records, corr.ctypes.data))
+    if loss is None:
+        capi.check(capi.lib().psulvsb_icp_batch_host(pairs, B, C.byref(p), res, records, corr.ctypes.data))
+    else:
+        capi.check(capi.lib().psulvsb_icp_robust_batch_host(pairs, B, C.byref(p), _icp_loss(loss, point_to_plane), res,
+                                                            records, corr.ctypes.data))
     return _batch_results(res, records, nrec, corr, sizes)
 
 
 def icp_batch_device(d_srcs, d_tgts, R0s, t0s, max_correspondence_distance: float, *, d_target_normals=None,
                      point_to_plane: bool = False, max_iterations: int = 30, relative_fitness: float = 1e-6,
-                     relative_rmse: float = 1e-6, trace: bool = False, work=None) -> list:
+                     relative_rmse: float = 1e-6, trace: bool = False, work=None,
+                     loss: Optional[RobustKernel] = None) -> list:
     """psulvsb_icp_batch on sequences of CUDA tensors [n, 3] float64 and the current stream.  The small results (and the
     traces) are read back, which waits for the stream; the correspondences stay on the device as views into one tensor.
-    `work`: an optional uint8 CUDA tensor of at least psulvsb_icp_batch_workspace_bytes bytes to reuse."""
+    `work`: an optional uint8 CUDA tensor of at least psulvsb_icp_batch_workspace_bytes bytes to reuse.  loss: as `icp`
+    (psulvsb_icp_robust_batch)."""
     import torch
 
     from .stages import _dev, _stream
@@ -217,8 +283,11 @@ def icp_batch_device(d_srcs, d_tgts, R0s, t0s, max_correspondence_distance: floa
     rec = torch.empty(B * nrec * C.sizeof(capi.IcpIteration) if trace and B else 1, dtype=torch.uint8, device=dev)
     corr = torch.empty(max(sum(ns for ns, _ in sizes), 1), dtype=torch.int32, device=dev)
     p = _params(max_correspondence_distance, point_to_plane, max_iterations, relative_fitness, relative_rmse)
-    capi.check(L.psulvsb_icp_batch(_stream(), pairs, B, C.byref(p), _dev(work), _dev(out),
-                                   _dev(rec) if trace else None, _dev(corr)))
+    tail = (_dev(work), _dev(out), _dev(rec) if trace else None, _dev(corr))
+    if loss is None:
+        capi.check(L.psulvsb_icp_batch(_stream(), pairs, B, C.byref(p), *tail))
+    else:
+        capi.check(L.psulvsb_icp_robust_batch(_stream(), pairs, B, C.byref(p), _icp_loss(loss, point_to_plane), *tail))
     res = (capi.IcpResult * max(B, 1)).from_buffer_copy(out.cpu().numpy().tobytes())
     records = None
     if trace and B:
@@ -235,10 +304,11 @@ def _normals(n, cloud, what) -> np.ndarray:
 
 def gicp(src, tgt, src_normals, tgt_normals, R0, t0, max_correspondence_distance: float, *, epsilon: float = 1e-3,
          max_iterations: int = 30, relative_fitness: float = 1e-6, relative_rmse: float = 1e-6,
-         trace: bool = False) -> IcpResult:
+         trace: bool = False, loss: Optional[RobustKernel] = None) -> IcpResult:
     """psulvsb_gicp_host: refine (R0, t0) so that tgt ~ R src + t with generalized ICP.  src, src_normals 3 x n_s; tgt,
     tgt_normals 3 x n_t.  Each point's covariance is I - (1 - epsilon) n n^T (a non-finite or zero normal gives I, and
-    the point stays a candidate); 0 < epsilon <= 1, Open3D's default 1e-3."""
+    the point stays a candidate); 0 < epsilon <= 1, Open3D's default 1e-3.  loss: a robust kernel applied to each row
+    of the whitened residual (psulvsb_gicp_robust_host)."""
     s, q = _cm(src, "src"), _cm(tgt, "tgt")
     ns, nt = _normals(src_normals, s, "src_normals"), _normals(tgt_normals, q, "tgt_normals")
     p = _params(max_correspondence_distance, False, max_iterations, relative_fitness, relative_rmse)
@@ -246,18 +316,23 @@ def gicp(src, tgt, src_normals, tgt_normals, R0, t0, max_correspondence_distance
     res = capi.IcpResult()
     records = (capi.IcpIteration * (max(int(max_iterations), 0) + 1))() if trace else None
     corr = np.empty(s.shape[1], dtype=np.int32)
-    capi.check(capi.lib().psulvsb_gicp_host(s.ctypes.data, s.shape[1], ns.ctypes.data, q.ctypes.data, q.shape[1],
-                                            nt.ctypes.data, C.byref(p), float(epsilon), R, t, C.byref(res), records,
-                                            corr.ctypes.data))
+    head = (s.ctypes.data, s.shape[1], ns.ctypes.data, q.ctypes.data, q.shape[1], nt.ctypes.data, C.byref(p),
+            float(epsilon))
+    tail = (R, t, C.byref(res), records, corr.ctypes.data)
+    if loss is None:
+        capi.check(capi.lib().psulvsb_gicp_host(*head, *tail))
+    else:
+        capi.check(capi.lib().psulvsb_gicp_robust_host(*head, loss._c(), *tail))
     return _result(res, records, corr)
 
 
 def gicp_device(d_src, d_tgt, d_src_normals, d_tgt_normals, R0, t0, max_correspondence_distance: float, *,
                 epsilon: float = 1e-3, max_iterations: int = 30, relative_fitness: float = 1e-6,
-                relative_rmse: float = 1e-6, trace: bool = False, work=None) -> IcpResult:
+                relative_rmse: float = 1e-6, trace: bool = False, work=None,
+                loss: Optional[RobustKernel] = None) -> IcpResult:
     """psulvsb_gicp on CUDA tensors [n, 3] float64 (normals the same shape as their clouds) and the current stream; the
     outputs as `icp_device`.  `work`: an optional uint8 CUDA tensor of at least psulvsb_icp_workspace_bytes(n_s, n_t)
-    bytes to reuse."""
+    bytes to reuse.  loss: as `gicp` (psulvsb_gicp_robust)."""
     import torch
 
     from .stages import _dev, _stream
@@ -276,10 +351,13 @@ def gicp_device(d_src, d_tgt, d_src_normals, d_tgt_normals, R0, t0, max_correspo
     corr = torch.empty(max(ns, 1), dtype=torch.int32, device=dev)
     p = _params(max_correspondence_distance, False, max_iterations, relative_fitness, relative_rmse)
     R, t = _transform(R0, t0)
-    capi.check(capi.lib().psulvsb_gicp(_stream(), _dev(d_src) if ns else None, ns,
-                                       _dev(d_src_normals) if ns else None, _dev(d_tgt) if nt else None, nt,
-                                       _dev(d_tgt_normals) if nt else None, C.byref(p), float(epsilon), R, t,
-                                       _dev(work), _dev(out), _dev(rec) if trace else None, _dev(corr)))
+    head = (_stream(), _dev(d_src) if ns else None, ns, _dev(d_src_normals) if ns else None,
+            _dev(d_tgt) if nt else None, nt, _dev(d_tgt_normals) if nt else None, C.byref(p), float(epsilon))
+    tail = (R, t, _dev(work), _dev(out), _dev(rec) if trace else None, _dev(corr))
+    if loss is None:
+        capi.check(capi.lib().psulvsb_gicp(*head, *tail))
+    else:
+        capi.check(capi.lib().psulvsb_gicp_robust(*head, loss._c(), *tail))
     res = capi.IcpResult.from_buffer_copy(out.cpu().numpy().tobytes())
     records = None
     if trace:
@@ -300,10 +378,10 @@ def _gicp_pairs(ptrs, sizes, R, t):
 
 def gicp_batch(srcs, tgts, src_normals, tgt_normals, R0s, t0s, max_correspondence_distance: float, *,
                epsilon: float = 1e-3, max_iterations: int = 30, relative_fitness: float = 1e-6,
-               relative_rmse: float = 1e-6, trace: bool = False) -> list:
+               relative_rmse: float = 1e-6, trace: bool = False, loss: Optional[RobustKernel] = None) -> list:
     """psulvsb_gicp_batch_host: refine B pairs with generalized ICP in one call with shared parameters.  srcs, tgts,
     src_normals, tgt_normals: sequences of 3 x n arrays; R0s [B, 3, 3], t0s [B, 3].  Returns one IcpResult per pair,
-    each equal bit for bit to `gicp` on that pair alone."""
+    each equal bit for bit to `gicp` on that pair alone.  loss: as `gicp` (psulvsb_gicp_robust_batch_host)."""
     s = [_cm(a, "src") for a in srcs]
     q = [_cm(a, "tgt") for a in tgts]
     B = len(s)
@@ -320,16 +398,22 @@ def gicp_batch(srcs, tgts, src_normals, tgt_normals, R0s, t0s, max_correspondenc
     res = (capi.IcpResult * max(B, 1))()
     records = (capi.IcpIteration * (B * nrec))() if trace and B else None
     corr = np.empty(sum(ns for ns, _ in sizes), dtype=np.int32)
-    capi.check(capi.lib().psulvsb_gicp_batch_host(pairs, B, C.byref(p), float(epsilon), res, records,
-                                                  corr.ctypes.data))
+    if loss is None:
+        capi.check(capi.lib().psulvsb_gicp_batch_host(pairs, B, C.byref(p), float(epsilon), res, records,
+                                                      corr.ctypes.data))
+    else:
+        capi.check(capi.lib().psulvsb_gicp_robust_batch_host(pairs, B, C.byref(p), float(epsilon), loss._c(), res,
+                                                             records, corr.ctypes.data))
     return _batch_results(res, records, nrec, corr, sizes)
 
 
 def gicp_batch_device(d_srcs, d_tgts, d_src_normals, d_tgt_normals, R0s, t0s, max_correspondence_distance: float, *,
                       epsilon: float = 1e-3, max_iterations: int = 30, relative_fitness: float = 1e-6,
-                      relative_rmse: float = 1e-6, trace: bool = False, work=None) -> list:
+                      relative_rmse: float = 1e-6, trace: bool = False, work=None,
+                      loss: Optional[RobustKernel] = None) -> list:
     """psulvsb_gicp_batch on sequences of CUDA tensors [n, 3] float64 and the current stream; the outputs as
-    `icp_batch_device`.  `work`: an optional uint8 CUDA tensor of at least psulvsb_gicp_batch_workspace_bytes bytes."""
+    `icp_batch_device`.  `work`: an optional uint8 CUDA tensor of at least psulvsb_gicp_batch_workspace_bytes bytes.
+    loss: as `gicp` (psulvsb_gicp_robust_batch)."""
     import torch
 
     from .stages import _dev, _stream
@@ -358,8 +442,11 @@ def gicp_batch_device(d_srcs, d_tgts, d_src_normals, d_tgt_normals, R0s, t0s, ma
     rec = torch.empty(B * nrec * C.sizeof(capi.IcpIteration) if trace and B else 1, dtype=torch.uint8, device=dev)
     corr = torch.empty(max(sum(ns for ns, _ in sizes), 1), dtype=torch.int32, device=dev)
     p = _params(max_correspondence_distance, False, max_iterations, relative_fitness, relative_rmse)
-    capi.check(L.psulvsb_gicp_batch(_stream(), pairs, B, C.byref(p), float(epsilon), _dev(work), _dev(out),
-                                    _dev(rec) if trace else None, _dev(corr)))
+    tail = (_dev(work), _dev(out), _dev(rec) if trace else None, _dev(corr))
+    if loss is None:
+        capi.check(L.psulvsb_gicp_batch(_stream(), pairs, B, C.byref(p), float(epsilon), *tail))
+    else:
+        capi.check(L.psulvsb_gicp_robust_batch(_stream(), pairs, B, C.byref(p), float(epsilon), loss._c(), *tail))
     res = (capi.IcpResult * max(B, 1)).from_buffer_copy(out.cpu().numpy().tobytes())
     records = None
     if trace and B:
