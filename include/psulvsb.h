@@ -687,6 +687,87 @@ int psulvsb_gicp_robust_batch_host(const psulvsb_gicp_pair_t* pairs, int B, cons
                                    double epsilon, const psulvsb_robust_kernel_t* loss, psulvsb_icp_result_t* results,
                                    psulvsb_icp_iteration_t* trace, int* corr);
 
+/* ---- Colored ICP (Park, Zhou and Koltun, ICCV 2017; Open3D's registration_colored_icp with
+ * TransformationEstimationForColoredICP(lambda_geometric, kernel)), DESIGN.md section 11 "Colored ICP".  The loop,
+ * stop rule, correspondences (a target point with a non-finite normal is no candidate), fitness, the unweighted
+ * inlier_rmse, trace, statuses and minimum count (6) are those of psulvsb_icp in point-to-plane mode; only the update
+ * changes.  Colours are column-major 3 x n doubles, Open3D's [0, 1] RGB (not range-checked); a point's intensity is
+ * I = ((r + g) + b) / 3.  The call first computes the target's colour gradients (psulvsb_color_gradients_batch with
+ * radius 2 d and max_nn 30, Open3D's KDTreeSearchParamHybrid(2 d, 30)), then each correspondence (p' = T_k p, its
+ * target q with normal n, used as given, and gradient g) adds two rows to point-to-plane's 6x6 system:
+ *   geometric    r = sqrt(lambda) ((p' - q).n)                         J = sqrt(lambda) [p' x n, n]
+ *   photometric  r = sqrt(1 - lambda) (I_s(p) - (g.(p' - q) + I_t(q)))  J = sqrt(1 - lambda) [p' x m, m]
+ * with m = -(g - (g.n) n), each weighted by rho(r) of the loss (NULL: L2).  params->point_to_plane must be 0 (the entry
+ * point is the mode).  lambda_geometric in [0, 1] (Open3D's default 0.968); with lambda 1 and the L2 loss the call is
+ * bit-identical to psulvsb_icp in point-to-plane mode.  Non-finite colours reach the 6x6 system, whose non-finite rule
+ * stops the loop with PSULVSB_ICP_NO_UPDATE.  The tests compare with a numpy restatement
+ * (tests/colored_icp_restatement.py). */
+typedef struct psulvsb_colored_icp_pair {
+  const double* src;         /* 3 x n_s, column-major                                                  */
+  int n_s;
+  const double* src_colors;  /* 3 x n_s, required when n_s > 0                                         */
+  const double* tgt;         /* 3 x n_t                                                                */
+  int n_t;
+  const double* tgt_colors;  /* 3 x n_t, required when n_t > 0                                         */
+  const double* tgt_normals; /* 3 x n_t, required when n_t > 0                                         */
+  double R0[9];              /* column-major                                                           */
+  double t0[3];
+} psulvsb_colored_icp_pair_t;
+
+/* Device scratch of psulvsb_colored_icp / psulvsb_colored_icp_batch (depends on the sizes only; it holds the target
+ * gradients, 24 bytes per target point, besides the grids); 0 for a negative size, B <= 0 or a NULL pairs array. */
+unsigned long long psulvsb_colored_icp_workspace_bytes(int n_s, int n_t);
+unsigned long long psulvsb_colored_icp_batch_workspace_bytes(const psulvsb_colored_icp_pair_t* pairs, int B);
+/* psulvsb_icp's arguments, outputs and layouts plus the colours, lambda_geometric and an optional robust kernel (read
+ * before the call returns); a single call is a batch of one, so d_work is required even for an empty cloud.
+ * PSULVSB_ERR_INVALID before any device work for everything psulvsb_icp refuses, point_to_plane != 0, a
+ * lambda_geometric outside [0, 1] or NaN, a NULL colour or normal array of a non-empty cloud, and the loss refusals of
+ * psulvsb_icp_robust (an unknown type, a k that is not finite and > 0). */
+int psulvsb_colored_icp(void* stream, const double* d_src, int n_s, const double* d_src_colors, const double* d_tgt,
+                        int n_t, const double* d_tgt_colors, const double* d_tgt_normals,
+                        const psulvsb_icp_params_t* params, double lambda_geometric,
+                        const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3], void* d_work,
+                        psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr);
+/* The same on host buffers, synchronous: clouds, colours and normals go up in one copy, one download at the end. */
+int psulvsb_colored_icp_host(const double* src, int n_s, const double* src_colors, const double* tgt, int n_t,
+                             const double* tgt_colors, const double* tgt_normals, const psulvsb_icp_params_t* params,
+                             double lambda_geometric, const psulvsb_robust_kernel_t* loss, const double R0[9],
+                             const double t0[3], psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace,
+                             int* corr);
+/* psulvsb_icp_batch with colored ICP's update: the layouts, refusals (PSULVSB_ERR_UNSUPPORTED included) and the
+ * guarantee that pair b's outputs are bit-identical to psulvsb_colored_icp_host on that pair alone are
+ * psulvsb_icp_batch's, plus psulvsb_colored_icp's refusals. */
+int psulvsb_colored_icp_batch(void* stream, const psulvsb_colored_icp_pair_t* pairs, int B,
+                              const psulvsb_icp_params_t* params, double lambda_geometric,
+                              const psulvsb_robust_kernel_t* loss, void* d_work, psulvsb_icp_result_t* d_results,
+                              psulvsb_icp_iteration_t* d_trace, int* d_corr);
+int psulvsb_colored_icp_batch_host(const psulvsb_colored_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                                   double lambda_geometric, const psulvsb_robust_kernel_t* loss,
+                                   psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr);
+
+/* ---- Colour gradients alone: the first stage of colored ICP (Open3D's InitializePointCloudForColoredICP), on
+ * FPFH's grid.  The neighbourhood of point i is the hybrid one of psulvsb_normals (the max_nn smallest keys (FP32
+ * squared distance, index) within `radius`, i itself included); with nn kept points, nn < 4 gives g = 0.  Every kept
+ * j != i gives the row a_j = (q_j - ((q_j - q_i).n_i) n_i) - q_i with b_j = I_j - I_i, one more row (nn - 1) n_i has
+ * b = 0, and g solves A^T A g = A^T b by a 3x3 FP64 Cholesky (sums in the walk's order); a non-positive pivot, a
+ * non-finite g or a non-finite n_i gives g = 0.  Results are bit-identical from call to call, and cloud c's are
+ * bit-identical to a batch of cloud c alone.  radius finite and > 0, 4 <= max_nn <= 32.  Cloud c's gradients are
+ * columns [sum_{a<c} n_a, ...) of the 3 x (sum n) doubles.  PSULVSB_ERR_INVALID before any device work for B < 0, a bad
+ * radius or max_nn, a negative size, a NULL array of a non-empty cloud or a required NULL;
+ * PSULVSB_ERR_UNSUPPORTED when the sizes add up to 2^31 or more.  B = 0 does nothing.  The _host variant takes host
+ * buffers and is synchronous. */
+typedef struct psulvsb_color_cloud {
+  const double* points;  /* 3 x n, column-major                                                           */
+  int n;
+  const double* colors;  /* 3 x n                                                                        */
+  const double* normals; /* 3 x n                                                                        */
+} psulvsb_color_cloud_t;
+unsigned long long psulvsb_color_gradients_batch_workspace_bytes(const psulvsb_color_cloud_t* clouds, int B);
+int psulvsb_color_gradients_batch(void* stream, const psulvsb_color_cloud_t* clouds, int B, double radius, int max_nn,
+                                  void* d_work, double* d_gradients);
+int psulvsb_color_gradients_batch_host(const psulvsb_color_cloud_t* clouds, int B, double radius, int max_nn,
+                                       double* gradients);
+
 /* Clique escalation (registration.cc:1000-1085 -> teaser/src/graph.cc:12-125, PMC exact maximum clique) of the
  * graph with n_vertices vertices and the given edges (uint2 endpoint pairs).  A deterministic greedy maximal
  * clique (most neighbours among the remaining candidates first, ties: lowest index) gives the lower bound;

@@ -46,6 +46,10 @@ SYMBOLS = [
     "psulvsb_voxel_down_sample_workspace_bytes", "psulvsb_voxel_down_sample", "psulvsb_voxel_down_sample_host",
     "psulvsb_voxel_down_sample_batch_workspace_bytes", "psulvsb_voxel_down_sample_batch",
     "psulvsb_voxel_down_sample_batch_host",
+    "psulvsb_colored_icp_workspace_bytes", "psulvsb_colored_icp_batch_workspace_bytes", "psulvsb_colored_icp",
+    "psulvsb_colored_icp_host", "psulvsb_colored_icp_batch", "psulvsb_colored_icp_batch_host",
+    "psulvsb_color_gradients_batch_workspace_bytes", "psulvsb_color_gradients_batch",
+    "psulvsb_color_gradients_batch_host",
 ]
 UNIQUE_ID_BYTES = 128
 
@@ -221,6 +225,31 @@ class RobustKernel(C.Structure):
     _fields_ = [
         ("type", C.c_int),
         ("k", C.c_double),
+    ]
+
+
+class ColoredIcpPair(C.Structure):
+    """psulvsb_colored_icp_pair_t: one colored-ICP problem of a batch (R0 column-major)."""
+    _fields_ = [
+        ("src", C.c_void_p),
+        ("n_s", C.c_int),
+        ("src_colors", C.c_void_p),
+        ("tgt", C.c_void_p),
+        ("n_t", C.c_int),
+        ("tgt_colors", C.c_void_p),
+        ("tgt_normals", C.c_void_p),
+        ("R0", C.c_double * 9),
+        ("t0", C.c_double * 3),
+    ]
+
+
+class ColorCloud(C.Structure):
+    """psulvsb_color_cloud_t: one cloud of a colour-gradient batch."""
+    _fields_ = [
+        ("points", C.c_void_p),
+        ("n", C.c_int),
+        ("colors", C.c_void_p),
+        ("normals", C.c_void_p),
     ]
 
 
@@ -412,6 +441,23 @@ def _declare(L: C.CDLL) -> None:
     L.psulvsb_match_batch_workspace_bytes.restype = _ull
     L.psulvsb_match_batch.argtypes = [_vp, C.POINTER(MatchPair), C.c_int, C.c_int, C.c_int, C.c_double, _vp, _vp, _vp]
     L.psulvsb_match_batch_host.argtypes = [C.POINTER(MatchPair), C.c_int, C.c_int, C.c_int, C.c_double, _vp, _vp]
+    _dp = C.POINTER(C.c_double)
+    L.psulvsb_colored_icp_workspace_bytes.argtypes = [C.c_int, C.c_int]
+    L.psulvsb_colored_icp_workspace_bytes.restype = _ull
+    L.psulvsb_colored_icp_batch_workspace_bytes.argtypes = [C.POINTER(ColoredIcpPair), C.c_int]
+    L.psulvsb_colored_icp_batch_workspace_bytes.restype = _ull
+    L.psulvsb_colored_icp.argtypes = [_vp, _vp, C.c_int, _vp, _vp, C.c_int, _vp, _vp, C.POINTER(IcpParams), C.c_double,
+                                      _rk, _dp, _dp, _vp, _vp, _vp, _vp]
+    L.psulvsb_colored_icp_host.argtypes = [_vp, C.c_int, _vp, _vp, C.c_int, _vp, _vp, C.POINTER(IcpParams),
+                                           C.c_double, _rk, _dp, _dp, _vp, _vp, _vp]
+    L.psulvsb_colored_icp_batch.argtypes = [_vp, C.POINTER(ColoredIcpPair), C.c_int, C.POINTER(IcpParams), C.c_double,
+                                            _rk, _vp, _vp, _vp, _vp]
+    L.psulvsb_colored_icp_batch_host.argtypes = [C.POINTER(ColoredIcpPair), C.c_int, C.POINTER(IcpParams),
+                                                 C.c_double, _rk, _vp, _vp, _vp]
+    L.psulvsb_color_gradients_batch_workspace_bytes.argtypes = [C.POINTER(ColorCloud), C.c_int]
+    L.psulvsb_color_gradients_batch_workspace_bytes.restype = _ull
+    L.psulvsb_color_gradients_batch.argtypes = [_vp, C.POINTER(ColorCloud), C.c_int, C.c_double, C.c_int, _vp, _vp]
+    L.psulvsb_color_gradients_batch_host.argtypes = [C.POINTER(ColorCloud), C.c_int, C.c_double, C.c_int, _vp]
     for name in SYMBOLS:
         getattr(L, name)  # AttributeError here = the library does not export what the header declares
 

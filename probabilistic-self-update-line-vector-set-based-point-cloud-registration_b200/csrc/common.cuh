@@ -238,4 +238,18 @@ __device__ __forceinline__ int warp_sum_int(int v) {
   return v;
 }
 
+// ------------------------------------------------------------------------------------------
+// the colour-gradient stage (k8_features.cu), which colored ICP (k9_icp.cu) runs on its targets
+// ------------------------------------------------------------------------------------------
+// a point's intensity ((r + g) + b) / 3 in FP64, from its colour (Open3D's colored ICP)
+__device__ __forceinline__ double intensity(const double* rgb) {
+  return __ddiv_rn(dadd(dadd(rgb[0], rgb[1]), rgb[2]), 3.0);
+}
+// device scratch of run_color_gradients (sizes only)
+size_t color_gradients_scratch(const psulvsb_color_cloud_t* clouds, int B);
+// the batch on the device (clouds checked, radius and max_nn valid): cloud c's gradients at columns
+// [sum_{a<c} n_a, ...) of the 3 x (sum n) doubles `gradients`; asynchronous on st
+int run_color_gradients(cudaStream_t st, const psulvsb_color_cloud_t* clouds, int B, double radius, int max_nn,
+                        void* work, double* gradients);
+
 }  // namespace psulvsb

@@ -15,6 +15,10 @@
 //   k9_robust_p2l_correspond, k9_robust_gicp_correspond
 //                      the same passes with a robust kernel: each point-to-plane row, and each row of GICP's whitened
 //                      residual, weighted by rho(r) (tests/robust_icp_restatement.py);
+//   k9_colored_correspond
+//                      colored ICP's pass: a geometric and a photometric row per correspondence, each weighted by
+//                      rho(r), in point-to-plane's partials (tests/colored_icp_restatement.py); the target's colour
+//                      gradients come from k8_color_gradients (k8_features.cu), run once per call before the grids;
 //   k9_icp_cross       (point-to-point) the centred cross-covariance H over the correspondences, per-CTA sums;
 //   k9_icp_step        one CTA per pair: the pair's CTA sums in a fixed order, trace record k, the stop rule, the
 //                      update U, T <- U T.
@@ -25,6 +29,7 @@
 // is bit-identical from call to call.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <string>
@@ -82,6 +87,13 @@ struct IcpPair {
 };
 // the pair table is part of the workspace, whose size psulvsb_icp_[batch_]workspace_bytes publish
 static_assert(sizeof(IcpPair) == 152, "IcpPair's size fixes the published workspace sizes");
+
+// colored ICP's side table of the workspace, indexed by pair: what k9_colored_correspond reads besides the IcpPair
+struct ColorPair {
+  const double* src_colors;  // 3 x ns
+  const double* tgt_colors;  // 3 x nt
+  const double* grad;        // 3 x nt: the target's colour gradients
+};
 
 __device__ __forceinline__ long long icp_cell(double x, double c, double inv_h) {
   return (long long)floor(dmul(dsub(x, c), inv_h));
@@ -357,6 +369,61 @@ __device__ __forceinline__ void robust_row_terms(double px, double py, double pz
   for (int a = 0; a < 6; ++a) c[21 + a] = ACC ? dadd(c[21 + a], dmul(u[a], r)) : dmul(u[a], r);
 }
 
+// ---- colored ICP's terms of one correspondence (DESIGN.md section 11, "Colored ICP"); every operation in the order
+// written, which tests/colored_icp_restatement.py repeats elementwise in numpy
+
+// J = s [p' x o, o]
+__device__ __forceinline__ void scaled_row(double px, double py, double pz, const double o[3], double s, double J[6]) {
+  J[0] = dmul(s, dsub(dmul(py, o[2]), dmul(pz, o[1])));
+  J[1] = dmul(s, dsub(dmul(pz, o[0]), dmul(px, o[2])));
+  J[2] = dmul(s, dsub(dmul(px, o[1]), dmul(py, o[0])));
+  J[3] = dmul(s, o[0]);
+  J[4] = dmul(s, o[1]);
+  J[5] = dmul(s, o[2]);
+}
+
+// c[0, 27) of the row (J, r) weighted by rho(r), u = rho(r) J: J^T J (upper triangle row by row) as u_a J_e and J^T r
+// as u_a r.  ACC adds them to c, except that a term equal to zero leaves its entry as it is: an IEEE sum would turn a
+// -0 there into +0, and lambda = 1 would then no longer reproduce point-to-plane's partials bit for bit.
+template <bool ACC>
+__device__ __forceinline__ void weighted_row(const double J[6], double r, const psulvsb_robust_kernel_t& loss,
+                                             double* __restrict__ c) {
+  const double rho = robust_weight(loss, r);
+  double u[6];
+#pragma unroll
+  for (int a = 0; a < 6; ++a) u[a] = dmul(rho, J[a]);
+  int v = 0;
+#pragma unroll
+  for (int a = 0; a < 6; ++a)
+#pragma unroll
+    for (int e = a; e < 6; ++e, ++v) {
+      const double t = dmul(u[a], J[e]);
+      c[v] = !ACC ? t : (t == 0.0 ? c[v] : dadd(c[v], t));
+    }
+#pragma unroll
+  for (int a = 0; a < 6; ++a) {
+    const double t = dmul(u[a], r);
+    c[21 + a] = !ACC ? t : (t == 0.0 ? c[21 + a] : dadd(c[21 + a], t));
+  }
+}
+
+// d = p' - q, n the target normal, g the target's colour gradient, Is and It the intensities; sl = sqrt(lambda),
+// sc = sqrt(1 - lambda).  The geometric row r = sl (d . n), J = sl [p' x n, n] is written, then the photometric row
+// r = sc (Is - (g . d + It)), J = sc [p' x m, m] with m = -(g - (g . n) n) is added (Open3D's ComputeTransformation
+// of TransformationEstimationForColoredICP).
+__device__ __forceinline__ void colored_terms(double px, double py, double pz, const double d[3], const double n[3],
+                                              const double g[3], double Is, double It, double sl, double sc,
+                                              const psulvsb_robust_kernel_t& loss, double* __restrict__ c) {
+  double J[6];
+  scaled_row(px, py, pz, n, sl, J);
+  weighted_row<false>(J, dmul(sl, dadd(dadd(dmul(d[0], n[0]), dmul(d[1], n[1])), dmul(d[2], n[2]))), loss, c);
+  const double gn = dadd(dadd(dmul(g[0], n[0]), dmul(g[1], n[1])), dmul(g[2], n[2]));
+  const double m[3] = {-dsub(g[0], dmul(gn, n[0])), -dsub(g[1], dmul(gn, n[1])), -dsub(g[2], dmul(gn, n[2]))};
+  const double gd = dadd(dadd(dmul(g[0], d[0]), dmul(g[1], d[1])), dmul(g[2], d[2]));
+  scaled_row(px, py, pz, m, sc, J);
+  weighted_row<true>(J, dmul(sc, dsub(Is, dadd(gd, It))), loss, c);
+}
+
 // beta(lambda) = w / ((2 sqrt2 a)(sqrt2 + a)), a = sqrt(2 - w lambda): the coefficient of v v^T in C^-1/2 for the
 // eigenvalue w lambda of w (m m^T + n n^T) along v, |v|^2 = 2 lambda
 __device__ __forceinline__ double whiten_beta(double w, double lambda) {
@@ -401,14 +468,16 @@ __device__ __forceinline__ void whitening(const double m[3], const double n[3], 
 
 // ---- evaluation of T_k: corr[i] = the target at the smallest d^2 <= dd (ties: lowest index) or -1, and the CTA sums
 // of what the step needs (point-to-point: count, sum d^2, sum p', sum q; point-to-plane: count, sum d^2, J^T J, J^T r;
-// GICP: count, sum d^2, A^T M A, A^T M d with w = 1 - epsilon; ROBUST: the same layout, the terms weighted by `loss`);
-// the body of k9_icp_correspond, k9_gicp_correspond and the robust passes
-template <int MODE, bool ROBUST = false>
+// GICP: count, sum d^2, A^T M A, A^T M d with w = 1 - epsilon; ROBUST: the same layout, the terms weighted by `loss`;
+// COLOR (point-to-plane): count, sum d^2 and colored ICP's terms with sl = sqrt(lambda), sc = sqrt(1 - lambda));
+// the body of k9_icp_correspond, k9_gicp_correspond, the robust passes and k9_colored_correspond
+template <int MODE, bool ROBUST = false, bool COLOR = false>
 __device__ __forceinline__ void correspond(const IcpPair* __restrict__ pairs, const int* __restrict__ tile_first, int B,
                                            const double4* __restrict__ rec, const int* __restrict__ start,
                                            double inv_h, const IcpState* __restrict__ states, double dd, double w,
                                            psulvsb_robust_kernel_t loss, int* __restrict__ corr,
-                                           double* __restrict__ partials) {
+                                           double* __restrict__ partials, const ColorPair* __restrict__ colors = nullptr,
+                                           double sl = 0.0, double sc = 0.0) {
   // the pair, its bucket mask and its start table are read from shared memory at each use: held in registers across
   // the 27-cell walk they push the point-to-plane instantiation past 128 registers (4 CTAs per SM) into spills
   __shared__ volatile int s_pair, s_start;
@@ -478,6 +547,13 @@ __device__ __forceinline__ void correspond(const IcpPair* __restrict__ pairs, co
         c[5] = qx;
         c[6] = qy;
         c[7] = qz;
+      } else if constexpr (COLOR) {
+        const double* nrm = pairs[s_pair].nrm + 3 * (size_t)bj;
+        const ColorPair& cp = colors[s_pair];
+        const double d[3] = {dsub(px, qx), dsub(py, qy), dsub(pz, qz)}, n[3] = {nrm[0], nrm[1], nrm[2]};
+        const double g[3] = {cp.grad[3 * (size_t)bj], cp.grad[3 * (size_t)bj + 1], cp.grad[3 * (size_t)bj + 2]};
+        colored_terms(px, py, pz, d, n, g, intensity(cp.src_colors + 3 * (size_t)i),
+                      intensity(cp.tgt_colors + 3 * (size_t)bj), sl, sc, loss, c + 2);
       } else if constexpr (ROBUST) {
         const double d[3] = {dsub(px, qx), dsub(py, qy), dsub(pz, qz)};
         if constexpr (MODE == P2L) {
@@ -565,6 +641,17 @@ __global__ void __launch_bounds__(ICP_THREADS)
                               const IcpState* __restrict__ states, double dd, double w, psulvsb_robust_kernel_t loss,
                               int* __restrict__ corr, double* __restrict__ partials) {
   correspond<GICP, true>(pairs, tile_first, B, rec, start, inv_h, states, dd, w, loss, corr, partials);
+}
+
+// colored ICP, sl = sqrt(lambda), sc = sqrt(1 - lambda): point-to-plane's partials of the geometric and photometric rows
+__global__ void __launch_bounds__(ICP_THREADS)
+    k9_colored_correspond(const IcpPair* __restrict__ pairs, const ColorPair* __restrict__ colors,
+                          const int* __restrict__ tile_first, int B, const double4* __restrict__ rec,
+                          const int* __restrict__ start, double inv_h, const IcpState* __restrict__ states, double dd,
+                          double sl, double sc, psulvsb_robust_kernel_t loss, int* __restrict__ corr,
+                          double* __restrict__ partials) {
+  correspond<P2L, false, true>(pairs, tile_first, B, rec, start, inv_h, states, dd, 0.0, loss, corr, partials, colors,
+                               sl, sc);
 }
 
 // ---- point-to-point: H = sum (p' - mu_p)(q - mu_q)^T over the correspondences of T_k
@@ -852,13 +939,62 @@ void empty_result(const double* R0, const double* t0, psulvsb_icp_result_t* res,
 }
 
 // what a call minimises: the mode, GICP's source normals (one pointer per pair, else nullptr), w = 1 - epsilon and
-// the robust kernel of point-to-plane / GICP (nullptr: none)
+// the robust kernel of point-to-plane / GICP (nullptr: none); colored ICP (point-to-plane) adds the pairs' colours
+// and lambda_geometric
 struct Objective {
   Mode mode;
   const double* const* src_normals;
   double w;
   const psulvsb_robust_kernel_t* loss = nullptr;
+  const double* const* src_colors = nullptr;  // one pointer per pair: colored ICP, else nullptr
+  const double* const* tgt_colors = nullptr;
+  double lambda = 1.0;
 };
+
+// colored ICP's gradient stage: Open3D's KDTreeSearchParamHybrid(2 d, 30)
+constexpr int COLOR_MAX_NN = 30;
+
+// the gradient stage's clouds: pair b's target when the pair is live, else empty (sizes only without obj)
+std::vector<psulvsb_color_cloud_t> target_clouds(const psulvsb_icp_pair_t* pairs, int B, const Objective* obj) {
+  std::vector<psulvsb_color_cloud_t> c((size_t)B);
+  for (int b = 0; b < B; ++b) {
+    const bool on = live(pairs[b]);
+    c[b] = psulvsb_color_cloud_t{pairs[b].tgt, on ? pairs[b].n_t : 0, obj ? obj->tgt_colors[b] : nullptr,
+                                 pairs[b].tgt_normals};
+  }
+  return c;
+}
+
+// colored ICP's workspace: ICP's layout, and the gradient stage's scratch aliased over it (the stream orders them);
+// then the side table ColorPair[B] and the live targets' gradients (3 x nt), which persist through the rounds
+size_t colored_layout(const psulvsb_icp_pair_t* pairs, int B, char* base, ColorPair** cp, double** grad) {
+  const IcpSizes z = icp_sizes(pairs, B);
+  const std::vector<psulvsb_color_cloud_t> clouds = target_clouds(pairs, B, nullptr);
+  size_t off = std::max(icp_layout(z, nullptr, nullptr), color_gradients_scratch(clouds.data(), B));
+  if (cp) *cp = reinterpret_cast<ColorPair*>(base + off);
+  off += up256(sizeof(ColorPair) * (size_t)B);
+  if (grad) *grad = reinterpret_cast<double*>(base + off);
+  return off + up256(24 * (size_t)z.nt);
+}
+
+// colored ICP before its grids (B >= 1): the live targets' gradients, then the side table
+int colored_prologue(cudaStream_t st, const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t& prm,
+                     const Objective& obj, void* work, ColorPair** d_cp) {
+  double* grad;
+  colored_layout(pairs, B, static_cast<char*>(work), d_cp, &grad);
+  const std::vector<psulvsb_color_cloud_t> clouds = target_clouds(pairs, B, &obj);
+  if (int rc = run_color_gradients(st, clouds.data(), B, 2.0 * prm.max_correspondence_distance, COLOR_MAX_NN, work,
+                                   grad))
+    return rc;
+  std::vector<ColorPair> cp((size_t)B);
+  long long t0 = 0;
+  for (int b = 0; b < B; ++b) {
+    cp[b] = ColorPair{obj.src_colors[b], obj.tgt_colors[b], grad + 3 * t0};
+    t0 += clouds[b].n;
+  }
+  PSU_CUDA(cudaMemcpyAsync(*d_cp, cp.data(), sizeof(ColorPair) * (size_t)B, cudaMemcpyHostToDevice, st));
+  return PSULVSB_OK;
+}
 
 Objective icp_objective(const psulvsb_icp_params_t& prm) {
   return Objective{prm.point_to_plane ? P2L : P2P, nullptr, 0.0};
@@ -869,6 +1005,9 @@ Objective icp_objective(const psulvsb_icp_params_t& prm) {
 int run_icp(cudaStream_t st, const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t& prm, Objective obj,
             void* work, psulvsb_icp_result_t* d_results, psulvsb_icp_iteration_t* d_trace, int* d_corr) {
   const IcpSizes z = icp_sizes(pairs, B);
+  ColorPair* d_cp = nullptr;
+  if (obj.src_colors)
+    if (int rc = colored_prologue(st, pairs, B, prm, obj, work, &d_cp)) return rc;
   IcpWork w;
   icp_layout(z, static_cast<char*>(work), &w);
   const double d = prm.max_correspondence_distance;
@@ -923,9 +1062,14 @@ int run_icp(cudaStream_t st, const psulvsb_icp_pair_t* pairs, int B, const psulv
     PSU_CHECK_LAUNCH("k9_icp_grid_order");
     const StepParams sp{prm.max_iterations, prm.relative_fitness, prm.relative_rmse};
     const double dd = d * d;
+    const double sl = std::sqrt(obj.lambda), sc = std::sqrt(1.0 - obj.lambda);
+    const psulvsb_robust_kernel_t loss = obj.loss ? *obj.loss : psulvsb_robust_kernel_t{PSULVSB_LOSS_L2, 1.0};
     for (int k = 0; k <= prm.max_iterations; ++k) {
       if (obj.mode == P2L) {
-        if (obj.loss)
+        if (d_cp)
+          k9_colored_correspond<<<tiles, ICP_THREADS, 0, st>>>(w.pair, d_cp, w.tile_first, B, w.rec, w.start, inv_h,
+                                                               w.state, dd, sl, sc, loss, w.corr, w.partials);
+        else if (obj.loss)
           k9_robust_p2l_correspond<<<tiles, ICP_THREADS, 0, st>>>(w.pair, w.tile_first, B, w.rec, w.start, inv_h,
                                                                   w.state, dd, *obj.loss, w.corr, w.partials);
         else
@@ -965,17 +1109,19 @@ int run_icp(cudaStream_t st, const psulvsb_icp_pair_t* pairs, int B, const psulv
 // trace records and correspondences come back in one
 int run_icp_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_params_t& prm, Objective obj,
                  psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr, const char* who) {
-  const bool tn = obj.mode != P2P, sn = obj.mode == GICP;
+  const bool tn = obj.mode != P2P, sn = obj.mode == GICP, col = obj.src_colors != nullptr;
   const IcpSizes z = icp_sizes(pairs, B);
   const size_t nrec = (size_t)prm.max_iterations + 1, NB = (size_t)B;
   // outputs first and contiguous, so that one copy brings them back
   const size_t o_trace = up256(sizeof(psulvsb_icp_result_t) * NB),
                o_corr = o_trace + (trace ? sizeof(psulvsb_icp_iteration_t) * nrec * NB : 0),
                o_end = o_corr + (corr ? 4 * (size_t)z.ns : 0), o_in = up256(o_end);
-  const size_t in_bytes = 24 * (size_t)(z.ns * (sn ? 2 : 1) + z.nt * (tn ? 2 : 1));
+  long long ns_live = 0;  // the colours go up for live pairs only
+  for (int b = 0; b < B; ++b) ns_live += live(pairs[b]) ? pairs[b].n_s : 0;
+  const size_t in_bytes = 24 * (size_t)(z.ns * (sn ? 2 : 1) + z.nt * (tn ? 2 : 1) + (col ? ns_live + z.nt : 0));
   const size_t o_work = up256(o_in + in_bytes);
-  // the live pairs' src, tgt (and target normals, then source normals) in pair order: pair b's src at in_off[b], the
-  // rest after it
+  // the live pairs' src, tgt (and target normals, then source normals, then source and target colours) in pair order:
+  // pair b's src at in_off[b], the rest after it
   std::vector<char> in(in_bytes);
   std::vector<size_t> in_off(NB);
   size_t off = 0;
@@ -991,15 +1137,20 @@ int run_icp_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_param
     put(q.tgt, q.n_t);
     if (tn) put(q.tgt_normals, q.n_t);
     if (sn) put(obj.src_normals[b], q.n_s);
+    if (col) {
+      put(obj.src_colors[b], q.n_s);
+      put(obj.tgt_colors[b], q.n_t);
+    }
   }
+  const size_t work_bytes = col ? colored_layout(pairs, B, nullptr, nullptr, nullptr) : icp_layout(z, nullptr, nullptr);
   void* buf = nullptr;
-  if (cudaMalloc(&buf, o_work + icp_layout(z, nullptr, nullptr)) != cudaSuccess) {
+  if (cudaMalloc(&buf, o_work + work_bytes) != cudaSuccess) {
     cudaGetLastError();
     return fail(PSULVSB_ERR_CUDA, std::string(who) + ": cudaMalloc failed");
   }
   char* base = static_cast<char*>(buf);
   std::vector<psulvsb_icp_pair_t> dev(pairs, pairs + B);
-  std::vector<const double*> dev_snrm(NB, nullptr);
+  std::vector<const double*> dev_snrm(NB, nullptr), dev_scol(NB, nullptr), dev_tcol(NB, nullptr);
   for (int b = 0; b < B; ++b) {
     psulvsb_icp_pair_t& q = dev[b];
     const double* src = reinterpret_cast<const double*>(base + o_in + in_off[b]);
@@ -1008,9 +1159,16 @@ int run_icp_host(const psulvsb_icp_pair_t* pairs, int B, const psulvsb_icp_param
     q.tgt = on ? src + 3 * (size_t)q.n_s : nullptr;
     q.tgt_normals = on && tn ? src + 3 * ((size_t)q.n_s + q.n_t) : nullptr;
     dev_snrm[b] = on && sn ? src + 3 * ((size_t)q.n_s + 2 * (size_t)q.n_t) : nullptr;
+    // colored ICP: point-to-plane's layout (src, tgt, target normals) followed by the source and target colours
+    dev_scol[b] = on && col ? src + 3 * ((size_t)q.n_s + 2 * (size_t)q.n_t) : nullptr;
+    dev_tcol[b] = on && col ? src + 3 * (2 * (size_t)q.n_s + 2 * (size_t)q.n_t) : nullptr;
   }
   Objective dev_obj = obj;
   dev_obj.src_normals = dev_snrm.data();
+  if (col) {
+    dev_obj.src_colors = dev_scol.data();
+    dev_obj.tgt_colors = dev_tcol.data();
+  }
   std::vector<char> out(o_end);
   int rc = PSULVSB_OK;
   auto step = [&](cudaError_t e, const char* what) {
@@ -1229,6 +1387,68 @@ int gicp_batch_host(const psulvsb_gicp_pair_t* pairs, int B, const psulvsb_icp_p
   return run_icp_host(icp.data(), B, *params, obj, results, trace, corr, who);
 }
 
+// colored ICP takes ICP's parameters in point-to-point form (the entry point is the mode), lambda in [0, 1] and an
+// optional robust kernel
+bool colored_args_ok(const psulvsb_icp_params_t* p, double lambda, const psulvsb_robust_kernel_t* loss) {
+  return icp_params_ok(p) && p->point_to_plane == 0 && lambda >= 0.0 && lambda <= 1.0 && (!loss || loss_ok(loss));
+}
+
+Objective colored_objective(const double* const* src_colors, const double* const* tgt_colors, double lambda,
+                            const psulvsb_robust_kernel_t* loss) {
+  Objective obj{P2L, nullptr, 0.0, loss};
+  obj.src_colors = src_colors;
+  obj.tgt_colors = tgt_colors;
+  obj.lambda = lambda;
+  return obj;
+}
+
+// colored pairs as ICP pairs (target normals included) and their colours; PSULVSB_ERR_INVALID for a non-empty cloud
+// without its colours or normals, else pairs_check's verdict
+int colored_pairs(const psulvsb_colored_icp_pair_t* g, int B, const psulvsb_icp_params_t* params,
+                  std::vector<psulvsb_icp_pair_t>& pairs, std::vector<const double*>& scol,
+                  std::vector<const double*>& tcol, const char* who) {
+  pairs.resize((size_t)B);
+  scol.resize((size_t)B);
+  tcol.resize((size_t)B);
+  for (int b = 0; b < B; ++b) {
+    const psulvsb_colored_icp_pair_t& q = g[b];
+    if ((q.n_s > 0 && !q.src_colors) || (q.n_t > 0 && (!q.tgt_colors || !q.tgt_normals)))
+      return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad pair " + std::to_string(b) + " (colours, normals)");
+    pairs[b] = one_pair(q.src, q.n_s, q.tgt, q.n_t, q.tgt_normals, q.R0, q.t0);
+    scol[b] = q.src_colors;
+    tcol[b] = q.tgt_colors;
+  }
+  return pairs_check(pairs.data(), B, params, who);
+}
+
+int colored_batch(void* stream, const psulvsb_colored_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                  double lambda, const psulvsb_robust_kernel_t* loss, void* d_work, psulvsb_icp_result_t* d_results,
+                  psulvsb_icp_iteration_t* d_trace, int* d_corr, const char* who) {
+  if (B < 0 || !colored_args_ok(params, lambda, loss) || (B > 0 && (!pairs || !d_work || !d_results)))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  std::vector<psulvsb_icp_pair_t> icp;
+  std::vector<const double*> scol, tcol;
+  if (int rc = colored_pairs(pairs, B, params, icp, scol, tcol, who)) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = need_device()) return rc;
+  return run_icp((cudaStream_t)stream, icp.data(), B, *params, colored_objective(scol.data(), tcol.data(), lambda, loss),
+                 d_work, d_results, d_trace, d_corr);
+}
+
+int colored_batch_host(const psulvsb_colored_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                       double lambda, const psulvsb_robust_kernel_t* loss, psulvsb_icp_result_t* results,
+                       psulvsb_icp_iteration_t* trace, int* corr, const char* who) {
+  if (B < 0 || !colored_args_ok(params, lambda, loss) || (B > 0 && (!pairs || !results)))
+    return fail(PSULVSB_ERR_INVALID, std::string(who) + ": bad argument");
+  std::vector<psulvsb_icp_pair_t> icp;
+  std::vector<const double*> scol, tcol;
+  if (int rc = colored_pairs(pairs, B, params, icp, scol, tcol, who)) return rc;
+  if (B == 0) return PSULVSB_OK;
+  if (int rc = need_device()) return rc;
+  return run_icp_host(icp.data(), B, *params, colored_objective(scol.data(), tcol.data(), lambda, loss), results,
+                      trace, corr, who);
+}
+
 }  // namespace
 
 }  // namespace psulvsb
@@ -1389,6 +1609,71 @@ int psulvsb_gicp_robust_batch_host(const psulvsb_gicp_pair_t* pairs, int B, cons
   if (!psulvsb::loss_ok(loss)) return fail(PSULVSB_ERR_INVALID, "psulvsb_gicp_robust_batch_host: bad argument");
   return psulvsb::gicp_batch_host(pairs, B, params, epsilon, loss, results, trace, corr,
                                   "psulvsb_gicp_robust_batch_host");
+}
+
+unsigned long long psulvsb_colored_icp_workspace_bytes(int n_s, int n_t) {
+  if (n_s < 0 || n_t < 0) return 0ull;
+  const psulvsb_icp_pair_t p{nullptr, n_s, nullptr, n_t, nullptr, {}, {}};
+  return (unsigned long long)psulvsb::colored_layout(&p, 1, nullptr, nullptr, nullptr);
+}
+
+unsigned long long psulvsb_colored_icp_batch_workspace_bytes(const psulvsb_colored_icp_pair_t* pairs, int B) {
+  if (B <= 0 || !pairs) return 0ull;
+  std::vector<psulvsb_icp_pair_t> sizes((size_t)B);
+  for (int b = 0; b < B; ++b) {
+    if (pairs[b].n_s < 0 || pairs[b].n_t < 0) return 0ull;
+    sizes[b].n_s = pairs[b].n_s;
+    sizes[b].n_t = pairs[b].n_t;
+  }
+  return (unsigned long long)psulvsb::colored_layout(sizes.data(), B, nullptr, nullptr, nullptr);
+}
+
+// the single calls are batches of one: an empty cloud gives T0 through k9_icp_bounds, as a batch's empty pair does
+static psulvsb_colored_icp_pair_t colored_pair(const double* src, int n_s, const double* src_colors, const double* tgt,
+                                               int n_t, const double* tgt_colors, const double* tgt_normals,
+                                               const double R0[9], const double t0[3]) {
+  psulvsb_colored_icp_pair_t p{src, n_s, src_colors, tgt, n_t, tgt_colors, tgt_normals, {}, {}};
+  if (R0) std::memcpy(p.R0, R0, sizeof p.R0);
+  if (t0) std::memcpy(p.t0, t0, sizeof p.t0);
+  return p;
+}
+
+int psulvsb_colored_icp(void* stream, const double* d_src, int n_s, const double* d_src_colors, const double* d_tgt,
+                        int n_t, const double* d_tgt_colors, const double* d_tgt_normals,
+                        const psulvsb_icp_params_t* params, double lambda_geometric,
+                        const psulvsb_robust_kernel_t* loss, const double R0[9], const double t0[3], void* d_work,
+                        psulvsb_icp_result_t* d_result, psulvsb_icp_iteration_t* d_trace, int* d_corr) {
+  if (!R0 || !t0) return fail(PSULVSB_ERR_INVALID, "psulvsb_colored_icp: bad argument");
+  const psulvsb_colored_icp_pair_t p =
+      colored_pair(d_src, n_s, d_src_colors, d_tgt, n_t, d_tgt_colors, d_tgt_normals, R0, t0);
+  return psulvsb::colored_batch(stream, &p, 1, params, lambda_geometric, loss, d_work, d_result, d_trace, d_corr,
+                                "psulvsb_colored_icp");
+}
+
+int psulvsb_colored_icp_host(const double* src, int n_s, const double* src_colors, const double* tgt, int n_t,
+                             const double* tgt_colors, const double* tgt_normals, const psulvsb_icp_params_t* params,
+                             double lambda_geometric, const psulvsb_robust_kernel_t* loss, const double R0[9],
+                             const double t0[3], psulvsb_icp_result_t* result, psulvsb_icp_iteration_t* trace,
+                             int* corr) {
+  if (!R0 || !t0) return fail(PSULVSB_ERR_INVALID, "psulvsb_colored_icp_host: bad argument");
+  const psulvsb_colored_icp_pair_t p = colored_pair(src, n_s, src_colors, tgt, n_t, tgt_colors, tgt_normals, R0, t0);
+  return psulvsb::colored_batch_host(&p, 1, params, lambda_geometric, loss, result, trace, corr,
+                                     "psulvsb_colored_icp_host");
+}
+
+int psulvsb_colored_icp_batch(void* stream, const psulvsb_colored_icp_pair_t* pairs, int B,
+                              const psulvsb_icp_params_t* params, double lambda_geometric,
+                              const psulvsb_robust_kernel_t* loss, void* d_work, psulvsb_icp_result_t* d_results,
+                              psulvsb_icp_iteration_t* d_trace, int* d_corr) {
+  return psulvsb::colored_batch(stream, pairs, B, params, lambda_geometric, loss, d_work, d_results, d_trace, d_corr,
+                                "psulvsb_colored_icp_batch");
+}
+
+int psulvsb_colored_icp_batch_host(const psulvsb_colored_icp_pair_t* pairs, int B, const psulvsb_icp_params_t* params,
+                                   double lambda_geometric, const psulvsb_robust_kernel_t* loss,
+                                   psulvsb_icp_result_t* results, psulvsb_icp_iteration_t* trace, int* corr) {
+  return psulvsb::colored_batch_host(pairs, B, params, lambda_geometric, loss, results, trace, corr,
+                                     "psulvsb_colored_icp_batch_host");
 }
 
 }  // extern "C"

@@ -1,10 +1,11 @@
 """Correspondences from two raw clouds: FPFH descriptors, the two-way descriptor nearest neighbour and FGR's matcher;
-surface normals alone (radius or hybrid neighbourhood) on the same grid; and the voxel-grid filter that comes first.
+surface normals alone (radius or hybrid neighbourhood) on the same grid; the voxel-grid filter that comes first; and
+the colour gradients of colored ICP (`color_gradients`, on the same grid; icp.colored_icp computes them itself).
 
 What upstream TEASER++ gets from teaser::FPFHEstimation and teaser::Matcher (over PCL and FLANN), on the GPU through
 the C ABI (include/psulvsb.h, csrc/k8_features.cu).  Host arrays in, host arrays out, except fpfh_device /
 nearest_neighbours_device / fpfh_batch_device / match_batch_device / normals_device / normals_batch_device /
-voxel_down_sample_device / voxel_down_sample_batch_device, which take and return CUDA tensors on the current stream.
+voxel_down_sample_device / voxel_down_sample_batch_device / color_gradients_batch_device, which take and return CUDA tensors on the current stream.
 The _batch functions compute B clouds or B pairs in one call; each item's result is bit-identical to the single call
 on it alone.
 """
@@ -235,6 +236,83 @@ def normals_batch_device(d_clouds, radius: float, max_nn: int = 0, viewpoints=No
     N = sum(sizes)
     out = torch.empty((max(N, 1), 3), dtype=torch.float64, device=dev)
     capi.check(L.psulvsb_normals_batch(_stream(), arr, B, float(radius), int(max_nn), _dev(work), _dev(out)))
+    views, o = [], 0
+    for n in sizes:
+        views.append(out[o:o + n])
+        o += n
+    return out[:N], views
+
+
+def _color_clouds(ptrs, sizes):
+    """psulvsb_color_cloud_t[B] from (points, colors, normals) pointers and n per cloud."""
+    arr = (capi.ColorCloud * max(len(sizes), 1))()
+    for c, ((pp, pc, pn), n) in enumerate(zip(ptrs, sizes)):
+        arr[c].points, arr[c].n, arr[c].colors, arr[c].normals = pp, n, pc, pn
+    return arr
+
+
+def _same_shape(a, cloud, what) -> np.ndarray:
+    a = _cm(a)
+    if a.shape != cloud.shape:
+        raise ValueError(f"{what}: one per point is needed, got {a.shape} for {cloud.shape}")
+    return a
+
+
+def color_gradients(points, colors, normals, radius: float, max_nn: int = 30) -> np.ndarray:
+    """The colour gradient of every point (3 x n float64; Open3D's InitializePointCloudForColoredICP): points, colors
+    ([0, 1] RGB) and normals 3 x n.  The hybrid neighbourhood (`radius`, 4 <= max_nn <= 32) of `normals`; 0 where
+    fewer than 4 points are kept, the normal is not finite or the 3x3 solve fails.  A batch of one cloud."""
+    return color_gradients_batch([points], [colors], [normals], radius, max_nn)[0]
+
+
+def color_gradients_batch(clouds, colors, normals, radius: float, max_nn: int = 30) -> list:
+    """psulvsb_color_gradients_batch_host: B clouds (3 x n_c each) with their colours and normals in one call.  Returns
+    one 3 x n_c float64 gradient array per cloud, each equal bit for bit to a batch of that cloud alone."""
+    ps = [_cm(p) for p in clouds]
+    B = len(ps)
+    if len(colors) != B or len(normals) != B:
+        raise ValueError(f"{B} clouds, {len(colors)} colour and {len(normals)} normal sets")
+    cs = [_same_shape(c, p, "colors") for c, p in zip(colors, ps)]
+    ns = [_same_shape(n, p, "normals") for n, p in zip(normals, ps)]
+    sizes = [p.shape[1] for p in ps]
+    arr = _color_clouds([(p.ctypes.data, c.ctypes.data, n.ctypes.data) if p.shape[1] else (None, None, None)
+                         for p, c, n in zip(ps, cs, ns)], sizes)
+    out = np.zeros((max(sum(sizes), 1), 3), dtype=np.float64)
+    capi.check(capi.lib().psulvsb_color_gradients_batch_host(arr, B, float(radius), int(max_nn), out.ctypes.data))
+    res, o = [], 0
+    for n in sizes:
+        res.append(np.asfortranarray(out[o:o + n].T))
+        o += n
+    return res
+
+
+def color_gradients_batch_device(d_clouds, d_colors, d_normals, radius: float, max_nn: int = 30, work=None):
+    """psulvsb_color_gradients_batch on CUDA tensors [n_c, 3] float64 and the current stream.  Returns (gradients
+    [sum n, 3], views): views[c] = cloud c's rows.  `work`: an optional uint8 CUDA tensor of at least
+    psulvsb_color_gradients_batch_workspace_bytes bytes to reuse."""
+    import torch
+
+    from .stages import _dev, _stream
+
+    B = len(d_clouds)
+    if len(d_colors) != B or len(d_normals) != B:
+        raise ValueError(f"{B} clouds, {len(d_colors)} colour and {len(d_normals)} normal sets")
+    for p, c, n in zip(d_clouds, d_colors, d_normals):
+        if tuple(c.shape) != tuple(p.shape) or tuple(n.shape) != tuple(p.shape):
+            raise ValueError("one colour and one normal per point are needed")
+    sizes = [int(p.shape[0]) for p in d_clouds]
+    arr = _color_clouds([(_dev(p), _dev(c), _dev(n)) if k else (None, None, None)
+                         for p, c, n, k in zip(d_clouds, d_colors, d_normals, sizes)], sizes)
+    L = capi.lib()
+    dev = d_clouds[0].device if B else torch.device("cuda")
+    nbytes = L.psulvsb_color_gradients_batch_workspace_bytes(arr, B)
+    if work is None:
+        work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=dev)
+    elif work.numel() < nbytes:
+        raise ValueError("work is smaller than psulvsb_color_gradients_batch_workspace_bytes(clouds, B)")
+    N = sum(sizes)
+    out = torch.empty((max(N, 1), 3), dtype=torch.float64, device=dev)
+    capi.check(L.psulvsb_color_gradients_batch(_stream(), arr, B, float(radius), int(max_nn), _dev(work), _dev(out)))
     views, o = [], 0
     for n in sizes:
         views.append(out[o:o + n])

@@ -11,6 +11,9 @@ or hybrid normals of `features.normals` / `features.normals_batch` (on the grid,
 normals `features.fpfh` returns or the k-NN normals of `stages.estimate_normals`.
 Every call takes `loss=`, a robust kernel of the point-to-plane or generalized-ICP update under Open3D's names
 (`L2Loss`, `HuberLoss`, `CauchyLoss`, `GMLoss`, `TukeyLoss`; DESIGN.md section 11, "Robust kernels").
+`colored_icp`, `colored_icp_device`, `colored_icp_batch` and `colored_icp_batch_device` are colored ICP (Open3D's
+registration_colored_icp; DESIGN.md section 11, "Colored ICP"): point-to-plane's loop with a geometric and a
+photometric row per correspondence; they need both clouds' [0, 1] RGB colours and the target's normals.
 Convention: q ~ R p + t.
 """
 from __future__ import annotations
@@ -447,6 +450,161 @@ def gicp_batch_device(d_srcs, d_tgts, d_src_normals, d_tgt_normals, R0s, t0s, ma
         capi.check(L.psulvsb_gicp_batch(_stream(), pairs, B, C.byref(p), float(epsilon), *tail))
     else:
         capi.check(L.psulvsb_gicp_robust_batch(_stream(), pairs, B, C.byref(p), float(epsilon), loss._c(), *tail))
+    res = (capi.IcpResult * max(B, 1)).from_buffer_copy(out.cpu().numpy().tobytes())
+    records = None
+    if trace and B:
+        records = (capi.IcpIteration * (B * nrec)).from_buffer_copy(rec.cpu().numpy().tobytes())
+    return _batch_results(res, records, nrec, corr, sizes)
+
+
+def _colored_params(d, max_iterations, relative_fitness, relative_rmse) -> capi.IcpParams:
+    return _params(d, False, max_iterations, relative_fitness, relative_rmse)
+
+
+def _loss_c(loss):
+    return None if loss is None else loss._c()
+
+
+def colored_icp(src, tgt, src_colors, tgt_colors, tgt_normals, R0, t0, max_correspondence_distance: float, *,
+                lambda_geometric: float = 0.968, loss: Optional[RobustKernel] = None, max_iterations: int = 30,
+                relative_fitness: float = 1e-6, relative_rmse: float = 1e-6, trace: bool = False) -> IcpResult:
+    """psulvsb_colored_icp_host: refine (R0, t0) so that tgt ~ R src + t with colored ICP.  src, src_colors 3 x n_s;
+    tgt, tgt_colors, tgt_normals 3 x n_t; colours are [0, 1] RGB.  lambda_geometric in [0, 1] weighs the geometric
+    rows against the photometric ones (1: point-to-plane ICP); loss: a robust kernel applied to each row, None = L2.
+    The target's colour gradients are computed inside the call (features.color_gradients with radius 2 d, max_nn 30)."""
+    s, q = _cm(src, "src"), _cm(tgt, "tgt")
+    sc, tc, tn = (_normals(src_colors, s, "src_colors"), _normals(tgt_colors, q, "tgt_colors"),
+                  _normals(tgt_normals, q, "tgt_normals"))
+    p = _colored_params(max_correspondence_distance, max_iterations, relative_fitness, relative_rmse)
+    R, t = _transform(R0, t0)
+    res = capi.IcpResult()
+    records = (capi.IcpIteration * (max(int(max_iterations), 0) + 1))() if trace else None
+    corr = np.empty(s.shape[1], dtype=np.int32)
+    capi.check(capi.lib().psulvsb_colored_icp_host(s.ctypes.data, s.shape[1], sc.ctypes.data, q.ctypes.data,
+                                                   q.shape[1], tc.ctypes.data, tn.ctypes.data, C.byref(p),
+                                                   float(lambda_geometric), _loss_c(loss), R, t, C.byref(res), records,
+                                                   corr.ctypes.data))
+    return _result(res, records, corr)
+
+
+def colored_icp_device(d_src, d_tgt, d_src_colors, d_tgt_colors, d_tgt_normals, R0, t0,
+                       max_correspondence_distance: float, *, lambda_geometric: float = 0.968,
+                       loss: Optional[RobustKernel] = None, max_iterations: int = 30, relative_fitness: float = 1e-6,
+                       relative_rmse: float = 1e-6, trace: bool = False, work=None) -> IcpResult:
+    """psulvsb_colored_icp on CUDA tensors [n, 3] float64 (colours and normals the same shape as their clouds) and the
+    current stream; the outputs as `icp_device`.  `work`: an optional uint8 CUDA tensor of at least
+    psulvsb_colored_icp_workspace_bytes(n_s, n_t) bytes to reuse."""
+    import torch
+
+    from .stages import _dev, _stream
+
+    ns, nt = d_src.shape[0], d_tgt.shape[0]
+    if tuple(d_src_colors.shape) != tuple(d_src.shape) or any(tuple(a.shape) != tuple(d_tgt.shape)
+                                                               for a in (d_tgt_colors, d_tgt_normals)):
+        raise ValueError("one colour per point and one normal per target point are needed")
+    dev = d_src.device
+    nbytes = capi.lib().psulvsb_colored_icp_workspace_bytes(ns, nt)
+    if work is None:
+        work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=dev)
+    elif work.numel() < nbytes:
+        raise ValueError("work is smaller than psulvsb_colored_icp_workspace_bytes(n_s, n_t)")
+    nrec = max(int(max_iterations), 0) + 1
+    out = torch.empty(C.sizeof(capi.IcpResult), dtype=torch.uint8, device=dev)
+    rec = torch.empty(nrec * C.sizeof(capi.IcpIteration) if trace else 1, dtype=torch.uint8, device=dev)
+    corr = torch.empty(max(ns, 1), dtype=torch.int32, device=dev)
+    p = _colored_params(max_correspondence_distance, max_iterations, relative_fitness, relative_rmse)
+    R, t = _transform(R0, t0)
+    ptr = lambda x: _dev(x) if x.shape[0] else None                  # noqa: E731
+    capi.check(capi.lib().psulvsb_colored_icp(_stream(), ptr(d_src), ns, ptr(d_src_colors), ptr(d_tgt), nt,
+                                              ptr(d_tgt_colors), ptr(d_tgt_normals), C.byref(p),
+                                              float(lambda_geometric), _loss_c(loss), R, t, _dev(work), _dev(out),
+                                              _dev(rec) if trace else None, _dev(corr)))
+    res = capi.IcpResult.from_buffer_copy(out.cpu().numpy().tobytes())
+    records = None
+    if trace:
+        records = (capi.IcpIteration * nrec).from_buffer_copy(rec.cpu().numpy().tobytes())
+    return _result(res, records, corr[:ns])
+
+
+def _colored_pairs(ptrs, sizes, R, t):
+    """psulvsb_colored_icp_pair_t[B] from (src, src_colors, tgt, tgt_colors, tgt_normals) pointers and (n_s, n_t)."""
+    pairs = (capi.ColoredIcpPair * max(len(sizes), 1))()
+    for b, ((ps, psc, pt, ptc, ptn), (ns, nt)) in enumerate(zip(ptrs, sizes)):
+        q = pairs[b]
+        q.src, q.n_s, q.src_colors, q.tgt, q.n_t, q.tgt_colors, q.tgt_normals = ps, ns, psc, pt, nt, ptc, ptn
+        q.R0[:] = R[b].flatten(order="F").tolist()
+        q.t0[:] = t[b].tolist()
+    return pairs
+
+
+def colored_icp_batch(srcs, tgts, src_colors, tgt_colors, tgt_normals, R0s, t0s, max_correspondence_distance: float,
+                      *, lambda_geometric: float = 0.968, loss: Optional[RobustKernel] = None,
+                      max_iterations: int = 30, relative_fitness: float = 1e-6, relative_rmse: float = 1e-6,
+                      trace: bool = False) -> list:
+    """psulvsb_colored_icp_batch_host: refine B pairs with colored ICP in one call with shared parameters.  srcs, tgts,
+    src_colors, tgt_colors, tgt_normals: sequences of 3 x n arrays; R0s [B, 3, 3], t0s [B, 3].  Returns one IcpResult
+    per pair, each equal bit for bit to `colored_icp` on that pair alone."""
+    s = [_cm(a, "src") for a in srcs]
+    q = [_cm(a, "tgt") for a in tgts]
+    B = len(s)
+    if len(q) != B or len(src_colors) != B or len(tgt_colors) != B or len(tgt_normals) != B:
+        raise ValueError(f"{B} sources, {len(q)} targets, {len(src_colors)} and {len(tgt_colors)} colour sets, "
+                         f"{len(tgt_normals)} normal sets")
+    sc = [_normals(a, c, "src_colors") for a, c in zip(src_colors, s)]
+    tc = [_normals(a, c, "tgt_colors") for a, c in zip(tgt_colors, q)]
+    tn = [_normals(a, c, "tgt_normals") for a, c in zip(tgt_normals, q)]
+    R, t = _batch_transforms(R0s, t0s, B)
+    sizes = [(a.shape[1], b.shape[1]) for a, b in zip(s, q)]
+    pairs = _colored_pairs([(a.ctypes.data, b.ctypes.data, c.ctypes.data, d.ctypes.data, e.ctypes.data)
+                            for a, b, c, d, e in zip(s, sc, q, tc, tn)], sizes, R, t)
+    p = _colored_params(max_correspondence_distance, max_iterations, relative_fitness, relative_rmse)
+    nrec = max(int(max_iterations), 0) + 1
+    res = (capi.IcpResult * max(B, 1))()
+    records = (capi.IcpIteration * (B * nrec))() if trace and B else None
+    corr = np.empty(sum(ns for ns, _ in sizes), dtype=np.int32)
+    capi.check(capi.lib().psulvsb_colored_icp_batch_host(pairs, B, C.byref(p), float(lambda_geometric),
+                                                         _loss_c(loss), res, records, corr.ctypes.data))
+    return _batch_results(res, records, nrec, corr, sizes)
+
+
+def colored_icp_batch_device(d_srcs, d_tgts, d_src_colors, d_tgt_colors, d_tgt_normals, R0s, t0s,
+                             max_correspondence_distance: float, *, lambda_geometric: float = 0.968,
+                             loss: Optional[RobustKernel] = None, max_iterations: int = 30,
+                             relative_fitness: float = 1e-6, relative_rmse: float = 1e-6, trace: bool = False,
+                             work=None) -> list:
+    """psulvsb_colored_icp_batch on sequences of CUDA tensors [n, 3] float64 and the current stream; the outputs as
+    `icp_batch_device`.  `work`: an optional uint8 CUDA tensor of at least psulvsb_colored_icp_batch_workspace_bytes
+    bytes to reuse."""
+    import torch
+
+    from .stages import _dev, _stream
+
+    B = len(d_srcs)
+    if len(d_tgts) != B or len(d_src_colors) != B or len(d_tgt_colors) != B or len(d_tgt_normals) != B:
+        raise ValueError(f"{B} sources, {len(d_tgts)} targets, {len(d_src_colors)} and {len(d_tgt_colors)} colour "
+                         f"sets, {len(d_tgt_normals)} normal sets")
+    for c, a in list(zip(d_srcs, d_src_colors)) + list(zip(d_tgts, d_tgt_colors)) + list(zip(d_tgts, d_tgt_normals)):
+        if tuple(a.shape) != tuple(c.shape):
+            raise ValueError("one colour per point and one normal per target point are needed")
+    R, t = _batch_transforms(R0s, t0s, B)
+    sizes = [(a.shape[0], b.shape[0]) for a, b in zip(d_srcs, d_tgts)]
+    ptr = lambda x: _dev(x) if x.shape[0] else None                  # noqa: E731
+    pairs = _colored_pairs([(ptr(a), ptr(b), ptr(c), ptr(d), ptr(e)) for a, b, c, d, e in
+                            zip(d_srcs, d_src_colors, d_tgts, d_tgt_colors, d_tgt_normals)], sizes, R, t)
+    L = capi.lib()
+    nbytes = L.psulvsb_colored_icp_batch_workspace_bytes(pairs, B)
+    dev = d_srcs[0].device if B else torch.device("cuda")
+    if work is None:
+        work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=dev)
+    elif work.numel() < nbytes:
+        raise ValueError("work is smaller than psulvsb_colored_icp_batch_workspace_bytes(pairs, B)")
+    nrec = max(int(max_iterations), 0) + 1
+    out = torch.empty(max(B, 1) * C.sizeof(capi.IcpResult), dtype=torch.uint8, device=dev)
+    rec = torch.empty(B * nrec * C.sizeof(capi.IcpIteration) if trace and B else 1, dtype=torch.uint8, device=dev)
+    corr = torch.empty(max(sum(ns for ns, _ in sizes), 1), dtype=torch.int32, device=dev)
+    p = _colored_params(max_correspondence_distance, max_iterations, relative_fitness, relative_rmse)
+    capi.check(L.psulvsb_colored_icp_batch(_stream(), pairs, B, C.byref(p), float(lambda_geometric), _loss_c(loss),
+                                           _dev(work), _dev(out), _dev(rec) if trace else None, _dev(corr)))
     res = (capi.IcpResult * max(B, 1)).from_buffer_copy(out.cpu().numpy().tobytes())
     records = None
     if trace and B:
