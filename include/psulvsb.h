@@ -768,6 +768,29 @@ int psulvsb_color_gradients_batch(void* stream, const psulvsb_color_cloud_t* clo
 int psulvsb_color_gradients_batch_host(const psulvsb_color_cloud_t* clouds, int B, double radius, int max_nn,
                                        double* gradients);
 
+/* ---- Voxel downsampling with colours (DESIGN.md section 10, "Voxel downsampling with colours"): the voxel filter
+ * above on a cloud with a colour per point (3 x n doubles, [0, 1] RGB, not range-checked), as Open3D's
+ * VoxelDownSample does on a cloud with colours.  The voxels, their order and the counts are bit for bit those of the
+ * plain calls on the same points.  A voxel's colour is the sum of its members' colours per channel (FP64 from 0.0, in
+ * ascending input index, no FMA) divided once by the count; column c of the colour output belongs to column c of the
+ * voxel output.  A point dropped for a non-finite coordinate takes its colour with it; a non-finite colour of a kept
+ * point reaches its own voxel's channel only.  Refusals, zero counts and the device rules are the plain calls', and a
+ * NULL colour array of a non-empty cloud is PSULVSB_ERR_INVALID before any device work.  Batch items are
+ * psulvsb_color_cloud_t (`normals` is ignored).  Workspaces depend on the sizes only; the _host variants upload points
+ * and colours in one copy. */
+unsigned long long psulvsb_voxel_down_sample_colors_workspace_bytes(int n);
+int psulvsb_voxel_down_sample_colors(void* stream, const double* d_pts, const double* d_colors, int n,
+                                     double voxel_size, void* d_work, double* d_out /* 3 x n capacity */,
+                                     double* d_out_colors /* 3 x n capacity */, int* d_count);
+int psulvsb_voxel_down_sample_colors_host(const double* pts, const double* colors, int n, double voxel_size,
+                                          double* out /* 3 x n */, double* out_colors /* 3 x n */, int* n_out);
+unsigned long long psulvsb_voxel_down_sample_colors_batch_workspace_bytes(const psulvsb_color_cloud_t* clouds, int B);
+int psulvsb_voxel_down_sample_colors_batch(void* stream, const psulvsb_color_cloud_t* clouds, int B,
+                                           double voxel_size, void* d_work, double* d_out, double* d_out_colors,
+                                           int* d_counts);
+int psulvsb_voxel_down_sample_colors_batch_host(const psulvsb_color_cloud_t* clouds, int B, double voxel_size,
+                                                double* out, double* out_colors, int* counts);
+
 /* Clique escalation (registration.cc:1000-1085 -> teaser/src/graph.cc:12-125, PMC exact maximum clique) of the
  * graph with n_vertices vertices and the given edges (uint2 endpoint pairs).  A deterministic greedy maximal
  * clique (most neighbours among the remaining candidates first, ties: lowest index) gives the lower bound;

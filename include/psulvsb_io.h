@@ -51,6 +51,10 @@ int psulvsb_prefilter_reduce_batch(int B, const double* const* src_normals, cons
 /* PLY: number of vertices, then their x, y, z as float (teaser::PointXYZ is 3 x float). */
 int psulvsb_ply_vertex_count(const char* path, long long* n);
 int psulvsb_ply_read_xyz(const char* path, float* xyz, long long capacity, long long* n);
+/* The same vertices with their colours, read in the same pass: the vertex properties red, green and blue, uchar / uint8
+ * values divided by 255, float / double values as stored; rgb has xyz's layout (3 doubles per vertex).  A missing
+ * channel or any other type is PSULVSB_ERR_INVALID with a message. */
+int psulvsb_ply_read_xyz_rgb(const char* path, float* xyz, double* rgb, long long capacity, long long* n);
 
 /* Correspondence text files.  A first line holding a single integer (the count-header variant) is
  * skipped; malformed lines are skipped like the reference's `if (iss >> ...)`. */

@@ -50,6 +50,9 @@ SYMBOLS = [
     "psulvsb_colored_icp_host", "psulvsb_colored_icp_batch", "psulvsb_colored_icp_batch_host",
     "psulvsb_color_gradients_batch_workspace_bytes", "psulvsb_color_gradients_batch",
     "psulvsb_color_gradients_batch_host",
+    "psulvsb_voxel_down_sample_colors_workspace_bytes", "psulvsb_voxel_down_sample_colors",
+    "psulvsb_voxel_down_sample_colors_host", "psulvsb_voxel_down_sample_colors_batch_workspace_bytes",
+    "psulvsb_voxel_down_sample_colors_batch", "psulvsb_voxel_down_sample_colors_batch_host",
 ]
 UNIQUE_ID_BYTES = 128
 
@@ -244,7 +247,7 @@ class ColoredIcpPair(C.Structure):
 
 
 class ColorCloud(C.Structure):
-    """psulvsb_color_cloud_t: one cloud of a colour-gradient batch."""
+    """psulvsb_color_cloud_t: one cloud of a colour-gradient or colour voxel-filter batch."""
     _fields_ = [
         ("points", C.c_void_p),
         ("n", C.c_int),
@@ -458,6 +461,16 @@ def _declare(L: C.CDLL) -> None:
     L.psulvsb_color_gradients_batch_workspace_bytes.restype = _ull
     L.psulvsb_color_gradients_batch.argtypes = [_vp, C.POINTER(ColorCloud), C.c_int, C.c_double, C.c_int, _vp, _vp]
     L.psulvsb_color_gradients_batch_host.argtypes = [C.POINTER(ColorCloud), C.c_int, C.c_double, C.c_int, _vp]
+    L.psulvsb_voxel_down_sample_colors_workspace_bytes.argtypes = [C.c_int]
+    L.psulvsb_voxel_down_sample_colors_workspace_bytes.restype = _ull
+    L.psulvsb_voxel_down_sample_colors.argtypes = [_vp, _vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp]
+    L.psulvsb_voxel_down_sample_colors_host.argtypes = [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp]
+    L.psulvsb_voxel_down_sample_colors_batch_workspace_bytes.argtypes = [C.POINTER(ColorCloud), C.c_int]
+    L.psulvsb_voxel_down_sample_colors_batch_workspace_bytes.restype = _ull
+    L.psulvsb_voxel_down_sample_colors_batch.argtypes = [_vp, C.POINTER(ColorCloud), C.c_int, C.c_double, _vp, _vp,
+                                                         _vp, _vp]
+    L.psulvsb_voxel_down_sample_colors_batch_host.argtypes = [C.POINTER(ColorCloud), C.c_int, C.c_double, _vp, _vp,
+                                                              _vp]
     for name in SYMBOLS:
         getattr(L, name)  # AttributeError here = the library does not export what the header declares
 

@@ -1,5 +1,5 @@
 // host_io.cpp -- host-side helpers of the callers around the hot path (include/psulvsb_io.h):
-// PLY vertex reader, correspondence files.  (The pre-filter and reduced-set builder are device code: k7_prefilter.cu.)
+// PLY vertex reader (positions, and colours on request), correspondence files.  (The pre-filter and reduced-set builder are device code: k7_prefilter.cu.)
 // Plain C++17, no CUDA, no third-party dependency (the reference uses PCL/Eigen/tinyply here).
 #include <algorithm>
 #include <climits>
@@ -130,8 +130,12 @@ unsigned long long list_count(const unsigned char* p, int size, bool swap) {
   return load_scalar<uint32_t>(p, swap);
 }
 
-// reads the vertex element; xyz == nullptr: only counts
-int ply_read(const char* path, float* xyz, long long capacity, long long* n_out) {
+// a colour channel's value: uchar / uint8 over 255, float / double as stored
+double color_value(double v, const PlyProp& pr) { return pr.kind == 'u' ? v / 255.0 : v; }
+
+// reads the vertex element; xyz == nullptr: only counts.  rgb != nullptr: the red, green and blue properties too
+// (uchar / uint8, float or double; anything else, or a missing channel, is refused)
+int ply_read(const char* path, float* xyz, double* rgb, long long capacity, long long* n_out) {
   if (!path || !n_out) return fail(PSULVSB_ERR_INVALID, "ply: NULL argument");
   std::ifstream f(path, std::ios::binary);
   if (!f.is_open()) return fail(PSULVSB_ERR_INVALID, std::string("ply: cannot open ") + path);
@@ -153,6 +157,20 @@ int ply_read(const char* path, float* xyz, long long capacity, long long* n_out)
     if (V.props[p].name == "z") iz = (int)p;
   }
   if (ix < 0 || iy < 0 || iz < 0) return fail(PSULVSB_ERR_INVALID, "ply: vertex element lacks x / y / z");
+  int ic[3] = {-1, -1, -1};
+  if (rgb) {
+    static const char* const kChannel[3] = {"red", "green", "blue"};
+    for (int k = 0; k < 3; ++k) {
+      for (size_t p = 0; p < V.props.size(); ++p)
+        if (V.props[p].name == kChannel[k]) ic[k] = (int)p;
+      if (ic[k] < 0)
+        return fail(PSULVSB_ERR_INVALID, std::string("ply: vertex element lacks ") + kChannel[k] + " in " + path);
+      const PlyProp& pr = V.props[(size_t)ic[k]];
+      if (pr.is_list || !((pr.kind == 'u' && pr.size == 1) || pr.kind == 'f'))
+        return fail(PSULVSB_ERR_INVALID, std::string("ply: unsupported type of vertex property ") + kChannel[k] +
+                                             " (uchar / uint8, float or double) in " + path);
+    }
+  }
   f.clear();
   f.seekg(h.data_begin);
   const bool host_le = [] { const uint16_t one = 1; return *reinterpret_cast<const unsigned char*>(&one) == 1; }();
@@ -174,6 +192,9 @@ int ply_read(const char* path, float* xyz, long long capacity, long long* n_out)
           if ((int)p == ix) xyz[3 * r + 0] = (float)v;
           if ((int)p == iy) xyz[3 * r + 1] = (float)v;
           if ((int)p == iz) xyz[3 * r + 2] = (float)v;
+          if (rgb)
+            for (int k = 0; k < 3; ++k)
+              if ((int)p == ic[k]) rgb[3 * r + k] = color_value(v, E.props[p]);
         }
       } else {
         for (size_t p = 0; p < E.props.size(); ++p) {
@@ -190,6 +211,9 @@ int ply_read(const char* path, float* xyz, long long capacity, long long* n_out)
               if ((int)p == ix) xyz[3 * r + 0] = (float)scalar_as_double(buf, pr, swap);
               if ((int)p == iy) xyz[3 * r + 1] = (float)scalar_as_double(buf, pr, swap);
               if ((int)p == iz) xyz[3 * r + 2] = (float)scalar_as_double(buf, pr, swap);
+              if (rgb)
+                for (int k = 0; k < 3; ++k)
+                  if ((int)p == ic[k]) rgb[3 * r + k] = color_value(scalar_as_double(buf, pr, swap), pr);
             }
           }
         }
@@ -243,10 +267,14 @@ int corr_read(const char* path, double* src, double* dst, long long capacity, lo
 
 extern "C" {
 
-int psulvsb_ply_vertex_count(const char* path, long long* n) { return ply_read(path, nullptr, 0, n); }
+int psulvsb_ply_vertex_count(const char* path, long long* n) { return ply_read(path, nullptr, nullptr, 0, n); }
 int psulvsb_ply_read_xyz(const char* path, float* xyz, long long capacity, long long* n) {
   if (!xyz) return fail(PSULVSB_ERR_INVALID, "psulvsb_ply_read_xyz: NULL output");
-  return ply_read(path, xyz, capacity, n);
+  return ply_read(path, xyz, nullptr, capacity, n);
+}
+int psulvsb_ply_read_xyz_rgb(const char* path, float* xyz, double* rgb, long long capacity, long long* n) {
+  if (!xyz || !rgb) return fail(PSULVSB_ERR_INVALID, "psulvsb_ply_read_xyz_rgb: NULL output");
+  return ply_read(path, xyz, rgb, capacity, n);
 }
 int psulvsb_corr_count(const char* path, long long* n) { return corr_read(path, nullptr, nullptr, 0, n); }
 int psulvsb_corr_read(const char* path, double* src, double* dst, long long capacity, long long* n) {

@@ -1,5 +1,6 @@
 """Correspondences from two raw clouds: FPFH descriptors, the two-way descriptor nearest neighbour and FGR's matcher;
-surface normals alone (radius or hybrid neighbourhood) on the same grid; the voxel-grid filter that comes first; and
+surface normals alone (radius or hybrid neighbourhood) on the same grid; the voxel-grid filter that comes first
+(`colors=` carries a colour per point through it); and
 the colour gradients of colored ICP (`color_gradients`, on the same grid; icp.colored_icp computes them itself).
 
 What upstream TEASER++ gets from teaser::FPFHEstimation and teaser::Matcher (over PCL and FLANN), on the GPU through
@@ -320,84 +321,133 @@ def color_gradients_batch_device(d_clouds, d_colors, d_normals, radius: float, m
     return out[:N], views
 
 
-def voxel_down_sample(points, voxel_size: float) -> np.ndarray:
+def voxel_down_sample(points, voxel_size: float, colors=None):
     """psulvsb_voxel_down_sample_host (Open3D's voxel_down_sample): 3xN points -> 3xM float64 voxel means, in ascending
-    order of each voxel's lowest input index.  Points with a non-finite coordinate are dropped."""
+    order of each voxel's lowest input index.  Points with a non-finite coordinate are dropped.  colors: 3xN [0, 1]
+    RGB, one per point (psulvsb_voxel_down_sample_colors_host): returns (voxels, voxel colours 3xM), the voxels bit for
+    bit those without colours, each colour the mean of its voxel's members' colours."""
     p = _cm(points)
     n = p.shape[1]
     out = np.zeros((3, max(n, 1)), dtype=np.float64, order="F")
     m = C.c_int(0)
-    capi.check(capi.lib().psulvsb_voxel_down_sample_host(p.ctypes.data if n else None, n, float(voxel_size),
-                                                         out.ctypes.data, C.byref(m)))
-    return out[:, :m.value].copy(order="F")
+    if colors is None:
+        capi.check(capi.lib().psulvsb_voxel_down_sample_host(p.ctypes.data if n else None, n, float(voxel_size),
+                                                             out.ctypes.data, C.byref(m)))
+        return out[:, :m.value].copy(order="F")
+    c = _same_shape(colors, p, "colors")
+    oc = np.zeros((3, max(n, 1)), dtype=np.float64, order="F")
+    capi.check(capi.lib().psulvsb_voxel_down_sample_colors_host(p.ctypes.data if n else None,
+                                                                c.ctypes.data if n else None, n, float(voxel_size),
+                                                                out.ctypes.data, oc.ctypes.data, C.byref(m)))
+    return out[:, :m.value].copy(order="F"), oc[:, :m.value].copy(order="F")
 
 
-def voxel_down_sample_device(d_pts, voxel_size: float, work=None):
+def voxel_down_sample_device(d_pts, voxel_size: float, work=None, colors=None):
     """psulvsb_voxel_down_sample on a CUDA tensor [N, 3] float64 (== column-major 3xN) and the current stream, without
     a host round trip.  Returns (voxels [N, 3], count [1] int32): the first count[0] rows are the voxels, the rest is
     unspecified.  `work`: an optional uint8 CUDA tensor of at least psulvsb_voxel_down_sample_workspace_bytes(N) bytes
-    to reuse."""
+    to reuse.  colors: a CUDA tensor [N, 3] float64 of [0, 1] RGB (psulvsb_voxel_down_sample_colors): returns (voxels,
+    voxel colours [N, 3], count), `work` then sized by psulvsb_voxel_down_sample_colors_workspace_bytes(N)."""
     import torch
 
     from .stages import _dev, _stream
 
     n = d_pts.shape[0]
-    nbytes = capi.lib().psulvsb_voxel_down_sample_workspace_bytes(n)
+    L = capi.lib()
+    if colors is not None and tuple(colors.shape) != tuple(d_pts.shape):
+        raise ValueError("colors: one colour per point is needed")
+    name = "psulvsb_voxel_down_sample_workspace_bytes" if colors is None else \
+        "psulvsb_voxel_down_sample_colors_workspace_bytes"
+    nbytes = getattr(L, name)(n)
     if work is None:
         work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=d_pts.device)
     elif work.numel() < nbytes:
-        raise ValueError("work is smaller than psulvsb_voxel_down_sample_workspace_bytes(n)")
+        raise ValueError(f"work is smaller than {name}(n)")
     out = torch.empty((max(n, 1), 3), dtype=torch.float64, device=d_pts.device)
     count = torch.empty(1, dtype=torch.int32, device=d_pts.device)
-    capi.check(capi.lib().psulvsb_voxel_down_sample(_stream(), _dev(d_pts) if n else None, n, float(voxel_size),
-                                                    _dev(work), _dev(out), _dev(count)))
-    return out[:n], count
+    if colors is None:
+        capi.check(L.psulvsb_voxel_down_sample(_stream(), _dev(d_pts) if n else None, n, float(voxel_size), _dev(work),
+                                               _dev(out), _dev(count)))
+        return out[:n], count
+    oc = torch.empty((max(n, 1), 3), dtype=torch.float64, device=d_pts.device)
+    capi.check(L.psulvsb_voxel_down_sample_colors(_stream(), _dev(d_pts) if n else None, _dev(colors) if n else None,
+                                                  n, float(voxel_size), _dev(work), _dev(out), _dev(oc), _dev(count)))
+    return out[:n], oc[:n], count
 
 
-def voxel_down_sample_batch(clouds, voxel_size: float) -> list:
+def voxel_down_sample_batch(clouds, voxel_size: float, colors=None) -> list:
     """psulvsb_voxel_down_sample_batch_host: B clouds (3 x n_c each) with a shared voxel size in one call.  Returns one
-    3 x m_c float64 array per cloud, each equal bit for bit to `voxel_down_sample` on that cloud alone."""
+    3 x m_c float64 array per cloud, each equal bit for bit to `voxel_down_sample` on that cloud alone.  colors: one
+    3 x n_c colour array per cloud (psulvsb_voxel_down_sample_colors_batch_host): returns (voxel list, colour list)."""
     ps = [_cm(p) for p in clouds]
     B = len(ps)
     sizes = [p.shape[1] for p in ps]
-    arr = _clouds([p.ctypes.data if p.shape[1] else None for p in ps], sizes, _viewpoints(None, B))
     out = np.zeros((max(sum(sizes), 1), 3), dtype=np.float64)
     counts = np.zeros(max(B, 1), dtype=np.int32)
-    capi.check(capi.lib().psulvsb_voxel_down_sample_batch_host(arr, B, float(voxel_size), out.ctypes.data,
-                                                               counts.ctypes.data))
-    res, o = [], 0
+    oc = None
+    if colors is None:
+        arr = _clouds([p.ctypes.data if p.shape[1] else None for p in ps], sizes, _viewpoints(None, B))
+        capi.check(capi.lib().psulvsb_voxel_down_sample_batch_host(arr, B, float(voxel_size), out.ctypes.data,
+                                                                   counts.ctypes.data))
+    else:
+        if len(colors) != B:
+            raise ValueError(f"{B} clouds and {len(colors)} colour sets")
+        cs = [_same_shape(c, p, "colors") for c, p in zip(colors, ps)]
+        arr = _color_clouds([(p.ctypes.data, c.ctypes.data, None) if p.shape[1] else (None, None, None)
+                             for p, c in zip(ps, cs)], sizes)
+        oc = np.zeros_like(out)
+        capi.check(capi.lib().psulvsb_voxel_down_sample_colors_batch_host(arr, B, float(voxel_size), out.ctypes.data,
+                                                                          oc.ctypes.data, counts.ctypes.data))
+    res, cres, o = [], [], 0
     for c, n in enumerate(sizes):
         res.append(np.asfortranarray(out[o:o + int(counts[c])].T))
+        if oc is not None:
+            cres.append(np.asfortranarray(oc[o:o + int(counts[c])].T))
         o += n
-    return res
+    return res if oc is None else (res, cres)
 
 
-def voxel_down_sample_batch_device(d_clouds, voxel_size: float, work=None):
+def voxel_down_sample_batch_device(d_clouds, voxel_size: float, work=None, colors=None):
     """psulvsb_voxel_down_sample_batch on CUDA tensors [n_c, 3] float64 and the current stream, without a host round
     trip.  Returns (voxels [sum n, 3] float64, counts [B] int32, offsets): cloud c's voxels are
     voxels[offsets[c]:offsets[c] + counts[c]], offsets[c] = sum of the sizes before it.  `work`: an optional uint8 CUDA
-    tensor of at least psulvsb_voxel_down_sample_batch_workspace_bytes bytes to reuse."""
+    tensor of at least psulvsb_voxel_down_sample_batch_workspace_bytes bytes to reuse.  colors: one CUDA tensor
+    [n_c, 3] float64 per cloud (psulvsb_voxel_down_sample_colors_batch): returns (voxels, voxel colours [sum n, 3],
+    counts, offsets), `work` then sized by psulvsb_voxel_down_sample_colors_batch_workspace_bytes."""
     import torch
 
     from .stages import _dev, _stream
 
     B = len(d_clouds)
     sizes = [int(p.shape[0]) for p in d_clouds]
-    arr = _clouds([_dev(p) if n else None for p, n in zip(d_clouds, sizes)], sizes, _viewpoints(None, B))
     L = capi.lib()
+    if colors is None:
+        arr = _clouds([_dev(p) if n else None for p, n in zip(d_clouds, sizes)], sizes, _viewpoints(None, B))
+        name = "psulvsb_voxel_down_sample_batch_workspace_bytes"
+    else:
+        if len(colors) != B or any(tuple(c.shape) != tuple(p.shape) for c, p in zip(colors, d_clouds)):
+            raise ValueError("colors: one colour tensor per cloud, one colour per point, is needed")
+        arr = _color_clouds([(_dev(p), _dev(c), None) if n else (None, None, None)
+                             for p, c, n in zip(d_clouds, colors, sizes)], sizes)
+        name = "psulvsb_voxel_down_sample_colors_batch_workspace_bytes"
     dev = d_clouds[0].device if B else torch.device("cuda")
-    nbytes = L.psulvsb_voxel_down_sample_batch_workspace_bytes(arr, B)
+    nbytes = getattr(L, name)(arr, B)
     if work is None:
         work = torch.empty(max(1, nbytes), dtype=torch.uint8, device=dev)
     elif work.numel() < nbytes:
-        raise ValueError("work is smaller than psulvsb_voxel_down_sample_batch_workspace_bytes(clouds, B)")
+        raise ValueError(f"work is smaller than {name}(clouds, B)")
     offsets = np.concatenate([[0], np.cumsum(sizes, dtype=np.int64)]).astype(np.int64)
     N = int(offsets[-1])
     out = torch.empty((max(N, 1), 3), dtype=torch.float64, device=dev)
     counts = torch.empty(max(B, 1), dtype=torch.int32, device=dev)
-    capi.check(L.psulvsb_voxel_down_sample_batch(_stream(), arr, B, float(voxel_size), _dev(work), _dev(out),
-                                                 _dev(counts)))
-    return out[:N], counts[:B], offsets[:B]
+    if colors is None:
+        capi.check(L.psulvsb_voxel_down_sample_batch(_stream(), arr, B, float(voxel_size), _dev(work), _dev(out),
+                                                     _dev(counts)))
+        return out[:N], counts[:B], offsets[:B]
+    oc = torch.empty((max(N, 1), 3), dtype=torch.float64, device=dev)
+    capi.check(L.psulvsb_voxel_down_sample_colors_batch(_stream(), arr, B, float(voxel_size), _dev(work), _dev(out),
+                                                        _dev(oc), _dev(counts)))
+    return out[:N], oc[:N], counts[:B], offsets[:B]
 
 
 def match_caps(n_srcs, n_tgts, crosscheck: bool = True, tuple_test: bool = False) -> list:

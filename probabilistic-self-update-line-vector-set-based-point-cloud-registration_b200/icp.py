@@ -14,6 +14,9 @@ Every call takes `loss=`, a robust kernel of the point-to-plane or generalized-I
 `colored_icp`, `colored_icp_device`, `colored_icp_batch` and `colored_icp_batch_device` are colored ICP (Open3D's
 registration_colored_icp; DESIGN.md section 11, "Colored ICP"): point-to-plane's loop with a geometric and a
 photometric row per correspondence; they need both clouds' [0, 1] RGB colours and the target's normals.
+`multiscale_colored_icp`, `multiscale_colored_icp_batch` and `multiscale_colored_icp_batch_device` run Open3D's
+coarse-to-fine recipe on the raw coloured clouds (DESIGN.md section 11, "Multi-scale colored ICP"): per voxel size, the
+colour-carrying voxel filter, the targets' hybrid normals and colored ICP from the previous scale's result.
 Convention: q ~ R p + t.
 """
 from __future__ import annotations
@@ -610,3 +613,91 @@ def colored_icp_batch_device(d_srcs, d_tgts, d_src_colors, d_tgt_colors, d_tgt_n
     if trace and B:
         records = (capi.IcpIteration * (B * nrec)).from_buffer_copy(rec.cpu().numpy().tobytes())
     return _batch_results(res, records, nrec, corr, sizes)
+
+
+MULTISCALE_MAX_NN = 30   # Open3D's KDTreeSearchParamHybrid(2 v, 30) for the target normals of each scale
+
+
+def _scales(voxel_sizes, max_correspondence_distances, max_iterations):
+    """(v_s, d_s, iterations_s) per scale: d_s = v_s by default; one iteration count for all scales or one per scale."""
+    vs = [float(v) for v in voxel_sizes]
+    ds = vs if max_correspondence_distances is None else [float(d) for d in max_correspondence_distances]
+    its = [int(max_iterations)] * len(vs) if np.ndim(max_iterations) == 0 else [int(k) for k in max_iterations]
+    if not vs or len(ds) != len(vs) or len(its) != len(vs):
+        raise ValueError(f"{len(vs)} voxel sizes, {len(ds)} distances and {len(its)} iteration counts: one per scale "
+                         "(at least one scale) is needed")
+    return list(zip(vs, ds, its))
+
+
+def multiscale_colored_icp_batch(srcs, tgts, src_colors, tgt_colors, R0s, t0s, voxel_sizes, *,
+                                 max_correspondence_distances=None, max_iterations=30, lambda_geometric: float = 0.968,
+                                 loss: Optional[RobustKernel] = None, relative_fitness: float = 1e-6,
+                                 relative_rmse: float = 1e-6) -> list:
+    """Open3D's multi-scale colored ICP (its colored point-cloud registration recipe) for B pairs: for each scale s, in
+    the order given, both clouds of every pair are downsampled with their colours at voxel size v_s
+    (features.voxel_down_sample_batch over all 2 B clouds in one call), the B target voxel sets get hybrid normals
+    (features.normals_batch, radius 2 v_s, max_nn 30), and `colored_icp_batch` refines every pair on the voxels at
+    distance d_s (default v_s), starting from its result at scale s - 1 whatever its status (R0s, t0s at the first
+    scale).  Source normals are not computed.  max_iterations: an int or one count per scale.  srcs, tgts, src_colors,
+    tgt_colors: sequences of 3 x n arrays ([0, 1] RGB); R0s [B, 3, 3], t0s [B, 3].  Returns out[s][b], the IcpResult of
+    pair b at scale s; the last scale's are the answer.  Correspondences index that scale's voxel clouds, which the
+    deterministic filter reproduces.  The wrapper adds no arithmetic: each scale equals the three calls composed by
+    hand."""
+    from . import features
+
+    B = len(srcs)
+    if len(tgts) != B or len(src_colors) != B or len(tgt_colors) != B:
+        raise ValueError(f"{B} sources, {len(tgts)} targets, {len(src_colors)} and {len(tgt_colors)} colour sets")
+    R, t = _batch_transforms(R0s, t0s, B)
+    out = []
+    for v, d, its in _scales(voxel_sizes, max_correspondence_distances, max_iterations):
+        vox, col = features.voxel_down_sample_batch(list(srcs) + list(tgts), v, colors=list(src_colors) + list(tgt_colors))
+        nrm = features.normals_batch(vox[B:], 2.0 * v, MULTISCALE_MAX_NN)
+        res = colored_icp_batch(vox[:B], vox[B:], col[:B], col[B:], nrm, R, t, d, lambda_geometric=lambda_geometric,
+                                loss=loss, max_iterations=its, relative_fitness=relative_fitness,
+                                relative_rmse=relative_rmse)
+        out.append(res)
+        R = np.array([r.R for r in res]).reshape(B, 3, 3)
+        t = np.array([r.t for r in res]).reshape(B, 3)
+    return out
+
+
+def multiscale_colored_icp(src, tgt, src_colors, tgt_colors, R0, t0, voxel_sizes, **kw) -> list:
+    """`multiscale_colored_icp_batch` on one pair: one IcpResult per scale, the last one the answer."""
+    res = multiscale_colored_icp_batch([src], [tgt], [src_colors], [tgt_colors],
+                                       np.asarray(R0, dtype=np.float64).reshape(1, 3, 3),
+                                       np.asarray(t0, dtype=np.float64).reshape(1, 3), voxel_sizes, **kw)
+    return [r[0] for r in res]
+
+
+def multiscale_colored_icp_batch_device(d_srcs, d_tgts, d_src_colors, d_tgt_colors, R0s, t0s, voxel_sizes, *,
+                                        max_correspondence_distances=None, max_iterations=30,
+                                        lambda_geometric: float = 0.968, loss: Optional[RobustKernel] = None,
+                                        relative_fitness: float = 1e-6, relative_rmse: float = 1e-6) -> list:
+    """`multiscale_colored_icp_batch` on sequences of CUDA tensors [n, 3] float64 and the current stream, through
+    features.voxel_down_sample_batch_device, features.normals_batch_device and `colored_icp_batch_device`.  Each scale
+    reads the 2 B voxel counts to the host once (they size the normal and ICP launches), and the transforms pass
+    through the host between scales, because colored_icp_batch_device reads its results back; both waits are on the
+    stream.  Returns out[s][b] as the host variant, correspondences on the device."""
+    from . import features
+
+    B = len(d_srcs)
+    if len(d_tgts) != B or len(d_src_colors) != B or len(d_tgt_colors) != B:
+        raise ValueError(f"{B} sources, {len(d_tgts)} targets, {len(d_src_colors)} and {len(d_tgt_colors)} colour "
+                         "sets")
+    R, t = _batch_transforms(R0s, t0s, B)
+    out = []
+    for v, d, its in _scales(voxel_sizes, max_correspondence_distances, max_iterations):
+        vox, col, counts, offsets = features.voxel_down_sample_batch_device(
+            list(d_srcs) + list(d_tgts), v, colors=list(d_src_colors) + list(d_tgt_colors))
+        m = counts.cpu().numpy()
+        vv = [vox[o:o + k] for o, k in zip(offsets, m)]
+        cv = [col[o:o + k] for o, k in zip(offsets, m)]
+        _, nrm = features.normals_batch_device(vv[B:], 2.0 * v, MULTISCALE_MAX_NN)
+        res = colored_icp_batch_device(vv[:B], vv[B:], cv[:B], cv[B:], nrm, R, t, d,
+                                       lambda_geometric=lambda_geometric, loss=loss, max_iterations=its,
+                                       relative_fitness=relative_fitness, relative_rmse=relative_rmse)
+        out.append(res)
+        R = np.array([r.R for r in res]).reshape(B, 3, 3)
+        t = np.array([r.t for r in res]).reshape(B, 3)
+    return out

@@ -10,7 +10,7 @@ from . import capi
 
 IO_SYMBOLS = ["psulvsb_histogram_outlier_removal", "psulvsb_mask_filter", "psulvsb_prefilter_reduce",
               "psulvsb_prefilter_reduce_batch", "psulvsb_ply_vertex_count",
-              "psulvsb_ply_read_xyz", "psulvsb_corr_count", "psulvsb_corr_read", "psulvsb_gtmat_read",
+              "psulvsb_ply_read_xyz", "psulvsb_ply_read_xyz_rgb", "psulvsb_corr_count", "psulvsb_corr_read", "psulvsb_gtmat_read",
               "psulvsb_gtlog_read"]
 
 _dp = C.POINTER(C.c_double)
@@ -31,6 +31,7 @@ def _lib():
         L.psulvsb_prefilter_reduce_batch.argtypes = [C.c_int, pp, pp, pp, pp, _ip, pp, pp, pp, pp, _ip, _ip]
         L.psulvsb_ply_vertex_count.argtypes = [C.c_char_p, _llp]
         L.psulvsb_ply_read_xyz.argtypes = [C.c_char_p, _fp, C.c_longlong, _llp]
+        L.psulvsb_ply_read_xyz_rgb.argtypes = [C.c_char_p, _fp, _dp, C.c_longlong, _llp]
         L.psulvsb_corr_count.argtypes = [C.c_char_p, _llp]
         L.psulvsb_corr_read.argtypes = [C.c_char_p, _dp, _dp, C.c_longlong, _llp]
         L.psulvsb_gtmat_read.argtypes = [C.c_char_p, _dp]
@@ -122,6 +123,18 @@ def read_ply_xyz(path: str) -> np.ndarray:
     xyz = np.zeros((max(n.value, 1), 3), dtype=np.float32)
     capi.check(_lib().psulvsb_ply_read_xyz(path.encode(), xyz.ctypes.data_as(_fp), n.value, C.byref(n)))
     return np.asfortranarray(xyz[:n.value].T.astype(np.float64))
+
+
+def read_ply_xyz_rgb(path: str):
+    """Vertices and colours of a PLY file: (3xN float64 positions, read as float32 like `read_ply_xyz`; 3xN float64
+    [0, 1] RGB from the red, green and blue properties, uchar / uint8 over 255, float / double as stored)."""
+    n = C.c_longlong(0)
+    capi.check(_lib().psulvsb_ply_vertex_count(path.encode(), C.byref(n)))
+    xyz = np.zeros((max(n.value, 1), 3), dtype=np.float32)
+    rgb = np.zeros((max(n.value, 1), 3), dtype=np.float64)
+    capi.check(_lib().psulvsb_ply_read_xyz_rgb(path.encode(), xyz.ctypes.data_as(_fp), rgb.ctypes.data_as(_dp),
+                                               n.value, C.byref(n)))
+    return np.asfortranarray(xyz[:n.value].T.astype(np.float64)), np.asfortranarray(rgb[:n.value].T)
 
 
 def read_correspondences(path: str):
